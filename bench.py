@@ -2,7 +2,7 @@
 """Benchmark of the categorical-memory hot path (BASELINE.json metric) on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dtype f32|bf16]
-                    [--workload cfg2_module_os8_b8] [--labels blocky|iid]
+                    [--workload cfg2_module_os8_b8] [--labels blocky|iid] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic input: ``Memory_sup.forward(query, labels,
 memory_writing=True, writing_detach=False)`` + backward of ``<G, updated_query> + 0.02*readloss + 0.4*div +
@@ -16,7 +16,13 @@ The metric is feature-map Mpixels/s. Prints ONE JSON line (rank 0).
 * ``roofline``   the dominant kernel: algorithmic bytes / its CUDA-event duration measured inside the timed region
 * ``cpu_baseline`` the reference's own module (byte-compiled into oracle/_ref/, else the oracle/ port) timed on this host's cores on a bounded sample
 ``--impl reference`` times that CPU arm instead (all host threads, the workload's full batch) and prints the same
-line shape. Timed regions are blocks of ``--steps`` steps repeated until >= 0.5 s; the median block is reported.
+line shape. Each timed region of the workload runs exactly ``--steps`` steps after ``--warmup`` untimed ones (``e2e``
+half as many, at least 5, after 3); the short runs of the other configs repeat fixed blocks and report the median block
+(``timing`` gives each region's blocks and their milliseconds). ``--impl reference`` is the exception: it warms up with
+at most 2 steps (the eval read with exactly 2), and on the training workloads it stops timing after 120 s (at least 3
+steps), since a full-batch CPU step can take seconds; ``sample`` reports the steps it timed.
+``--dump-outputs DIR`` writes what the headline path computed in its last timed step; the inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 Under torchrun (N>1) every rank runs its own batch (weak scaling); the write path all-reduces the class sums.
 """
 import argparse
@@ -44,7 +50,8 @@ LOSS_W = dict(read=0.02, div=0.4, cls=0.2)
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    # 600 steps of the ~0.83 ms default step keep the headline's single timed window at about 0.5 s
+    ap.add_argument("--steps", type=int, default=600)
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--dtype", default="f32", choices=["f32", "bf16"])
@@ -56,7 +63,59 @@ def parse():
     ap.add_argument("--overlap-write", action="store_true", help="write branch on a side stream (parallel graph branch)")
     ap.add_argument("--no-graph", action="store_true", help="headline = kernel-by-kernel launches instead of the CUDA graph")
     ap.add_argument("--no-extra", action="store_true", help="skip the short runs of the other BASELINE configs (cfg 3/4/5)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the headline path computed in its last timed step as DIR/<name>.npy (float32, or "
+                         "float64 where the output is); outputs above %d elements are replaced by a fixed seeded sample "
+                         "of %d of their elements" % (DUMP_FULL_MAX, DUMP_SAMPLE))
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
+
+
+# ------------------------------------------------------------------------------------------ output dump
+
+DUMP_FULL_MAX = 1 << 21   # outputs up to this many elements are written whole
+DUMP_SAMPLE = 1 << 20     # larger ones as this many elements at seeded flat positions (the same for every run)
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_arrays(named):
+    """{name: tensor} -> {name: float32 | float64 numpy array}, sampled as --dump-outputs describes. Call right after the
+    timed steps: the tensors are the step's static outputs and the next step overwrites them."""
+    out = {}
+    for name, t in named.items():
+        if t.numel() > DUMP_FULL_MAX:
+            g = torch.Generator().manual_seed(synth.SEED)
+            idx = torch.randint(t.numel(), (DUMP_SAMPLE,), generator=g).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        out[name] = t.to(torch.float64 if t.dtype == torch.float64 else torch.float32).cpu().numpy()
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d byte bound" % (total, DUMP_MAX_BYTES))
+    return out
+
+
+def write_dump(out_dir, arrays):
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def step_outputs(uq, sq, sm, rl, wl, memory=None, grad_query=None, param_grads=()):
+    """The arrays a caller of Memory_sup.forward (+ backward) receives, by name; int zeros of an absent loss are left out.
+    Detached: a kept reference to the step's autograd graph would keep its AccumulateGrad nodes alive, and a later CUDA
+    graph capture of the same parameters on another stream then fails."""
+    named = {"updated_query": uq, "score_query": sq, "score_memory": sm}
+    for n, v in (("readloss", rl), ("div_loss", wl[0]), ("cls_loss", wl[1]), ("m_items", memory), ("grad_query", grad_query)):
+        if torch.is_tensor(v):
+            named[n] = v
+    for n, g in param_grads:
+        if g is not None:
+            named["grad." + n] = g
+    return {n: t.detach() for n, t in named.items()}
 
 
 def tensor_peak(dt):
@@ -348,6 +407,10 @@ def eval_read_main(args, wl):
     capi.enable_kernel_timing(False)
     gstep = GraphedStep(mem, x, None, memory_writing=False, autocast_dtype=torch.bfloat16 if dt == torch.bfloat16 else None)
     ms_graph, clocks = run(gstep.replay, args.steps, args.warmup, clocks=True)
+    if args.dump_outputs and rank == 0:
+        o = gstep.outputs
+        write_dump(args.dump_outputs, dump_arrays(step_outputs(o["updated_query"], o["score_query"], o["score_memory"],
+                                                               o["readloss"], o["writeloss"])))
 
     res_host = torch.empty(N, dtype=torch.uint8).pin_memory()
 
@@ -655,14 +718,21 @@ def main():
     M0 = mem.m_items.clone()
     gw = [torch.tensor(LOSS_W[k], device=dev) for k in ("read", "div", "cls")]
     autocast = torch.autocast("cuda", dtype=torch.bfloat16, enabled=(dt == torch.bfloat16))
+    # --dump-outputs: module_step records its outputs on the call that counts "calls_left" down to 0
+    last_step = {"calls_left": 0}
 
     def module_step(xin, lab):
         mem.m_items = M0
         xin.grad = None
         mem.zero_grad(set_to_none=True)
         with autocast:
-            uq, _, _, rl, wlss = mem(xin, lab, True, False)
+            uq, sq, sm, rl, wlss = mem(xin, lab, True, False)
         torch.autograd.backward([uq, rl, wlss[0], wlss[1]], [G.to(uq.dtype), gw[0], gw[1], gw[2]])
+        if last_step["calls_left"]:
+            last_step["calls_left"] -= 1
+            if last_step["calls_left"] == 0:
+                last_step["outputs"] = step_outputs(uq, sq, sm, rl, wlss, mem.m_items, xin.grad,
+                                                    [(n, p.grad) for n, p in mem.named_parameters()])
         return rl, wlss
 
     Wc, bc = mem.clsfier.weight, mem.clsfier.bias
@@ -731,8 +801,8 @@ def main():
     def timed(fn, steps, warmup, sample_clocks=False, kernel_timing=False, min_total_ms=0.0, tag=None):
         """W warm-up steps, then blocks of EXACTLY `steps` steps, each bracketed by barrier + synchronize and timed
         with CUDA events on the launching stream (max over ranks per block); blocks repeat until `min_total_ms` of timed
-        work has accumulated and the MEDIAN block is returned -- a single 20-step block of a 0.8 ms step is 16 ms of
-        signal, too little to be stable."""
+        work has accumulated and the MEDIAN block is returned. The measurements that --steps sizes run one block, so that
+        --steps is the number of timed steps."""
         for _ in range(warmup):
             fn()
         torch.cuda.synchronize()
@@ -777,8 +847,9 @@ def main():
         return ms, launches, ktimes, (sampler.summary() if sampler else None)
 
     # whole module, device-resident inputs, one Python-side launch per kernel
+    last_step["calls_left"] = args.warmup + args.steps if args.dump_outputs else 0
     ms, launches, _, clocks = timed(lambda: module_step(x, labels), args.steps, args.warmup, sample_clocks=True,
-                                    min_total_ms=300.0, tag="eager_launch")
+                                    tag="eager_launch")
     ms_per_step = ms / args.steps
     value = world * N / (ms_per_step * 1e-3) / 1e6
     eager_launch = {"value": value, "unit": UNIT, "ms_per_step": ms_per_step, "gpu_launches": launches,
@@ -801,8 +872,13 @@ def main():
                                 memory_writing=True, writing_detach=False, carry_memory=True,
                                 autocast_dtype=torch.bfloat16 if dt == torch.bfloat16 else None)
             mem.overlap_write = overlap_eager
-            ms_g, _, _, clocks_g = timed(gstep.replay, args.steps, args.warmup, sample_clocks=True, min_total_ms=500.0,
-                                         tag="value")
+            ms_g, _, _, clocks_g = timed(gstep.replay, args.steps, args.warmup, sample_clocks=True, tag="value")
+            if args.dump_outputs:
+                o = gstep.outputs
+                names = [n for n, p in mem.named_parameters() if p.requires_grad]   # GraphedStep's order of param_grads
+                last_step["outputs"] = step_outputs(o["updated_query"], o["score_query"], o["score_memory"], o["readloss"],
+                                                    o["writeloss"], o["memory"], gstep.query_grad,
+                                                    zip(names, gstep.param_grads))
             graph_info = {"kernels_per_replay": gstep.kernels_per_replay}
             ms_per_step = ms_g / args.steps
             value = world * N / (ms_per_step * 1e-3) / 1e6
@@ -811,6 +887,9 @@ def main():
         except Exception as e:  # report the eagerly launched number rather than nothing
             graph_info = {"error": str(e)[:300]}
             mem.overlap_write = bool(args.overlap_write) or world > 1
+    if args.dump_outputs and rank == 0:
+        write_dump(args.dump_outputs, dump_arrays(last_step["outputs"]))
+    last_step.pop("outputs", None)
 
     # per-kernel durations measured live (events around every C-ABI launch) in a second timed region
     # (each step starts behind a ~3 ms device-side sleep so that the host has queued the whole step before the first kernel
@@ -984,7 +1063,7 @@ def main():
         except Exception as e:
             core_graph, core_fn = None, core_step
             core_launch = "one Python-side launch per kernel (capture failed: %s)" % str(e)[:120]
-    ms_c, launches_c, _, _ = timed(core_fn, args.steps, args.warmup, min_total_ms=300.0, tag="core")
+    ms_c, launches_c, _, _ = timed(core_fn, args.steps, args.warmup, tag="core")
     ms_core = ms_c / args.steps
     a_train = 10 * C * esz + 8 * r + 8 * K
     core_gbps = N * a_train / (ms_core * 1e-3) / 1e9
@@ -1001,7 +1080,7 @@ def main():
     for i in range(2):
         consumed[i].record()
     upload(0)
-    ms_e, _, _, _ = timed(e2e_pipelined_step, n_e, 3, min_total_ms=300.0, tag="e2e")
+    ms_e, _, _, _ = timed(e2e_pipelined_step, n_e, 3, tag="e2e")
     ms_e2e = ms_e / n_e
     # the same with the labels handed over as uint8 class ids (the module accepts both; 1/8 of the label bytes on the bus)
     e2e_u8 = None
@@ -1015,7 +1094,7 @@ def main():
             consumed[i].record()
         slot[0] = 0
         upload(0)
-        ms_u8, _, _, _ = timed(e2e_pipelined_step, n_e, 3, min_total_ms=200.0)
+        ms_u8, _, _, _ = timed(e2e_pipelined_step, n_e, 3)
         ms_u8 /= n_e
         e2e_u8 = {"value": world * N / (ms_u8 * 1e-3) / 1e6, "ms_per_step": ms_u8,
                   "h2d_bytes_per_step": x_host.numel() * x_host.element_size() + lab_host8.numel(),

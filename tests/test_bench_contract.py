@@ -6,6 +6,8 @@ import sys
 
 import pytest
 
+from oracle import ref_loader
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -26,7 +28,7 @@ def test_reference_arm_line(extra):
     assert line["steps"] == 2 and line["warmup"] == 1 and line["n_gpus"] == 1 and line["vs_baseline"] is None
     assert "workload" in line["config"] and "model" not in line["config"]
     cb = line["cpu_baseline"]
-    have_ref = os.path.isfile(os.path.join(ROOT, "oracle", "_ref", "reference_memory.bytecode")) or os.path.isdir("/root/reference/network")
+    have_ref = ref_loader.reference_available() or ref_loader.compiled_reference_available()
     assert cb["kind"] == ("reference" if have_ref else "port")   # the reference's own module whenever it is available
     assert cb["cores"] >= 1 and cb["value"] == line["value"] and cb["sample"]
     e2e = line["e2e"]

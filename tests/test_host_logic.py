@@ -93,20 +93,34 @@ def test_product_never_imports_the_oracle():
             assert not any("oracle" in ln for ln in imports), fn + " must not import oracle/"
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference tree not mounted (GPU box)")
-def test_attribute_surface_matches_the_live_reference():
-    ref = build_reference_memory(19, 64)
-    mem = _mem()
-    for name in ("memory_size", "feature_dim", "momentum", "initial_momentum", "temperature", "gumbel_read", "m_items",
-                 "mem_cls", "output", "writenet", "clsfier", "celoss", "writeTF"):
-        assert hasattr(ref, name) and hasattr(mem, name), name
-    assert [n for n, _ in ref.named_modules()] == [n for n, _ in mem.named_modules()]
-    for m in ("forward", "read", "write", "get_score"):
-        assert callable(getattr(mem, m))
+def _surface(m):
     import inspect
 
-    assert list(inspect.signature(ref.forward).parameters) == list(inspect.signature(mem.forward).parameters)
-    assert list(inspect.signature(type(ref).__init__).parameters) == list(inspect.signature(type(mem).__init__).parameters)[:-1]
+    return {"named_modules": [n for n, _ in m.named_modules()], "forward": list(inspect.signature(m.forward).parameters),
+            "init": list(inspect.signature(type(m).__init__).parameters)}
+
+
+def test_attribute_surface_matches_the_live_reference():
+    """Against the reference's surface stored in tests/golden/reference_surface.json, and against the live reference
+    module as well where its source tree is mounted (PINMEM_REFERENCE_ROOT)."""
+    import json
+    import os
+
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_surface.json")) as fh:
+        ref = json.load(fh)
+    if reference_available():
+        live = build_reference_memory(19, 64)
+        assert all(hasattr(live, name) for name in ref["attributes"])
+        assert _surface(live) == {k: ref[k] for k in ("named_modules", "forward", "init")}
+    mem = _mem()
+    for name in ref["attributes"]:
+        assert hasattr(mem, name), name
+    for m in ("forward", "read", "write", "get_score"):
+        assert callable(getattr(mem, m))
+    got = _surface(mem)
+    assert got["named_modules"] == ref["named_modules"]
+    assert got["forward"] == ref["forward"]
+    assert got["init"][:-1] == ref["init"] and got["init"][-1] == "device"
 
 
 def test_bn_args_counter_is_bumped_once_and_only_deferred_for_cuda_buffers():
