@@ -54,7 +54,7 @@ enum pm_readloss_ws_layout {
 #define PM_COLPART_ROWS 296
 
 /* Bumped with every prototype change; the binding refuses a library whose pm_version() differs. */
-#define PM_ABI_VERSION 206
+#define PM_ABI_VERSION 207
 int pm_version(void);
 const char* pm_status_string(int code);
 /* Row stride (floats) of the internal score buffers for K slots: 20 for K<=19, else 32. */
@@ -382,6 +382,32 @@ int pm_update_fwd_peer(const void* peer_bufs, int rank, int world, unsigned* epo
 int pm_update_bwd_peer(const void* peer_bufs, int rank, int world, unsigned* epoch, const float* dM_new, const float* g_div,
                        const float* g_cls, const float* M_new, const float* saved, const float* W_cls, const float* b_cls,
                        float momentum, float* dS, float* dW_cls, float* db_cls, float* aux, int C, int K, void* stream);
+
+/* 64-bit words of the segmentation-metrics workspace (`ws`, zero it before every pm_seg_eval call). */
+enum pm_seg_eval_ws_layout {
+    PM_SEG_WS_LOSS_SUM = 0, /* double: sum over valid label pixels of (LSE - logit[y])                   */
+    PM_SEG_WS_VALID = 1,    /* uint64: V, label pixels with a class id in [0,K)                           */
+    PM_SEG_WS_BAD = 2,      /* uint64: label values outside [0,K) u {255} (excluded like 255, and counted) */
+    PM_SEG_WS_COUNTER = 3,  /* uint64: CTA arrival ticket                                                 */
+    PM_SEG_WS_WORDS = 4
+};
+
+/*
+ * Segmentation validation metrics (csrc/pm_segeval.cu). Replaces, per validation batch, the up-sampling of the head's
+ * output to label size (network/deepv3plus.py:575-578, mynn.py:57-62), the criterion on it, `argmax` and the host-side
+ * `fast_hist` (utils/misc.py:65-73) of the validation loop (train.py:847-939) and the whole-image eval
+ * (eval.py:277-286,304-337) -- the [B,K,Hm,Wm] logits are never written and nothing is copied to the host.
+ *   logits     [B,K,h,w] NCHW in `dtype`; bilinearly up-sampled (align_corners=True) to [Hm,Wm] with ATen's arithmetic,
+ *              used as they are when h == Hm and w == Wm. Hm >= h, Wm >= w, K in 1..31.
+ *   labels     [B,Hm,Wm] int64 (labels_are_u8 = 0) or uint8 (1); 255 = ignore. Values outside [0,K) are excluded from
+ *              the confusion matrix and the loss (fast_hist's mask); those other than 255 are counted in ws[PM_SEG_WS_BAD].
+ *   confusion  [K,K] int64, ACCUMULATED: confusion[label][pred] += 1 per label pixel with a valid label.
+ *   pred       [B,Hm,Wm] uint8 out (argmax, first maximal class; written for every pixel, ignored ones included) or NULL.
+ *   ws         PM_SEG_WS_WORDS 64-bit words, ZEROED by the caller (layout above).
+ *   out        float[1] out: mean cross-entropy over the valid label pixels (NaN when there is none, like torch).
+ */
+int pm_seg_eval(const void* logits, int dtype, int B, int K, int h, int w, const void* labels, int labels_are_u8, int Hm,
+                int Wm, int64_t* confusion, uint8_t* pred, void* ws, float* out, void* stream);
 
 #ifdef __cplusplus
 }

@@ -2,7 +2,7 @@
 import sys
 
 __all__ = ["Memory_sup", "Writingnet", "initialize_weights", "install", "enable_sharded_update", "GraphedStep", "PrototypePool", "initialize_memory",
-           "upsampled_cross_entropy"]
+           "upsampled_cross_entropy", "SegMetrics"]
 
 
 def __getattr__(name):
@@ -15,7 +15,7 @@ def __getattr__(name):
         from .sharding import enable_sharded_update
 
         return enable_sharded_update
-    if name in ("PrototypePool", "initialize_memory", "upsampled_cross_entropy"):
+    if name in ("PrototypePool", "initialize_memory", "upsampled_cross_entropy", "SegMetrics"):
         from . import callers
 
         return getattr(callers, name)

@@ -14,9 +14,15 @@
   count. The bilinear weights are transposed onto the feature grid by ``pm_readloss_fwd`` (with all-zero logits and one
   spare slot its gradient IS ``W/K' - onehot`` scattered back), and ``pm_read_bwd_dM`` contracts them with the
   normalised features -- the [B,C,Hm,Wm] up-sampled map (1.2 GB at 8 x 768 x 768) never exists.
+* ``SegMetrics`` -- validation (train.py:847-939, eval.py:277-286,304-337): the criterion on the up-sampled head output,
+  its argmax and ``fast_hist`` (utils/misc.py:65-73) in one ``pm_seg_eval`` launch per batch; the confusion matrix stays
+  on the device and is all-reduced once at the end (train.py:927-929). At a Cityscapes validation image that removes
+  160 MB of up-sampled logits, a 16.8 MB prediction copy to the host and a NumPy bincount over 2.1 M pixels.
 
 CUDA only, like the rest of the package.
 """
+import os
+
 import torch
 import torch.nn.functional as F
 
@@ -141,3 +147,64 @@ def class_mean_vectors(features, labels, num_class):
     counts = ws.view(torch.int64)[capi.WS_HIST: capi.WS_HIST + K].to(torch.float32)
     safe = torch.where(counts == 0, torch.ones_like(counts), counts)
     return sums[:K] / safe.unsqueeze(1), counts
+
+
+class SegMetrics:
+    """Validation metrics of a segmentation head: mean cross-entropy per batch and the accumulated ``[K,K]`` confusion
+    matrix (rows = label, columns = prediction, ``fast_hist``'s layout), both computed on the device.
+
+    ``group``: a ``sharding.ShardGroup`` whose ranks' matrices ``finalize`` sums, or None (this process only).
+    ``device`` defaults to CUDA (``PINMEM_B200_DEVICE`` only serves CPU unit tests of ``finalize``'s host logic).
+    """
+
+    def __init__(self, num_classes, device=None, group=None):
+        self.K, self.group = int(num_classes), group
+        if not 1 <= self.K <= 31:
+            raise RuntimeError("pinmem_b200: SegMetrics supports 1..31 classes")
+        dev = torch.device(device if device is not None else os.environ.get("PINMEM_B200_DEVICE", "cuda"))
+        self.confusion = torch.zeros(self.K, self.K, dtype=torch.int64, device=dev)
+        self.last_bad_labels = None   # device int64 scalar: label values of the last batch outside [0,K) and != 255
+
+    def add(self, logits, labels, predictions=False):
+        """logits [B,K,h,w] fp32|bf16 (before the head's up-sampling, or already at label size), labels [B,Hm,Wm] int64|uint8
+        with 255 = ignore, Hm >= h, Wm >= w. Returns the batch's mean cross-entropy over its valid label pixels (0-d fp32
+        device tensor, NaN when there is none); with ``predictions`` also the argmax map [B,Hm,Wm] uint8."""
+        capi.require_cuda(logits, labels)
+        if logits.device != self.confusion.device or labels.device != self.confusion.device:
+            raise RuntimeError(f"pinmem_b200: SegMetrics lives on {self.confusion.device}, got tensors on {logits.device} "
+                               f"and {labels.device}")
+        if logits.dim() != 4 or labels.dim() != 3 or labels.shape[0] != logits.shape[0] or logits.shape[1] != self.K:
+            raise RuntimeError(f"pinmem_b200: logits must be [B,{self.K},h,w] and labels [B,Hm,Wm], got "
+                               f"{tuple(logits.shape)} and {tuple(labels.shape)}")
+        if labels.dtype not in (torch.int64, torch.uint8):
+            raise RuntimeError("pinmem_b200: labels must be int64 (or uint8 class ids)")
+        capi.dtype_code(logits)
+        if labels.shape[1] < logits.shape[2] or labels.shape[2] < logits.shape[3]:
+            raise RuntimeError("pinmem_b200: SegMetrics up-samples only: labels must be at least the logits' size")
+        dev = logits.device
+        buf = torch.zeros(capi.SEG_WS_WORDS + 1, dtype=torch.int64, device=dev)   # workspace words | loss (fp32 bits)
+        ws, out = buf[: capi.SEG_WS_WORDS], buf[capi.SEG_WS_WORDS:].view(torch.float32)
+        pred = torch.empty(labels.shape, dtype=torch.uint8, device=dev) if predictions else None
+        capi.seg_eval(logits.detach().contiguous(), labels.contiguous(), self.confusion, pred, ws, out)
+        self.last_bad_labels = ws[capi.SEG_WS_BAD]
+        loss = out[0]
+        return (loss, pred) if predictions else loss
+
+    def reset(self):
+        self.confusion.zero_()
+
+    def finalize(self):
+        """(confusion [K,K] int64 summed over the group, iou [K] float64, mean_iou): iou = diag / (rowsum + colsum - diag),
+        NaN for a class absent from both labels and predictions; mean_iou = nanmean(iou) (0-d float64)."""
+        conf = self.confusion
+        if self.group is not None:
+            conf = sharding.all_reduce_sum_(conf.clone(), self.group)
+        iou = segmentation_iou(conf)
+        return conf, iou, iou.nanmean()
+
+
+def segmentation_iou(confusion):
+    """Per-class IoU of a [K,K] confusion matrix (rows = label, columns = prediction) in float64."""
+    c = confusion.to(torch.float64)
+    diag = c.diagonal()
+    return diag / (c.sum(1) + c.sum(0) - diag)

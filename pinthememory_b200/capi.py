@@ -16,7 +16,10 @@ WS_WORDS = 40  # PM_WS_WORDS
 WS_HIST = 4    # PM_WS_HIST
 WS_BAD = 2     # PM_WS_BAD
 
-ABI_VERSION = 206  # PM_ABI_VERSION of include/pinmem_b200.h the argtypes below were written against
+SEG_WS_WORDS = 4  # PM_SEG_WS_WORDS
+SEG_WS_BAD = 2    # PM_SEG_WS_BAD
+
+ABI_VERSION = 207  # PM_ABI_VERSION of include/pinmem_b200.h the argtypes below were written against
 
 _c_p = ctypes.c_void_p
 _c_i = ctypes.c_int
@@ -74,6 +77,7 @@ PROTOTYPES = {
     "pm_readloss_fwd8": [_c_p, _c_p, _c_f] + [_c_i] * 6 + [_c_p] * 4,
     "pm_memory_losses_fwd": [_c_p] * 3 + [_c_i] * 2 + [_c_p] * 4,
     "pm_memory_losses_bwd": [_c_p] * 6 + [_c_i] * 2 + [_c_p] * 4,
+    "pm_seg_eval": [_c_p] + [_c_i] * 5 + [_c_p] + [_c_i] * 3 + [_c_p] * 5,
 }
 EXPORTED_SYMBOLS = sorted(list(PROTOTYPES) + ["pm_status_string"])
 
@@ -524,6 +528,14 @@ def readloss_fwd8(s, lab8, temperature, B, h, w, K, ds_rl, ws, out):
     Hm, Wm = lab8.shape[1], lab8.shape[2]
     _call("pm_readloss_fwd8", _ptr(s), _ptr(lab8), float(temperature), B, h, w, Hm, Wm, K, _ptr(ds_rl), _ptr(ws), _ptr(out),
           _stream())
+
+
+def seg_eval(logits, labels, confusion, pred, ws, out):
+    """Up-sample + argmax + cross-entropy + confusion increments in one label pass (csrc/pm_segeval.cu)."""
+    B, K, h, w = logits.shape
+    Hm, Wm = labels.shape[1], labels.shape[2]
+    _call("pm_seg_eval", _ptr(logits), dtype_code(logits), B, K, h, w, _ptr(labels), int(labels.dtype == torch.uint8), Hm, Wm,
+          _ptr(confusion), _ptr(pred), _ptr(ws), _ptr(out), _stream())
 
 
 def readloss(s, labels, temperature, B, h, w, K, ds_rl, ws, out):
