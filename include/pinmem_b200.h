@@ -54,7 +54,7 @@ enum pm_readloss_ws_layout {
 #define PM_COLPART_ROWS 296
 
 /* Bumped with every prototype change; the binding refuses a library whose pm_version() differs. */
-#define PM_ABI_VERSION 207
+#define PM_ABI_VERSION 208
 int pm_version(void);
 const char* pm_status_string(int code);
 /* Row stride (floats) of the internal score buffers for K slots: 20 for K<=19, else 32. */
@@ -408,6 +408,29 @@ enum pm_seg_eval_ws_layout {
  */
 int pm_seg_eval(const void* logits, int dtype, int B, int K, int h, int w, const void* labels, int labels_are_u8, int Hm,
                 int Wm, int64_t* confusion, uint8_t* pred, void* ws, float* out, void* stream);
+
+/*
+ * Decoder up-sample + concat (csrc/pm_upcat.cu). Replaces the DeepLabV3+ decoder step after the memory module
+ * (network/deepv3plus.py:569-572): `Upsample(dec0_up, low_level.size()[2:])` (mynn.py:57-62, bilinear,
+ * align_corners=True) and `torch.cat([dec0_fine, dec0_up], 1)` -- the up-sampled map is written straight into its
+ * channels of the concatenated output and never exists on its own.
+ *   fine    [B,Cf,H,W] NCHW in `dtype` (may be NULL when Cf == 0; Cf = 0 is a plain up-sample)
+ *   coarse  [B,Cc,h,w] NCHW in `dtype`; H >= h, W >= w (up-sampling only)
+ *   out     [B,Cf+Cc,H,W] out: planes [0,Cf) = fine, planes [Cf,Cf+Cc) = coarse up-sampled with ATen's arithmetic
+ *           (upsample_bilinear2d_out_frame bit for bit; equal sizes copy).
+ * B <= 65535 and Cf + Cc <= 65535 (grid limits), H * W < 2^31.
+ */
+int pm_upcat_fwd(const void* fine, const void* coarse, void* out, int dtype, int B, int Cf, int Cc, int h, int w, int H, int W,
+                 void* stream);
+/*
+ * Backward of pm_upcat_fwd with respect to `coarse`. Replaces upsample_bilinear2d_backward (atomics, registered as
+ * non-deterministic) after the copy of the gradient's coarse-channel slice made by cat's backward.
+ *   g         [B,Cf+Cc,H,W] NCHW in `dtype`: the gradient of `out`; only its planes [Cf,Cf+Cc) are read, in place.
+ *   d_coarse  [B,Cc,h,w] out: the exact transpose of the forward's interpolation (the same taps and fp32 weights),
+ *             accumulated in fp32 in a fixed order and stored once per element: bitwise reproducible.
+ * The gradient of `fine` is g's planes [0,Cf) as they are (what cat's backward returns); no kernel touches it.
+ */
+int pm_upcat_bwd(const void* g, void* d_coarse, int dtype, int B, int Cf, int Cc, int h, int w, int H, int W, void* stream);
 
 #ifdef __cplusplus
 }

@@ -2,7 +2,7 @@
 import sys
 
 __all__ = ["Memory_sup", "Writingnet", "initialize_weights", "install", "enable_sharded_update", "GraphedStep", "PrototypePool", "initialize_memory",
-           "upsampled_cross_entropy", "SegMetrics"]
+           "upsampled_cross_entropy", "SegMetrics", "upsample_concat"]
 
 
 def __getattr__(name):
@@ -15,7 +15,7 @@ def __getattr__(name):
         from .sharding import enable_sharded_update
 
         return enable_sharded_update
-    if name in ("PrototypePool", "initialize_memory", "upsampled_cross_entropy", "SegMetrics"):
+    if name in ("PrototypePool", "initialize_memory", "upsampled_cross_entropy", "SegMetrics", "upsample_concat"):
         from . import callers
 
         return getattr(callers, name)

@@ -18,6 +18,11 @@
   its argmax and ``fast_hist`` (utils/misc.py:65-73) in one ``pm_seg_eval`` launch per batch; the confusion matrix stays
   on the device and is all-reduced once at the end (train.py:927-929). At a Cityscapes validation image that removes
   160 MB of up-sampled logits, a 16.8 MB prediction copy to the host and a NumPy bincount over 2.1 M pixels.
+* ``upsample_concat`` -- the decoder step after the memory module (network/deepv3plus.py:569-572):
+  ``cat([dec0_fine, Upsample(dec0_up, low_level.size()[2:])], 1)`` as one ``pm_upcat_fwd`` launch that writes the
+  up-sampled channels straight into the concatenated map, and a deterministic gather backward (``pm_upcat_bwd``) that
+  reads the gradient's coarse channels in place. torch's own backward uses atomics and raises under
+  ``torch.use_deterministic_algorithms(True)``.
 
 CUDA only, like the rest of the package.
 """
@@ -208,3 +213,48 @@ def segmentation_iou(confusion):
     c = confusion.to(torch.float64)
     diag = c.diagonal()
     return diag / (c.sum(1) + c.sum(0) - diag)
+
+
+class _UpsampleConcat(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, fine, coarse):
+        B, Cf, H, W = fine.shape
+        out = torch.empty(B, Cf + coarse.shape[1], H, W, dtype=fine.dtype, device=fine.device)
+        capi.upcat_fwd(fine.detach().contiguous(), coarse.detach().contiguous(), out)
+        ctx.Cf, ctx.coarse_shape = Cf, coarse.shape   # shapes only: the backward needs no saved tensor
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        if not g.is_contiguous():
+            g = g.contiguous()
+        d_coarse = None
+        if ctx.needs_input_grad[1]:
+            d_coarse = torch.empty(ctx.coarse_shape, dtype=g.dtype, device=g.device)
+            capi.upcat_bwd(g, d_coarse, ctx.Cf)
+        d_fine = g.narrow(1, 0, ctx.Cf) if ctx.needs_input_grad[0] else None
+        return d_fine, d_coarse
+
+
+def upsample_concat(fine, coarse):
+    """``torch.cat([fine, F.interpolate(coarse, fine.shape[-2:], mode="bilinear", align_corners=True)], 1)`` fused.
+
+    fine [B,Cf,H,W] and coarse [B,Cc,h,w]: CUDA, the same device, dtype (fp32|bf16) and batch, H >= h, W >= w; Cf may
+    be 0. The forward equals torch's bit for bit. Differentiable w.r.t. both inputs: the gradient of ``fine`` is the
+    incoming gradient's first Cf channels (a view, as with torch.cat), that of ``coarse`` comes from a deterministic
+    kernel (fp32 accumulation in a fixed order, no atomics).
+    """
+    capi.require_cuda(fine, coarse)
+    if fine.dim() != 4 or coarse.dim() != 4:
+        raise RuntimeError(f"pinmem_b200: upsample_concat takes [B,C,H,W] tensors, got {tuple(fine.shape)} and "
+                           f"{tuple(coarse.shape)}")
+    if fine.device != coarse.device:
+        raise RuntimeError(f"pinmem_b200: upsample_concat got tensors on {fine.device} and {coarse.device}")
+    if fine.dtype != coarse.dtype:
+        raise RuntimeError(f"pinmem_b200: upsample_concat got {fine.dtype} and {coarse.dtype}")
+    capi.dtype_code(fine)
+    if fine.shape[0] != coarse.shape[0]:
+        raise RuntimeError(f"pinmem_b200: upsample_concat got batches of {fine.shape[0]} and {coarse.shape[0]}")
+    if fine.shape[2] < coarse.shape[2] or fine.shape[3] < coarse.shape[3]:
+        raise RuntimeError("pinmem_b200: upsample_concat up-samples only: fine must be at least coarse's size")
+    return _UpsampleConcat.apply(fine, coarse)

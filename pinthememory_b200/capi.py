@@ -19,7 +19,7 @@ WS_BAD = 2     # PM_WS_BAD
 SEG_WS_WORDS = 4  # PM_SEG_WS_WORDS
 SEG_WS_BAD = 2    # PM_SEG_WS_BAD
 
-ABI_VERSION = 207  # PM_ABI_VERSION of include/pinmem_b200.h the argtypes below were written against
+ABI_VERSION = 208  # PM_ABI_VERSION of include/pinmem_b200.h the argtypes below were written against
 
 _c_p = ctypes.c_void_p
 _c_i = ctypes.c_int
@@ -78,6 +78,8 @@ PROTOTYPES = {
     "pm_memory_losses_fwd": [_c_p] * 3 + [_c_i] * 2 + [_c_p] * 4,
     "pm_memory_losses_bwd": [_c_p] * 6 + [_c_i] * 2 + [_c_p] * 4,
     "pm_seg_eval": [_c_p] + [_c_i] * 5 + [_c_p] + [_c_i] * 3 + [_c_p] * 5,
+    "pm_upcat_fwd": [_c_p] * 3 + [_c_i] * 8 + [_c_p],
+    "pm_upcat_bwd": [_c_p] * 2 + [_c_i] * 8 + [_c_p],
 }
 EXPORTED_SYMBOLS = sorted(list(PROTOTYPES) + ["pm_status_string"])
 
@@ -536,6 +538,21 @@ def seg_eval(logits, labels, confusion, pred, ws, out):
     Hm, Wm = labels.shape[1], labels.shape[2]
     _call("pm_seg_eval", _ptr(logits), dtype_code(logits), B, K, h, w, _ptr(labels), int(labels.dtype == torch.uint8), Hm, Wm,
           _ptr(confusion), _ptr(pred), _ptr(ws), _ptr(out), _stream())
+
+
+def upcat_fwd(fine, coarse, out):
+    """out [B,Cf+Cc,H,W] = cat(fine, bilinear up-sample of coarse, align_corners=True) in one kernel (csrc/pm_upcat.cu)."""
+    B, Cf, H, W = fine.shape
+    _, Cc, h, w = coarse.shape
+    _call("pm_upcat_fwd", _ptr(fine) if Cf else None, _ptr(coarse), _ptr(out), dtype_code(coarse), B, Cf, Cc, h, w, H, W,
+          _stream())
+
+
+def upcat_bwd(g, d_coarse, Cf):
+    """d_coarse [B,Cc,h,w] from the planes [Cf,Cf+Cc) of the contiguous gradient g [B,Cf+Cc,H,W], read in place."""
+    B, _, H, W = g.shape
+    _, Cc, h, w = d_coarse.shape
+    _call("pm_upcat_bwd", _ptr(g), _ptr(d_coarse), dtype_code(g), B, Cf, Cc, h, w, H, W, _stream())
 
 
 def readloss(s, labels, temperature, B, h, w, K, ds_rl, ws, out):

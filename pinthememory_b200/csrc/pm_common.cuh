@@ -159,6 +159,26 @@ __device__ __forceinline__ int src_index(float scale, int dst, int n_in, float* 
     return i0;
 }
 
+// ATen's align_corners=True source index and lambda (upsample_bilinear2d_out_frame): src = scale * dst in fp32,
+// i0 = trunc(src) clamped to n_in - 1, lambda = src - i0. Round-to-nearest intrinsics keep nvcc from contracting them
+// into an FFMA, so the tap set is exactly torch's.
+__device__ __forceinline__ int tap(float scale, int dst, int n_in, float* lambda) {
+    const float src = __fmul_rn(scale, (float)dst);
+    int i0 = (int)src;
+    if (i0 > n_in - 1) i0 = n_in - 1;
+    *lambda = __fsub_rn(src, (float)i0);
+    return i0;
+}
+
+// ATen's interpolated value h0λ·(w0λ·a + w1λ·b) + h1λ·(w0λ·c + w1λ·d) as nvcc contracts it in torch's sm_100 build
+// (fp32 and bf16 instantiations alike): fma(h0, fma(w0, a, w1 * b), h1 * fma(w0, c, w1 * d)).
+__device__ __forceinline__ float lerp4(float h0, float h1, float w0, float w1, float a, float b, float c, float d) {
+    return __fmaf_rn(h0, __fmaf_rn(w0, a, __fmul_rn(w1, b)), __fmul_rn(h1, __fmaf_rn(w0, c, __fmul_rn(w1, d))));
+}
+__device__ __forceinline__ float2 lerp4(float2 h0, float2 h1, float2 w0, float2 w1, float2 a, float2 b, float2 c, float2 d) {
+    return __ffma2_rn(h0, __ffma2_rn(w0, a, __fmul2_rn(w1, b)), __fmul2_rn(h1, __ffma2_rn(w0, c, __fmul2_rn(w1, d))));
+}
+
 // The (<=4) label taps a feature pixel samples when the (K+1)-channel one-hot label map is
 // bilinearly down-sampled to the feature grid (reference memory.py:220-223). Equal classes
 // are merged; unused slots get weight 0. Class K is the ignore slot.

@@ -36,22 +36,6 @@ __device__ __forceinline__ float lg2a(float x) {
     return y;
 }
 
-// ATen's source index and lambda for align_corners=True, without contraction into an FFMA.
-__device__ __forceinline__ int tap(float scale, int dst, int n_in, float* lambda) {
-    const float src = __fmul_rn(scale, (float)dst);
-    int i0 = (int)src;
-    if (i0 > n_in - 1) i0 = n_in - 1;
-    *lambda = __fsub_rn(src, (float)i0);
-    return i0;
-}
-
-__device__ __forceinline__ float lerp4(float h0, float h1, float w0, float w1, float a, float b, float c, float d) {
-    return __fmaf_rn(h0, __fmaf_rn(w0, a, __fmul_rn(w1, b)), __fmul_rn(h1, __fmaf_rn(w0, c, __fmul_rn(w1, d))));
-}
-__device__ __forceinline__ float2 lerp4(float2 h0, float2 h1, float2 w0, float2 w1, float2 a, float2 b, float2 c, float2 d) {
-    return __ffma2_rn(h0, __ffma2_rn(w0, a, __fmul2_rn(w1, b)), __fmul2_rn(h1, __ffma2_rn(w0, c, __fmul2_rn(w1, d))));
-}
-
 template <typename T>
 __device__ __forceinline__ float ld_logit(const T* p);
 template <>
