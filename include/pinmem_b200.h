@@ -54,7 +54,7 @@ enum pm_readloss_ws_layout {
 #define PM_COLPART_ROWS 296
 
 /* Bumped with every prototype change; the binding refuses a library whose pm_version() differs. */
-#define PM_ABI_VERSION 208
+#define PM_ABI_VERSION 209
 int pm_version(void);
 const char* pm_status_string(int code);
 /* Row stride (floats) of the internal score buffers for K slots: 20 for K<=19, else 32. */
@@ -223,7 +223,8 @@ int pm_write_bwd(const float* dS, const void* f, const int64_t* labels, void* df
  *   pm_bn_apply       y = [relu]((x - mean) * invstd * gamma + beta [+ residual]); optionally also a packed ReLU
  *                     mask (1 bit per element, pm_bn_mask_words(B,C,hw) uint32 words; needs hw % 4 == 0) that the
  *                     backward passes read instead of y
- *   pm_bn_bwd_reduce  g = dy * (y > 0 if relu) (from relu_mask if given, else from y);  dbeta = sum g,  dgamma = sum g * xhat
+ *   pm_bn_bwd_reduce_rows  g = dy * (y > 0 if relu) (from relu_mask if given, else from y);  dbeta = sum g,
+ *                     dgamma = sum g * xhat
  *   pm_bn_bwd_apply   dx = gamma * invstd * (g - [training](dbeta + xhat * dgamma) / (B*hw));  dres = g (or NULL)
  */
 int pm_bn_stats(const void* x, int B, int C, int hw, int dtype, float eps, float* mean, float* invstd,
@@ -245,17 +246,8 @@ int pm_bn_apply_stats(const void* x, const double* stats, double count, float ep
  *   count_dev  NULL, or the element count in device memory, used instead of `count`: SyncBatchNorm (the reference under
  *              --syncbn, train.py:95) all-reduces [stats | count] over the ranks and normalises with the global statistics
  *              without a device->host read. */
-int pm_bn_bwd_reduce(const void* dy, const void* y, const uint32_t* relu_mask, const void* x, const float* mean,
-                     const float* invstd, int relu, float* dgamma, float* dbeta, int B, int C, int hw, int dtype,
-                     void* stream);
-/* pm_bn_bwd_reduce with every channel split over 4 CTAs (256 channels alone are 1.7 waves of long serial loops on 148
- * SMs); scratch: pm_bn_bwd_scratch_bytes(C) bytes, ZEROED by the caller; partials are added in split order (deterministic). */
-int pm_bn_bwd_scratch_bytes(int C);
-int pm_bn_bwd_reduce_split(const void* dy, const void* y, const uint32_t* relu_mask, const void* x, const float* mean,
-                           const float* invstd, int relu, float* dgamma, float* dbeta, int B, int C, int hw, int dtype,
-                           void* scratch, void* stream);
-/* pm_bn_bwd_reduce with one CTA per (image, channel) row -- bn_bwd_apply's access pattern, ~1.6x the bandwidth of one CTA
- * per channel. scratch: pm_bn_bwd_rows_scratch_bytes(B, C) bytes, 8-byte aligned, zeroed ONCE when allocated (the kernel
+/* pm_bn_bwd_reduce_rows runs one CTA per (image, channel) row -- bn_bwd_apply's access pattern, ~1.6x the bandwidth of
+ * one CTA per channel. scratch: pm_bn_bwd_rows_scratch_bytes(B, C) bytes, 8-byte aligned, zeroed ONCE when allocated (the kernel
  * leaves its arrival counters at zero); the B row partials of a channel are added in image order (deterministic). Use one
  * scratch per stream that may run this entry concurrently. */
 int pm_bn_bwd_rows_scratch_bytes(int B, int C);
@@ -308,7 +300,7 @@ int pm_bn_eval_affine(const float* gamma, const float* beta, const float* runnin
  * the forward's expression) and the dz tiles are stored to dZ [B,K,hw] for the weight-gradient GEMM.
  *   dY, Z, dZ [B,K,hw] fp32 (K = the convolution's OUTPUT channels)      A_hi/A_lo = pm_conv1x1_prep(W, transpose = 1)
  *   dX [B,M,hw] fp32 (M = the convolution's INPUT channels)              mean/invstd/gamma/beta [K], dgamma/dbeta [K] =
- *   the sums pm_bn_bwd_reduce produced; training = 0: eval-mode BatchNorm (dz = gamma*invstd*g); n = B*hw.
+ *   the sums pm_bn_bwd_reduce_rows produced; training = 0: eval-mode BatchNorm (dz = gamma*invstd*g); n = B*hw.
  */
 int pm_conv1x1_dgrad_bnbwd(const void* dY, const void* Z, const void* A_hi, const void* A_lo, void* dX, void* dZ,
                            const float* mean, const float* invstd, const float* gamma, const float* beta, const float* dgamma,

@@ -19,7 +19,7 @@ WS_BAD = 2     # PM_WS_BAD
 SEG_WS_WORDS = 4  # PM_SEG_WS_WORDS
 SEG_WS_BAD = 2    # PM_SEG_WS_BAD
 
-ABI_VERSION = 208  # PM_ABI_VERSION of include/pinmem_b200.h the argtypes below were written against
+ABI_VERSION = 209  # PM_ABI_VERSION of include/pinmem_b200.h the argtypes below were written against
 
 _c_p = ctypes.c_void_p
 _c_i = ctypes.c_int
@@ -52,9 +52,6 @@ PROTOTYPES = {
     "pm_bn_stats": [_c_p] + [_c_i] * 4 + [_c_f] + [_c_p] * 4 + [_c_f, _c_p],
     "pm_bn_mask_words": [_c_i] * 3,
     "pm_bn_apply": [_c_p] * 8 + [_c_i] * 5 + [_c_p],
-    "pm_bn_bwd_reduce": [_c_p] * 6 + [_c_i] + [_c_p] * 2 + [_c_i] * 4 + [_c_p],
-    "pm_bn_bwd_scratch_bytes": [_c_i],
-    "pm_bn_bwd_reduce_split": [_c_p] * 6 + [_c_i] + [_c_p] * 2 + [_c_i] * 4 + [_c_p] * 2,
     "pm_bn_bwd_rows_scratch_bytes": [_c_i] * 2,
     "pm_bn_bwd_reduce_rows": [_c_p] * 6 + [_c_i] + [_c_p] * 2 + [_c_i] * 4 + [_c_p] * 2,
     "pm_bn_bwd_apply": [_c_p] * 9 + [_c_i] * 2 + [_c_p] * 2 + [_c_i] * 4 + [_c_p],
@@ -370,17 +367,8 @@ def _bn_rows_scratch(x, B, C):
 
 def bn_bwd_reduce(dy, y, relu_mask, x, mean, invstd, relu, dgamma, dbeta):
     B, C, h, w = x.shape
-    if not os.environ.get("PINMEM_B200_BN_REDUCE_PER_CHANNEL"):  # one CTA per (image, channel) row: 48 -> ~30 us at cfg 2
-        _call("pm_bn_bwd_reduce_rows", _ptr(dy), _ptr(y), _ptr(relu_mask), _ptr(x), _ptr(mean), _ptr(invstd), int(relu),
-              _ptr(dgamma), _ptr(dbeta), B, C, h * w, dtype_code(x), _ptr(_bn_rows_scratch(x, B, C)), _stream())
-        return
-    if os.environ.get("PINMEM_B200_BN_SPLIT"):   # measured 55.7 us vs 51 us unsplit at cfg 2: off by default (A/B switch)
-        scratch = torch.zeros(load().pm_bn_bwd_scratch_bytes(C) // 8 + 1, dtype=torch.float64, device=x.device)
-        _call("pm_bn_bwd_reduce_split", _ptr(dy), _ptr(y), _ptr(relu_mask), _ptr(x), _ptr(mean), _ptr(invstd), int(relu),
-              _ptr(dgamma), _ptr(dbeta), B, C, h * w, dtype_code(x), _ptr(scratch), _stream())
-        return
-    _call("pm_bn_bwd_reduce", _ptr(dy), _ptr(y), _ptr(relu_mask), _ptr(x), _ptr(mean), _ptr(invstd), int(relu),
-          _ptr(dgamma), _ptr(dbeta), B, C, h * w, dtype_code(x), _stream())
+    _call("pm_bn_bwd_reduce_rows", _ptr(dy), _ptr(y), _ptr(relu_mask), _ptr(x), _ptr(mean), _ptr(invstd), int(relu),
+          _ptr(dgamma), _ptr(dbeta), B, C, h * w, dtype_code(x), _ptr(_bn_rows_scratch(x, B, C)), _stream())
 
 
 def bn_bwd_apply(dy, y, relu_mask, x, mean, invstd, gamma, dgamma, dbeta, relu, training, dx, dres):
@@ -556,9 +544,9 @@ def upcat_bwd(g, d_coarse, Cf):
 
 
 def readloss(s, labels, temperature, B, h, w, K, ds_rl, ws, out):
-    """Read loss on int64 | uint8 labels: one label pass (pack + histogram + bad-label count) and the second-generation
-    kernel for K <= 19, the first kernel (int64 labels, any K <= 31) otherwise or with PINMEM_B200_READLOSS_V1 set."""
-    if K <= 19 and not os.environ.get("PINMEM_B200_READLOSS_V1"):
+    """Read loss on int64 | uint8 labels: one label pass (pack + histogram + bad-label count) and the packed-label kernels
+    for K <= 19, the first kernel (int64 labels, any K <= 31) otherwise."""
+    if K <= 19:
         lab8 = labels_pack(labels, K, ws)
         readloss_fwd8(s, lab8, temperature, B, h, w, K, ds_rl, ws, out)
         return lab8

@@ -218,91 +218,9 @@ __global__ void __launch_bounds__(256) bn_apply_kernel(const T* __restrict__ x, 
     }
 }
 
-// one CTA per channel: dbeta = sum g, dgamma = sum g * xhat, g = dy * (y > 0 if relu)
-template <typename T, int VN>
-__global__ void __launch_bounds__(BN_THREADS) bn_bwd_reduce_kernel(const T* __restrict__ dy, const T* __restrict__ y,
-                                                                   const unsigned* __restrict__ relu_mask,
-                                                                   const T* __restrict__ x, const float* __restrict__ mean,
-                                                                   const float* __restrict__ invstd, int relu,
-                                                                   float* __restrict__ dgamma, float* __restrict__ dbeta,
-                                                                   int B, int C, int hw, double* __restrict__ scratch) {
-    // grid (C, S): a channel's B*hw elements are split over S CTAs (256 channels alone are 1.7 waves of long serial loops
-    // on 148 SMs); partial sums meet in `scratch` ([S][C][2] doubles + C arrival counters, zeroed by the caller) and the
-    // last CTA of a channel adds them in split order -- deterministic. S = 1 (scratch NULL) is the single-CTA form.
-    __shared__ double red[BN_THREADS / 32];
-    __shared__ int last_sm;
-    const int c = blockIdx.x, S = gridDim.y, sp = blockIdx.y;
-    const float m = mean[c], is = invstd[c];
-    float sg = 0.f, sgx = 0.f;
-    if constexpr (VN != 0) {
-        const int nv = hw / VN, total = B * nv, wpr = (nv + 32 / VN - 1) / (32 / VN);
-        const int per = (total + S - 1) / S, i0 = sp * per, i1 = min(total, i0 + per);
-#pragma unroll 4
-        for (int i = i0 + threadIdx.x; i < i1; i += BN_THREADS) {
-            const int b = i / nv, j = i - b * nv;
-            const size_t off = ((size_t)b * C + c) * hw + VN * j;
-            typename VecSel<T, VN>::type g, yy, xx;
-            g.load(dy + off);
-            xx.load(x + off);
-            unsigned bits = (1u << VN) - 1u;
-            if (relu) {
-                if (relu_mask != nullptr) {
-                    bits = mask_bits<VN>(relu_mask + ((size_t)b * C + c) * wpr, j);
-                } else {
-                    yy.load(y + off);
-                    bits = 0u;
-#pragma unroll
-                    for (int e = 0; e < VN; ++e) bits |= (yy.get(e) > 0.f ? 1u : 0u) << e;
-                }
-            }
-#pragma unroll
-            for (int e = 0; e < VN; ++e) {
-                const float gv = ((bits >> e) & 1u) ? g.get(e) : 0.f;
-                sg += gv;
-                sgx = fmaf(gv, (xx.get(e) - m) * is, sgx);
-            }
-        }
-    } else {
-        const int total = B * hw;
-        const int per = (total + S - 1) / S, i0 = sp * per, i1 = min(total, i0 + per);
-        for (int i = i0 + threadIdx.x; i < i1; i += BN_THREADS) {
-            const int b = i / hw, j = i - b * hw;
-            const size_t off = ((size_t)b * C + c) * hw + j;
-            const float gv = (!relu || ldf(y + off) > 0.f) ? ldf(dy + off) : 0.f;
-            sg += gv;
-            sgx = fmaf(gv, (ldf(x + off) - m) * is, sgx);
-        }
-    }
-    const double SG = block_sum_double((double)sg, red);
-    const double SGX = block_sum_double((double)sgx, red);
-    if (S == 1) {
-        if (threadIdx.x == 0) {
-            dbeta[c] = (float)SG;
-            dgamma[c] = (float)SGX;
-        }
-        return;
-    }
-    if (threadIdx.x == 0) {
-        scratch[((size_t)sp * C + c) * 2] = SG;
-        scratch[((size_t)sp * C + c) * 2 + 1] = SGX;
-        __threadfence();
-        unsigned* counters = reinterpret_cast<unsigned*>(scratch + (size_t)S * C * 2);
-        last_sm = atomicAdd(counters + c, 1u) == (unsigned)S - 1;
-        if (last_sm) {
-            __threadfence();
-            double a = 0.0, b2 = 0.0;
-            for (int q = 0; q < S; ++q) {
-                a += __ldcg(scratch + ((size_t)q * C + c) * 2);
-                b2 += __ldcg(scratch + ((size_t)q * C + c) * 2 + 1);
-            }
-            dbeta[c] = (float)a;
-            dgamma[c] = (float)b2;
-        }
-    }
-}
-
-// The same sums with one CTA per (b, c) ROW -- the access pattern of bn_bwd_apply, which streams at ~90 % of the copy peak
-// where one CTA per channel reaches ~50 %: 8 x as many CTAs, each reading two contiguous rows front to back. A row's two
+// dbeta = sum g, dgamma = sum g * xhat, g = dy * (y > 0 if relu), with one CTA per (b, c) ROW -- the access pattern of
+// bn_bwd_apply, which streams at ~90 % of the copy peak where one CTA per channel reaches ~50 %: each CTA reads two
+// contiguous rows front to back. A row's two
 // partial sums go to `partials` [B][C][2] (doubles); the CTA that completes a channel (per-channel arrival counter) adds
 // the B partials in image order -- deterministic -- and RESETS the counter, so the scratch only has to be zeroed when it is
 // allocated, not per call.
@@ -566,49 +484,7 @@ static int bn_apply_impl(const void* x, const float* mean, const float* invstd, 
     return 0;
 }
 
-#define PM_BN_SPLITS 4
-extern "C" int pm_bn_bwd_scratch_bytes(int C) { return C > 0 ? PM_BN_SPLITS * C * 2 * 8 + C * 4 : 0; }
-
-static int bn_bwd_reduce_impl(const void* dy, const void* y, const uint32_t* relu_mask, const void* x, const float* mean,
-                              const float* invstd, int relu, float* dgamma, float* dbeta, int B, int C, int hw, int dtype,
-                              double* scratch, void* stream);
-
-extern "C" int pm_bn_bwd_reduce(const void* dy, const void* y, const uint32_t* relu_mask, const void* x, const float* mean,
-                                const float* invstd, int relu, float* dgamma, float* dbeta, int B, int C, int hw, int dtype,
-                                void* stream) {
-    return bn_bwd_reduce_impl(dy, y, relu_mask, x, mean, invstd, relu, dgamma, dbeta, B, C, hw, dtype, nullptr, stream);
-}
-/* the same with each channel split over PM_BN_SPLITS CTAs; scratch: pm_bn_bwd_scratch_bytes(C) bytes, ZEROED, 8-byte aligned */
-extern "C" int pm_bn_bwd_reduce_split(const void* dy, const void* y, const uint32_t* relu_mask, const void* x,
-                                      const float* mean, const float* invstd, int relu, float* dgamma, float* dbeta, int B,
-                                      int C, int hw, int dtype, void* scratch, void* stream) {
-    if (!scratch || ((uintptr_t)scratch & 7)) return PM_ERR_NULL;
-    return bn_bwd_reduce_impl(dy, y, relu_mask, x, mean, invstd, relu, dgamma, dbeta, B, C, hw, dtype, (double*)scratch, stream);
-}
-
-static int bn_bwd_reduce_impl(const void* dy, const void* y, const uint32_t* relu_mask, const void* x, const float* mean,
-                              const float* invstd, int relu, float* dgamma, float* dbeta, int B, int C, int hw, int dtype,
-                              double* scratch, void* stream) {
-    if (!dy || !x || !mean || !invstd || !dgamma || !dbeta || (relu && !y && !relu_mask)) return PM_ERR_NULL;
-    if (int e = bn_check(B, C, hw, dtype)) return e;
-    const int vec = pm::vec_ok(hw, dy, y, x, nullptr, nullptr, dtype);
-    if (relu && !y && !vec) return PM_ERR_ALIGN;
-    cudaStream_t st = (cudaStream_t)stream;
-    const dim3 grid(C, scratch != nullptr ? PM_BN_SPLITS : 1);
-    if (dtype == PM_F32) {
-        if (vec) pm::bn_bwd_reduce_kernel<float, 4><<<grid, pm::BN_THREADS, 0, st>>>((const float*)dy, (const float*)y, relu_mask, (const float*)x, mean, invstd, relu, dgamma, dbeta, B, C, hw, scratch);
-        else pm::bn_bwd_reduce_kernel<float, 0><<<grid, pm::BN_THREADS, 0, st>>>((const float*)dy, (const float*)y, relu_mask, (const float*)x, mean, invstd, relu, dgamma, dbeta, B, C, hw, scratch);
-    } else {
-        typedef __nv_bfloat16 bf;
-        if (vec == 8) pm::bn_bwd_reduce_kernel<bf, 8><<<grid, pm::BN_THREADS, 0, st>>>((const bf*)dy, (const bf*)y, relu_mask, (const bf*)x, mean, invstd, relu, dgamma, dbeta, B, C, hw, scratch);
-        else if (vec) pm::bn_bwd_reduce_kernel<bf, 4><<<grid, pm::BN_THREADS, 0, st>>>((const bf*)dy, (const bf*)y, relu_mask, (const bf*)x, mean, invstd, relu, dgamma, dbeta, B, C, hw, scratch);
-        else pm::bn_bwd_reduce_kernel<bf, 0><<<grid, pm::BN_THREADS, 0, st>>>((const bf*)dy, (const bf*)y, relu_mask, (const bf*)x, mean, invstd, relu, dgamma, dbeta, B, C, hw, scratch);
-    }
-    PM_CHECK_LAUNCH();
-    return 0;
-}
-
-/* pm_bn_bwd_reduce with one CTA per (image, channel) row (csrc/pm_bn.cu: bn_bwd_reduce_rows_kernel). scratch:
+/* BatchNorm backward sums with one CTA per (image, channel) row (bn_bwd_reduce_rows_kernel). scratch:
  * pm_bn_bwd_rows_scratch_bytes(B, C) bytes, 8-byte aligned, zeroed ONCE when allocated (the kernel leaves its arrival
  * counters at zero); one scratch per stream that may run this concurrently. */
 extern "C" int pm_bn_bwd_rows_scratch_bytes(int B, int C) { return (B > 0 && C > 0) ? B * C * 2 * 8 + C * 4 : 0; }

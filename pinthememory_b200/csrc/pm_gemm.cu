@@ -74,61 +74,6 @@ __device__ __forceinline__ void split_tile_trunc(const float4* __restrict__ raw,
         lo[i] = l;
     }
 }
-// ---- "mixed" error compensation (fp32 I/O, default): D = tf32(A).tf32(X)  +  [bf16(A_lo) | bf16(A_hi)] . [bf16(X) ; bf16(X_lo)]
-// The two correction products are 2^-11 of the main one, so 8 mantissa bits are plenty for THEIR operands: they run as
-// one bf16 MMA pass over a K-concatenated operand pair (kind::f16 retires K = 16 per instruction, twice the TF32 rate),
-// i.e. 2 tensor passes instead of 3 for the same ~2e-6 result. x_hi is what the tensor core keeps of the raw fp32
-// container (truncation), x_lo = x - x_hi; the weights are split once per call (round-to-nearest hi).
-__device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
-    const __nv_bfloat162 p = __floats2bfloat162_rn(a, b);
-    return *reinterpret_cast<const uint32_t*>(&p);
-}
-__device__ __forceinline__ float tf32_resid(float x) { return x - __uint_as_float(__float_as_uint(x) & 0xffffe000u); }
-
-// MN-major activation tile (form 1). raw: fp32 [KB rows][NT pixels] as 32-pixel chunks of [KB][128 B] with 32-byte
-// atoms swizzled by (row & 3) (SWIZZLE_128B_ATOM_32B). out: bf16 [2*KB rows][NT pixels] as 64-pixel chunks of
-// [2*KB][128 B] with 16-byte chunks swizzled by (row & 7) (SWIZZLE_128B); per group of 16 channels rows
-// [32g, 32g+16) = bf16(x) and [32g+16, 32g+32) = bf16(x_lo) -- the K order of the prepared weight operand.
-template <int KB, int NT>
-__device__ __forceinline__ void mix_tile_mn(const unsigned char* __restrict__ raw, unsigned char* __restrict__ out, int t,
-                                            int nthreads) {
-    constexpr int NC32 = NT / 32, ATOMS = KB * NC32 * 4;
-    for (int i = t; i < ATOMS; i += nthreads) {
-        const int a = i & 3, k = (i >> 2) % KB, c = (i >> 2) / KB;
-        const float4* src = reinterpret_cast<const float4*>(raw + c * (KB * 128) + k * 128 + ((a ^ (k & 3)) << 5));
-        const float4 v0 = src[0], v1 = src[1];
-        uint4 hi, lo;
-        hi.x = pack_bf16(v0.x, v0.y), hi.y = pack_bf16(v0.z, v0.w), hi.z = pack_bf16(v1.x, v1.y), hi.w = pack_bf16(v1.z, v1.w);
-        lo.x = pack_bf16(tf32_resid(v0.x), tf32_resid(v0.y)), lo.y = pack_bf16(tf32_resid(v0.z), tf32_resid(v0.w));
-        lo.z = pack_bf16(tf32_resid(v1.x), tf32_resid(v1.y)), lo.w = pack_bf16(tf32_resid(v1.z), tf32_resid(v1.w));
-        const int j = ((c & 1) << 2) | a;                 // 16-byte chunk of the 64-pixel row
-        const int r0 = ((k >> 4) << 5) | (k & 15), r1 = r0 + 16;
-        unsigned char* base = out + (c >> 1) * (2 * KB * 128);
-        *reinterpret_cast<uint4*>(base + r0 * 128 + ((j ^ (r0 & 7)) << 4)) = hi;
-        *reinterpret_cast<uint4*>(base + r1 * 128 + ((j ^ (r1 & 7)) << 4)) = lo;
-    }
-}
-// K-major tile (form 2: K = pixels). raw: fp32 [rows][32 pixels] (128-byte rows, 16-byte chunks swizzled by row & 7);
-// out: bf16 [rows][64] (128-byte rows, same swizzle). hi_first = false: [bf16(x_lo) | bf16(x)] (the A operand);
-// hi_first = true: [bf16(x) | bf16(x_lo)] (the B operand) -- so that the concatenated K pairs lo.x with x.lo.
-__device__ __forceinline__ void mix_tile_k(const unsigned char* __restrict__ raw, unsigned char* __restrict__ out, int rows,
-                                           bool hi_first, int t, int nthreads) {
-    for (int i = t; i < rows * 4; i += nthreads) {
-        const int m = i & 3, r = i >> 2;  // pixels 8m .. 8m+7 of row r = fp32 chunks 2m, 2m+1
-        const unsigned char* rr = raw + r * 128;
-        const float4 v0 = *reinterpret_cast<const float4*>(rr + (((2 * m) ^ (r & 7)) << 4));
-        const float4 v1 = *reinterpret_cast<const float4*>(rr + (((2 * m + 1) ^ (r & 7)) << 4));
-        uint4 hi, lo;
-        hi.x = pack_bf16(v0.x, v0.y), hi.y = pack_bf16(v0.z, v0.w), hi.z = pack_bf16(v1.x, v1.y), hi.w = pack_bf16(v1.z, v1.w);
-        lo.x = pack_bf16(tf32_resid(v0.x), tf32_resid(v0.y)), lo.y = pack_bf16(tf32_resid(v0.z), tf32_resid(v0.w));
-        lo.z = pack_bf16(tf32_resid(v1.x), tf32_resid(v1.y)), lo.w = pack_bf16(tf32_resid(v1.z), tf32_resid(v1.w));
-        unsigned char* ro = out + r * 128;
-        const int jh = hi_first ? m : 4 + m, jl = hi_first ? 4 + m : m;
-        *reinterpret_cast<uint4*>(ro + ((jh ^ (r & 7)) << 4)) = hi;
-        *reinterpret_cast<uint4*>(ro + ((jl ^ (r & 7)) << 4)) = lo;
-    }
-}
-
 __device__ __forceinline__ float tf32_rn(float x) { return __uint_as_float((__float_as_uint(x) + 0x00001000u) & 0xffffe000u); }
 __device__ __forceinline__ void split_tile(float4* __restrict__ raw, float4* __restrict__ lo, int n4, int t, int nthreads) {
     for (int i = t; i < n4; i += nthreads) {
@@ -193,21 +138,17 @@ __device__ __forceinline__ void bnbwd_tile(float4* __restrict__ dy_hi, float4* _
 //   mapAl : fp32 only, the "lo" part
 //   mapY  : [B*M rows][hw] output, box [32 rows][PXC pixels]
 //   CTA tile: MT x 128 output rows (starting at 128*m_tile0) x NT pixels of one image; persistent over tiles.
-//   CL > 1: clusters of CL CTAs work on CL consecutive pixel tiles in lock step and share the weight blocks -- each
-//   CTA loads 1/CL of them and TMA-multicasts them to the whole cluster (the weights are re-read for every pixel tile,
-//   so at CL = 1 the L2 -> SM traffic is ~4x the activation bytes and bounds the kernel); ring slots are released
-//   cluster-wide (tcgen05.commit multicast onto every CTA's `empty` barrier).
 // =================================================================================================================
-template <typename T, int MT, int NT, int KB, int CL, bool MIX>
+template <typename T, int MT, int NT, int KB>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
     conv1x1_nn_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant__ CUtensorMap mapAh,
                       const __grid_constant__ CUtensorMap mapAl, const __grid_constant__ CUtensorMap mapY, int K, int M,
                       int m_tile0, int tiles_per_img, int total_tiles, int accumulate, double* __restrict__ stats,
-                      const float* __restrict__ ep_scale, const float* __restrict__ ep_shift, int ep_relu, int dbg,
+                      const float* __restrict__ ep_scale, const float* __restrict__ ep_shift, int ep_relu,
                       const __grid_constant__ CUtensorMap mapZ, const __grid_constant__ CUtensorMap mapDZ, const BnBwdArgs bn) {
     using TR = GemmTraits<T>;
     constexpr int PXC = TR::PXC, UK = TR::UK, KSTEPS = KB / UK;
-    const bool bnbwd = TR::SPLIT && !MIX && bn.mean != nullptr;  // X = dy, Z = saved conv output: dz formed in the split stage
+    const bool bnbwd = TR::SPLIT && bn.mean != nullptr;  // X = dy, Z = saved conv output: dz formed in the split stage
     constexpr int NCH = NT / PXC;                      // 128-byte pixel chunks per tile
     constexpr int XCHUNK = KB * 128;                   // bytes of one [KB rows][128 B] chunk
     constexpr int XBYTES = NCH * XCHUNK;               // = NT * KB * sizeof(T)
@@ -224,8 +165,6 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
     static_assert(STAGES >= 2, "ring too small");
     static_assert(MT * NT <= 512, "accumulators exceed TMEM");
     constexpr uint32_t IDESC = umma_idesc(TR::FMT, false, true, 128, NT);
-    constexpr uint32_t IDESC_B = umma_idesc(UMMA_FMT_BF16, false, true, 128, NT);  // the bf16 correction pass (MIX)
-    static_assert(!MIX || (TR::SPLIT && KB % 16 == 0 && NT % 64 == 0), "mixed compensation: fp32 I/O, 16-channel groups");
 
     extern __shared__ unsigned char smem_raw[];
     unsigned char* smem = smem_align(smem_raw, 1024);
@@ -243,7 +182,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
     if (threadIdx.x == 0) {
         for (int i = 0; i < STAGES; ++i) {
             mbar_init(&full[i], 1);
-            mbar_init(&empty[i], CL);
+            mbar_init(&empty[i], 1);
             mbar_init(&xfull[i], 4);  // one arrival per operand-split warp
             mbar_init(&sfree[i], 1);
         }
@@ -259,22 +198,15 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
     if (warp == 1) tmem_alloc(tmem_slot, 512);
     tc_fence_before();
     __syncthreads();
-    if (CL > 1) cluster_sync_all();  // every CTA's barriers are initialised before a peer multicasts onto them
     tc_fence_after();
     const uint32_t tmem = *tmem_slot;
     const int nkb = (K + KB - 1) / KB;
-    // Work: tile group g = cluster index + i * clusters; this CTA takes tile CL*g + rank. A group past the end of an
-    // odd tile count repeats the last tile (same loads, same MMAs -- the ring must stay in lock step) and stores nothing.
-    const int crank = CL > 1 ? (int)cluster_ctarank() : 0;
-    const int ngroups = (total_tiles + CL - 1) / CL, gstride = gridDim.x / CL;
-    const int g0 = blockIdx.x / CL;
+    const int tile0 = blockIdx.x, tile_stride = gridDim.x;  // persistent CTAs: tiles tile0, tile0 + tile_stride, ...
 
     if (warp == 0) {
         if (lane == 0) {  // ---------------------------------------------------------------- TMA producer
             uint32_t it = 0;
-            for (int g = g0; g < ngroups; g += gstride) {
-                int tile = g * CL + crank;
-                if (tile >= total_tiles) tile = total_tiles - 1;
+            for (int tile = tile0; tile < total_tiles; tile += tile_stride) {
                 const int b = tile / tiles_per_img, px0 = (tile - b * tiles_per_img) * NT;
                 for (int kb = 0; kb < nkb; ++kb, ++it) {
                     const int s = it % STAGES;
@@ -293,12 +225,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
 #pragma unroll
                     for (int j = 0; j < NOPA * MT; ++j) {  // weight blocks: [hi of every row tile | lo of every row tile]
                         const int mt = j % MT;
-                        const CUtensorMap* mp = j < MT ? &mapAh : &mapAl;
-                        const int col = (MIX && j >= MT) ? 2 * kb * KB : kb * KB;  // the bf16 operand is 2K columns wide
-                        if (CL == 1) tma_load_2d(sa + j * TILE_A, mp, col, (m_tile0 + mt) * 128, &full[s]);
-                        else if (j % CL == crank)
-                            tma_load_2d_multicast(sa + j * TILE_A, mp, col, (m_tile0 + mt) * 128, &full[s],
-                                                  (uint16_t)((1u << CL) - 1));
+                        tma_load_2d(sa + j * TILE_A, j < MT ? &mapAh : &mapAl, kb * KB, (m_tile0 + mt) * 128, &full[s]);
                     }
                 }
             }
@@ -306,7 +233,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
     } else if (warp == 1) {
         if (lane == 0) {  // ---------------------------------------------------------------- MMA issuer
             uint32_t it = 0, tc = 0;
-            for (int g = g0; g < ngroups; g += gstride, ++tc) {
+            for (int tile = tile0; tile < total_tiles; tile += tile_stride, ++tc) {
                 const int a = tc % ACC;
                 mbar_wait(&acce[a], ((tc / ACC) & 1) ^ 1);
                 tc_fence_after();
@@ -325,17 +252,14 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
                         // tf32 has one MN-major layout: 32-byte swizzle atoms, K groups of 4 rows (512 bytes apart)
                         constexpr uint32_t XL = sizeof(T) == 4 ? UMMA_SW128_BASE32B : UMMA_SW128;
                         constexpr uint32_t XSBO = sizeof(T) == 4 ? 512u : 1024u;
-                        const uint32_t lbo = (dbg & 1) ? XSBO : (uint32_t)XCHUNK, sbo = (dbg & 1) ? (uint32_t)XCHUNK : XSBO;
-                        const uint64_t bh = umma_desc(sx + ks * (UK * 128), lbo, sbo, XL);
-                        const uint64_t bl = umma_desc(sx + XBYTES + ks * (UK * 128), lbo, sbo, XL);
+                        const uint64_t bh = umma_desc(sx + ks * (UK * 128), XCHUNK, XSBO, XL);
+                        const uint64_t bl = umma_desc(sx + XBYTES + ks * (UK * 128), XCHUNK, XSBO, XL);
                         const uint32_t first = (kb | ks) ? 1u : 0u;
 #pragma unroll
                         for (int mt = 0; mt < MT; ++mt) {
                             const uint32_t d = tmem + (uint32_t)((a * MT + mt) * NT);
                             const uint64_t ah = umma_desc(sa + mt * TILE_A + ks * 32, 16, ASBO, ASWZ);
-                            if (MIX) {
-                                umma_issue<T>(d, ah, bh, IDESC, first);
-                            } else if (TR::SPLIT) {
+                            if (TR::SPLIT) {
                                 const uint64_t al = umma_desc(sa + (MT + mt) * TILE_A + ks * 32, 16, ASBO, ASWZ);
                                 umma_issue<T>(d, al, bh, IDESC, first);
                                 umma_issue<T>(d, ah, bl, IDESC, 1u);
@@ -345,22 +269,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
                             }
                         }
                     }
-                    if (MIX) {
-                        // correction pass: [bf16(A_lo) | bf16(A_hi)] (K-major, 2*KB wide) . [bf16(X) ; bf16(X_lo)] (MN-major,
-                        // 64-pixel chunks of [2*KB rows][128 B]), K = 16 per instruction
-                        const int ksb = 2 * ksteps * UK / 16;
-                        for (int ks = 0; ks < ksb; ++ks) {
-                            const uint64_t bb = umma_desc(sx + XBYTES + ks * (16 * 128), 2 * KB * 128, 1024, UMMA_SW128);
-#pragma unroll
-                            for (int mt = 0; mt < MT; ++mt) {
-                                const uint32_t d = tmem + (uint32_t)((a * MT + mt) * NT);
-                                const uint64_t ab = umma_desc(sa + (MT + mt) * TILE_A + ks * 32, 16, ASBO, ASWZ);
-                                umma_bf16(d, ab, bb, IDESC_B, 1u);
-                            }
-                        }
-                    }
-                    if (CL == 1) umma_commit(&empty[s]);
-                    else umma_commit_multicast(&empty[s], (uint16_t)((1u << CL) - 1));
+                    umma_commit(&empty[s]);
                 }
                 umma_commit(&accf[a]);
             }
@@ -373,8 +282,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
 #pragma unroll
         for (int mt = 0; mt < MT; ++mt) sum[mt] = 0.0, sq[mt] = 0.0;
         uint32_t tc = 0;
-        for (int g = g0; g < ngroups; g += gstride, ++tc) {
-            const int tile = g * CL + crank;
+        for (int tile = tile0; tile < total_tiles; tile += tile_stride, ++tc) {
             const int b = tile / tiles_per_img, px0 = (tile - b * tiles_per_img) * NT;
             const int a = tc % ACC;
             mbar_wait(&accf[a], (tc / ACC) & 1);
@@ -382,7 +290,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
 #pragma unroll
             for (int mt = 0; mt < MT; ++mt) {
                 const int row0 = (m_tile0 + mt) * 128 + q * 32;
-                if (row0 >= M || tile >= total_tiles) continue;  // padded rows / the repeated tile of a short group
+                if (row0 >= M) continue;  // padded rows
                 // optional per-row affine (+ ReLU) of the output: the eval-mode BatchNorm (+ ReLU) that follows the
                 // convolution, folded into the epilogue (this thread's row = one output channel)
                 const float sc = ep_scale != nullptr ? __ldg(ep_scale + row0 + lane) : 1.f;
@@ -496,17 +404,13 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
         if constexpr (TR::SPLIT) {
             const int t = threadIdx.x - 6 * 32;
             uint32_t it = 0;
-            for (int g = g0; g < ngroups; g += gstride) {
-                int tile = g * CL + crank;
-                const bool real_tile = tile < total_tiles;
-                if (!real_tile) tile = total_tiles - 1;
+            for (int tile = tile0; tile < total_tiles; tile += tile_stride) {
                 const int b = tile / tiles_per_img, px0 = (tile - b * tiles_per_img) * NT;
                 for (int kb = 0; kb < nkb; ++kb, ++it) {
                     const int s = it % STAGES;
                     mbar_wait(&full[s], (it / STAGES) & 1);
                     unsigned char* st = smem + s * STAGE;
-                    if (MIX) mix_tile_mn<KB, NT>(st, st + XBYTES, t, 128);
-                    else if (bnbwd) bnbwd_tile<KB>(reinterpret_cast<float4*>(st), reinterpret_cast<float4*>(st + XBYTES), XBYTES / 16, t, 128, kb * KB, bn);
+                    if (bnbwd) bnbwd_tile<KB>(reinterpret_cast<float4*>(st), reinterpret_cast<float4*>(st + XBYTES), XBYTES / 16, t, 128, kb * KB, bn);
                     else split_tile_trunc(reinterpret_cast<float4*>(st), reinterpret_cast<float4*>(st + XBYTES), XBYTES / 16, t, 128);
                     fence_proxy_async_smem();
                     __syncwarp();
@@ -516,10 +420,8 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
                         // weight-gradient GEMM reads it later) while the MMAs consume the same buffers; the stage may be
                         // refilled once the MMAs AND this store have read it
                         mbar_wait(&xfull[s], (it / STAGES) & 1);
-                        if (real_tile) {
 #pragma unroll
-                            for (int c = 0; c < NCH; ++c) tma_store_2d(&mapDZ, px0 + c * PXC, b * K + kb * KB, st + c * XCHUNK);
-                        }
+                        for (int c = 0; c < NCH; ++c) tma_store_2d(&mapDZ, px0 + c * PXC, b * K + kb * KB, st + c * XCHUNK);
                         bulk_commit();
                         bulk_wait_read<1>();  // every store but the one just issued has left shared memory
                         if (it > 0) mbar_arrive(&sfree[(it - 1) % STAGES]);
@@ -531,7 +433,6 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
     }
     tc_fence_before();
     __syncthreads();
-    if (CL > 1) cluster_sync_all();  // no CTA leaves while a peer may still multicast into it or arrive on its barriers
     if (warp == 1) {
         tc_fence_after();
         tmem_dealloc(tmem, 512);
@@ -545,46 +446,6 @@ constexpr size_t nn_smem_bytes() {
     constexpr int STAGE = NOPA * (NT * KB * (int)sizeof(T) + MT * 128 * KB * (int)sizeof(T));
     constexpr int STAGES = (GEMM_RING_BYTES / STAGE) > 4 ? 4 : (GEMM_RING_BYTES / STAGE);
     return (size_t)STAGES * STAGE + 4 * 2 * 4096 + 256 + 1024;
-}
-
-static int gemm_dbg() {  // PM_GEMM_DBG: bring-up switches (bit 0 swaps LBO/SBO of the MN-major operand descriptor)
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("PM_GEMM_DBG");
-        v = e ? atoi(e) : 0;
-    }
-    return v;
-}
-
-static int gemm_mix() {
-    // PM_GEMM_MIX=1: TF32 + one bf16 correction pass instead of three TF32 passes. Measured at cfg 2: forward 51 vs 56 us,
-    // input gradient 76 vs 80 us -- but 1.1e-6 instead of 4e-7 at K = 64 (the correction operands carry 8 mantissa bits),
-    // which pushes the module's ill-conditioned gradients past the 1e-5 parity bar on two fixtures. Parity first: off.
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("PM_GEMM_MIX");
-        v = (e && e[0] == '1') ? 1 : 0;
-    }
-    return v;
-}
-
-static int gemm_narrow() {  // PM_GEMM_NARROW=1: keep the 128-pixel fp32 tiles (A/B switch for the profiles)
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("PM_GEMM_NARROW");
-        v = (e && e[0] == '1') ? 1 : 0;
-    }
-    return v;
-}
-
-static int gemm_cluster() {  // PM_GEMM_CLUSTER = 1 | 2 | 4 (default 1): CTAs sharing the weight blocks by TMA multicast
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("PM_GEMM_CLUSTER");
-        v = e ? atoi(e) : 1;  // measured: multicast at cluster sizes <= 4 does not reduce the SM's ingest, and lock step costs
-        if (v != 1 && v != 2 && v != 4) v = 1;
-    }
-    return v;
 }
 
 template <typename T, int MT, int NT, int KB>
@@ -603,10 +464,7 @@ static int launch_nn(const void* X, const void* Ah, const void* Al, void* Y, dou
     constexpr int ASW = KB * (int)sizeof(T) == 128 ? 1 : 3;  // TMA swizzle of the weight boxes: 128-byte or 64-byte rows
     if (!make_map_2d<T>(&mX, X, (size_t)B * K, hw, KB, TR::PXC, sizeof(T) == 4 ? 2 : 1)) return PM_ERR_ALIGN;
     if (!make_map_2d<T>(&mAh, Ah, Mpad, K, 128, KB, ASW)) return PM_ERR_ALIGN;
-    const bool mix = TR::SPLIT && gemm_mix() && K % 16 == 0 && bn.mean == nullptr;
-    if (mix) {
-        if (!make_map_2d<__nv_bfloat16>(&mAl, Al, Mpad, 2 * (size_t)K, 128, 2 * KB, ASW)) return PM_ERR_ALIGN;
-    } else if (TR::SPLIT) {
+    if (TR::SPLIT) {
         if (!make_map_2d<T>(&mAl, Al, Mpad, K, 128, KB, ASW)) return PM_ERR_ALIGN;
     } else {
         mAl = mAh;
@@ -615,42 +473,11 @@ static int launch_nn(const void* X, const void* Ah, const void* Al, void* Y, dou
     if (bn.mean == nullptr) mZ = mX, mDZ = mX;  // unused
     const int tiles_per_img = (hw + NT - 1) / NT, total = B * tiles_per_img;
     const size_t smem = nn_smem_bytes<T, MT, NT, KB>();
-    // clusters of CL CTAs share the weight blocks by TMA multicast; the NOPA*MT blocks of a stage must split evenly
-    constexpr int NBLK = (TR::SPLIT ? 2 : 1) * MT;
-    constexpr int CLMAX = NBLK >= 4 ? 4 : NBLK;
-    int cl = gemm_cluster();
-    if (cl > CLMAX) cl = CLMAX;
-    if (total < 2 * cl) cl = 1;
-    cudaLaunchConfig_t cfg{};
-    cudaLaunchAttribute attr[1];
-    cfg.blockDim = dim3(GEMM_THREADS);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = cl, attr[0].val.clusterDim.y = 1, attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr, cfg.numAttrs = 1;
-    int groups = (total + cl - 1) / cl, clusters = 148 / cl;
-    if (clusters > groups) clusters = groups;
-    cfg.gridDim = dim3(clusters * cl);
-    const int dbg = gemm_dbg();
-    cudaError_t e;
-#define PM_NN_LAUNCH(CL_)                                                                                             \
-    {                                                                                                                 \
-        auto kern = mix ? conv1x1_nn_kernel<T, MT, NT, KB, CL_, TR::SPLIT> : conv1x1_nn_kernel<T, MT, NT, KB, CL_, false>; \
-        e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                       \
-        if (e != cudaSuccess) return (int)e;                                                                          \
-        e = cudaLaunchKernelEx(&cfg, kern, mX, mAh, mAl, mY, K, M, m_tile0, tiles_per_img, total, accumulate, stats,     \
-                               ep_scale, ep_shift, ep_relu, dbg, mZ, mDZ, bn);                                   \
-    }
-    if (cl == 4) {
-        if constexpr (CLMAX >= 4) PM_NN_LAUNCH(4) else return PM_ERR_SHAPE;
-    } else if (cl == 2) {
-        if constexpr (CLMAX >= 2) PM_NN_LAUNCH(2) else return PM_ERR_SHAPE;
-    } else {
-        PM_NN_LAUNCH(1)
-    }
-#undef PM_NN_LAUNCH
+    const int grid = total < 148 ? total : 148;
+    cudaError_t e = cudaFuncSetAttribute(conv1x1_nn_kernel<T, MT, NT, KB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
+    conv1x1_nn_kernel<T, MT, NT, KB><<<grid, GEMM_THREADS, smem, st>>>(mX, mAh, mAl, mY, K, M, m_tile0, tiles_per_img, total,
+                                                                      accumulate, stats, ep_scale, ep_shift, ep_relu, mZ, mDZ, bn);
     e = cudaGetLastError();
     return e == cudaSuccess ? 0 : (int)e;
 }
@@ -665,7 +492,7 @@ static int launch_nn(const void* X, const void* Ah, const void* Al, void* Y, dou
 // =================================================================================================================
 constexpr int WG_NMAX = 288;
 
-template <typename T, bool MIX>
+template <typename T>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
     conv1x1_wgrad_kernel(const __grid_constant__ CUtensorMap mapG, const __grid_constant__ CUtensorMap mapX, int M, int N,
                          int Ntot, int n0, int NW, int hw, int chunks_per_img, int blocks_per_chunk, float* __restrict__ part,
@@ -746,13 +573,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
                     for (int j = 0; j < NI; ++j) {
                         const uint32_t d = tmem + (uint32_t)(j * NW);
                         const uint64_t bh = umma_desc(sb + j * NW * 128 + ks * 32, 16, 1024);
-                        if (MIX) {
-                            // main TF32 pass + the bf16 correction over the concatenated K ([lo | x] . [x ; lo]): each
-                            // K step covers 16 bf16 = 32 bytes of the 128-byte rows, like a TF32 step
-                            const uint64_t bb = umma_desc(sb + BBYTES + j * NW * 128 + ks * 32, 16, 1024);
-                            umma_issue<T>(d, ah, bh, IDESC, first);
-                            umma_bf16(d, al, bb, umma_idesc(UMMA_FMT_BF16, false, false, 128, NW), 1u);
-                        } else if (TR::SPLIT) {
+                        if (TR::SPLIT) {
                             const uint64_t bl = umma_desc(sb + BBYTES + j * NW * 128 + ks * 32, 16, 1024);
                             umma_issue<T>(d, al, bh, IDESC, first);
                             umma_issue<T>(d, ah, bl, IDESC, 1u);
@@ -791,14 +612,9 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
                 const int s = kb % STAGES;
                 mbar_wait(&full[s], (kb / STAGES) & 1);
                 unsigned char* st = smem + s * STAGE;
-                if (MIX) {
-                    mix_tile_k(st, st + TILE_A_BYTES, 128, false, t, 128);
-                    mix_tile_k(st + 2 * TILE_A_BYTES, st + 2 * TILE_A_BYTES + BBYTES, N, true, t, 128);
-                } else {
-                    split_tile_trunc(reinterpret_cast<float4*>(st), reinterpret_cast<float4*>(st + TILE_A_BYTES), TILE_A_BYTES / 16, t, 128);
-                    split_tile_trunc(reinterpret_cast<float4*>(st + 2 * TILE_A_BYTES), reinterpret_cast<float4*>(st + 2 * TILE_A_BYTES + BBYTES),
-                                     N * 8, t, 128);
-                }
+                split_tile_trunc(reinterpret_cast<float4*>(st), reinterpret_cast<float4*>(st + TILE_A_BYTES), TILE_A_BYTES / 16, t, 128);
+                split_tile_trunc(reinterpret_cast<float4*>(st + 2 * TILE_A_BYTES), reinterpret_cast<float4*>(st + 2 * TILE_A_BYTES + BBYTES),
+                                 N * 8, t, 128);
                 fence_proxy_async_smem();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&xfull[s]);
@@ -885,13 +701,9 @@ static int launch_wgrad(const void* dY, const void* X, float* part, float* dW, i
     if (!make_map_2d<T>(&mX, X, (size_t)B * Ntot, hw, NW, TR::PXC, true)) return PM_ERR_ALIGN;
     const size_t smem = wgrad_smem_bytes<T>();
     dim3 grid(B * cpi, Mpad / 128);
-    // measured at cfg 2: the mixed pass does not pay here (77 vs 74.5 us) -- this kernel is bound by shared-memory traffic
-    // and by the operand ingest of a 128 x 288 tile, and the bf16 conversion costs the split warps more than the MMAs save
-    static const bool wg_mix = getenv("PM_GEMM_WGRAD_MIX") != nullptr;
-    auto kern = (TR::SPLIT && wg_mix) ? conv1x1_wgrad_kernel<T, TR::SPLIT> : conv1x1_wgrad_kernel<T, false>;
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(conv1x1_wgrad_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
-    kern<<<grid, GEMM_THREADS, smem, st>>>(mG, mX, M, N, Ntot, n0, NW, hw, cpi, bpc, part, Mpad);
+    conv1x1_wgrad_kernel<T><<<grid, GEMM_THREADS, smem, st>>>(mG, mX, M, N, Ntot, n0, NW, hw, cpi, bpc, part, Mpad);
     e = cudaGetLastError();
     if (e != cudaSuccess) return (int)e;
     const int n4 = M * (N / 4);
@@ -902,11 +714,9 @@ static int launch_wgrad(const void* dY, const void* X, float* part, float* dW, i
 
 // A[m][k] = W[m][k] (transpose = 0, W is [M][K]) or W[k][m] (transpose = 1, W is [K][M]); rows M..Mpad-1 are zero.
 // fp32: hi = W rounded to nearest TF32, lo = W - hi (both fp32 [Mpad][K]); bf16: hi = bf16(W).
-// fp32, mixed compensation (mix != 0): `lo` is instead the bf16 operand of the correction pass, [Mpad][2K]: per group g of 16
-// channels, columns [32g, 32g+16) = bf16(W - hi) and [32g+16, 32g+32) = bf16(hi) (same bytes as an fp32 [Mpad][K]).
 template <typename T>
 __global__ void conv1x1_prep_kernel(const float* __restrict__ W, int M, int K, int Mpad, int transpose, T* __restrict__ hi,
-                                    T* __restrict__ lo, int mix) {
+                                    T* __restrict__ lo) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= Mpad * K) return;
     const int m = i / K, k = i - m * K;
@@ -914,13 +724,7 @@ __global__ void conv1x1_prep_kernel(const float* __restrict__ W, int M, int K, i
     if constexpr (sizeof(T) == 4) {
         const float h = tf32_rn(v);
         hi[i] = h;
-        if (mix) {
-            __nv_bfloat16* lb = reinterpret_cast<__nv_bfloat16*>(lo) + (size_t)m * 2 * K + ((k >> 4) << 5) + (k & 15);
-            lb[0] = __float2bfloat16_rn(v - h);
-            lb[16] = __float2bfloat16_rn(h);
-        } else {
-            lo[i] = v - h;
-        }
+        lo[i] = v - h;
     } else {
         hi[i] = __float2bfloat16_rn(v);
     }
@@ -930,7 +734,7 @@ __global__ void conv1x1_prep_kernel(const float* __restrict__ W, int M, int K, i
 // input-gradient GEMM is produced next to the forward one instead of by a second launch in the backward pass
 template <typename T>
 __global__ void conv1x1_prep_both_kernel(const float* __restrict__ W, int R, int S, T* __restrict__ hi, T* __restrict__ lo,
-                                         T* __restrict__ hiT, T* __restrict__ loT, int mix, double* __restrict__ zero,
+                                         T* __restrict__ hiT, T* __restrict__ loT, double* __restrict__ zero,
                                          int zero_n) {
     // the statistics buffer of the BatchNorm that follows the forward GEMM is zeroed here (this launch precedes the GEMM
     // on the same stream) instead of by a fill kernel of its own
@@ -947,13 +751,7 @@ __global__ void conv1x1_prep_both_kernel(const float* __restrict__ W, int R, int
     if constexpr (sizeof(T) == 4) {
         const float h = tf32_rn(v);
         h_out[i] = h;
-        if (mix && K % 16 == 0) {
-            __nv_bfloat16* lb = reinterpret_cast<__nv_bfloat16*>(l_out) + (size_t)m * 2 * K + ((k >> 4) << 5) + (k & 15);
-            lb[0] = __float2bfloat16_rn(v - h);
-            lb[16] = __float2bfloat16_rn(h);
-        } else {
-            l_out[i] = v - h;
-        }
+        l_out[i] = v - h;
     } else {
         h_out[i] = __float2bfloat16_rn(v);
     }
@@ -974,9 +772,9 @@ int pm_conv1x1_prep_both(const float* W, int R, int S, int dtype, void* A_hi, vo
     cudaStream_t st = (cudaStream_t)stream;
     const dim3 grid((n + 255) / 256, 2);
     if (dtype == PM_F32)
-        conv1x1_prep_both_kernel<float><<<grid, 256, 0, st>>>(W, R, S, (float*)A_hi, (float*)A_lo, (float*)At_hi, (float*)At_lo, gemm_mix(), zero, zero_n);
+        conv1x1_prep_both_kernel<float><<<grid, 256, 0, st>>>(W, R, S, (float*)A_hi, (float*)A_lo, (float*)At_hi, (float*)At_lo, zero, zero_n);
     else
-        conv1x1_prep_both_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(W, R, S, (__nv_bfloat16*)A_hi, nullptr, (__nv_bfloat16*)At_hi, nullptr, 0, zero, zero_n);
+        conv1x1_prep_both_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(W, R, S, (__nv_bfloat16*)A_hi, nullptr, (__nv_bfloat16*)At_hi, nullptr, zero, zero_n);
     PM_CHECK_LAUNCH();
     return 0;
 }
@@ -988,10 +786,9 @@ int pm_conv1x1_prep(const float* W, int M, int K, int transpose, int dtype, void
     const int Mpad = (M + 127) / 128 * 128, n = Mpad * K;
     cudaStream_t st = (cudaStream_t)stream;
     if (dtype == PM_F32)
-        conv1x1_prep_kernel<float><<<(n + 255) / 256, 256, 0, st>>>(W, M, K, Mpad, transpose, (float*)A_hi, (float*)A_lo,
-                                                                    (gemm_mix() && K % 16 == 0) ? 1 : 0);
+        conv1x1_prep_kernel<float><<<(n + 255) / 256, 256, 0, st>>>(W, M, K, Mpad, transpose, (float*)A_hi, (float*)A_lo);
     else
-        conv1x1_prep_kernel<__nv_bfloat16><<<(n + 255) / 256, 256, 0, st>>>(W, M, K, Mpad, transpose, (__nv_bfloat16*)A_hi, nullptr, 0);
+        conv1x1_prep_kernel<__nv_bfloat16><<<(n + 255) / 256, 256, 0, st>>>(W, M, K, Mpad, transpose, (__nv_bfloat16*)A_hi, nullptr);
     PM_CHECK_LAUNCH();
     return 0;
 }
@@ -1022,7 +819,7 @@ static int conv1x1_fwd_impl(const void* X, const void* A_hi, const void* A_lo, v
             const void* Zi = first ? Z : nullptr;
             void* DZo = first ? DZ : nullptr;
             const BnBwdArgs* bi = first ? bn : nullptr;
-            if (wide && !gemm_narrow())
+            if (wide)
                 rc = mt == 2 ? launch_nn<float, 2, 256, 16>(Xin, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st, Zi, DZo, bi)
                              : launch_nn<float, 1, 256, 16>(Xin, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st, Zi, DZo, bi);
             else

@@ -7,7 +7,6 @@
 // K x C memory sits transposed in shared memory (Mt[c][KP]: a channel's K values are five broadcast
 // 128-bit loads) and all multiply-adds are packed FFMA2 (fp32x2), which is what reaches the fp32 peak
 // on sm_100 (profiles/microbench/ffma2.cu: 65.9 vs 46.8 TFLOP/s for scalar FFMA).
-#include <cstdlib>
 
 #include "pm_common.cuh"
 #include "pm_tma.cuh"
@@ -1307,9 +1306,8 @@ int launch_read_bwd_tiled(const void* du, const void* x, const float* M, const f
         CUtensorMap tm_x, tm_du;
         cudaError_t e;
         if constexpr (sizeof(T) == 2 && (C == 128 || C == 256)) {
-            static const bool off = getenv("PM_BF16_MMA_OFF") != nullptr;  // A/B switch
             CUtensorMap tm_dx;
-            if (!off && dx_add == nullptr && tma_enabled() && make_map_2d<T>(&tm_x, x, (size_t)B * C, hw, C, TP, 3) &&
+            if (dx_add == nullptr && tma_enabled() && make_map_2d<T>(&tm_x, x, (size_t)B * C, hw, C, TP, 3) &&
                 make_map_2d<T>(&tm_du, du, (size_t)B * UC, hw, C, TP, 3) && make_map_2d<T>(&tm_dx, dx, (size_t)B * C, hw, C, TP, 3)) {
                 constexpr int NS = 2;
                 const size_t sm = sizeof(T) * (size_t)NS * 2 * C * TP + sizeof(float) * ((size_t)NS * TP * KP + 2 * DXB_WARPS * TP) +

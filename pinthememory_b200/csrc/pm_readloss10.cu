@@ -1,9 +1,9 @@
 // Feature-cohesion read loss, fourth kernel: warps that own their cells end to end.
 //
-// The third kernel (pm_readloss9.cu) has the right instruction mix in its label loop but spends more than half of its time
-// in per-CTA phases: tile load -> barrier -> rows -> barrier -> y-weighting -> barrier -> flush -> reduction -> ticket, at
-// two CTAs per SM (profiles/r2f_ncu_full.txt, DESIGN.md section 6). Here nothing is CTA-wide until the very last
-// instruction:
+// The third kernel (a thread per label row, since removed) had the right instruction mix in its label loop but spent
+// more than half of its time in per-CTA phases: tile load -> barrier -> rows -> barrier -> y-weighting -> barrier -> flush
+// -> reduction -> ticket, at two CTAs per SM (profiles/r2f_ncu_full.txt, DESIGN.md section 6). Here nothing is CTA-wide
+// until the very last instruction:
 //   * a warp = 16 neighbouring cells of one cell row x 2 lanes per cell; each lane of a pair carries HALF of the 20 slots
 //     (float2 slot pairs 2j + half): E, ratio, the two row sums and the four tap accumulators are 5 float2 each = 80
 //     registers, so the kernel stays at 128 registers (16 warps per SM) while a thread still walks ALL label rows of its

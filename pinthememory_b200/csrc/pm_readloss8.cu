@@ -22,7 +22,6 @@
 // loss and ds_rl stay below 3e-6 (tests/test_gpu_parity.py). The weights lambda_x / lambda_y themselves are computed
 // exactly as PyTorch does (fp32 `scale * dst`, floor, clamp).
 #include "pm_common.cuh"
-#include <cstdlib>
 
 namespace pm {
 
@@ -396,22 +395,9 @@ __global__ void __launch_bounds__(RL8_THREADS, 2)
 
 }  // namespace pm
 
-// third-generation kernel (pm_readloss9.cu): 0 = launched, -1 = shape outside its fixed-point range
-int pm_readloss_rows_launch(const float* s, const uint8_t* lab8, float temperature, int B, int h, int w, int Hm, int Wm, int K,
-                            float* ds_rl, void* ws, float* out, cudaStream_t st);
+// cells kernel (pm_readloss10.cu): 0 = launched, -1 = shape outside its fixed-point range
 int pm_readloss_cells_launch(const float* s, const uint8_t* lab8, float temperature, int B, int h, int w, int Hm, int Wm, int K,
                              float* ds_rl, void* ws, float* out, cudaStream_t st);
-// PINMEM_B200_READLOSS_GEN = 2 | 3 | 4 (default 4): which kernel generation runs (A/B switch for the profiles);
-// PINMEM_B200_READLOSS_GEN2=1 is the older spelling of GEN=2. Generation 3 needs cells of >= 6 label pixels, generation 4
-// of >= 3 (PM_RL_MINRATIO); narrower cells take generation 2.
-static int readloss_gen() {   // read on every call (a getenv): tests flip it inside one process
-    const char* e = getenv("PINMEM_B200_READLOSS_GEN");
-    int v = e ? atoi(e) : 4;
-    const char* e2 = getenv("PINMEM_B200_READLOSS_GEN2");
-    if (e2 && e2[0] == '1') v = 2;
-    if (v < 2 || v > 4) v = 4;
-    return v;
-}
 
 extern "C" int pm_readloss_fwd8(const float* s, const uint8_t* lab8, float temperature, int B, int h, int w, int Hm, int Wm,
                                 int K, float* ds_rl, void* ws, float* out, void* stream) {
@@ -420,12 +406,8 @@ extern "C" int pm_readloss_fwd8(const float* s, const uint8_t* lab8, float tempe
     if (B <= 0 || h <= 0 || w <= 0 || Hm <= 0 || Wm <= 0 || !(temperature > 0.f)) return PM_ERR_SHAPE;
     if (((uintptr_t)s & 15) || ((uintptr_t)ds_rl & 15) || ((uintptr_t)ws & 7)) return PM_ERR_ALIGN;
     const int minratio = 3;   // narrower cells (label map < 3x the feature map) keep the one-thread-per-cell kernel
-    if (readloss_gen() == 4 && w > 1 && (Wm - 1) / (w - 1) >= minratio) {
+    if (w > 1 && (Wm - 1) / (w - 1) >= minratio) {
         const int rc = pm_readloss_cells_launch(s, lab8, temperature, B, h, w, Hm, Wm, K, ds_rl, ws, out, (cudaStream_t)stream);
-        if (rc >= 0) return rc;
-    }
-    if (readloss_gen() >= 3) {
-        const int rc = pm_readloss_rows_launch(s, lab8, temperature, B, h, w, Hm, Wm, K, ds_rl, ws, out, (cudaStream_t)stream);
         if (rc >= 0) return rc;
     }
     using namespace pm;

@@ -72,32 +72,6 @@ __device__ __forceinline__ void umma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 
-// the same, arriving on the barrier at this offset in every CTA of `cta_mask` (cluster-wide ring slots)
-__device__ __forceinline__ void umma_commit_multicast(uint64_t* bar, uint16_t cta_mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                     smem_u32(bar)),
-                 "h"(cta_mask)
-                 : "memory");
-}
-// TMA load whose box lands at the same shared-memory offset of every CTA in `cta_mask` (and completes on the
-// barrier at the same offset in each of them): one L2 read feeds the whole cluster
-__device__ __forceinline__ void tma_load_2d_multicast(void* dst, const CUtensorMap* map, int c0, int c1, uint64_t* bar,
-                                                      uint16_t cta_mask) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%2, "
-        "%3}], [%4], %5;" ::"r"(smem_u32(dst)),
-        "l"(reinterpret_cast<uint64_t>(map)), "r"(c0), "r"(c1), "r"(smem_u32(bar)), "h"(cta_mask)
-        : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\nbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-
 // 32 lanes x 32 consecutive columns: thread = lane (row of D), r[j] = column j. Warp w may only touch lanes
 // 32*(w%4) .. 32*(w%4)+31. Follow with tmem_ld_wait() before using r.
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {

@@ -1,5 +1,4 @@
 // Memory write, pipelined variants (fast path when hw is a multiple of the 16-byte chunk).
-#include <cstdlib>
 
 #include "pm_common.cuh"
 #include "pm_tma.cuh"
@@ -916,14 +915,11 @@ int write_reduce_tiled(const void* f, const void* labels, int lab_u8, float* SD,
             default: return PM_ERR_CHANNELS;
         }
     } else {
-        static const bool mma_off = getenv("PM_BF16_MMA_OFF") != nullptr;  // A/B switch: the run-length FFMA2 kernel
-        if (!mma_off) {
-            switch (C) {  // tensor-core variant (whole 32-channel warps, >= 64 threads for the tile loads)
-                case 64: return launch_write_reduce_mma16<64, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st);
-                case 128: return launch_write_reduce_mma16<128, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st);
-                case 256: return launch_write_reduce_mma16<256, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st);
-                default: break;
-            }
+        switch (C) {  // tensor-core variant (whole 32-channel warps, >= 64 threads for the tile loads)
+            case 64: return launch_write_reduce_mma16<64, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st);
+            case 128: return launch_write_reduce_mma16<128, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st);
+            case 256: return launch_write_reduce_mma16<256, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st);
+            default: break;  // C = 32: the run-length FFMA2 kernel
         }
         if (K <= 19) { PM_WT_SWITCH_C(__nv_bfloat16, 20, launch_write_reduce_tiled, f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st) }
         else { PM_WT_SWITCH_C(__nv_bfloat16, 32, launch_write_reduce_tiled, f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st) }

@@ -114,7 +114,7 @@ class _ReadFn(torch.autograd.Function):
         # orders it before the write kernels that consume the packed map) and the column softmax on a second side stream
         # under the read loss: two small kernels (17 + 11 us at cfg 2) leave the main chain. Captured, they are parallel
         # branches of the graph.
-        use_pack = labels is not None and K <= 19 and not os.environ.get("PINMEM_B200_READLOSS_V1")
+        use_pack = labels is not None and K <= 19
         branch = bool(branch) and x.is_cuda
         lab8 = None
         if branch:

@@ -42,7 +42,6 @@ def noise():
     capi.conv1x1_wgrad(a, b)
 
 
-print("cluster", os.environ.get("PM_GEMM_CLUSTER"))
 diag(8, 256, 256, 48, 48, False)
 diag(8, 256, 256, 48, 48, True)
 diag(8, 256, 256, 48, 48, True, pre=noise)

@@ -47,8 +47,8 @@ ENTRY_OF = [("readloss8_kernel", "pm_readloss_fwd8"), ("labels_pack_kernel", "pm
             ("bn_stats_kernel", "pm_bn_stats"), ("bn_apply_kernel", "pm_bn_apply"),
             ("write_reduce_mma_kernel", "pm_write_reduce_fwd"), ("write_reduce_tiled_kernel", "pm_write_reduce_fwd"),
             ("update_fwd_kernel", "pm_update_fwd"), ("update_bwd_kernel", "pm_update_bwd"),
-            ("write_bwd_tiled_kernel", "pm_write_bwd"), ("bn_bwd_reduce_kernel", "pm_bn_bwd_reduce"), ("bn_bwd_reduce_rows_kernel", "pm_bn_bwd_reduce_rows"),
-            ("readloss_rows_kernel", "pm_readloss_fwd8"), ("readloss_cells_kernel", "pm_readloss_fwd8"),
+            ("write_bwd_tiled_kernel", "pm_write_bwd"), ("bn_bwd_reduce_rows_kernel", "pm_bn_bwd_reduce_rows"),
+            ("readloss8_kernel", "pm_readloss_fwd8"), ("readloss_cells_kernel", "pm_readloss_fwd8"),
             ("bn_bwd_apply_kernel", "pm_bn_bwd_apply"), ("read_bwd_ds_tiled_kernel", "pm_read_bwd.ds"), ("read_bwd_ds_planes_kernel", "pm_read_bwd.ds"),
             ("read_bwd_dx_tiled_kernel", "pm_read_bwd.dx"), ("read_bwd_dx_tma_kernel", "pm_read_bwd.dx")]
 
