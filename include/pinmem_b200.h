@@ -54,7 +54,7 @@ enum pm_readloss_ws_layout {
 #define PM_COLPART_ROWS 296
 
 /* Bumped with every prototype change; the binding refuses a library whose pm_version() differs. */
-#define PM_ABI_VERSION 209
+#define PM_ABI_VERSION 210
 int pm_version(void);
 const char* pm_status_string(int code);
 /* Row stride (floats) of the internal score buffers for K slots: 20 for K<=19, else 32. */
@@ -423,6 +423,40 @@ int pm_upcat_fwd(const void* fine, const void* coarse, void* out, int dtype, int
  * The gradient of `fine` is g's planes [0,Cf) as they are (what cat's backward returns); no kernel touches it.
  */
 int pm_upcat_bwd(const void* g, void* d_coarse, int dtype, int B, int Cf, int Cc, int h, int w, int H, int W, void* stream);
+
+/*
+ * Ordered (bitwise reproducible) variants of the entries whose kernels combine per-CTA partials with float atomics.
+ * Each takes the same arguments as its counterpart plus a caller-owned, 16-byte aligned `scratch` of at least the size
+ * the matching *_scratch_bytes query returns (a negative pm_status for arguments the entry would reject). The kernels
+ * store every CTA's partial to scratch (its contents on entry do not matter) and a second kernel adds the partials in
+ * ascending CTA order, so the same inputs on the same GPU model give the same bits on every call. Outputs keep their
+ * counterparts' semantics: the sums are ADDED into SD / dM / stats, which the caller zeroes (or accumulates into), and
+ * ds_rl / out / ws are as pm_readloss_fwd leaves them (ds_rl is stored, not added).
+ *
+ * pm_readloss_fwd_ordered: pm_readloss_fwd (memory.py:173-176), any K <= 31, int64 labels.
+ * pm_readloss_fwd8_ordered: pm_readloss_fwd8 on the packed map (K <= 19), always on the one-thread-per-cell kernel.
+ *   Scratch: pm_readloss_scratch_bytes(B, h, w, Hm, Wm, K, packed) with packed = 0 / 1 for the two.
+ */
+int pm_readloss_scratch_bytes(int B, int h, int w, int Hm, int Wm, int K, int packed);
+int pm_readloss_fwd_ordered(const float* s, const int64_t* labels, float temperature, int B, int h, int w, int Hm, int Wm,
+                            int K, float* ds_rl, void* ws, float* out, float* scratch, void* stream);
+int pm_readloss_fwd8_ordered(const float* s, const uint8_t* lab8, float temperature, int B, int h, int w, int Hm, int Wm,
+                             int K, float* ds_rl, void* ws, float* out, float* scratch, void* stream);
+/* pm_write_reduce_fwd / _fwd8 (memory.py:215,220-231): class sums|counts added into SD [K+1, C+4]. */
+int pm_write_reduce_scratch_bytes(int B, int C, int h, int w, int K);
+int pm_write_reduce_fwd_ordered(const void* f, const int64_t* labels, float* SD, float* scratch, int B, int C, int h, int w,
+                                int Hm, int Wm, int K, int dtype, void* stream);
+int pm_write_reduce_fwd8_ordered(const void* f, const uint8_t* lab8, float* SD, float* scratch, int B, int C, int h, int w,
+                                 int Hm, int Wm, int K, int dtype, void* stream);
+/* pm_read_bwd_dM (autograd of memory.py:171,328 with respect to the memory): dM [K,C] added into. */
+int pm_read_bwd_dM_scratch_bytes(int B, int C, int h, int w, int K);
+int pm_read_bwd_dM_ordered(const void* du, const void* x, const float* score_m, const float* ds, float* dM, float* scratch,
+                           int B, int C, int h, int w, int K, int dtype, void* stream);
+/* pm_conv1x1_fwd with statistics (memory.py:74-76,103-105, conv + BatchNorm batch statistics), accumulate = 0: stats
+ * [sum | sum of squares] (fp64, 8-byte aligned, as are the scratch words) added into. */
+int pm_conv1x1_stats_scratch_bytes(int B, int M, int hw, int dtype);
+int pm_conv1x1_fwd_ordered(const void* X, const void* A_hi, const void* A_lo, void* Y, double* stats, double* scratch, int B,
+                           int K, int M, int hw, int dtype, void* stream);
 
 #ifdef __cplusplus
 }

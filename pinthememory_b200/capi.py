@@ -19,7 +19,7 @@ WS_BAD = 2     # PM_WS_BAD
 SEG_WS_WORDS = 4  # PM_SEG_WS_WORDS
 SEG_WS_BAD = 2    # PM_SEG_WS_BAD
 
-ABI_VERSION = 209  # PM_ABI_VERSION of include/pinmem_b200.h the argtypes below were written against
+ABI_VERSION = 210  # PM_ABI_VERSION of include/pinmem_b200.h the argtypes below were written against
 
 _c_p = ctypes.c_void_p
 _c_i = ctypes.c_int
@@ -77,6 +77,16 @@ PROTOTYPES = {
     "pm_seg_eval": [_c_p] + [_c_i] * 5 + [_c_p] + [_c_i] * 3 + [_c_p] * 5,
     "pm_upcat_fwd": [_c_p] * 3 + [_c_i] * 8 + [_c_p],
     "pm_upcat_bwd": [_c_p] * 2 + [_c_i] * 8 + [_c_p],
+    "pm_readloss_scratch_bytes": [_c_i] * 7,
+    "pm_readloss_fwd_ordered": [_c_p, _c_p, _c_f] + [_c_i] * 6 + [_c_p] * 5,
+    "pm_readloss_fwd8_ordered": [_c_p, _c_p, _c_f] + [_c_i] * 6 + [_c_p] * 5,
+    "pm_write_reduce_scratch_bytes": [_c_i] * 5,
+    "pm_write_reduce_fwd_ordered": [_c_p] * 4 + [_c_i] * 8 + [_c_p],
+    "pm_write_reduce_fwd8_ordered": [_c_p] * 4 + [_c_i] * 8 + [_c_p],
+    "pm_read_bwd_dM_scratch_bytes": [_c_i] * 5,
+    "pm_read_bwd_dM_ordered": [_c_p] * 6 + [_c_i] * 6 + [_c_p],
+    "pm_conv1x1_stats_scratch_bytes": [_c_i] * 4,
+    "pm_conv1x1_fwd_ordered": [_c_p] * 6 + [_c_i] * 5 + [_c_p],
 }
 EXPORTED_SYMBOLS = sorted(list(PROTOTYPES) + ["pm_status_string"])
 
@@ -189,7 +199,9 @@ def score_stride(K):
 # with CUDA events on the launching stream to get per-kernel durations live.
 
 LAUNCHES = 0
-_KERNELS_PER_CALL = {"pm_conv1x1_dgrad_bnbwd": 2, "pm_colsoftmax": 3, "pm_colsoftmax_apply": 1, "pm_read_bwd": 2, "pm_read_bwd_planes": 2, "pm_conv1x1_wgrad": 2}
+_KERNELS_PER_CALL = {"pm_readloss_fwd_ordered": 2, "pm_readloss_fwd8_ordered": 2, "pm_write_reduce_fwd_ordered": 2,
+                     "pm_write_reduce_fwd8_ordered": 2, "pm_read_bwd_dM_ordered": 2, "pm_conv1x1_fwd_ordered": 2,
+                     "pm_conv1x1_dgrad_bnbwd": 2, "pm_colsoftmax": 3, "pm_colsoftmax_apply": 1, "pm_read_bwd": 2, "pm_read_bwd_planes": 2, "pm_conv1x1_wgrad": 2}
 PLANES = 32  # PM_PLANES: score planes appended to q in the score-plane read
 _timing = None  # name -> list of (start_event, end_event) when enabled
 
@@ -233,6 +245,19 @@ def _call(name, *args):
 # --------------------------------------------------------------------------------------------- calls
 
 
+def deterministic():
+    """torch's own switch, read at call time as torch's kernels read it: when set, the wrappers below whose default kernels
+    combine per-CTA partials with float atomics call the ordered entries instead (bitwise reproducible on one GPU model)."""
+    return torch.are_deterministic_algorithms_enabled()
+
+
+def _scratch(nbytes, device, what):
+    """Scratch of an ordered entry from torch's allocator (its contents on entry do not matter)."""
+    if nbytes < 0:
+        _check(nbytes, what)
+    return torch.empty(max(int(nbytes), 16), dtype=torch.uint8, device=device)
+
+
 def planes_ok(x):
     """The score-plane read runs only on the pipelined kernels: 16-byte rows and pointers."""
     hw = x.shape[2] * x.shape[3]
@@ -259,6 +284,11 @@ def colsoftmax_workspace_floats(K):
 
 def readloss_fwd(s, labels, temperature, B, h, w, K, ds_rl, ws, out):
     Hm, Wm = labels.shape[1], labels.shape[2]
+    if deterministic():
+        scratch = _scratch(load().pm_readloss_scratch_bytes(B, h, w, Hm, Wm, K, 0), s.device, "pm_readloss_scratch_bytes")
+        _call("pm_readloss_fwd_ordered", _ptr(s), _ptr(labels), float(temperature), B, h, w, Hm, Wm, K, _ptr(ds_rl), _ptr(ws),
+              _ptr(out), _ptr(scratch), _stream())
+        return
     _call("pm_readloss_fwd", _ptr(s), _ptr(labels), float(temperature), B, h, w, Hm, Wm, K, _ptr(ds_rl),
                                   _ptr(ws), _ptr(out), _stream())
 
@@ -278,6 +308,11 @@ def read_bwd(du, x, M, score_m, ds_rl, g_loss, rl_out, dx, ds, K, planes=False, 
 
 def read_bwd_dM(du, x, score_m, ds, dM, K):
     B, C, h, w = x.shape
+    if deterministic():
+        scratch = _scratch(load().pm_read_bwd_dM_scratch_bytes(B, C, h, w, K), x.device, "pm_read_bwd_dM_scratch_bytes")
+        _call("pm_read_bwd_dM_ordered", _ptr(du), _ptr(x), _ptr(score_m), _ptr(ds), _ptr(dM), _ptr(scratch), B, C, h, w, K,
+              dtype_code(x), _stream())
+        return
     _call("pm_read_bwd_dM", _ptr(du), _ptr(x), _ptr(score_m), _ptr(ds), _ptr(dM), B, C, h, w, K,
                                  dtype_code(x), _stream())
 
@@ -302,6 +337,11 @@ def write_reduce_fwd(f, labels, SD, K):
     """labels: int64 class ids, or the packed uint8 map of labels_pack (class K = ignore)."""
     B, C, h, w = f.shape
     Hm, Wm = labels.shape[1], labels.shape[2]
+    if deterministic():
+        scratch = _scratch(load().pm_write_reduce_scratch_bytes(B, C, h, w, K), f.device, "pm_write_reduce_scratch_bytes")
+        _call("pm_write_reduce_fwd8_ordered" if labels.dtype == torch.uint8 else "pm_write_reduce_fwd_ordered", _ptr(f),
+              _ptr(labels), _ptr(SD), _ptr(scratch), B, C, h, w, Hm, Wm, K, dtype_code(f), _stream())
+        return
     _call("pm_write_reduce_fwd8" if labels.dtype == torch.uint8 else "pm_write_reduce_fwd", _ptr(f), _ptr(labels), _ptr(SD), B, C, h, w, Hm, Wm, K, dtype_code(f),
                                       _stream())
 
@@ -425,6 +465,12 @@ def conv1x1_fwd(x, A_hi, A_lo, M, y=None, stats=None, accumulate=False):
     B, K, h, w = x.shape
     if y is None:
         y = torch.empty(B, M, h, w, dtype=x.dtype, device=x.device)
+    if stats is not None and not accumulate and deterministic():
+        nbytes = load().pm_conv1x1_stats_scratch_bytes(B, M, h * w, dtype_code(x))
+        scratch = _scratch(nbytes, x.device, "pm_conv1x1_stats_scratch_bytes")
+        _call("pm_conv1x1_fwd_ordered", _ptr(x), _ptr(A_hi), _ptr(A_lo), _ptr(y), _ptr(stats), _ptr(scratch), B, K, M, h * w,
+              dtype_code(x), _stream())
+        return y
     _call("pm_conv1x1_fwd", _ptr(x), _ptr(A_hi), _ptr(A_lo), _ptr(y), _ptr(stats), B, K, M, h * w, int(bool(accumulate)),
           dtype_code(x), _stream())
     return y
@@ -516,6 +562,11 @@ def labels_pack(labels, K, ws):
 
 def readloss_fwd8(s, lab8, temperature, B, h, w, K, ds_rl, ws, out):
     Hm, Wm = lab8.shape[1], lab8.shape[2]
+    if deterministic():
+        scratch = _scratch(load().pm_readloss_scratch_bytes(B, h, w, Hm, Wm, K, 1), s.device, "pm_readloss_scratch_bytes")
+        _call("pm_readloss_fwd8_ordered", _ptr(s), _ptr(lab8), float(temperature), B, h, w, Hm, Wm, K, _ptr(ds_rl), _ptr(ws),
+              _ptr(out), _ptr(scratch), _stream())
+        return
     _call("pm_readloss_fwd8", _ptr(s), _ptr(lab8), float(temperature), B, h, w, Hm, Wm, K, _ptr(ds_rl), _ptr(ws), _ptr(out),
           _stream())
 

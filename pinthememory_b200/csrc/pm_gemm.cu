@@ -23,6 +23,7 @@
 //     stage and a TMA store (or TMA reduce-add when the caller accumulates into an existing gradient).
 #include "pm_common.cuh"
 #include "pm_umma.cuh"
+#include "pm_internal.h"
 
 namespace pm {
 
@@ -139,7 +140,7 @@ __device__ __forceinline__ void bnbwd_tile(float4* __restrict__ dy_hi, float4* _
 //   mapY  : [B*M rows][hw] output, box [32 rows][PXC pixels]
 //   CTA tile: MT x 128 output rows (starting at 128*m_tile0) x NT pixels of one image; persistent over tiles.
 // =================================================================================================================
-template <typename T, int MT, int NT, int KB>
+template <typename T, int MT, int NT, int KB, bool ORD = false>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
     conv1x1_nn_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant__ CUtensorMap mapAh,
                       const __grid_constant__ CUtensorMap mapAl, const __grid_constant__ CUtensorMap mapY, int K, int M,
@@ -395,8 +396,13 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
             for (int mt = 0; mt < MT; ++mt) {
                 const int row = (m_tile0 + mt) * 128 + q * 32 + lane;
                 if (row < M) {
-                    atomicAdd(&stats[row], sum[mt]);
-                    atomicAdd(&stats[M + row], sq[mt]);
+                    if constexpr (ORD) {  // ordered instantiation: stats is the partial scratch, this CTA's slot is [blockIdx.x]
+                        stats[(size_t)blockIdx.x * 2 * M + row] = sum[mt];
+                        stats[(size_t)blockIdx.x * 2 * M + M + row] = sq[mt];
+                    } else {
+                        atomicAdd(&stats[row], sum[mt]);
+                        atomicAdd(&stats[M + row], sq[mt]);
+                    }
                 }
             }
         }
@@ -448,7 +454,7 @@ constexpr size_t nn_smem_bytes() {
     return (size_t)STAGES * STAGE + 4 * 2 * 4096 + 256 + 1024;
 }
 
-template <typename T, int MT, int NT, int KB>
+template <typename T, int MT, int NT, int KB, bool ORD = false>
 static int launch_nn(const void* X, const void* Ah, const void* Al, void* Y, double* stats, int B, int K, int M, int Mpad,
                      int hw, int m_tile0, int accumulate, const float* ep_scale, const float* ep_shift, int ep_relu,
                      cudaStream_t st, const void* Z = nullptr, void* DZ = nullptr, const BnBwdArgs* bnargs = nullptr) {
@@ -474,9 +480,9 @@ static int launch_nn(const void* X, const void* Ah, const void* Al, void* Y, dou
     const int tiles_per_img = (hw + NT - 1) / NT, total = B * tiles_per_img;
     const size_t smem = nn_smem_bytes<T, MT, NT, KB>();
     const int grid = total < 148 ? total : 148;
-    cudaError_t e = cudaFuncSetAttribute(conv1x1_nn_kernel<T, MT, NT, KB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(conv1x1_nn_kernel<T, MT, NT, KB, ORD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
-    conv1x1_nn_kernel<T, MT, NT, KB><<<grid, GEMM_THREADS, smem, st>>>(mX, mAh, mAl, mY, K, M, m_tile0, tiles_per_img, total,
+    conv1x1_nn_kernel<T, MT, NT, KB, ORD><<<grid, GEMM_THREADS, smem, st>>>(mX, mAh, mAl, mY, K, M, m_tile0, tiles_per_img, total,
                                                                       accumulate, stats, ep_scale, ep_shift, ep_relu, mZ, mDZ, bn);
     e = cudaGetLastError();
     return e == cudaSuccess ? 0 : (int)e;
@@ -793,6 +799,8 @@ int pm_conv1x1_prep(const float* W, int M, int K, int transpose, int dtype, void
     return 0;
 }
 
+extern "C++" {  // (a template inside the extern "C" block)
+template <bool ORD = false>
 static int conv1x1_fwd_impl(const void* X, const void* A_hi, const void* A_lo, void* Y, double* stats, int B, int K, int M, int hw,
                             int accumulate, const float* ep_scale, const float* ep_shift, int ep_relu, int dtype, void* stream,
                             const void* Z = nullptr, void* DZ = nullptr, const BnBwdArgs* bn = nullptr) {
@@ -820,23 +828,47 @@ static int conv1x1_fwd_impl(const void* X, const void* A_hi, const void* A_lo, v
             void* DZo = first ? DZ : nullptr;
             const BnBwdArgs* bi = first ? bn : nullptr;
             if (wide)
-                rc = mt == 2 ? launch_nn<float, 2, 256, 16>(Xin, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st, Zi, DZo, bi)
-                             : launch_nn<float, 1, 256, 16>(Xin, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st, Zi, DZo, bi);
+                rc = mt == 2 ? launch_nn<float, 2, 256, 16, ORD>(Xin, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st, Zi, DZo, bi)
+                             : launch_nn<float, 1, 256, 16, ORD>(Xin, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st, Zi, DZo, bi);
             else
-                rc = mt == 2 ? launch_nn<float, 2, 128, 32>(Xin, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st, Zi, DZo, bi)
-                             : launch_nn<float, 1, 128, 32>(Xin, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st, Zi, DZo, bi);
+                rc = mt == 2 ? launch_nn<float, 2, 128, 32, ORD>(Xin, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st, Zi, DZo, bi)
+                             : launch_nn<float, 1, 128, 32, ORD>(Xin, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st, Zi, DZo, bi);
         } else {
-            rc = mt == 2 ? launch_nn<__nv_bfloat16, 2, 128, 64>(X, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st)
-                         : launch_nn<__nv_bfloat16, 1, 128, 64>(X, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st);
+            rc = mt == 2 ? launch_nn<__nv_bfloat16, 2, 128, 64, ORD>(X, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st)
+                         : launch_nn<__nv_bfloat16, 1, 128, 64, ORD>(X, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st);
         }
         if (rc) return rc;
     }
     return 0;
 }
+}  // extern "C++"
 
 int pm_conv1x1_fwd(const void* X, const void* A_hi, const void* A_lo, void* Y, double* stats, int B, int K, int M, int hw,
                    int accumulate, int dtype, void* stream) {
     return conv1x1_fwd_impl(X, A_hi, A_lo, Y, stats, B, K, M, hw, accumulate, nullptr, nullptr, 0, dtype, stream);
+}
+
+// CTAs of the forward GEMM: each stores one [sum | sum of squares] partial in the ordered variant
+static int conv1x1_fwd_ctas(int B, int hw, int dtype) {
+    const bool wide = dtype == PM_F32 && (long long)B * ((hw + 255) / 256) >= 96;   // as conv1x1_fwd_impl chooses NT
+    const long long total = (long long)B * ((hw + (wide ? 255 : 127)) / (wide ? 256 : 128));
+    return (int)(total < 148 ? total : 148);
+}
+
+int pm_conv1x1_stats_scratch_bytes(int B, int M, int hw, int dtype) {
+    if (dtype != PM_F32 && dtype != PM_BF16) return PM_ERR_DTYPE;
+    if (B <= 0 || hw <= 0 || M <= 0 || M % 32 || M > 512) return PM_ERR_SHAPE;
+    return conv1x1_fwd_ctas(B, hw, dtype) * 2 * M * (int)sizeof(double);
+}
+
+int pm_conv1x1_fwd_ordered(const void* X, const void* A_hi, const void* A_lo, void* Y, double* stats, double* scratch, int B,
+                           int K, int M, int hw, int dtype, void* stream) {
+    if (!stats || !scratch) return PM_ERR_NULL;
+    if (((uintptr_t)stats | (uintptr_t)scratch) & 7) return PM_ERR_ALIGN;
+    // every CTA stores its fp64 [sum | sq] rows to `scratch` (all row tiles of one call share the grid), then one
+    // fixed-order reduction adds them into stats
+    if (int rc = conv1x1_fwd_impl<true>(X, A_hi, A_lo, Y, scratch, B, K, M, hw, 0, nullptr, nullptr, 0, dtype, stream)) return rc;
+    return pm::reduce_partials_f64(stats, scratch, conv1x1_fwd_ctas(B, hw, dtype), 2LL * M, (cudaStream_t)stream);
 }
 
 int pm_conv1x1_dgrad_bnbwd(const void* dY, const void* Z, const void* A_hi, const void* A_lo, void* dX, void* dZ,

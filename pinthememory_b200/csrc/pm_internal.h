@@ -16,8 +16,21 @@ int read_bwd_tiled(const void* du, const void* x, const float* M, const float* p
                    const float* g_loss, const float* rl_out, void* dx, const void* dx_add, float* ds, int B, int C, int hw,
                    int K, int dtype, int planes, cudaStream_t st);
 
+// part != NULL: the ordered instantiation stores each CTA's [K+1][C+4] tile to part[blockIdx.x] and sets *ncta to the
+// grid size (at most PM_ORD_CTAS) instead of adding into SD
 int write_reduce_tiled(const void* f, const void* labels, int lab_u8, float* SD, int B, int C, int h, int w, int Hm, int Wm,
-                       int K, int dtype, cudaStream_t st);
+                       int K, int dtype, cudaStream_t st, float* part = nullptr, int* ncta = nullptr);
+
+// CTA cap of the ordered class-sum kernels: bounds their partial scratch (persistent CTAs take the tiles in turn)
+constexpr int PM_ORD_CTAS = 296;
+
+// pm_ordered.cu: dst[i] += sum_g part[g*n + i] with g ascending
+int reduce_partials_f32(float* dst, const float* part, int G, long long n, cudaStream_t st);
+int reduce_partials_f64(double* dst, const double* part, int G, long long n, cudaStream_t st);
+// ds_rl and the loss of the ordered read-loss kernels from their stored tap tiles ([ncta][(TY+1)][(TX+1)][KP]) and
+// per-CTA loss partials (log2 units)
+int readloss_gather(const float* tiles, const float* lossp, int ncta, int B, int h, int w, int KP, int TY, int TX, int tiles_x,
+                    int tiles_y, int K, float temperature, float* ds_rl, unsigned long long* ws, float* out, cudaStream_t st);
 
 int write_bwd_tiled(const float* dS, const void* f, const void* labels, int lab_u8, void* df, int B, int C, int h, int w, int Hm,
                     int Wm, int K, int dtype, cudaStream_t st);

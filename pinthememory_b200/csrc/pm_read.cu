@@ -352,7 +352,7 @@ __global__ void __launch_bounds__(RD_THREADS) read_bwd_kernel(const T* __restric
 
 constexpr int DM_P = 32;
 
-template <typename T, int C, int KP>
+template <typename T, int C, int KP, bool ORD = false>
 __global__ void __launch_bounds__(C) read_bwd_dM_kernel(const T* __restrict__ du, const T* __restrict__ x,
                                                          const float* __restrict__ p_in, const float* __restrict__ ds,
                                                          float* __restrict__ dM, int hw, int K, int tiles_per_img,
@@ -416,9 +416,16 @@ __global__ void __launch_bounds__(C) read_bwd_dM_kernel(const T* __restrict__ du
         }
         __syncthreads();
     }
+    if constexpr (ORD) {  // ordered instantiation: dM is the partial scratch, this CTA's [K][C] slot is [blockIdx.x]
+        float* dst = dM + (size_t)blockIdx.x * K * C;
 #pragma unroll
-    for (int k = 0; k < KP; ++k)
-        if (k < K) atomicAdd(dM + (size_t)k * C + tid, acc[k]);
+        for (int k = 0; k < KP; ++k)
+            if (k < K) dst[(size_t)k * C + tid] = acc[k];
+    } else {
+#pragma unroll
+        for (int k = 0; k < KP; ++k)
+            if (k < K) atomicAdd(dM + (size_t)k * C + tid, acc[k]);
+    }
 }
 
 // ----------------------------------------------------------------------- get_score on an NHWC query
@@ -487,14 +494,15 @@ int launch_read_bwd(const void* du, const void* x, const float* M, const float* 
 
 template <typename T, int C, int KP>
 int launch_read_bwd_dM(const void* du, const void* x, const float* p, const float* ds, float* dM, int B, int hw,
-                       int K, cudaStream_t st) {
+                       int K, cudaStream_t st, float* part = nullptr, int* ncta = nullptr) {
     constexpr int LD = DM_P + 1;
     const size_t smem = sizeof(float) * ((size_t)2 * C * LD + 2 * DM_P * KP + (C / 32) * DM_P + DM_P);
-    auto kern = read_bwd_dM_kernel<T, C, KP>;
+    auto kern = part ? read_bwd_dM_kernel<T, C, KP, true> : read_bwd_dM_kernel<T, C, KP>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
     const int tiles = (hw + DM_P - 1) / DM_P, ntiles = B * tiles;
     const int grid = ntiles < 148 ? ntiles : 148;
+    if (part) dM = part, *ncta = grid;
     kern<<<grid, C, smem, st>>>((const T*)du, (const T*)x, p, ds, dM, hw, K, tiles, ntiles);
     PM_CHECK_LAUNCH();
     return 0;
@@ -600,6 +608,29 @@ extern "C" int pm_read_bwd_dM(const void* du, const void* x, const float* score_
     if (!x || !score_m || !ds || !dM) return PM_ERR_NULL;  // du NULL: only the ds (x) q term (planes mode)
     if (int e = check_common(B, C, h, w, K, dtype)) return e;
     PM_DISPATCH(PM_DISPATCH_C, launch_read_bwd_dM, du, x, score_m, ds, dM, B, h * w, K, (cudaStream_t)stream);
+}
+
+extern "C" int pm_read_bwd_dM_scratch_bytes(int B, int C, int h, int w, int K) {
+    if (C != 32 && C != 64 && C != 128 && C != 256) return PM_ERR_CHANNELS;
+    if (K < 1 || K > 31) return PM_ERR_SLOTS;
+    if (B <= 0 || h <= 0 || w <= 0 || (long long)B * h * w > 0x7fffffffLL / 64) return PM_ERR_SHAPE;
+    const long long ntiles = (long long)B * ((h * w + pm::DM_P - 1) / pm::DM_P);
+    return (int)((ntiles < 148 ? ntiles : 148) * K * C * (long long)sizeof(float));
+}
+
+extern "C" int pm_read_bwd_dM_ordered(const void* du, const void* x, const float* score_m, const float* ds, float* dM,
+                                      float* scratch, int B, int C, int h, int w, int K, int dtype, void* stream) {
+    if (!x || !score_m || !ds || !dM || !scratch) return PM_ERR_NULL;
+    if (int e = check_common(B, C, h, w, K, dtype)) return e;
+    if ((uintptr_t)scratch & 15) return PM_ERR_ALIGN;
+    int ncta = 0;
+    // every CTA stores its [K][C] partial to `scratch`, then one fixed-order reduction adds them into dM
+    const int rc = [&]() -> int {
+        PM_DISPATCH(PM_DISPATCH_C, launch_read_bwd_dM, du, x, score_m, ds, dM, B, h * w, K, (cudaStream_t)stream, scratch,
+                    &ncta);
+    }();
+    if (rc) return rc;
+    return pm::reduce_partials_f32(dM, scratch, ncta, (long long)K * C, (cudaStream_t)stream);
 }
 
 extern "C" int pm_score_nhwc(const float* q, const float* M, float* s, int N, int C, int K, void* stream) {

@@ -21,6 +21,7 @@
 // large enough for that to underflow (> 60 in log2 units: tiny T or un-normalised queries) additionally
 // take the per-pixel max.
 #include "pm_common.cuh"
+#include "pm_internal.h"
 
 namespace pm {
 
@@ -61,7 +62,9 @@ __device__ __forceinline__ int first_ge(int c, float scale, int n_out, int n_in)
     return y;
 }
 
-template <int KP, int RL_TX>
+// ORD = true (ordered instantiation): ds_rl is the tile scratch and `out` the per-CTA loss partials; each CTA stores its
+// whole tap tile and its loss to slot [blockIdx.x] instead of adding them with atomics (readloss_gather combines them)
+template <int KP, int RL_TX, bool ORD = false>
 __global__ void __launch_bounds__(RL_THREADS, 2)
     readloss_kernel(const float* __restrict__ s, const long long* __restrict__ labels, float inv_T, float temperature,
                     int h, int w, int Hm, int Wm, int K, float sy, float sx, int RS, int TYC, int tiles_x, int tiles_y,
@@ -324,15 +327,20 @@ __global__ void __launch_bounds__(RL_THREADS, 2)
             __syncthreads();
         }
     }
-    // flush taps that exist (clamped duplicates were folded and stay zero)
-    for (int i = tid; i < tile_elems / 4; i += NT) {
-        int e = i / (KP / 4), q = i - e * (KP / 4);
-        int ty = e / RL_LDX, tx = e - ty * RL_LDX;
-        int fy = fy0 + ty, fx = fx0 + tx;
-        if (fy < h && fx < w) {
-            float4 v = reinterpret_cast<const float4*>(ds_tile)[i];
-            if (v.x != 0.f || v.y != 0.f || v.z != 0.f || v.w != 0.f)
-                atomicAdd(reinterpret_cast<float4*>(ds_rl + ((size_t)(b * h + fy) * w + fx) * KP) + q, v);
+    if constexpr (ORD) {
+        float4* dst = reinterpret_cast<float4*>(ds_rl + (size_t)blockIdx.x * tile_elems);
+        for (int i = tid; i < tile_elems / 4; i += NT) dst[i] = reinterpret_cast<const float4*>(ds_tile)[i];
+    } else {
+        // flush taps that exist (clamped duplicates were folded and stay zero)
+        for (int i = tid; i < tile_elems / 4; i += NT) {
+            int e = i / (KP / 4), q = i - e * (KP / 4);
+            int ty = e / RL_LDX, tx = e - ty * RL_LDX;
+            int fy = fy0 + ty, fx = fx0 + tx;
+            if (fy < h && fx < w) {
+                float4 v = reinterpret_cast<const float4*>(ds_tile)[i];
+                if (v.x != 0.f || v.y != 0.f || v.z != 0.f || v.w != 0.f)
+                    atomicAdd(reinterpret_cast<float4*>(ds_rl + ((size_t)(b * h + fy) * w + fx) * KP) + q, v);
+            }
         }
     }
     // label histogram + loss sum
@@ -346,9 +354,11 @@ __global__ void __launch_bounds__(RL_THREADS, 2)
     if (tid == 0) {
         float tot = 0.f;
         for (int i = 0; i < NT / 32; ++i) tot += red[i];
-        atomicAdd(reinterpret_cast<double*>(ws + PM_WS_LOSS_SUM), (double)tot * 0.6931471805599453);
+        if constexpr (ORD) out[blockIdx.x] = tot;
+        else atomicAdd(reinterpret_cast<double*>(ws + PM_WS_LOSS_SUM), (double)tot * 0.6931471805599453);
     }
     if (tid <= K && hist_sm[tid] != 0) atomicAdd(ws + PM_WS_HIST + tid, (unsigned long long)hist_sm[tid]);
+    if constexpr (ORD) return;
     // last CTA: readloss = loss_sum / V ; scale = 1 / (V*T)
     __threadfence();
     __syncthreads();
@@ -365,24 +375,34 @@ __global__ void __launch_bounds__(RL_THREADS, 2)
     }
 }
 
-template <int KP, int RL_TX>
-static int launch_readloss_tx(const float* s, const long long* labels, float temperature, int B, int h, int w, int Hm,
-                           int Wm, int K, float* ds_rl, unsigned long long* ws, float* out, cudaStream_t st) {
-    // PyTorch's align_corners scale: (in-1)/(out-1) in fp32, 0 when out == 1
-    const float sy = Hm > 1 ? (float)(h - 1) / (float)(Hm - 1) : 0.f;
-    const float sx = Wm > 1 ? (float)(w - 1) / (float)(Wm - 1) : 0.f;
+// row-split factor and tiling of the first kernel (shared by the launch and the ordered variant's scratch size)
+static void rl_tiling(int B, int h, int w, int Hm, int RL_TX, int* RS_out, int* TYC_out, int* tiles_x, int* tiles_y) {
     // row-split factor: enough threads to fill the chip when there are few cells
     const long long cells = (long long)B * h * w;
     const int rows_per_cell = h > 1 ? (Hm + h - 2) / (h - 1) : Hm;
     int RS = 1;
     while (RS < 4 && cells * RS * 2 < 148LL * 512 && RS * 2 <= rows_per_cell) RS *= 2;
     const int TYC = (RL_THREADS / 2 / RL_TX) / RS;
-    const int tiles_x = (w + RL_TX - 1) / RL_TX, tiles_y = (h + TYC - 1) / TYC;
+    *RS_out = RS, *TYC_out = TYC;
+    *tiles_x = (w + RL_TX - 1) / RL_TX, *tiles_y = (h + TYC - 1) / TYC;
+}
+
+// cells per CTA along x (see RL_THREADS)
+static int rl_tx(int w) { return (w + 31) / 32 * 32 - w >= 16 ? 16 : 32; }
+
+template <int KP, int RL_TX, bool ORD>
+static int launch_readloss_tx(const float* s, const long long* labels, float temperature, int B, int h, int w, int Hm,
+                           int Wm, int K, float* ds_rl, unsigned long long* ws, float* out, cudaStream_t st) {
+    // PyTorch's align_corners scale: (in-1)/(out-1) in fp32, 0 when out == 1
+    const float sy = Hm > 1 ? (float)(h - 1) / (float)(Hm - 1) : 0.f;
+    const float sx = Wm > 1 ? (float)(w - 1) / (float)(Wm - 1) : 0.f;
+    int RS, TYC, tiles_x, tiles_y;
+    rl_tiling(B, h, w, Hm, RL_TX, &RS, &TYC, &tiles_x, &tiles_y);
     const size_t smem = sizeof(float) * ((size_t)2 * (TYC + 1) * (RL_TX + 1) * KP + (size_t)4 * (KP / 2) * RL_THREADS +
                                          (size_t)KP * (RL_THREADS / 2) + KP + 8);
     const long long grid = (long long)B * tiles_x * tiles_y;
     if (grid > 0x7fffffffLL) return PM_ERR_SHAPE;
-    auto kern = readloss_kernel<KP, RL_TX>;
+    auto kern = readloss_kernel<KP, RL_TX, ORD>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
     kern<<<(int)grid, RL_THREADS, smem, st>>>(s, labels, 1.f / temperature, temperature, h, w, Hm, Wm, K, sy, sx, RS,
@@ -391,12 +411,27 @@ static int launch_readloss_tx(const float* s, const long long* labels, float tem
     return e == cudaSuccess ? 0 : (int)e;
 }
 
-template <int KP>
+template <int KP, bool ORD = false>
 static int launch_readloss(const float* s, const long long* labels, float temperature, int B, int h, int w, int Hm,
                            int Wm, int K, float* ds_rl, unsigned long long* ws, float* out, cudaStream_t st) {
-    const int pad32 = (w + 31) / 32 * 32 - w;
-    if (pad32 >= 16) return launch_readloss_tx<KP, 16>(s, labels, temperature, B, h, w, Hm, Wm, K, ds_rl, ws, out, st);
-    return launch_readloss_tx<KP, 32>(s, labels, temperature, B, h, w, Hm, Wm, K, ds_rl, ws, out, st);
+    if (rl_tx(w) == 16) return launch_readloss_tx<KP, 16, ORD>(s, labels, temperature, B, h, w, Hm, Wm, K, ds_rl, ws, out, st);
+    return launch_readloss_tx<KP, 32, ORD>(s, labels, temperature, B, h, w, Hm, Wm, K, ds_rl, ws, out, st);
+}
+
+long long readloss8_scratch_bytes(int B, int h, int w, int Hm, int Wm);   // pm_readloss8.cu
+
+struct RlGeometry {
+    int TX, TYC, tiles_x, tiles_y;
+    long long grid, tile_elems;
+};
+static RlGeometry rl_geometry(int B, int h, int w, int Hm, int KP) {
+    RlGeometry g;
+    int RS;
+    g.TX = rl_tx(w);
+    rl_tiling(B, h, w, Hm, g.TX, &RS, &g.TYC, &g.tiles_x, &g.tiles_y);
+    g.grid = (long long)B * g.tiles_x * g.tiles_y;
+    g.tile_elems = (long long)(g.TYC + 1) * (g.TX + 1) * KP;
+    return g;
 }
 
 }  // namespace pm
@@ -412,4 +447,37 @@ extern "C" int pm_readloss_fwd(const float* s, const int64_t* labels, float temp
     unsigned long long* w64 = (unsigned long long*)ws;
     if (K <= 19) return pm::launch_readloss<20>(s, lab, temperature, B, h, w, Hm, Wm, K, ds_rl, w64, out, st);
     return pm::launch_readloss<32>(s, lab, temperature, B, h, w, Hm, Wm, K, ds_rl, w64, out, st);
+}
+
+extern "C" int pm_readloss_scratch_bytes(int B, int h, int w, int Hm, int Wm, int K, int packed) {
+    if (K < 1 || K > (packed ? 19 : 31)) return PM_ERR_SLOTS;
+    if (B <= 0 || h <= 0 || w <= 0 || Hm <= 0 || Wm <= 0) return PM_ERR_SHAPE;
+    long long bytes;
+    if (packed) {
+        bytes = pm::readloss8_scratch_bytes(B, h, w, Hm, Wm);
+    } else {
+        const pm::RlGeometry g = pm::rl_geometry(B, h, w, Hm, K <= 19 ? 20 : 32);
+        bytes = (g.grid * g.tile_elems + (g.grid + 3) / 4 * 4) * (long long)sizeof(float);
+    }
+    return bytes > 0x7fffffffLL ? PM_ERR_SHAPE : (int)bytes;
+}
+
+extern "C" int pm_readloss_fwd_ordered(const float* s, const int64_t* labels, float temperature, int B, int h, int w, int Hm,
+                                       int Wm, int K, float* ds_rl, void* ws, float* out, float* scratch, void* stream) {
+    if (!s || !labels || !ds_rl || !ws || !out || !scratch) return PM_ERR_NULL;
+    if (K < 1 || K > 31) return PM_ERR_SLOTS;
+    if (B <= 0 || h <= 0 || w <= 0 || Hm <= 0 || Wm <= 0 || !(temperature > 0.f)) return PM_ERR_SHAPE;
+    if (((uintptr_t)s & 15) || ((uintptr_t)ds_rl & 15) || ((uintptr_t)ws & 7) || ((uintptr_t)scratch & 15)) return PM_ERR_ALIGN;
+    const cudaStream_t st = (cudaStream_t)stream;
+    const long long* lab = (const long long*)labels;
+    unsigned long long* w64 = (unsigned long long*)ws;
+    const int KP = K <= 19 ? 20 : 32;
+    const pm::RlGeometry g = pm::rl_geometry(B, h, w, Hm, KP);
+    if (g.grid > 0x7fffffffLL) return PM_ERR_SHAPE;
+    float* lossp = scratch + (size_t)g.grid * g.tile_elems;
+    const int rc = KP == 20 ? pm::launch_readloss<20, true>(s, lab, temperature, B, h, w, Hm, Wm, K, scratch, w64, lossp, st)
+                            : pm::launch_readloss<32, true>(s, lab, temperature, B, h, w, Hm, Wm, K, scratch, w64, lossp, st);
+    if (rc) return rc;
+    return pm::readloss_gather(scratch, lossp, (int)g.grid, B, h, w, KP, g.TYC, g.TX, g.tiles_x, g.tiles_y, K, temperature,
+                               ds_rl, w64, out, st);
 }

@@ -22,6 +22,7 @@
 // loss and ds_rl stay below 3e-6 (tests/test_gpu_parity.py). The weights lambda_x / lambda_y themselves are computed
 // exactly as PyTorch does (fp32 `scale * dst`, floor, clamp).
 #include "pm_common.cuh"
+#include "pm_internal.h"
 
 namespace pm {
 
@@ -202,6 +203,9 @@ __device__ __forceinline__ void cell_rows(const CellCtx& c, RunState& rs, float*
     }
 }
 
+// ORD = true (ordered instantiation): ds_rl is the tile scratch and `out` the per-CTA loss partials; each CTA stores its
+// whole tap tile and its loss to slot [blockIdx.x] instead of adding them with atomics (readloss_gather combines them)
+template <bool ORD = false>
 __global__ void __launch_bounds__(RL8_THREADS, 2)
     readloss8_kernel(const float* __restrict__ s, const unsigned char* __restrict__ lab8, float inv_T, float temperature, int h,
                      int w, int Hm, int Wm, int K, float sy, float sx, int RS, int TYC, int tiles_x, int tiles_y,
@@ -358,15 +362,20 @@ __global__ void __launch_bounds__(RL8_THREADS, 2)
             __syncthreads();
         }
     }
-    // flush taps that exist (clamped duplicates were folded and stay zero)
-    for (int i = tid; i < tile_elems / 4; i += NT) {
-        const int e = i / (KP / 4), q = i - e * (KP / 4);
-        const int ty = e / LDX, tx = e - ty * LDX;
-        const int fy = fy0 + ty, fx = fx0 + tx;
-        if (fy < h && fx < w) {
-            const float4 v = reinterpret_cast<const float4*>(ds_tile)[i];
-            if (v.x != 0.f || v.y != 0.f || v.z != 0.f || v.w != 0.f)
-                atomicAdd(reinterpret_cast<float4*>(ds_rl + ((size_t)(b * h + fy) * w + fx) * KP) + q, v);
+    if constexpr (ORD) {
+        float4* dst = reinterpret_cast<float4*>(ds_rl + (size_t)blockIdx.x * tile_elems);
+        for (int i = tid; i < tile_elems / 4; i += NT) dst[i] = reinterpret_cast<const float4*>(ds_tile)[i];
+    } else {
+        // flush taps that exist (clamped duplicates were folded and stay zero)
+        for (int i = tid; i < tile_elems / 4; i += NT) {
+            const int e = i / (KP / 4), q = i - e * (KP / 4);
+            const int ty = e / LDX, tx = e - ty * LDX;
+            const int fy = fy0 + ty, fx = fx0 + tx;
+            if (fy < h && fx < w) {
+                const float4 v = reinterpret_cast<const float4*>(ds_tile)[i];
+                if (v.x != 0.f || v.y != 0.f || v.z != 0.f || v.w != 0.f)
+                    atomicAdd(reinterpret_cast<float4*>(ds_rl + ((size_t)(b * h + fy) * w + fx) * KP) + q, v);
+            }
         }
     }
     lossacc = warp_sum(lossacc);
@@ -375,8 +384,10 @@ __global__ void __launch_bounds__(RL8_THREADS, 2)
     if (tid == 0) {
         float tot = 0.f;
         for (int i = 0; i < NT / 32; ++i) tot += red[i];
-        atomicAdd(reinterpret_cast<double*>(ws + PM_WS_LOSS_SUM), (double)tot * 0.6931471805599453);
+        if constexpr (ORD) out[blockIdx.x] = tot;
+        else atomicAdd(reinterpret_cast<double*>(ws + PM_WS_LOSS_SUM), (double)tot * 0.6931471805599453);
     }
+    if constexpr (ORD) return;
     // last CTA: readloss = loss_sum / V ; scale = 1 / (V*T)   (V from the histogram pm_labels_pack left in ws)
     __threadfence();
     __syncthreads();
@@ -391,6 +402,48 @@ __global__ void __launch_bounds__(RL8_THREADS, 2)
             out[1] = (float)(1.0 / ((double)V * (double)temperature));
         }
     }
+}
+
+struct Rl8Geometry {
+    float sy, sx;
+    int RS, TYC, tiles_x, tiles_y;
+    long long grid, tile_elems;  // CTAs; floats of one CTA's (TYC+1) x (RL8_TX+1) x RL8_KP tap tile
+};
+
+static Rl8Geometry rl8_geometry(int B, int h, int w, int Hm, int Wm) {
+    Rl8Geometry g;
+    // PyTorch's align_corners scale: (in-1)/(out-1) in fp32, 0 when out == 1
+    g.sy = Hm > 1 ? (float)(h - 1) / (float)(Hm - 1) : 0.f;
+    g.sx = Wm > 1 ? (float)(w - 1) / (float)(Wm - 1) : 0.f;
+    // row-split factor: enough CTAs to fill the chip when there are few cells (output stride 16, small batches)
+    const long long cells = (long long)B * h * w;
+    const int rows_per_cell = h > 1 ? (Hm + h - 2) / (h - 1) : Hm;
+    g.RS = 1;
+    while (g.RS < 4 && cells * g.RS < 4LL * 148 * RL8_THREADS && g.RS * 2 <= rows_per_cell) g.RS *= 2;
+    g.TYC = (RL8_THREADS / RL8_TX) / g.RS;
+    g.tiles_x = (w + RL8_TX - 1) / RL8_TX, g.tiles_y = (h + g.TYC - 1) / g.TYC;
+    g.grid = (long long)B * g.tiles_x * g.tiles_y;
+    g.tile_elems = (long long)(g.TYC + 1) * (RL8_TX + 1) * RL8_KP;
+    return g;
+}
+
+template <bool ORD>
+static int launch_readloss8(const float* s, const uint8_t* lab8, float temperature, int B, int h, int w, int Hm, int Wm, int K,
+                            float* ds_rl, unsigned long long* ws, float* out, cudaStream_t st) {
+    const Rl8Geometry g = rl8_geometry(B, h, w, Hm, Wm);
+    const size_t smem = sizeof(float) * ((size_t)2 * g.tile_elems + (size_t)4 * RL8_KP * RL8_THREADS + 8);
+    if (g.grid > 0x7fffffffLL) return PM_ERR_SHAPE;
+    cudaError_t e = cudaFuncSetAttribute(readloss8_kernel<ORD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return (int)e;
+    readloss8_kernel<ORD><<<(int)g.grid, RL8_THREADS, smem, st>>>(s, lab8, 1.f / temperature, temperature, h, w, Hm, Wm, K, g.sy,
+                                                                  g.sx, g.RS, g.TYC, g.tiles_x, g.tiles_y, ds_rl, ws, out);
+    e = cudaGetLastError();
+    return e == cudaSuccess ? 0 : (int)e;
+}
+
+long long readloss8_scratch_bytes(int B, int h, int w, int Hm, int Wm) {
+    const Rl8Geometry g = rl8_geometry(B, h, w, Hm, Wm);
+    return (g.grid * g.tile_elems + (g.grid + 3) / 4 * 4) * (long long)sizeof(float);
 }
 
 }  // namespace pm
@@ -410,25 +463,24 @@ extern "C" int pm_readloss_fwd8(const float* s, const uint8_t* lab8, float tempe
         const int rc = pm_readloss_cells_launch(s, lab8, temperature, B, h, w, Hm, Wm, K, ds_rl, ws, out, (cudaStream_t)stream);
         if (rc >= 0) return rc;
     }
+    return pm::launch_readloss8<false>(s, lab8, temperature, B, h, w, Hm, Wm, K, ds_rl, (unsigned long long*)ws, out,
+                                       (cudaStream_t)stream);
+}
+
+extern "C" int pm_readloss_fwd8_ordered(const float* s, const uint8_t* lab8, float temperature, int B, int h, int w, int Hm,
+                                        int Wm, int K, float* ds_rl, void* ws, float* out, float* scratch, void* stream) {
+    if (!s || !lab8 || !ds_rl || !ws || !out || !scratch) return PM_ERR_NULL;
+    if (K < 1 || K > 19) return PM_ERR_SLOTS;
+    if (B <= 0 || h <= 0 || w <= 0 || Hm <= 0 || Wm <= 0 || !(temperature > 0.f)) return PM_ERR_SHAPE;
+    if (((uintptr_t)s & 15) || ((uintptr_t)ds_rl & 15) || ((uintptr_t)ws & 7) || ((uintptr_t)scratch & 15)) return PM_ERR_ALIGN;
+    // readloss8_kernel takes every shape; the cells kernel is never used here (its warps scatter with REDs)
     using namespace pm;
-    // PyTorch's align_corners scale: (in-1)/(out-1) in fp32, 0 when out == 1
-    const float sy = Hm > 1 ? (float)(h - 1) / (float)(Hm - 1) : 0.f;
-    const float sx = Wm > 1 ? (float)(w - 1) / (float)(Wm - 1) : 0.f;
-    // row-split factor: enough CTAs to fill the chip when there are few cells (output stride 16, small batches)
-    const long long cells = (long long)B * h * w;
-    const int rows_per_cell = h > 1 ? (Hm + h - 2) / (h - 1) : Hm;
-    int RS = 1;
-    while (RS < 4 && cells * RS < 4LL * 148 * RL8_THREADS && RS * 2 <= rows_per_cell) RS *= 2;
-    const int TYC = (RL8_THREADS / RL8_TX) / RS;
-    const int tiles_x = (w + RL8_TX - 1) / RL8_TX, tiles_y = (h + TYC - 1) / TYC;
-    const size_t smem = sizeof(float) * ((size_t)2 * (TYC + 1) * (RL8_TX + 1) * RL8_KP + (size_t)4 * RL8_KP * RL8_THREADS + 8);
-    const long long grid = (long long)B * tiles_x * tiles_y;
-    if (grid > 0x7fffffffLL) return PM_ERR_SHAPE;
-    cudaError_t e = cudaFuncSetAttribute(readloss8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return (int)e;
-    readloss8_kernel<<<(int)grid, RL8_THREADS, smem, (cudaStream_t)stream>>>(s, lab8, 1.f / temperature, temperature, h, w, Hm, Wm,
-                                                                             K, sy, sx, RS, TYC, tiles_x, tiles_y, ds_rl,
-                                                                             (unsigned long long*)ws, out);
-    e = cudaGetLastError();
-    return e == cudaSuccess ? 0 : (int)e;
+    const Rl8Geometry g = rl8_geometry(B, h, w, Hm, Wm);
+    if (g.grid > 0x7fffffffLL) return PM_ERR_SHAPE;
+    float* lossp = scratch + (size_t)g.grid * g.tile_elems;
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (int rc = launch_readloss8<true>(s, lab8, temperature, B, h, w, Hm, Wm, K, scratch, (unsigned long long*)ws, lossp, st))
+        return rc;
+    return readloss_gather(scratch, lossp, (int)g.grid, B, h, w, RL8_KP, g.TYC, RL8_TX, g.tiles_x, g.tiles_y, K, temperature,
+                           ds_rl, (unsigned long long*)ws, out, st);
 }

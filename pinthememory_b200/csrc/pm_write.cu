@@ -16,7 +16,7 @@ namespace pm {
 
 constexpr int WR_P = 32;
 
-template <typename T, int C, int KP>
+template <typename T, int C, int KP, bool ORD = false>
 __global__ void __launch_bounds__(C) write_reduce_kernel(const T* __restrict__ f, const void* __restrict__ labels, int lab_u8,
                                                           float* __restrict__ SD, int h, int w, int Hm, int Wm, int K,
                                                           float sy, float sx, int tiles_per_img, int ntiles) {
@@ -96,11 +96,16 @@ __global__ void __launch_bounds__(C) write_reduce_kernel(const T* __restrict__ f
         if (tid == 0) S_tile[cur * CS + C] += accD;
     }
     __syncthreads();
-    for (int k = 0; k <= K; ++k) {
-        if (!((seen >> k) & 1u)) continue;
-        for (int i = tid; i < CS / 4; i += C)
-            atomicAdd(reinterpret_cast<float4*>(SD + (size_t)k * CS) + i,
-                      reinterpret_cast<const float4*>(S_tile + k * CS)[i]);
+    if constexpr (ORD) {  // ordered instantiation: SD is the partial scratch, this CTA's slot is [blockIdx.x]
+        float4* dst = reinterpret_cast<float4*>(SD + (size_t)blockIdx.x * (K + 1) * CS);
+        for (int i = tid; i < (K + 1) * CS / 4; i += C) dst[i] = reinterpret_cast<const float4*>(S_tile)[i];
+    } else {
+        for (int k = 0; k <= K; ++k) {
+            if (!((seen >> k) & 1u)) continue;
+            for (int i = tid; i < CS / 4; i += C)
+                atomicAdd(reinterpret_cast<float4*>(SD + (size_t)k * CS) + i,
+                          reinterpret_cast<const float4*>(S_tile + k * CS)[i]);
+        }
     }
 }
 
@@ -544,15 +549,16 @@ __global__ void __launch_bounds__(UP_THREADS) update_bwd_kernel(const float* __r
 
 template <typename T, int C, int KP>
 int launch_write_reduce(const void* f, const void* labels, int lab_u8, float* SD, int B, int h, int w, int Hm, int Wm, int K,
-                        cudaStream_t st) {
+                        cudaStream_t st, float* part, int* ncta) {
     constexpr int LD = WR_P + 1, CS = C + 4;
     const size_t smem = sizeof(float) * ((size_t)KP * CS + (size_t)C * LD + (C / 32) * WR_P + WR_P + 8 * WR_P);
-    auto kern = write_reduce_kernel<T, C, KP>;
+    auto kern = part ? write_reduce_kernel<T, C, KP, true> : write_reduce_kernel<T, C, KP>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
     const int hw = h * w, tiles = (hw + WR_P - 1) / WR_P, ntiles = B * tiles;
     int grid = 148 * 2;
     if (grid > ntiles) grid = ntiles;
+    if (part) SD = part, *ncta = grid;  // (grid <= PM_ORD_CTAS already)
     // down-sampling the label map to the feature grid: scale = (Hm-1)/(h-1)  (in = labels, out = features)
     const float sy = h > 1 ? (float)(Hm - 1) / (float)(h - 1) : 0.f;
     const float sx = w > 1 ? (float)(Wm - 1) / (float)(w - 1) : 0.f;
@@ -618,13 +624,24 @@ static int check_write(int B, int C, int h, int w, int Hm, int Wm, int K, int dt
 }
 
 static int write_reduce_any(const void* f, const void* labels, int lab_u8, float* SD, int B, int C, int h, int w, int Hm,
-                            int Wm, int K, int dtype, void* stream) {
+                            int Wm, int K, int dtype, void* stream, float* part = nullptr, int* ncta = nullptr) {
     if (!f || !labels || !SD) return PM_ERR_NULL;
     if (int e = check_write(B, C, h, w, Hm, Wm, K, dtype)) return e;
     if ((uintptr_t)SD & 15) return PM_ERR_ALIGN;
     if (pm::tiled_ok(f, nullptr, nullptr, h * w, dtype))
-        return pm::write_reduce_tiled(f, labels, lab_u8, SD, B, C, h, w, Hm, Wm, K, dtype, (cudaStream_t)stream);
-    PMW_DISPATCH(PMW_DISPATCH_C, launch_write_reduce, f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, (cudaStream_t)stream);
+        return pm::write_reduce_tiled(f, labels, lab_u8, SD, B, C, h, w, Hm, Wm, K, dtype, (cudaStream_t)stream, part, ncta);
+    PMW_DISPATCH(PMW_DISPATCH_C, launch_write_reduce, f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, (cudaStream_t)stream, part,
+                 ncta);
+}
+
+// ordered: every CTA stores its [K+1][C+4] tile to `scratch`, then one fixed-order reduction adds them into SD
+static int write_reduce_ordered(const void* f, const void* labels, int lab_u8, float* SD, float* scratch, int B, int C, int h,
+                                int w, int Hm, int Wm, int K, int dtype, void* stream) {
+    if (!scratch) return PM_ERR_NULL;
+    if ((uintptr_t)scratch & 15) return PM_ERR_ALIGN;
+    int ncta = 0;
+    if (int rc = write_reduce_any(f, labels, lab_u8, SD, B, C, h, w, Hm, Wm, K, dtype, stream, scratch, &ncta)) return rc;
+    return pm::reduce_partials_f32(SD, scratch, ncta, (long long)(K + 1) * (C + 4), (cudaStream_t)stream);
 }
 
 static int write_bwd_any(const float* dS, const void* f, const void* labels, int lab_u8, void* df, int B, int C, int h, int w,
@@ -643,6 +660,22 @@ extern "C" int pm_write_reduce_fwd(const void* f, const int64_t* labels, float* 
 extern "C" int pm_write_reduce_fwd8(const void* f, const uint8_t* lab8, float* SD, int B, int C, int h, int w, int Hm,
                                     int Wm, int K, int dtype, void* stream) {
     return write_reduce_any(f, lab8, 1, SD, B, C, h, w, Hm, Wm, K, dtype, stream);
+}
+extern "C" int pm_write_reduce_scratch_bytes(int B, int C, int h, int w, int K) {
+    if (C != 32 && C != 64 && C != 128 && C != 256) return PM_ERR_CHANNELS;
+    if (K < 1 || K > 31) return PM_ERR_SLOTS;
+    if (B <= 0 || h <= 0 || w <= 0 || (long long)B * h * w > 0x7fffffffLL / 64) return PM_ERR_SHAPE;
+    const long long ntiles = (long long)B * ((h * w + 31) / 32);   // 32-pixel tiles in every variant
+    const long long ncta = ntiles < pm::PM_ORD_CTAS ? ntiles : pm::PM_ORD_CTAS;
+    return (int)(ncta * (K + 1) * (C + 4) * (long long)sizeof(float));
+}
+extern "C" int pm_write_reduce_fwd_ordered(const void* f, const int64_t* labels, float* SD, float* scratch, int B, int C, int h,
+                                           int w, int Hm, int Wm, int K, int dtype, void* stream) {
+    return write_reduce_ordered(f, labels, 0, SD, scratch, B, C, h, w, Hm, Wm, K, dtype, stream);
+}
+extern "C" int pm_write_reduce_fwd8_ordered(const void* f, const uint8_t* lab8, float* SD, float* scratch, int B, int C, int h,
+                                            int w, int Hm, int Wm, int K, int dtype, void* stream) {
+    return write_reduce_ordered(f, lab8, 1, SD, scratch, B, C, h, w, Hm, Wm, K, dtype, stream);
 }
 extern "C" int pm_write_bwd(const float* dS, const void* f, const int64_t* labels, void* df, int B, int C, int h, int w,
                             int Hm, int Wm, int K, int dtype, void* stream) {

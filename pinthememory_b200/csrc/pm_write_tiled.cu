@@ -13,7 +13,7 @@ namespace pm {
 // XOR-swizzled chunks, so a thread reads 4 (fp32) / 8 (bf16) pixels of its channel per conflict-free
 // LDS.128; the label taps of the NEXT tile are fetched while the current one is reduced.
 
-template <typename T, int C, int KP>
+template <typename T, int C, int KP, bool ORD = false>
 __global__ void __launch_bounds__(C) write_reduce_tiled_kernel(const T* __restrict__ f, const void* __restrict__ labels, int lab_u8,
                                                                 float* __restrict__ SD, int h, int w, int Hm, int Wm,
                                                                 int K, float sy, float sx, int tiles_per_img,
@@ -189,11 +189,16 @@ __global__ void __launch_bounds__(C) write_reduce_tiled_kernel(const T* __restri
         if (tid == 0) S_tile[cur * CS + C] += accD;
     }
     __syncthreads();
-    for (int k = 0; k <= K; ++k) {
-        if (!((seen >> k) & 1u)) continue;
-        for (int i = tid; i < CS / 4; i += C)
-            atomicAdd(reinterpret_cast<float4*>(SD + (size_t)k * CS) + i,
-                      reinterpret_cast<const float4*>(S_tile + k * CS)[i]);
+    if constexpr (ORD) {  // ordered instantiation: SD is the partial scratch, this CTA's slot is [blockIdx.x]
+        float4* dst = reinterpret_cast<float4*>(SD + (size_t)blockIdx.x * (K + 1) * CS);
+        for (int i = tid; i < (K + 1) * CS / 4; i += C) dst[i] = reinterpret_cast<const float4*>(S_tile)[i];
+    } else {
+        for (int k = 0; k <= K; ++k) {
+            if (!((seen >> k) & 1u)) continue;
+            for (int i = tid; i < CS / 4; i += C)
+                atomicAdd(reinterpret_cast<float4*>(SD + (size_t)k * CS) + i,
+                          reinterpret_cast<const float4*>(S_tile + k * CS)[i]);
+        }
     }
 }
 
@@ -207,7 +212,7 @@ __global__ void __launch_bounds__(C) write_reduce_tiled_kernel(const T* __restri
 // fragmented the label map is (the run-length kernel above degenerates on noisy labels).
 
 // TMA = true: the tiles arrive as SWIZZLE_128B tensor-map boxes (the same chunk ^ (row & 7) layout) on an mbarrier ring
-template <int C, int KP, bool TMA>
+template <int C, int KP, bool TMA, bool ORD = false>
 __global__ void __launch_bounds__(C) write_reduce_mma_kernel(const __grid_constant__ CUtensorMap tm_f,
                                                               const float* __restrict__ f, const void* __restrict__ labels, int lab_u8,
                                                               float* __restrict__ SD, int h, int w, int Hm, int Wm,
@@ -403,11 +408,16 @@ __global__ void __launch_bounds__(C) write_reduce_mma_kernel(const __grid_consta
         S_tile[lane * CS + C + 1] = S_tile[lane * CS + C + 2] = S_tile[lane * CS + C + 3] = 0.f;
     }
     __syncthreads();
-    for (int k = 0; k <= K; ++k) {
-        if (!((seen >> k) & 1u)) continue;
-        for (int i = tid; i < CS / 4; i += C)
-            atomicAdd(reinterpret_cast<float4*>(SD + (size_t)k * CS) + i,
-                      reinterpret_cast<const float4*>(S_tile + k * CS)[i]);
+    if constexpr (ORD) {  // ordered instantiation: SD is the partial scratch, this CTA's slot is [blockIdx.x]
+        float4* dst = reinterpret_cast<float4*>(SD + (size_t)blockIdx.x * (K + 1) * CS);
+        for (int i = tid; i < (K + 1) * CS / 4; i += C) dst[i] = reinterpret_cast<const float4*>(S_tile)[i];
+    } else {
+        for (int k = 0; k <= K; ++k) {
+            if (!((seen >> k) & 1u)) continue;
+            for (int i = tid; i < CS / 4; i += C)
+                atomicAdd(reinterpret_cast<float4*>(SD + (size_t)k * CS) + i,
+                          reinterpret_cast<const float4*>(S_tile + k * CS)[i]);
+        }
     }
 }
 
@@ -416,7 +426,7 @@ __global__ void __launch_bounds__(C) write_reduce_mma_kernel(const __grid_consta
 // pixel pair (2t, 2t+1) an m16n8k16 B fragment wants, and with the 64-byte swizzle the eight rows of a fragment load
 // fall into distinct bank groups. 1/|f| scales the A operand (the label weights of the pixel) instead of the features,
 // so the bf16 feature values enter the product unrounded; A is split hi + lo (two MMAs).
-template <int C, int KP, bool TMA>
+template <int C, int KP, bool TMA, bool ORD = false>
 __global__ void __launch_bounds__(C) write_reduce_mma16_kernel(const __grid_constant__ CUtensorMap tm_f,
                                                                 const __nv_bfloat16* __restrict__ f,
                                                                 const void* __restrict__ labels, int lab_u8,
@@ -616,16 +626,21 @@ __global__ void __launch_bounds__(C) write_reduce_mma16_kernel(const __grid_cons
         S_tile[lane * CS + C + 1] = S_tile[lane * CS + C + 2] = S_tile[lane * CS + C + 3] = 0.f;
     }
     __syncthreads();
-    for (int k = 0; k <= K; ++k) {
-        if (!((seen >> k) & 1u)) continue;
-        for (int i = tid; i < CS / 4; i += C)
-            atomicAdd(reinterpret_cast<float4*>(SD + (size_t)k * CS) + i, reinterpret_cast<const float4*>(S_tile + k * CS)[i]);
+    if constexpr (ORD) {  // ordered instantiation: SD is the partial scratch, this CTA's slot is [blockIdx.x]
+        float4* dst = reinterpret_cast<float4*>(SD + (size_t)blockIdx.x * (K + 1) * CS);
+        for (int i = tid; i < (K + 1) * CS / 4; i += C) dst[i] = reinterpret_cast<const float4*>(S_tile)[i];
+    } else {
+        for (int k = 0; k <= K; ++k) {
+            if (!((seen >> k) & 1u)) continue;
+            for (int i = tid; i < CS / 4; i += C)
+                atomicAdd(reinterpret_cast<float4*>(SD + (size_t)k * CS) + i, reinterpret_cast<const float4*>(S_tile + k * CS)[i]);
+        }
     }
 }
 
 template <int C, int KP>
 int launch_write_reduce_mma16(const void* f, const void* labels, int lab_u8, float* SD, int B, int h, int w, int Hm, int Wm,
-                              int K, cudaStream_t st) {
+                              int K, cudaStream_t st, float* part, int* ncta) {
     using T = __nv_bfloat16;
     const size_t ring = sizeof(T) * (size_t)2 * C * 32, stile = sizeof(float) * (size_t)32 * (C + 4);
     const size_t smem = sizeof(float) * (32 * 40 + (C / 32) * 32 + 32 + 4) + (ring > stile ? ring : stile) + 1024;
@@ -634,7 +649,8 @@ int launch_write_reduce_mma16(const void* f, const void* labels, int lab_u8, flo
     const float sx = w > 1 ? (float)(Wm - 1) / (float)(w - 1) : 0.f;
     CUtensorMap tm_f;
     const bool tma = tma_enabled() && make_map_2d<T>(&tm_f, f, (size_t)B * C, hw, C, 32, 3);
-    auto kern = tma ? write_reduce_mma16_kernel<C, KP, true> : write_reduce_mma16_kernel<C, KP, false>;
+    auto kern = part ? (tma ? write_reduce_mma16_kernel<C, KP, true, true> : write_reduce_mma16_kernel<C, KP, false, true>)
+                     : (tma ? write_reduce_mma16_kernel<C, KP, true> : write_reduce_mma16_kernel<C, KP, false>);
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
     int per_sm = 1;
@@ -644,6 +660,10 @@ int launch_write_reduce_mma16(const void* f, const void* labels, int lab_u8, flo
     if (per_sm > 4) per_sm = 4;
     int grid = 148 * per_sm;
     if (grid > ntiles) grid = ntiles;
+    if (part) {
+        if (grid > PM_ORD_CTAS) grid = PM_ORD_CTAS;
+        SD = part, *ncta = grid;
+    }
     kern<<<grid, C, smem, st>>>(tm_f, (const T*)f, labels, lab_u8, SD, h, w, Hm, Wm, K, sy, sx, tiles, ntiles);
     e = cudaGetLastError();
     return e == cudaSuccess ? 0 : (int)e;
@@ -651,7 +671,7 @@ int launch_write_reduce_mma16(const void* f, const void* labels, int lab_u8, flo
 
 template <int C, int KP>
 int launch_write_reduce_mma(const void* f, const void* labels, int lab_u8, float* SD, int B, int h, int w, int Hm, int Wm, int K,
-                            cudaStream_t st) {
+                            cudaStream_t st, float* part, int* ncta) {
     const size_t ring = sizeof(float) * (size_t)2 * C * 32, stile = sizeof(float) * (size_t)32 * (C + 4);
     const size_t smem = sizeof(float) * (32 * 40 + (C / 32) * 32 + 32 + 4) + (ring > stile ? ring : stile) + 1024;
     const int hw = h * w, tiles = (hw + 31) / 32, ntiles = B * tiles;
@@ -659,7 +679,8 @@ int launch_write_reduce_mma(const void* f, const void* labels, int lab_u8, float
     const float sx = w > 1 ? (float)(Wm - 1) / (float)(w - 1) : 0.f;
     CUtensorMap tm_f;
     const bool tma = tma_enabled() && make_map_2d<float>(&tm_f, f, (size_t)B * C, hw, C, 32, true);
-    auto kern = tma ? write_reduce_mma_kernel<C, KP, true> : write_reduce_mma_kernel<C, KP, false>;
+    auto kern = part ? (tma ? write_reduce_mma_kernel<C, KP, true, true> : write_reduce_mma_kernel<C, KP, false, true>)
+                     : (tma ? write_reduce_mma_kernel<C, KP, true> : write_reduce_mma_kernel<C, KP, false>);
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
     int per_sm = 1;
@@ -669,6 +690,10 @@ int launch_write_reduce_mma(const void* f, const void* labels, int lab_u8, float
     if (per_sm > 4) per_sm = 4;
     int grid = 148 * per_sm;
     if (grid > ntiles) grid = ntiles;
+    if (part) {
+        if (grid > PM_ORD_CTAS) grid = PM_ORD_CTAS;
+        SD = part, *ncta = grid;
+    }
     kern<<<grid, C, smem, st>>>(tm_f, (const float*)f, labels, lab_u8, SD, h, w, Hm, Wm, K, sy, sx, tiles, ntiles);
     e = cudaGetLastError();
     return e == cudaSuccess ? 0 : (int)e;
@@ -676,10 +701,10 @@ int launch_write_reduce_mma(const void* f, const void* labels, int lab_u8, float
 
 template <typename T, int C, int KP>
 int launch_write_reduce_tiled(const void* f, const void* labels, int lab_u8, float* SD, int B, int h, int w, int Hm, int Wm,
-                              int K, cudaStream_t st) {
+                              int K, cudaStream_t st, float* part, int* ncta) {
     const size_t smem = sizeof(float) * ((size_t)KP * (C + 4) + (C / 32) * 32 + 32) + sizeof(float4) * 2 * 32 * 4 + 16 +
                         sizeof(T) * (size_t)2 * C * 32;
-    auto kern = write_reduce_tiled_kernel<T, C, KP>;
+    auto kern = part ? write_reduce_tiled_kernel<T, C, KP, true> : write_reduce_tiled_kernel<T, C, KP>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
     const int hw = h * w, tiles = (hw + 31) / 32, ntiles = B * tiles;
@@ -688,6 +713,10 @@ int launch_write_reduce_tiled(const void* f, const void* labels, int lab_u8, flo
     if (per_sm < 1) per_sm = 1;
     int grid = 148 * per_sm;
     if (grid > ntiles) grid = ntiles;
+    if (part) {
+        if (grid > PM_ORD_CTAS) grid = PM_ORD_CTAS;
+        SD = part, *ncta = grid;
+    }
     const float sy = h > 1 ? (float)(Hm - 1) / (float)(h - 1) : 0.f;
     const float sx = w > 1 ? (float)(Wm - 1) / (float)(w - 1) : 0.f;
     kern<<<grid, C, smem, st>>>((const T*)f, labels, lab_u8, SD, h, w, Hm, Wm, K, sy, sx, tiles, ntiles);
@@ -905,24 +934,24 @@ int launch_write_bwd_tiled(const float* dS, const void* f, const void* labels, i
     }
 
 int write_reduce_tiled(const void* f, const void* labels, int lab_u8, float* SD, int B, int C, int h, int w, int Hm, int Wm,
-                       int K, int dtype, cudaStream_t st) {
+                       int K, int dtype, cudaStream_t st, float* part, int* ncta) {
     if (dtype == PM_F32) {
         switch (C) {  // tensor-core variant for every fp32 case (K + 1 <= 32 classes fit two 16-row MMA tiles)
-            case 32: return launch_write_reduce_mma<32, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st);
-            case 64: return launch_write_reduce_mma<64, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st);
-            case 128: return launch_write_reduce_mma<128, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st);
-            case 256: return launch_write_reduce_mma<256, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st);
+            case 32: return launch_write_reduce_mma<32, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st, part, ncta);
+            case 64: return launch_write_reduce_mma<64, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st, part, ncta);
+            case 128: return launch_write_reduce_mma<128, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st, part, ncta);
+            case 256: return launch_write_reduce_mma<256, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st, part, ncta);
             default: return PM_ERR_CHANNELS;
         }
     } else {
         switch (C) {  // tensor-core variant (whole 32-channel warps, >= 64 threads for the tile loads)
-            case 64: return launch_write_reduce_mma16<64, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st);
-            case 128: return launch_write_reduce_mma16<128, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st);
-            case 256: return launch_write_reduce_mma16<256, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st);
+            case 64: return launch_write_reduce_mma16<64, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st, part, ncta);
+            case 128: return launch_write_reduce_mma16<128, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st, part, ncta);
+            case 256: return launch_write_reduce_mma16<256, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st, part, ncta);
             default: break;  // C = 32: the run-length FFMA2 kernel
         }
-        if (K <= 19) { PM_WT_SWITCH_C(__nv_bfloat16, 20, launch_write_reduce_tiled, f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st) }
-        else { PM_WT_SWITCH_C(__nv_bfloat16, 32, launch_write_reduce_tiled, f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st) }
+        if (K <= 19) { PM_WT_SWITCH_C(__nv_bfloat16, 20, launch_write_reduce_tiled, f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st, part, ncta) }
+        else { PM_WT_SWITCH_C(__nv_bfloat16, 32, launch_write_reduce_tiled, f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st, part, ncta) }
     }
 }
 

@@ -99,7 +99,9 @@ class _ReadFn(torch.autograd.Function):
         KP = capi.score_stride(K)
         UC = C + capi.PLANES if planes else 2 * C
         u = torch.empty(B, UC, h, w, dtype=x.dtype, device=dev)
-        s = torch.empty(N, KP, dtype=torch.float32, device=dev)
+        # deterministic mode: torch may fill `empty` with NaN; the read-loss kernels read whole padded rows of s, so its
+        # padding columns must be finite -- zero them rather than depend on what the allocation held
+        s = (torch.zeros if capi.deterministic() else torch.empty)(N, KP, dtype=torch.float32, device=dev)
         score_m = torch.empty(N, K, dtype=torch.float32, device=dev)
         score_q = torch.empty(N, K, dtype=torch.float32, device=dev)
         M = M.contiguous()
@@ -952,7 +954,7 @@ class Memory_sup(nn.Module):
             q = query.detach().to(torch.float32).contiguous()
             M = mem.detach().to(torch.float32).contiguous()
             KP = capi.score_stride(K)
-            s = torch.empty(N, KP, dtype=torch.float32, device=dev)
+            s = (torch.zeros if capi.deterministic() else torch.empty)(N, KP, dtype=torch.float32, device=dev)   # (see _ReadFn)
             capi.score_nhwc(q, M, s, N, C, K)
             if mask is not None:
                 labels = _check_labels(mask, Bq)
