@@ -5,7 +5,7 @@
 
 namespace pm {
 
-// true when the pipelined (16-byte async copy) kernels can be used for these feature pointers
+// true when the pipelined (TMA / 16-byte async copy) kernels can be used for these feature pointers
 bool tiled_ok(const void* p0, const void* p1, const void* p2, int hw, int dtype);
 
 int read_fwd_tiled(const void* x, const float* M, const float* gum_m, const float* gum_q, void* u, float* s, float* p,

@@ -1,9 +1,9 @@
 // Memory read, pipelined variants (the fast path when hw is a multiple of the 16-byte chunk).
 //
 // Persistent CTAs (2 per SM) walk tiles of 32 consecutive pixels x all C channels. Each tile is brought
-// into shared memory with 16-byte async copies (LDGSTS) into a 2-stage ring, so the next tile streams
-// from HBM while the current one is consumed and the feature values never occupy registers. The 8 warps
-// split the channels, a lane owns one pixel (conflict-free column reads of the dense [C][32] tile), the
+// into shared memory by TMA (the ds pass of the backward: 16-byte async copies, LDGSTS) into a 2-stage ring,
+// so the next tile streams from HBM while the current one is consumed and the feature values never occupy
+// registers. The 8 warps split the channels, a lane owns one pixel (conflict-free column reads of the dense [C][32] tile), the
 // K x C memory sits transposed in shared memory (Mt[c][KP]: a channel's K values are five broadcast
 // 128-bit loads) and all multiply-adds are packed FFMA2 (fp32x2), which is what reaches the fp32 peak
 // on sm_100 (profiles/microbench/ffma2.cu: 65.9 vs 46.8 TFLOP/s for scalar FFMA).
@@ -192,20 +192,6 @@ __device__ __forceinline__ void tile_weighted_sum_mma(const float* p_sm, const f
 __device__ __forceinline__ int bf16_tile_off(int row, int px) {  // element offset of (row, px) in a SWIZZLE_64B tile
     return row * 32 + ((((px >> 3) ^ ((row >> 1) & 3)) << 3) | (px & 7));
 }
-template <int ROWS, int NTHREADS>
-__device__ __forceinline__ void tile_load_async_mma16(__nv_bfloat16* smem_tile, const __nv_bfloat16* __restrict__ base, int hw,
-                                                      int px0) {
-    static_assert(NTHREADS % 4 == 0, "thread count must be a multiple of the chunks per row");
-    const int ch = threadIdx.x % 4;
-    const int px = px0 + ch * 8;
-    const bool valid = px < hw;
-    const __nv_bfloat16* src = base + (size_t)(threadIdx.x / 4) * hw + (valid ? px : 0);
-    const size_t step = (size_t)(NTHREADS / 4) * hw;
-    for (int row = threadIdx.x / 4; row < ROWS; row += NTHREADS / 4) {
-        cp_async16(smem_tile + row * 32 + ((ch ^ ((row >> 1) & 3)) << 3), src, valid);
-        src += step;
-    }
-}
 __device__ __forceinline__ void ldmatrix_x4_trans(unsigned (&r)[4], uint32_t saddr) {
     asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];"
                  : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
@@ -321,8 +307,8 @@ struct UseMma<__nv_bfloat16, CW> {
 // dispatch: load one tile for the dots phase in the layout the chosen contraction wants
 template <typename T, int C, int NTHREADS, bool MMA>
 __device__ __forceinline__ void dots_tile_load(T* smem_tile, const T* __restrict__ base, int hw, int px0) {
-    if constexpr (MMA && sizeof(T) == 4) tile_load_async_mma<C, NTHREADS>(reinterpret_cast<float*>(smem_tile), reinterpret_cast<const float*>(base), hw, px0);
-    else if constexpr (MMA) tile_load_async_mma16<C, NTHREADS>(reinterpret_cast<__nv_bfloat16*>(smem_tile), reinterpret_cast<const __nv_bfloat16*>(base), hw, px0);
+    static_assert(!MMA || sizeof(T) == 4, "the cp.async tensor-core layout is the fp32 one");
+    if constexpr (MMA) tile_load_async_mma<C, NTHREADS>(reinterpret_cast<float*>(smem_tile), reinterpret_cast<const float*>(base), hw, px0);
     else tile_load_async<T, C, NTHREADS>(smem_tile, base, hw, px0);
 }
 
@@ -335,8 +321,6 @@ __device__ __forceinline__ void store_partial(float* part, int wid, int lane, co
 
 // --------------------------------------------------------------------------------------------- forward
 
-// TMA = true: the x tiles arrive as tensor-map boxes (SWIZZLE_128B for the tensor-core layout, dense otherwise) on an
-// mbarrier ring; tm_x is unused with the cp.async ring.
 // exp(x) for x <= 0 (softmax terms after the maximum is subtracted): ex2.approx of x*log2(e) -- 2 instructions instead of
 // expf's ~10; the terms that matter have |x| of a few units, where the product's rounding is ~1e-7 relative (the read-loss
 // kernels have always computed their softmax this way)
@@ -346,7 +330,11 @@ __device__ __forceinline__ float fexp_nonpos(float x) {
     return y;
 }
 
-template <typename T, int C, int KP, int NSTAGE, bool TMA>
+// The x tiles arrive as tensor-map boxes (SWIZZLE_128B / SWIZZLE_64B for the tensor-core layouts, dense otherwise) on an
+// mbarrier ring. `x` itself is not read; it stays in the parameter list because the offsets of the parameters after it
+// steer ptxas: without it the bf16 tensor-core instantiations are scheduled differently (C = 128, K > 19: 87 registers
+// instead of 80).
+template <typename T, int C, int KP, int NSTAGE>
 __global__ void __launch_bounds__(TL_THREADS, 2)
     read_fwd_tiled_kernel(const __grid_constant__ CUtensorMap tm_x, const T* __restrict__ x,
                           const float* __restrict__ M, const float* __restrict__ gum_m,
@@ -376,30 +364,18 @@ __global__ void __launch_bounds__(TL_THREADS, 2)
 
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     int tile = blockIdx.x;
-    auto issue = [&](int t, int s) {  // TMA: one thread
+    auto issue = [&](int t, int s) {  // one thread
         const int b = t / tiles_per_img, px0 = (t - b * tiles_per_img) * TP;
         mbar_expect_tx(&full[s], (uint32_t)(C * TP * sizeof(T)));
         tma_load_2d(xs + s * C * TP, &tm_x, px0, b * C, &full[s]);
     };
-    if constexpr (TMA) {
-        if (tid == 0) {
+    if (tid == 0) {
 #pragma unroll
-            for (int s = 0; s < NSTAGE; ++s) mbar_init(&full[s], 1);
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        for (int s = 0; s < NSTAGE; ++s) mbar_init(&full[s], 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 #pragma unroll
-            for (int s = 0; s < NSTAGE; ++s)
-                if (tile + s * (int)gridDim.x < ntiles) issue(tile + s * gridDim.x, s);
-        }
-    } else {
-#pragma unroll
-        for (int s = 0; s < NSTAGE; ++s) {
-            const int t = tile + s * gridDim.x;
-            if (t < ntiles) {
-                const int b = t / tiles_per_img, px0 = (t - b * tiles_per_img) * TP;
-                dots_tile_load<T, C, TL_THREADS, MMA>(xs + s * C * TP, x + (size_t)b * C * hw, hw, px0);
-            }
-            cp_async_commit();
-        }
+        for (int s = 0; s < NSTAGE; ++s)
+            if (tile + s * (int)gridDim.x < ntiles) issue(tile + s * gridDim.x, s);
     }
     load_Mt<C, KP>(Mt, M, K);
     if constexpr (MMA16) load_Mb<C, KP>(Mb_hi, Mb_lo, M, K);
@@ -410,9 +386,8 @@ __global__ void __launch_bounds__(TL_THREADS, 2)
     int stage = 0;
     unsigned phase = 0;
     for (; tile < ntiles; tile += gridDim.x) {
-        if constexpr (!TMA) cp_async_wait<NSTAGE - 1>();
-        __syncthreads();  // Mt and the mbarriers are set up / the cp.async tile is visible
-        if constexpr (TMA) mbar_wait(&full[stage], phase);
+        __syncthreads();  // Mt and the mbarriers are set up
+        mbar_wait(&full[stage], phase);
         const T* xt = xs + stage * C * TP;
         const int b = tile / tiles_per_img, px0 = (tile - b * tiles_per_img) * TP;
         const int nvalid = min(TP, hw - px0);
@@ -574,18 +549,9 @@ __global__ void __launch_bounds__(TL_THREADS, 2)
         }
         __syncthreads();  // every read of this stage is done: refill it
         const int next = tile + NSTAGE * gridDim.x;
-        if constexpr (TMA) {
-            if (tid == 0 && next < ntiles) issue(next, stage);
-        } else {
-            if (next < ntiles) {
-                const int nb = next / tiles_per_img, npx0 = (next - nb * tiles_per_img) * TP;
-                dots_tile_load<T, C, TL_THREADS, MMA>(xs + stage * C * TP, x + (size_t)nb * C * hw, hw, npx0);
-            }
-            cp_async_commit();
-        }
+        if (tid == 0 && next < ntiles) issue(next, stage);
         if (++stage == NSTAGE) stage = 0, phase ^= 1u;
     }
-    if constexpr (!TMA) cp_async_wait<0>();
 
     if (colpart != nullptr) {  // per-CTA column (max,sum) partials, same layout as colsoftmax_stats_kernel
         __syncthreads();
@@ -681,12 +647,11 @@ int launch_read_fwd_tiled(const void* x, const float* M, const float* gum_m, con
     if (grid > ntiles) grid = ntiles;
     CUtensorMap tm_x;
     // fp32 tiles: 128-byte rows, SWIZZLE_128B; bf16 tiles: 64-byte rows, SWIZZLE_64B
-    const bool tma = tma_enabled() && make_map_2d<T>(&tm_x, x, (size_t)B * C, hw, C, TP, MMA16 ? 3 : (MMA ? 1 : 0));
-    auto kern = tma ? read_fwd_tiled_kernel<T, C, KP, NSTAGE, true> : read_fwd_tiled_kernel<T, C, KP, NSTAGE, false>;
+    if (!make_map_2d<T>(&tm_x, x, (size_t)B * C, hw, C, TP, MMA16 ? 3 : (MMA ? 1 : 0))) return PM_ERR_ALIGN;
+    auto kern = read_fwd_tiled_kernel<T, C, KP, NSTAGE>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
-    kern<<<grid, TL_THREADS, smem, st>>>(tm_x, (const T*)x, M, gum_m, gum_q, (T*)u, s, p, colpart, hw, K, tiles, ntiles,
-                                         planes);
+    kern<<<grid, TL_THREADS, smem, st>>>(tm_x, (const T*)x, M, gum_m, gum_q, (T*)u, s, p, colpart, hw, K, tiles, ntiles, planes);
     cudaError_t le = cudaGetLastError();
     return le == cudaSuccess ? 0 : (int)le;
 }
@@ -826,141 +791,13 @@ __global__ void __launch_bounds__(256)
 }
 
 // -------------------------------------------------------------------------------- backward, part B: dx
-// dq = dq0 + ds.M ; q = x/|x| ; dx = (dq - q (q.dq)) / |x|. One CTA per SM, 16 warps x (C/16) channels,
-// lanes = pixels; x, dq0 and the ds rows of a tile arrive through a 2-stage async-copy ring.
+// dq = dq0 + ds.M ; q = x/|x| ; dx = (dq - q (q.dq)) / |x|. One CTA per SM, 16 warps x (C/16) channels, lanes = pixels.
+// The x and dq0 tiles of a stage arrive as two 2-D tensor-map boxes ([C rows][32 pixels] of the [B*C, hw] / [B*UC, hw]
+// matrices) and the ds rows as one 1-D bulk copy, all completing on an mbarrier per stage that one thread issues (3
+// instructions). The kernel is LSU / shared-memory-pipe bound (DESIGN.md 6), and the async proxy keeps the tile fill off
+// that pipe. Columns past the end of an image row are zero-filled by the TMA unit.
 
 constexpr int DX_THREADS = 512, DX_WARPS = 16;
-
-template <typename T, int C, int KP, int NSTAGE>
-__global__ void __launch_bounds__(DX_THREADS, 1)
-    read_bwd_dx_tiled_kernel(const T* __restrict__ du, const T* __restrict__ x, const float* __restrict__ M,
-                             const float* __restrict__ ds, T* __restrict__ dx, const T* __restrict__ dx_add, int hw, int K,
-                             int tiles_per_img, int ntiles, int UC) {  // UC: channels per image of du (2C, or C + PM_PLANES)
-    constexpr int CW = C / DX_WARPS;
-    extern __shared__ __align__(16) unsigned char smraw[];
-    float* Mt = reinterpret_cast<float*>(smraw);        // [C][KP]
-    float* pn = Mt + C * KP;                            // [16][TP]
-    float* pd = pn + DX_WARPS * TP;                     // [16][TP]
-    float* dss = pd + DX_WARPS * TP;                    // [NSTAGE][TP][KP]
-    T* xs = reinterpret_cast<T*>(dss + NSTAGE * TP * KP);  // [NSTAGE][2][C][TP]: x tile, dq0 tile
-
-    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-    auto issue = [&](int t, int s) {
-        const int b = t / tiles_per_img, px0 = (t - b * tiles_per_img) * TP;
-        T* base = xs + (size_t)s * 2 * C * TP;
-        tile_load_async<T, C, DX_THREADS>(base, x + (size_t)b * C * hw, hw, px0);
-        tile_load_async<T, C, DX_THREADS>(base + C * TP, du + (size_t)b * UC * hw, hw, px0);
-        const size_t n0g = (size_t)b * hw + px0;
-        const int nvalid = min(TP, hw - px0);
-        for (int i = tid; i < TP * KP / 4; i += DX_THREADS)
-            cp_async16(dss + s * TP * KP + i * 4, ds + n0g * KP + (i * 4 < nvalid * KP ? i * 4 : 0), i * 4 < nvalid * KP);
-    };
-    int tile = blockIdx.x;
-#pragma unroll
-    for (int s = 0; s < NSTAGE; ++s) {
-        const int t = tile + s * gridDim.x;
-        if (t < ntiles) issue(t, s);
-        cp_async_commit();
-    }
-    for (int i = tid; i < C * KP; i += DX_THREADS) {
-        const int c = i / KP, k = i - c * KP;
-        Mt[i] = (k < K) ? __ldg(M + (size_t)k * C + c) : 0.f;
-    }
-
-    int stage = 0;
-    for (; tile < ntiles; tile += gridDim.x) {
-        cp_async_wait<NSTAGE - 1>();
-        __syncthreads();
-        const T* xt = xs + (size_t)stage * 2 * C * TP;
-        const T* qt = xt + C * TP;
-        const int b = tile / tiles_per_img, px0 = (tile - b * tiles_per_img) * TP;
-        const int nvalid = min(TP, hw - px0);
-        const T* xcol = xt + wid * CW * 32 + lane;
-        const T* qcol = qt + wid * CW * 32 + lane;
-        float xv[CW], n2 = 0.f;
-#pragma unroll
-        for (int j = 0; j < CW; ++j) {
-            xv[j] = to_float(xcol[j * 32]);
-            n2 = fmaf(xv[j], xv[j], n2);
-        }
-        pn[wid * TP + lane] = n2;
-        // dq = dq0 + ds . M for this warp's channels
-        float2 s2[KP / 2];
-        {
-            const float4* sr = reinterpret_cast<const float4*>(dss + stage * TP * KP + lane * KP);
-#pragma unroll
-            for (int q = 0; q < KP / 4; ++q) {
-                const float4 v = sr[q];
-                s2[2 * q] = f2(v.x, v.y);
-                s2[2 * q + 1] = f2(v.z, v.w);
-            }
-        }
-        float dq[CW];
-        const float4* mbase = reinterpret_cast<const float4*>(Mt + wid * CW * KP);
-#pragma unroll
-        for (int j = 0; j < CW; ++j) {
-            const float4* mrow = mbase + j * (KP / 4);
-            float2 acc = f2(to_float(qcol[j * 32]), 0.f);
-#pragma unroll
-            for (int q = 0; q < KP / 4; ++q) {
-                const float4 m = mrow[q];
-                acc = __ffma2_rn(s2[2 * q], f2(m.x, m.y), acc);
-                acc = __ffma2_rn(s2[2 * q + 1], f2(m.z, m.w), acc);
-            }
-            dq[j] = acc.x + acc.y;
-        }
-        __syncthreads();
-        float nn = 0.f;
-#pragma unroll
-        for (int w = 0; w < DX_WARPS; ++w) nn += pn[w * TP + lane];
-        const float nrm = sqrtf(nn), ir = 1.f / fmaxf(nrm, PM_NORM_EPS);
-        float dot = 0.f;
-#pragma unroll
-        for (int j = 0; j < CW; ++j) {
-            xv[j] *= ir;  // q
-            dot = fmaf(xv[j], dq[j], dot);
-        }
-        pd[wid * TP + lane] = dot;
-        __syncthreads();  // also: every read of this stage's tiles is done
-        const int next = tile + NSTAGE * gridDim.x;
-        if (next < ntiles) issue(next, stage);
-        cp_async_commit();
-        dot = 0.f;
-#pragma unroll
-        for (int w = 0; w < DX_WARPS; ++w) dot += pd[w * TP + lane];
-        if (nrm <= PM_NORM_EPS) dot = 0.f;  // F.normalize clamps the norm: no projection gradient below eps
-        if (lane < nvalid) {
-            const size_t o0 = ((size_t)b * C + wid * CW) * hw + px0 + lane;
-            T* dxp = dx + o0;
-            if (dx_add != nullptr) {  // a second gradient of x (the write branch's) summed here instead of by an add kernel
-                const T* ap = dx_add + o0;
-                float av[CW];
-#pragma unroll
-                for (int j = 0; j < CW; ++j) av[j] = ldf(ap + (size_t)j * hw);
-#pragma unroll
-                for (int j = 0; j < CW; ++j) {
-                    stf(dxp, (dq[j] - xv[j] * dot) * ir + av[j]);
-                    dxp += hw;
-                }
-            } else {
-#pragma unroll
-                for (int j = 0; j < CW; ++j) {
-                    stf(dxp, (dq[j] - xv[j] * dot) * ir);
-                    dxp += hw;
-                }
-            }
-        }
-        stage = (stage + 1 == NSTAGE) ? 0 : stage + 1;
-    }
-    cp_async_wait<0>();
-}
-
-// ---------------------------------------------------------------- backward, part B with a TMA tile ring
-// Same arithmetic as read_bwd_dx_tiled_kernel; the x and dq0 tiles arrive as two 2-D tensor-map boxes
-// ([C rows][32 pixels] of the [B*C, hw] / [B*UC, hw] matrices) and the ds rows as one 1-D bulk copy, all completing
-// on an mbarrier per stage. One thread issues a stage (3 instructions) instead of 512 threads issuing ~17 LDGSTS
-// each: the kernel is LSU / shared-memory-pipe bound (DESIGN.md 6), and the async proxy takes the tile fill off
-// that pipe. Columns past the end of an image row are zero-filled by the TMA unit.
 
 template <typename T, int C, int KP, int NSTAGE>
 __global__ void __launch_bounds__(DX_THREADS, 1)
@@ -1298,46 +1135,39 @@ int launch_read_bwd_tiled(const void* du, const void* x, const float* M, const f
         e = cudaGetLastError();
         if (e != cudaSuccess) return (int)e;
     }
-    {
-        const size_t smem = sizeof(float) * ((size_t)C * KP + 2 * DX_WARPS * TP + (size_t)NSTAGE * TP * KP) +
-                            sizeof(T) * (size_t)NSTAGE * 2 * C * TP;
-        int grid = 148;
-        if (grid > ntiles) grid = ntiles;
-        CUtensorMap tm_x, tm_du;
-        cudaError_t e;
-        if constexpr (sizeof(T) == 2 && (C == 128 || C == 256)) {
+    CUtensorMap tm_x, tm_du;
+    cudaError_t e;
+    if constexpr (sizeof(T) == 2 && (C == 128 || C == 256)) {
+        if (dx_add == nullptr) {
             CUtensorMap tm_dx;
-            if (dx_add == nullptr && tma_enabled() && make_map_2d<T>(&tm_x, x, (size_t)B * C, hw, C, TP, 3) &&
-                make_map_2d<T>(&tm_du, du, (size_t)B * UC, hw, C, TP, 3) && make_map_2d<T>(&tm_dx, dx, (size_t)B * C, hw, C, TP, 3)) {
-                constexpr int NS = 2;
-                const size_t sm = sizeof(T) * (size_t)NS * 2 * C * TP + sizeof(float) * ((size_t)NS * TP * KP + 2 * DXB_WARPS * TP) +
-                                  sizeof(unsigned) * 2 * 16 * (C + 8) + 1024;
-                auto kern = read_bwd_dx_bf16_kernel<C, KP, NS>;
-                e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-                if (e != cudaSuccess) return (int)e;
-                int g2 = 2 * 148;
-                if (g2 > ntiles) g2 = ntiles;
-                kern<<<g2, DXB_THREADS, sm, st>>>(tm_x, tm_du, tm_dx, M, ds, hw, K, tiles, ntiles, UC);
-                e = cudaGetLastError();
-                return e == cudaSuccess ? 0 : (int)e;
-            }
-        }
-        if (tma_enabled() && C <= 256 && make_map_2d<T>(&tm_x, x, (size_t)B * C, hw, C, TP, false) &&
-            make_map_2d<T>(&tm_du, du, (size_t)B * UC, hw, C, TP, false)) {
-            auto kern = read_bwd_dx_tma_kernel<T, C, KP, NSTAGE>;
-            e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem + 1024);
+            if (!make_map_2d<T>(&tm_x, x, (size_t)B * C, hw, C, TP, 3) || !make_map_2d<T>(&tm_du, du, (size_t)B * UC, hw, C, TP, 3) ||
+                !make_map_2d<T>(&tm_dx, dx, (size_t)B * C, hw, C, TP, 3))
+                return PM_ERR_ALIGN;
+            constexpr int NS = 2;
+            const size_t sm = sizeof(T) * (size_t)NS * 2 * C * TP + sizeof(float) * ((size_t)NS * TP * KP + 2 * DXB_WARPS * TP) +
+                              sizeof(unsigned) * 2 * 16 * (C + 8) + 1024;
+            auto kern = read_bwd_dx_bf16_kernel<C, KP, NS>;
+            e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
             if (e != cudaSuccess) return (int)e;
-            kern<<<grid, DX_THREADS, smem + 1024, st>>>(tm_x, tm_du, M, ds, (T*)dx, (const T*)dx_add, hw, K, tiles, ntiles, UC);
-        } else {
-            auto kern = read_bwd_dx_tiled_kernel<T, C, KP, NSTAGE>;
-            e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            if (e != cudaSuccess) return (int)e;
-            kern<<<grid, DX_THREADS, smem, st>>>((const T*)du, (const T*)x, M, ds, (T*)dx, (const T*)dx_add, hw, K, tiles, ntiles, UC);
+            int g2 = 2 * 148;
+            if (g2 > ntiles) g2 = ntiles;
+            kern<<<g2, DXB_THREADS, sm, st>>>(tm_x, tm_du, tm_dx, M, ds, hw, K, tiles, ntiles, UC);
+            e = cudaGetLastError();
+            return e == cudaSuccess ? 0 : (int)e;
         }
-        e = cudaGetLastError();
-        if (e != cudaSuccess) return (int)e;
     }
-    return 0;
+    if (!make_map_2d<T>(&tm_x, x, (size_t)B * C, hw, C, TP, false) || !make_map_2d<T>(&tm_du, du, (size_t)B * UC, hw, C, TP, false))
+        return PM_ERR_ALIGN;
+    const size_t smem = sizeof(float) * ((size_t)C * KP + 2 * DX_WARPS * TP + (size_t)NSTAGE * TP * KP) +
+                        sizeof(T) * (size_t)NSTAGE * 2 * C * TP + 1024;
+    auto kern = read_bwd_dx_tma_kernel<T, C, KP, NSTAGE>;
+    e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return (int)e;
+    int grid = 148;
+    if (grid > ntiles) grid = ntiles;
+    kern<<<grid, DX_THREADS, smem, st>>>(tm_x, tm_du, M, ds, (T*)dx, (const T*)dx_add, hw, K, tiles, ntiles, UC);
+    e = cudaGetLastError();
+    return e == cudaSuccess ? 0 : (int)e;
 }
 
 #define PM_TILED_SWITCH_C(T, KP, FN, ...)                   \

@@ -5,7 +5,6 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-#include <cstdlib>
 #include <mutex>
 
 namespace pm {
@@ -111,15 +110,6 @@ static bool make_map_2d(CUtensorMap* map, const void* base, size_t rows, size_t 
     const unsigned slot = next++ % SLOTS;
     keys[slot] = key, maps[slot] = *map, used[slot] = true;
     return true;
-}
-
-static int tma_enabled() {  // PM_TMA=0 keeps the per-thread cp.async rings (A/B switch)
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("PM_TMA");
-        v = (e && e[0] == '0') ? 0 : 1;
-    }
-    return v;
 }
 
 // round a shared-memory pointer up to a multiple of `a` bytes (a power of two); callers allocate the slack

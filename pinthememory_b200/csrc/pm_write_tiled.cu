@@ -211,10 +211,10 @@ __global__ void __launch_bounds__(C) write_reduce_tiled_kernel(const T* __restri
 // chunk-swizzled f tile (conflict-free) and are scaled by 1/|f| on the fly. Cost no longer depends on how
 // fragmented the label map is (the run-length kernel above degenerates on noisy labels).
 
-// TMA = true: the tiles arrive as SWIZZLE_128B tensor-map boxes (the same chunk ^ (row & 7) layout) on an mbarrier ring
-template <int C, int KP, bool TMA, bool ORD = false>
+// The tiles arrive as SWIZZLE_128B tensor-map boxes (16-byte chunk c of row r at chunk c ^ (r & 7)) on an mbarrier ring.
+template <int C, int KP, bool ORD = false>
 __global__ void __launch_bounds__(C) write_reduce_mma_kernel(const __grid_constant__ CUtensorMap tm_f,
-                                                              const float* __restrict__ f, const void* __restrict__ labels, int lab_u8,
+                                                              const void* __restrict__ labels, int lab_u8,
                                                               float* __restrict__ SD, int h, int w, int Hm, int Wm,
                                                               int K, float sy, float sx, int tiles_per_img,
                                                               int ntiles) {
@@ -259,32 +259,19 @@ __global__ void __launch_bounds__(C) write_reduce_mma_kernel(const __grid_consta
     };
 
     int tile = blockIdx.x;
-    auto issue = [&](int tl, int s) {  // TMA: one thread
+    auto issue = [&](int tl, int s) {  // one thread
         int b, px0;
         tile_coords(tl, b, px0);
         mbar_expect_tx(&full[s], (uint32_t)(C * 32 * sizeof(float)));
         tma_load_2d(ft + s * C * 32, &tm_f, px0, b * C, &full[s]);
     };
-    if constexpr (TMA) {
-        if (tid == 0) {
+    if (tid == 0) {
 #pragma unroll
-            for (int s = 0; s < NSTAGE; ++s) mbar_init(&full[s], 1);
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        for (int s = 0; s < NSTAGE; ++s) mbar_init(&full[s], 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 #pragma unroll
-            for (int s = 0; s < NSTAGE; ++s)
-                if (tile + s * (int)gridDim.x < ntiles) issue(tile + s * gridDim.x, s);
-        }
-    } else {
-#pragma unroll
-        for (int s = 0; s < NSTAGE; ++s) {
-            const int tl = tile + s * gridDim.x;
-            if (tl < ntiles) {
-                int b, px0;
-                tile_coords(tl, b, px0);
-                tile_load_async_swz<float, C, C>(ft + s * C * 32, f + (size_t)b * C * hw, hw, px0);
-            }
-            cp_async_commit();
-        }
+        for (int s = 0; s < NSTAGE; ++s)
+            if (tile + s * (int)gridDim.x < ntiles) issue(tile + s * gridDim.x, s);
     }
     LabelTaps tcur;
     if (wid == 0) tcur = taps_for(tile);
@@ -294,9 +281,8 @@ __global__ void __launch_bounds__(C) write_reduce_mma_kernel(const __grid_consta
     for (; tile < ntiles; tile += gridDim.x) {
         LabelTaps tnext;
         if (wid == 0) tnext = taps_for(tile + gridDim.x);  // loads in flight across this tile
-        if constexpr (!TMA) cp_async_wait<NSTAGE - 1>();
         __syncthreads();
-        if constexpr (TMA) mbar_wait(&full[stage], phase);
+        mbar_wait(&full[stage], phase);
         const float* xt = ft + stage * C * 32;
         for (int i = tid; i < 32 * OMLD / 4; i += C) reinterpret_cast<float4*>(om)[i] = make_float4(0.f, 0.f, 0.f, 0.f);
         {  // |f|^2 per pixel: lanes = pixels, each warp sums 32 of the C rows (rows wid, wid+NW, .. share a swizzle
@@ -373,20 +359,10 @@ __global__ void __launch_bounds__(C) write_reduce_mma_kernel(const __grid_consta
         }
         __syncthreads();  // stage and label table consumed
         const int next = tile + NSTAGE * gridDim.x;
-        if constexpr (TMA) {
-            if (tid == 0 && next < ntiles) issue(next, stage);
-        } else {
-            if (next < ntiles) {
-                int nb, npx0;
-                tile_coords(next, nb, npx0);
-                tile_load_async_swz<float, C, C>(ft + stage * C * 32, f + (size_t)nb * C * hw, hw, npx0);
-            }
-            cp_async_commit();
-        }
+        if (tid == 0 && next < ntiles) issue(next, stage);
         if (wid == 0) tcur = tnext;
         if (++stage == NSTAGE) stage = 0, phase ^= 1u;
     }
-    if constexpr (!TMA) cp_async_wait<0>();
     __syncthreads();
     // accumulators -> shared [32][CS] (over the tile ring), then one vector RED per touched class row
     float* S_tile = ft;
@@ -426,9 +402,8 @@ __global__ void __launch_bounds__(C) write_reduce_mma_kernel(const __grid_consta
 // pixel pair (2t, 2t+1) an m16n8k16 B fragment wants, and with the 64-byte swizzle the eight rows of a fragment load
 // fall into distinct bank groups. 1/|f| scales the A operand (the label weights of the pixel) instead of the features,
 // so the bf16 feature values enter the product unrounded; A is split hi + lo (two MMAs).
-template <int C, int KP, bool TMA, bool ORD = false>
+template <int C, int KP, bool ORD = false>
 __global__ void __launch_bounds__(C) write_reduce_mma16_kernel(const __grid_constant__ CUtensorMap tm_f,
-                                                                const __nv_bfloat16* __restrict__ f,
                                                                 const void* __restrict__ labels, int lab_u8,
                                                                 float* __restrict__ SD, int h, int w, int Hm, int Wm, int K,
                                                                 float sy, float sx, int tiles_per_img, int ntiles) {
@@ -472,38 +447,20 @@ __global__ void __launch_bounds__(C) write_reduce_mma16_kernel(const __grid_cons
         }
         return r;
     };
-    auto load_tile = [&](int tl, int s) {  // cp.async ring: all threads, the SWIZZLE_64B pattern by hand
-        int b, px0;
-        tile_coords(tl, b, px0);
-        const T* base = f + (size_t)b * C * hw;
-        const int ch = tid % 4, px = px0 + ch * 8;
-        const bool valid = px < hw;
-        for (int row = tid / 4; row < C; row += C / 4)
-            cp_async16(ft + (size_t)s * C * 32 + row * 32 + ((ch ^ ((row >> 1) & 3)) << 3), base + (size_t)row * hw + (valid ? px : 0),
-                       valid);
-    };
     int tile = blockIdx.x;
-    auto issue = [&](int tl, int s) {  // TMA: one thread
+    auto issue = [&](int tl, int s) {  // one thread
         int b, px0;
         tile_coords(tl, b, px0);
         mbar_expect_tx(&full[s], (uint32_t)(C * 32 * sizeof(T)));
         tma_load_2d(ft + (size_t)s * C * 32, &tm_f, px0, b * C, &full[s]);
     };
-    if constexpr (TMA) {
-        if (tid == 0) {
+    if (tid == 0) {
 #pragma unroll
-            for (int s = 0; s < NSTAGE; ++s) mbar_init(&full[s], 1);
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        for (int s = 0; s < NSTAGE; ++s) mbar_init(&full[s], 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 #pragma unroll
-            for (int s = 0; s < NSTAGE; ++s)
-                if (tile + s * (int)gridDim.x < ntiles) issue(tile + s * gridDim.x, s);
-        }
-    } else {
-#pragma unroll
-        for (int s = 0; s < NSTAGE; ++s) {
-            if (tile + s * (int)gridDim.x < ntiles) load_tile(tile + s * gridDim.x, s);
-            cp_async_commit();
-        }
+        for (int s = 0; s < NSTAGE; ++s)
+            if (tile + s * (int)gridDim.x < ntiles) issue(tile + s * gridDim.x, s);
     }
     LabelTaps tcur;
     if (wid == 0) tcur = taps_for(tile);
@@ -513,9 +470,8 @@ __global__ void __launch_bounds__(C) write_reduce_mma16_kernel(const __grid_cons
     for (; tile < ntiles; tile += gridDim.x) {
         LabelTaps tnext;
         if (wid == 0) tnext = taps_for(tile + gridDim.x);
-        if constexpr (!TMA) cp_async_wait<NSTAGE - 1>();
         __syncthreads();
-        if constexpr (TMA) mbar_wait(&full[stage], phase);
+        mbar_wait(&full[stage], phase);
         const T* xt = ft + (size_t)stage * C * 32;
         const unsigned* xw = reinterpret_cast<const unsigned*>(xt);
         for (int i = tid; i < 32 * OMLD / 4; i += C) reinterpret_cast<float4*>(om)[i] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -596,16 +552,10 @@ __global__ void __launch_bounds__(C) write_reduce_mma16_kernel(const __grid_cons
         }
         __syncthreads();
         const int next = tile + NSTAGE * gridDim.x;
-        if constexpr (TMA) {
-            if (tid == 0 && next < ntiles) issue(next, stage);
-        } else {
-            if (next < ntiles) load_tile(next, stage);
-            cp_async_commit();
-        }
+        if (tid == 0 && next < ntiles) issue(next, stage);
         if (wid == 0) tcur = tnext;
         if (++stage == NSTAGE) stage = 0, phase ^= 1u;
     }
-    if constexpr (!TMA) cp_async_wait<0>();
     __syncthreads();
     float* S_tile = reinterpret_cast<float*>(smraw);
 #pragma unroll
@@ -648,9 +598,8 @@ int launch_write_reduce_mma16(const void* f, const void* labels, int lab_u8, flo
     const float sy = h > 1 ? (float)(Hm - 1) / (float)(h - 1) : 0.f;
     const float sx = w > 1 ? (float)(Wm - 1) / (float)(w - 1) : 0.f;
     CUtensorMap tm_f;
-    const bool tma = tma_enabled() && make_map_2d<T>(&tm_f, f, (size_t)B * C, hw, C, 32, 3);
-    auto kern = part ? (tma ? write_reduce_mma16_kernel<C, KP, true, true> : write_reduce_mma16_kernel<C, KP, false, true>)
-                     : (tma ? write_reduce_mma16_kernel<C, KP, true> : write_reduce_mma16_kernel<C, KP, false>);
+    if (!make_map_2d<T>(&tm_f, f, (size_t)B * C, hw, C, 32, 3)) return PM_ERR_ALIGN;
+    auto kern = part ? write_reduce_mma16_kernel<C, KP, true> : write_reduce_mma16_kernel<C, KP>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
     int per_sm = 1;
@@ -664,7 +613,7 @@ int launch_write_reduce_mma16(const void* f, const void* labels, int lab_u8, flo
         if (grid > PM_ORD_CTAS) grid = PM_ORD_CTAS;
         SD = part, *ncta = grid;
     }
-    kern<<<grid, C, smem, st>>>(tm_f, (const T*)f, labels, lab_u8, SD, h, w, Hm, Wm, K, sy, sx, tiles, ntiles);
+    kern<<<grid, C, smem, st>>>(tm_f, labels, lab_u8, SD, h, w, Hm, Wm, K, sy, sx, tiles, ntiles);
     e = cudaGetLastError();
     return e == cudaSuccess ? 0 : (int)e;
 }
@@ -678,9 +627,8 @@ int launch_write_reduce_mma(const void* f, const void* labels, int lab_u8, float
     const float sy = h > 1 ? (float)(Hm - 1) / (float)(h - 1) : 0.f;
     const float sx = w > 1 ? (float)(Wm - 1) / (float)(w - 1) : 0.f;
     CUtensorMap tm_f;
-    const bool tma = tma_enabled() && make_map_2d<float>(&tm_f, f, (size_t)B * C, hw, C, 32, true);
-    auto kern = part ? (tma ? write_reduce_mma_kernel<C, KP, true, true> : write_reduce_mma_kernel<C, KP, false, true>)
-                     : (tma ? write_reduce_mma_kernel<C, KP, true> : write_reduce_mma_kernel<C, KP, false>);
+    if (!make_map_2d<float>(&tm_f, f, (size_t)B * C, hw, C, 32, true)) return PM_ERR_ALIGN;
+    auto kern = part ? write_reduce_mma_kernel<C, KP, true> : write_reduce_mma_kernel<C, KP>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
     int per_sm = 1;
@@ -694,7 +642,7 @@ int launch_write_reduce_mma(const void* f, const void* labels, int lab_u8, float
         if (grid > PM_ORD_CTAS) grid = PM_ORD_CTAS;
         SD = part, *ncta = grid;
     }
-    kern<<<grid, C, smem, st>>>(tm_f, (const float*)f, labels, lab_u8, SD, h, w, Hm, Wm, K, sy, sx, tiles, ntiles);
+    kern<<<grid, C, smem, st>>>(tm_f, labels, lab_u8, SD, h, w, Hm, Wm, K, sy, sx, tiles, ntiles);
     e = cudaGetLastError();
     return e == cudaSuccess ? 0 : (int)e;
 }
@@ -727,19 +675,17 @@ int launch_write_reduce_tiled(const void* f, const void* labels, int lab_u8, flo
 // ---------------------------------------------------------------------------- write backward (to f)
 // dv[n] = sum_taps w * dS[class]; df = (dv - v (v.dv)) / |f|, v = f/|f|. Persistent CTAs, 2 per SM (measured:
 // one 16-warp CTA with a 5-stage ring is 45% slower -- the per-tile barriers need a second CTA to hide
-// behind, bytes in flight are not the limit); the [C][32] tiles of f arrive through a 2-stage async-copy
-// ring, lanes = pixels, 8 warps split the channels,
+// behind, bytes in flight are not the limit); the [C][32] tiles of f arrive as 2-D tensor-map boxes on a
+// 2-stage mbarrier ring (one thread issues a stage), lanes = pixels, 8 warps split the channels,
 // dS sits in shared memory with row stride C+1 (lanes with different classes hit different banks). The
 // label taps of the next tile are fetched by warp 0 while the current tile is processed.
 
 constexpr int WBT_THREADS = 256, WBT_WARPS = 8, WBT_STAGES = 2;
 
-// TMA = true: the f tiles arrive as 2-D tensor-map boxes completing on one mbarrier per stage (one thread issues a
-// stage) instead of 8 LDGSTS per thread; `tm_f` is unused otherwise.
-template <typename T, int C, int KP, bool TMA>
+template <typename T, int C, int KP>
 __global__ void __launch_bounds__(WBT_THREADS, 2)
     write_bwd_tiled_kernel(const __grid_constant__ CUtensorMap tm_f, const float* __restrict__ dS,
-                           const T* __restrict__ f, const void* __restrict__ labels, int lab_u8,
+                           const void* __restrict__ labels, int lab_u8,
                            T* __restrict__ df, int h, int w, int Hm, int Wm, int K, float sy, float sx,
                            int tiles_per_img, int ntiles) {
     constexpr int NSTAGE = WBT_STAGES, CW = C / WBT_WARPS, LDS_ = C + 1;
@@ -776,32 +722,19 @@ __global__ void __launch_bounds__(WBT_THREADS, 2)
     };
 
     int tile = blockIdx.x;
-    auto issue = [&](int t, int s) {  // TMA: one thread
+    auto issue = [&](int t, int s) {  // one thread
         int b, px0;
         tile_coords(t, b, px0);
         mbar_expect_tx(&full[s], (uint32_t)(C * 32 * sizeof(T)));
         tma_load_2d(ft + s * C * 32, &tm_f, px0, b * C, &full[s]);
     };
-    if constexpr (TMA) {
-        if (tid == 0) {
+    if (tid == 0) {
 #pragma unroll
-            for (int s = 0; s < NSTAGE; ++s) mbar_init(&full[s], 1);
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        for (int s = 0; s < NSTAGE; ++s) mbar_init(&full[s], 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 #pragma unroll
-            for (int s = 0; s < NSTAGE; ++s)
-                if (tile + s * (int)gridDim.x < ntiles) issue(tile + s * gridDim.x, s);
-        }
-    } else {
-#pragma unroll
-        for (int s = 0; s < NSTAGE; ++s) {
-            const int t = tile + s * gridDim.x;
-            if (t < ntiles) {
-                int b, px0;
-                tile_coords(t, b, px0);
-                tile_load_async<T, C, WBT_THREADS>(ft + s * C * 32, f + (size_t)b * C * hw, hw, px0);
-            }
-            cp_async_commit();
-        }
+        for (int s = 0; s < NSTAGE; ++s)
+            if (tile + s * (int)gridDim.x < ntiles) issue(tile + s * gridDim.x, s);
     }
     for (int i = tid; i < KP * LDS_; i += WBT_THREADS) {
         const int k = i / LDS_, c = i - k * LDS_;
@@ -818,9 +751,8 @@ __global__ void __launch_bounds__(WBT_THREADS, 2)
     for (; tile < ntiles; tile += gridDim.x) {
         LabelTaps tn;
         if (wid == 0) tn = taps_for(tile + gridDim.x);  // loads in flight across this tile
-        if constexpr (!TMA) cp_async_wait<NSTAGE - 1>();
-        __syncthreads();  // dS / tap entries of this tile visible (and, with cp.async, the tile itself)
-        if constexpr (TMA) mbar_wait(&full[stage], phase);
+        __syncthreads();  // dS / tap entries of this tile visible
+        mbar_wait(&full[stage], phase);
         const T* xt = ft + stage * C * 32;
         int b, px0;
         tile_coords(tile, b, px0);
@@ -875,16 +807,7 @@ __global__ void __launch_bounds__(WBT_THREADS, 2)
         }
         __syncthreads();  // stage, entries and pn/pd consumed
         const int next = tile + NSTAGE * gridDim.x;
-        if constexpr (TMA) {
-            if (tid == 0 && next < ntiles) issue(next, stage);
-        } else {
-            if (next < ntiles) {
-                int nb, npx0;
-                tile_coords(next, nb, npx0);
-                tile_load_async<T, C, WBT_THREADS>(ft + stage * C * 32, f + (size_t)nb * C * hw, hw, npx0);
-            }
-            cp_async_commit();
-        }
+        if (tid == 0 && next < ntiles) issue(next, stage);
         if (wid == 0) {
             compact_taps(tn);
             store_entries(ebuf ^ 1, tn);
@@ -892,7 +815,6 @@ __global__ void __launch_bounds__(WBT_THREADS, 2)
         if (++stage == NSTAGE) stage = 0, phase ^= 1u;
         ebuf ^= 1;
     }
-    if constexpr (!TMA) cp_async_wait<0>();
 }
 
 template <typename T, int C, int KP>
@@ -906,20 +828,11 @@ int launch_write_bwd_tiled(const float* dS, const void* f, const void* labels, i
     const float sy = h > 1 ? (float)(Hm - 1) / (float)(h - 1) : 0.f;
     const float sx = w > 1 ? (float)(Wm - 1) / (float)(w - 1) : 0.f;
     CUtensorMap tm_f;
-    cudaError_t e;
-    if (tma_enabled() && make_map_2d<T>(&tm_f, f, (size_t)B * C, hw, C, 32, false)) {
-        auto kern = write_bwd_tiled_kernel<T, C, KP, true>;
-        e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return (int)e;
-        kern<<<grid, WBT_THREADS, smem, st>>>(tm_f, dS, (const T*)f, labels, lab_u8, (T*)df, h, w, Hm, Wm, K, sy,
-                                              sx, tiles, ntiles);
-    } else {
-        auto kern = write_bwd_tiled_kernel<T, C, KP, false>;
-        e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return (int)e;
-        kern<<<grid, WBT_THREADS, smem, st>>>(tm_f, dS, (const T*)f, labels, lab_u8, (T*)df, h, w, Hm, Wm, K, sy,
-                                              sx, tiles, ntiles);
-    }
+    if (!make_map_2d<T>(&tm_f, f, (size_t)B * C, hw, C, 32, false)) return PM_ERR_ALIGN;
+    auto kern = write_bwd_tiled_kernel<T, C, KP>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return (int)e;
+    kern<<<grid, WBT_THREADS, smem, st>>>(tm_f, dS, labels, lab_u8, (T*)df, h, w, Hm, Wm, K, sy, sx, tiles, ntiles);
     e = cudaGetLastError();
     return e == cudaSuccess ? 0 : (int)e;
 }

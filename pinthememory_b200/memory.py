@@ -85,8 +85,6 @@ class _ReadFn(torch.autograd.Function):
 
     last_bad = None   # device int64 scalar: label values outside [0,K) u {255} seen by the last read with labels
     last_lab8 = None  # the packed uint8 class map that read produced (None when the first-generation kernel ran)
-    pack_event = None  # recorded behind the label pass when it ran on the read's own stream and want_pack_event is set
-    want_pack_event = False
 
     @staticmethod
     def forward(ctx, x, M, labels, g_query, g_memory, temperature, K, planes=False, tee=False, branch=False):
@@ -149,12 +147,8 @@ class _ReadFn(torch.autograd.Function):
                 capi.readloss_fwd8(s, lab8, temperature, B, h, w, K, ds_rl, ws, rl_out)
                 _ReadFn.last_lab8 = lab8
             elif use_pack and x.is_cuda:
-                # one pass over the labels (packed uint8 classes + histogram + bad-label count), then the read loss on it; the
-                # event lets a write branch on another stream wait for exactly the pack (Memory_sup._forward_two_streams)
+                # one pass over the labels (packed uint8 classes + histogram + bad-label count), then the read loss on it
                 lab8 = capi.labels_pack(labels, K, ws)
-                if _ReadFn.want_pack_event:
-                    _ReadFn.pack_event = torch.cuda.Event()
-                    _ReadFn.pack_event.record(torch.cuda.current_stream(dev))
                 capi.readloss_fwd8(s, lab8, temperature, B, h, w, K, ds_rl, ws, rl_out)
                 _ReadFn.last_lab8 = lab8
             else:
@@ -395,7 +389,7 @@ class _ConvBnActFn(torch.autograd.Function):
         stats = None
         if pre is not None and pre[0][0].dtype != x.dtype:
             pre = None                # prepared for another compute dtype (autocast): redo it here
-        ctx.w_on_aux = pre is not None and not os.environ.get("PINMEM_B200_NO_WGRAD_BRANCH")
+        ctx.w_on_aux = pre is not None
         if pre is not None:           # operands (and the cleared statistics buffer) prepared ahead of time on a side stream
             (hi, lo), ctx.preT, stats = pre
             if not use_batch_stats:
@@ -472,8 +466,7 @@ class _ConvBnActFn(torch.autograd.Function):
             dist.all_reduce(sums, group=ctx.sync_group)
             sums = sums * (float(xc.shape[0] * xc.shape[2] * xc.shape[3]) / count).to(torch.float32)
             sg, sb = sums[:M].contiguous(), sums[M:].contiguous()
-        if (need_x and not ctx.has_res and xc.dtype == torch.float32 and M % 32 == 0 and ctx.beta32 is not None
-                and not os.environ.get("PINMEM_B200_NO_BNBWD_FUSION")):
+        if need_x and not ctx.has_res and xc.dtype == torch.float32 and M % 32 == 0 and ctx.beta32 is not None:
             # blocks without a residual (self.output): the BatchNorm backward rides in the operand path of the
             # input-gradient GEMM, which also stores dz for the weight-gradient GEMM -- no bn_bwd_apply pass
             hiT, loT = ctx.preT if ctx.preT is not None else capi.conv1x1_prep(W2, True, x.dtype)
@@ -605,14 +598,14 @@ def _inference_block(bn, x, residual):
     """conv + eval-mode BN (+ ReLU) can run as ONE kernel: no batch statistics, no residual, nothing to differentiate."""
     return (_bn_fast(bn, x) and not bn.training and bn.running_mean is not None and residual is None
             and not torch.is_grad_enabled() and bn.running_mean.dtype == torch.float32
-            and bn.running_var.dtype == torch.float32 and not os.environ.get("PINMEM_B200_LIBRARY_CONV"))
+            and bn.running_var.dtype == torch.float32)
 
 
 def _weight_bn_act(W, bn, x, residual, relu, prepared=None, affine=None, pre=None):
     if torch.is_autocast_enabled("cuda"):  # the nn.Conv2d this replaces would run in the autocast dtype
         x = x.to(torch.get_autocast_dtype("cuda"))
     M, K = W.shape[0], W.shape[1]
-    if _bn_fast(bn, x) and capi.conv1x1_ok(x, M, K) and not os.environ.get("PINMEM_B200_LIBRARY_CONV"):
+    if _bn_fast(bn, x) and capi.conv1x1_ok(x, M, K):
         x = x.contiguous()
         if _inference_block(bn, x, residual):
             # inference read (BASELINE config 5): the eval-mode BatchNorm and the ReLU ride in the GEMM epilogue
@@ -707,8 +700,7 @@ class Memory_sup(nn.Module):
         # extras (not in the reference)
         self.overlap_write = False     # run the write branch on a side stream next to the read (see forward)
         self.fold_memory_into_conv = True  # read hands [q ; score planes] to a convolution with the memory folded in
-        # the write branch's d/d(query) is summed inside the read's dx kernel (see read()); env switch for A/B runs
-        self.fuse_grad_sum = not os.environ.get("PINMEM_B200_NO_GRAD_SUM_FUSION")
+        self.fuse_grad_sum = True      # the write branch's d/d(query) is summed inside the read's dx kernel (see read())
         self.fold_min_pixels = 32768       # ... for feature maps of at least this many pixels per call
         self.shard_group = None        # set by sharding.enable_sharded_update()
         self.last_label_hist = None    # int64 [K+1] label histogram of the last read with labels
@@ -742,17 +734,7 @@ class Memory_sup(nn.Module):
         memory_in = self.m_items
         # the read's label pass runs on `side` too (before the write kernels that consume the packed map: stream order is
         # the dependency), its column softmax on a second side stream
-        self._branch_read = not os.environ.get("PINMEM_B200_NO_READ_BRANCHES")
-        _ReadFn.want_pack_event, _ReadFn.pack_event = not self._branch_read, None
-        try:
-            updated_query, score_query, score_memory, readloss = self.read(query, mask, True, _tee=True)   # main stream
-        finally:
-            branched, self._branch_read = self._branch_read, False
-            _ReadFn.want_pack_event = False
-        # (not branched: the packed label map is produced on the main stream; the write kernels that read it wait for the
-        # event recorded behind the pass -- see write())
-        self._pack_event = None if branched else _ReadFn.pack_event
-        _ReadFn.pack_event = None
+        updated_query, score_query, score_memory, readloss = self.read(query, mask, True, _tee=True, _branch=True)
         memory_after_read = self.m_items          # the detached view read() installed (memory.py:323-324)
         tee, self._tee = getattr(self, "_tee", None), None
         with torch.cuda.stream(side):
@@ -798,7 +780,7 @@ class Memory_sup(nn.Module):
             raise RuntimeError(f"pinmem_b200: m_items must be [{self.memory_size},{self.feature_dim}]")
         return M
 
-    def read(self, query, mask, memory_writing, _tee=False):
+    def read(self, query, mask, memory_writing, _tee=False, _branch=False):
         """memory.py:317-336. Returns (updated_query, score_query, score_memory, readloss)."""
         query = _check_features(query, "query")
         B, C, h, w = query.shape
@@ -823,8 +805,7 @@ class Memory_sup(nn.Module):
         # their three small kernels run on a side stream -- a parallel branch of a captured graph -- under the read kernels
         # instead of between them and the convolution (27 us of a 108 us step at one 1024x2048 image per GPU)
         pre = None
-        if (planes and _inference_block(self.output[1], query, None) and query.dtype in (torch.float32, torch.bfloat16)
-                and not os.environ.get("PINMEM_B200_NO_INFER_BRANCH")):
+        if planes and _inference_block(self.output[1], query, None) and query.dtype in (torch.float32, torch.bfloat16):
             cur = torch.cuda.current_stream(query.device)
             side = _SIDE_STREAMS.get(query.device)
             if side is None:
@@ -839,11 +820,9 @@ class Memory_sup(nn.Module):
         # clear the statistics buffer: two small launches) depends on parameters only -- it runs on the second side stream
         # under read_fwd instead of between the read loss and the convolution
         wpre = None
-        branch = bool(getattr(self, "_branch_read", False))
-        if (branch and planes and pre is None and torch.is_grad_enabled() and self.output[1].training
+        if (_branch and planes and pre is None and torch.is_grad_enabled() and self.output[1].training
                 and _bn_fast(self.output[1], query) and query.dtype in (torch.float32, torch.bfloat16)
-                and capi.conv1x1_ok(query, self.output[0].weight.shape[0], C + capi.PLANES)
-                and not os.environ.get("PINMEM_B200_LIBRARY_CONV")):
+                and capi.conv1x1_ok(query, self.output[0].weight.shape[0], C + capi.PLANES)):
             cur = torch.cuda.current_stream(query.device)
             aux = _stream_of(_AUX_STREAMS, query.device)
             aux.wait_stream(cur)
@@ -859,7 +838,7 @@ class Memory_sup(nn.Module):
                 if torch.is_tensor(t):
                     t.record_stream(cur)
         outs = _ReadFn.apply(query, M, labels, g_query, g_memory, float(self.temperature), self.memory_size, planes, tee,
-                             branch)
+                             _branch)
         if wpre is not None:   # (a branched _ReadFn joins the aux stream itself; this covers the read without labels / K > 19)
             torch.cuda.current_stream(query.device).wait_stream(_stream_of(_AUX_STREAMS, query.device))
         u, score_query, score_memory, readloss, hist = outs[:5]
@@ -879,9 +858,9 @@ class Memory_sup(nn.Module):
         if planes:
             # conv(W, [q ; p.M]) = W1.q + (W2.M^T).p : the memory is folded into the weight (a [C_out, 32] block) and
             # the convolution runs on [q ; score planes] -- C+32 input channels instead of 2C
-            infer = (_inference_block(self.output[1], u, None)
-                     and capi.conv1x1_ok(u, self.output[0].weight.shape[0], C + capi.PLANES))
-            prepared = (pre[0] if pre is not None else self._inference_weights(M, u)) if infer else None
+            # (`pre` exists exactly when this is an inference block: u has the query's device, rank and dtype)
+            infer = pre is not None and capi.conv1x1_ok(u, self.output[0].weight.shape[0], C + capi.PLANES)
+            prepared = pre[0] if infer else None
             if prepared is not None:
                 Wp = self._folded_shape
             elif wpre is not None:
@@ -889,7 +868,7 @@ class Memory_sup(nn.Module):
             else:
                 Wp = _FoldWeightFn.apply(self.output[0].weight, M)
             updated_query = weight_bn_act(Wp, self.output[1], u, None, True, "output", prepared,   # Wp [C_out, C+32, 1, 1]
-                                          pre[1] if (pre is not None and infer) else None,
+                                          pre[1] if infer else None,
                                           wpre[1] if (wpre is not None and prepared is None) else None)
         elif plain:
             updated_query = conv_bn_act(self.output[0], self.output[1], u, None, True, "output")
@@ -910,9 +889,6 @@ class Memory_sup(nn.Module):
         self._packed = None
         f = self.writenet(query)
         f = _check_features(f, "write feature")
-        ev, self._pack_event = getattr(self, "_pack_event", None), None
-        if ev is not None and labels.dtype == torch.uint8 and packed is not None:
-            torch.cuda.current_stream(query.device).wait_event(ev)   # two-stream mode: the packed map comes from the read's stream
         M_old = self._memory_for_kernels(query.device)
         if M_old.requires_grad and torch.is_grad_enabled():
             # memory.py:236 blends the NON-detached self.m_items[slot]; forward() never gets here with a grad-carrying

@@ -34,7 +34,7 @@ for _ in range(50):
     step()
 b.record()
 torch.cuda.synchronize()
-print("PM_TMA=%s core step: gpu %.3f ms, host %.3f ms" % (os.environ.get("PM_TMA", "1"), a.elapsed_time(b) / 50, (time.perf_counter() - t0) * 1e3 / 50))
+print("core step: gpu %.3f ms, host %.3f ms" % (a.elapsed_time(b) / 50, (time.perf_counter() - t0) * 1e3 / 50))
 capi.enable_kernel_timing(True)
 capi.reset_counters()
 for _ in range(20):

@@ -110,18 +110,11 @@ def test_graphed_gumbel_read_draws_fresh_noise_each_replay():
     assert_close(a.sum(-1), torch.ones_like(a.sum(-1)), 1e-5, "rows sum to one")
 
 
-@pytest.mark.parametrize("branches", [True, False])
 @pytest.mark.parametrize("graphed", [False, True])
-def test_two_stream_forward_matches_single_stream(graphed, branches, monkeypatch):
-    """overlap_write: the write branch on a side stream (a parallel branch when captured) changes nothing -- with the read's
-    own branches (label pass on the write stream, column softmax / weight work on a second side stream) and without them
-    (PINMEM_B200_NO_READ_BRANCHES: the write waits for an event recorded behind the label pass)."""
+def test_two_stream_forward_matches_single_stream(graphed):
+    """overlap_write: the write branch on a side stream (a parallel branch when captured) changes nothing, with the read's
+    own branches (label pass on the write stream, column softmax / weight work on a second side stream)."""
     from pinthememory_b200.graphed import GraphedStep
-
-    if branches:
-        monkeypatch.delenv("PINMEM_B200_NO_READ_BRANCHES", raising=False)
-    else:
-        monkeypatch.setenv("PINMEM_B200_NO_READ_BRANCHES", "1")
 
     B, C, h, w, Hm, Wm, K = 2, 64, 12, 16, 48, 64, 19
     plain, forked = _pair(K, C)
