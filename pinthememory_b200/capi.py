@@ -453,11 +453,12 @@ def conv1x1_prep_both(W2d, dtype, zero=None):
 
 
 def conv1x1_ok(x, M, K):
-    """Shapes/alignments the tcgen05 GEMMs take (everything the module produces on aligned feature maps)."""
+    """Shapes/alignments the tcgen05 GEMMs take (everything the module produces on aligned feature maps). The block's
+    input-gradient GEMM has K output rows, so K is held to the same 512-row limit as M."""
     hw = x.shape[2] * x.shape[3]
     esz = 4 if x.dtype == torch.float32 else 2
     return (x.is_cuda and x.dtype in (torch.float32, torch.bfloat16) and (hw * esz) % 16 == 0 and x.data_ptr() % 16 == 0
-            and K % (8 if esz == 4 else 16) == 0 and M % 32 == 0 and M <= 512 and K % 32 == 0 and K <= 1024)
+            and K % (8 if esz == 4 else 16) == 0 and M % 32 == 0 and M <= 512 and K % 32 == 0 and K <= 512)
 
 
 def conv1x1_fwd(x, A_hi, A_lo, M, y=None, stats=None, accumulate=False):
