@@ -54,7 +54,7 @@ enum pm_readloss_ws_layout {
 #define PM_COLPART_ROWS 296
 
 /* Bumped with every prototype change; the binding refuses a library whose pm_version() differs. */
-#define PM_ABI_VERSION 210
+#define PM_ABI_VERSION 211
 int pm_version(void);
 const char* pm_status_string(int code);
 /* Row stride (floats) of the internal score buffers for K slots: 20 for K<=19, else 32. */
@@ -111,6 +111,9 @@ int pm_readloss_fwd(const float* s, const int64_t* labels, float temperature, in
  *   x, M, score_m                  as in the forward (score_m carries the gumbel noise implicitly)
  *   ds_rl    [N,stride] fp32 or NULL; g_loss: device float* (upstream grad of readloss) or NULL;
  *   rl_out   the `out` array of pm_readloss_fwd (its [1] is the scale) or NULL
+ *            ds_rl is an additive [N,stride] term of the similarity gradient, scaled by g_loss[0] * rl_out[1]. When
+ *            score_query / score_memory carry gradients too, the caller passes the E of pm_score_bwd here (which already
+ *            holds the scaled read-loss term) with g_loss[0] = rl_out[1] = 1: a unit scale.
  *   dx       [B,C,h,w] dtype out
  *   ds       [N,stride] fp32 out or NULL: total gradient w.r.t. the similarities (input of pm_read_bwd_dM).
  *            Pass a buffer: the pipelined two-kernel path (score gradients, then dx) needs it as scratch;
@@ -170,6 +173,38 @@ int pm_score_nhwc(const float* q, const float* M, float* s, int N, int C, int K,
  * score_memory for that external get_score path: dense [N,K] row softmax of s (+ gumbel_m), memory.py:184/187.
  */
 int pm_rowsoftmax(const float* s, const float* gumbel_m, float* score_m, int N, int K, void* stream);
+
+/*
+ * Backward of the two score softmaxes: autograd of memory.py:181-187 (score_query = [gumbel-]softmax over all pixels of
+ * s, score_memory = [gumbel-]softmax over slots) for the read (memory.py:171,181-187) and for get_score (:167-189). The
+ * noise only shifts the inputs, so with and without it:
+ *   E[n,k] = p_m[n,k] (g_m[n,k] - sum_j p_m[n,j] g_m[n,j]) + p_q[n,k] (g_q[n,k] - c[k]) + g_loss[0] * rl_out[1] * ds_rl[n,k]
+ *   with c[k] = sum_n p_q[n,k] g_q[n,k] over all N pixels of the call.
+ *   score_q, g_q   [N,K] fp32 (score_query and its upstream gradient), both NULL: no column term
+ *   score_m, g_m   [N,K] fp32 (score_memory and its upstream gradient), both NULL: no row term
+ *   ds_rl, g_loss, rl_out   as in pm_read_bwd (all three or the term is absent)
+ *   E         [N,stride] fp32 out, 16-byte aligned; columns k >= K are written as zero. E is the gradient with respect to
+ *             the similarities s; pass it to pm_read_bwd[_planes] as ds_rl with a unit scale, or to pm_score_nhwc_bwd.
+ *   workspace pm_score_bwd_workspace_floats(K) floats, 8-byte aligned, contents on entry irrelevant (needed when g_q).
+ * Two launches (the column sums, then the element-wise pass; the first only with g_q). c is summed in fp64 in a fixed
+ * order: the result is bitwise reproducible on one GPU model, with or without torch's deterministic flag.
+ */
+int pm_score_bwd_workspace_floats(int K);
+int pm_score_bwd(const float* score_q, const float* g_q, const float* score_m, const float* g_m, const float* ds_rl,
+                 const float* g_loss, const float* rl_out, float* E, float* workspace, int N, int K, void* stream);
+
+/*
+ * Backward of pm_score_nhwc (get_score's s = q.M^T, memory.py:171 as called at :167-189; no normalisation: get_score
+ * takes an already normalised query).
+ *   q [N,C] fp32, M [K,C] fp32, E [N,stride] fp32 (from pm_score_bwd; 16-byte aligned)
+ *   dq [N,C] fp32 out or NULL: dq[n,:] = sum_k E[n,k] M[k,:]
+ *   dM [K,C] fp32 or NULL: dM += E^T.q (ADDED into: zero it first); per-CTA partials added in CTA order, no atomics
+ *   scratch: pm_score_nhwc_bwd_scratch_bytes(N, C, K) bytes, 16-byte aligned, contents on entry irrelevant (needed with dM)
+ * C <= 2048, K 1..31.
+ */
+int pm_score_nhwc_bwd_scratch_bytes(int N, int C, int K);
+int pm_score_nhwc_bwd(const float* q, const float* M, const float* E, float* dq, float* dM, float* scratch, int N, int C,
+                      int K, void* stream);
 
 /*
  * Memory write, class sums. Replaces memory.py:215 (normalise), :220-223 (255->K, one_hot(K+1),

@@ -19,7 +19,7 @@ WS_BAD = 2     # PM_WS_BAD
 SEG_WS_WORDS = 4  # PM_SEG_WS_WORDS
 SEG_WS_BAD = 2    # PM_SEG_WS_BAD
 
-ABI_VERSION = 210  # PM_ABI_VERSION of include/pinmem_b200.h the argtypes below were written against
+ABI_VERSION = 211  # PM_ABI_VERSION of include/pinmem_b200.h the argtypes below were written against
 
 _c_p = ctypes.c_void_p
 _c_i = ctypes.c_int
@@ -87,6 +87,10 @@ PROTOTYPES = {
     "pm_read_bwd_dM_ordered": [_c_p] * 6 + [_c_i] * 6 + [_c_p],
     "pm_conv1x1_stats_scratch_bytes": [_c_i] * 4,
     "pm_conv1x1_fwd_ordered": [_c_p] * 6 + [_c_i] * 5 + [_c_p],
+    "pm_score_bwd_workspace_floats": [_c_i],
+    "pm_score_bwd": [_c_p] * 9 + [_c_i] * 2 + [_c_p],
+    "pm_score_nhwc_bwd_scratch_bytes": [_c_i] * 3,
+    "pm_score_nhwc_bwd": [_c_p] * 6 + [_c_i] * 3 + [_c_p],
 }
 EXPORTED_SYMBOLS = sorted(list(PROTOTYPES) + ["pm_status_string"])
 
@@ -201,7 +205,8 @@ def score_stride(K):
 LAUNCHES = 0
 _KERNELS_PER_CALL = {"pm_readloss_fwd_ordered": 2, "pm_readloss_fwd8_ordered": 2, "pm_write_reduce_fwd_ordered": 2,
                      "pm_write_reduce_fwd8_ordered": 2, "pm_read_bwd_dM_ordered": 2, "pm_conv1x1_fwd_ordered": 2,
-                     "pm_conv1x1_dgrad_bnbwd": 2, "pm_colsoftmax": 3, "pm_colsoftmax_apply": 1, "pm_read_bwd": 2, "pm_read_bwd_planes": 2, "pm_conv1x1_wgrad": 2}
+                     "pm_conv1x1_dgrad_bnbwd": 2, "pm_colsoftmax": 3, "pm_colsoftmax_apply": 1, "pm_read_bwd": 2, "pm_read_bwd_planes": 2, "pm_conv1x1_wgrad": 2,
+                     "pm_score_bwd": 2, "pm_score_nhwc_bwd": 2}
 PLANES = 32  # PM_PLANES: score planes appended to q in the score-plane read
 _timing = None  # name -> list of (start_event, end_event) when enabled
 
@@ -331,6 +336,26 @@ def score_nhwc(q, M, s, N, C, K):
 
 def rowsoftmax(s, gumbel_m, score_m, N, K):
     _call("pm_rowsoftmax", _ptr(s), _ptr(gumbel_m), _ptr(score_m), N, K, _stream())
+
+
+def score_bwd(score_q, g_q, score_m, g_m, E, K, ds_rl=None, g_loss=None, rl_out=None):
+    """E [N,stride] = gradient w.r.t. the similarities of the two score softmaxes (either pair may be None) plus the scaled
+    read-loss term; score / gradient tensors are contiguous fp32 [N,K]. Order-fixed: two launches, no float atomics."""
+    N = E.shape[0]
+    ws = None
+    if g_q is not None:
+        ws = torch.empty(load().pm_score_bwd_workspace_floats(int(K)), dtype=torch.float32, device=E.device)
+    _call("pm_score_bwd", _ptr(score_q), _ptr(g_q), _ptr(score_m), _ptr(g_m), _ptr(ds_rl), _ptr(g_loss), _ptr(rl_out), _ptr(E),
+          _ptr(ws), N, K, _stream())
+
+
+def score_nhwc_bwd(q, M, E, dq, dM, K):
+    """dq [N,C] = E.M (or None), dM [K,C] += E^T.q (or None; partials added in CTA order)."""
+    N, C = q.shape
+    scratch = None
+    if dM is not None:
+        scratch = _scratch(load().pm_score_nhwc_bwd_scratch_bytes(N, C, K), q.device, "pm_score_nhwc_bwd_scratch_bytes")
+    _call("pm_score_nhwc_bwd", _ptr(q), _ptr(M), _ptr(E), _ptr(dq), _ptr(dM), _ptr(scratch), N, C, K, _stream())
 
 
 def write_reduce_fwd(f, labels, SD, K):

@@ -110,7 +110,7 @@ class GraphedStep:
             # after the backward: the read's saved memory IS self.memory
             self.memory.copy_(new_memory)
             new_memory = self.memory
-        return {"updated_query": uq.detach(), "score_query": sq, "score_memory": sm,
+        return {"updated_query": uq.detach(), "score_query": sq.detach(), "score_memory": sm.detach(),
                 "readloss": rl.detach() if torch.is_tensor(rl) else rl,
                 "writeloss": [w.detach() if torch.is_tensor(w) else w for w in wl],
                 "memory": new_memory}

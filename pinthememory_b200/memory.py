@@ -163,18 +163,21 @@ class _ReadFn(torch.autograd.Function):
         ctx.K, ctx.planes, ctx.UC = K, planes, UC
         ctx.has_loss = labels is not None
         ctx.set_materialize_grads(False)  # unused outputs (scores, histogram) arrive as None, not as zero fills
-        ctx.save_for_backward(x, M, score_m, ds_rl, rl_out)
-        ctx.mark_non_differentiable(score_q, score_m, hist)
+        # score_q is kept for the gradient of score_query (N*K*4 bytes, 5.6 MB at cfg 2: the one cost of differentiable
+        # scores on a step that does not use them)
+        ctx.save_for_backward(x, M, score_m, ds_rl, rl_out, score_q)
+        ctx.mark_non_differentiable(hist)
         if branch:
             cur.wait_stream(aux)                       # join: score_query is ready for whoever reads it on this stream
         outs = (u, score_q.view(B, h, w, K), score_m.view(B, h, w, K), readloss, hist)
         return outs + (x,) if tee else outs
 
     @staticmethod
-    def backward(ctx, du, _g_sq, _g_sm, g_loss, _g_hist, g_tee=None):
-        x, M, score_m, ds_rl, rl_out = ctx.saved_tensors
+    def backward(ctx, du, g_sq, g_sm, g_loss, _g_hist, g_tee=None):
+        x, M, score_m, ds_rl, rl_out, score_q = ctx.saved_tensors
         B, C, h, w = x.shape
         K = ctx.K
+        N = B * h * w
         need_dM = ctx.needs_input_grad[1]
         if du is None:
             du = torch.zeros(B, ctx.UC, h, w, dtype=x.dtype, device=x.device)
@@ -183,11 +186,21 @@ class _ReadFn(torch.autograd.Function):
             g_loss = g_loss.to(torch.float32).contiguous()
         else:
             g_loss = None
+        if g_loss is None:
+            ds_rl = rl_out = None
+        if g_sq is not None or g_sm is not None:
+            # gradients of score_query / score_memory: their softmax backward (plus the scaled read-loss term) forms one
+            # additive similarity gradient E, which the read backward takes in place of ds_rl with a unit scale
+            dense = lambda g: None if g is None else g.reshape(N, K).to(torch.float32).contiguous()
+            E = torch.empty(N, capi.score_stride(K), dtype=torch.float32, device=x.device)
+            capi.score_bwd(score_q if g_sq is not None else None, dense(g_sq), score_m if g_sm is not None else None,
+                           dense(g_sm), E, K, ds_rl=ds_rl, g_loss=g_loss, rl_out=rl_out)
+            ds_rl = E
+            g_loss = rl_out = torch.ones(2, dtype=torch.float32, device=x.device)
         dx = torch.empty_like(x)
-        ds = torch.empty(B * h * w, capi.score_stride(K), dtype=torch.float32, device=x.device)
+        ds = torch.empty(N, capi.score_stride(K), dtype=torch.float32, device=x.device)
         fused_add = g_tee is not None and ctx.planes and g_tee.dtype == x.dtype and g_tee.shape == x.shape
-        capi.read_bwd(du, x, M, score_m, ds_rl if g_loss is not None else None, g_loss,
-                      rl_out if g_loss is not None else None, dx, ds, K, planes=ctx.planes,
+        capi.read_bwd(du, x, M, score_m, ds_rl, g_loss, rl_out, dx, ds, K, planes=ctx.planes,
                       dx_add=g_tee.contiguous() if fused_add else None)
         if g_tee is not None and not fused_add:
             dx = dx + g_tee.to(dx.dtype)
@@ -918,36 +931,96 @@ class Memory_sup(nn.Module):
     def get_score(self, query, mask, mem):
         """memory.py:167-189 on an already normalised NHWC query (validation, train.py:891-896).
 
-        Forward only (the reference calls it under ``no_grad``): returns
-        (score_query [N,K], score_memory [N,K], readloss).
+        Returns (score_query [N,K], score_memory [N,K], readloss), readloss the int 0 without labels. As in the reference,
+        all three are differentiable with respect to ``query`` and ``mem`` when either requires grad (and grad mode is on);
+        otherwise the same kernels run without saving anything for a backward.
         """
         capi.require_cuda(query, mem)
-        Bq, h, w, C = query.shape
-        K = mem.shape[0]
-        N = Bq * h * w
-        dev = query.device
-        with torch.no_grad():
-            q = query.detach().to(torch.float32).contiguous()
-            M = mem.detach().to(torch.float32).contiguous()
-            KP = capi.score_stride(K)
-            s = (torch.zeros if capi.deterministic() else torch.empty)(N, KP, dtype=torch.float32, device=dev)   # (see _ReadFn)
-            capi.score_nhwc(q, M, s, N, C, K)
-            if mask is not None:
-                labels = _check_labels(mask, Bq)
-                buf = torch.zeros(N * KP + 2 * capi.WS_WORDS + 4, dtype=torch.float32, device=dev)
-                ws = buf[N * KP: N * KP + 2 * capi.WS_WORDS]
-                rl_out = buf[N * KP + 2 * capi.WS_WORDS:]
-                capi.readloss(s, labels, float(self.temperature), Bq, h, w, K, buf[: N * KP], ws, rl_out)
-                readloss = rl_out[0]
-                self.last_label_hist = ws.view(torch.int64)[capi.WS_HIST: capi.WS_HIST + K + 1]
-            else:
-                readloss = 0
-            g_query = g_memory = None
-            if self.gumbel_read:
-                g_query, g_memory = draw_gumbel_pair(N, K, dev)
-            score_query = torch.empty(N, K, dtype=torch.float32, device=dev)
-            score_memory = torch.empty(N, K, dtype=torch.float32, device=dev)
-            cs_ws = torch.empty(capi.colsoftmax_workspace_floats(K), dtype=torch.float32, device=dev)
-            capi.colsoftmax(s, g_query, score_query, cs_ws, N, K)
-            capi.rowsoftmax(s, g_memory, score_memory, N, K)
+        Bq = query.shape[0]
+        labels = _check_labels(mask, Bq) if mask is not None else None
+        if torch.is_grad_enabled() and (query.requires_grad or mem.requires_grad):
+            score_query, score_memory, readloss = _ScoreFn.apply(query, mem, labels, float(self.temperature), self.gumbel_read)
+            hist = _ScoreFn.last_hist
+        else:
+            with torch.no_grad():
+                score_query, score_memory, readloss, hist = _score_kernels(
+                    query.detach().to(torch.float32).contiguous(), mem.detach().to(torch.float32).contiguous(), labels,
+                    float(self.temperature), self.gumbel_read)[:4]
+        if labels is not None:
+            self.last_label_hist = hist
+        return score_query, score_memory, (readloss if labels is not None else 0)
+
+
+def _score_kernels(q, M, labels, temperature, gumbel):
+    """The kernels of get_score on a contiguous fp32 NHWC query [B,h,w,C] and memory [K,C]. Returns (score_query,
+    score_memory, readloss, label histogram, ds_rl, rl_out); the last four are None without labels."""
+    Bq, h, w, C = q.shape
+    K = M.shape[0]
+    N = Bq * h * w
+    dev = q.device
+    KP = capi.score_stride(K)
+    s = (torch.zeros if capi.deterministic() else torch.empty)(N, KP, dtype=torch.float32, device=dev)   # (see _ReadFn)
+    capi.score_nhwc(q, M, s, N, C, K)
+    readloss = hist = ds_rl = rl_out = None
+    if labels is not None:
+        buf = torch.zeros(N * KP + 2 * capi.WS_WORDS + 4, dtype=torch.float32, device=dev)
+        ws = buf[N * KP: N * KP + 2 * capi.WS_WORDS]
+        ds_rl, rl_out = buf[: N * KP], buf[N * KP + 2 * capi.WS_WORDS:]
+        capi.readloss(s, labels, temperature, Bq, h, w, K, ds_rl, ws, rl_out)
+        readloss = rl_out[0]
+        hist = ws.view(torch.int64)[capi.WS_HIST: capi.WS_HIST + K + 1]
+    g_query = g_memory = None
+    if gumbel:
+        g_query, g_memory = draw_gumbel_pair(N, K, dev)
+    score_query = torch.empty(N, K, dtype=torch.float32, device=dev)
+    score_memory = torch.empty(N, K, dtype=torch.float32, device=dev)
+    cs_ws = torch.empty(capi.colsoftmax_workspace_floats(K), dtype=torch.float32, device=dev)
+    capi.colsoftmax(s, g_query, score_query, cs_ws, N, K)
+    capi.rowsoftmax(s, g_memory, score_memory, N, K)
+    return score_query, score_memory, readloss, hist, ds_rl, rl_out
+
+
+class _ScoreFn(torch.autograd.Function):
+    """get_score with its autograd: query [B,h,w,C], mem [K,C] -> score_query, score_memory [N,K], readloss.
+
+    Backward: E = pm_score_bwd (both softmaxes and the read loss), then dq = E.M and dM = E^T.q (pm_score_nhwc_bwd). There is
+    no normalisation to differentiate: get_score takes the query as it is."""
+
+    last_hist = None  # the label histogram of the last call with labels
+
+    @staticmethod
+    def forward(ctx, query, mem, labels, temperature, gumbel):
+        q = query.detach().to(torch.float32).contiguous()
+        M = mem.detach().to(torch.float32).contiguous()
+        score_query, score_memory, readloss, _ScoreFn.last_hist, ds_rl, rl_out = _score_kernels(q, M, labels, temperature,
+                                                                                                gumbel)
+        if readloss is None:
+            readloss = torch.zeros((), dtype=torch.float32, device=q.device)
+        ctx.set_materialize_grads(False)
+        ctx.has_loss = labels is not None
+        ctx.qshape, ctx.qdtype, ctx.mdtype = query.shape, query.dtype, mem.dtype
+        ctx.save_for_backward(q, M, score_query, score_memory, ds_rl, rl_out)
         return score_query, score_memory, readloss
+
+    @staticmethod
+    def backward(ctx, g_sq, g_sm, g_rl):
+        q, M, score_query, score_memory, ds_rl, rl_out = ctx.saved_tensors
+        N, K = score_query.shape
+        C = q.shape[-1]
+        q = q.view(N, C)
+        dense = lambda g: None if g is None else g.reshape(N, K).to(torch.float32).contiguous()
+        if ctx.has_loss and g_rl is not None:
+            g_rl = g_rl.reshape(1).to(torch.float32).contiguous()
+        else:
+            g_rl = ds_rl = rl_out = None
+        E = torch.empty(N, capi.score_stride(K), dtype=torch.float32, device=q.device)
+        capi.score_bwd(score_query if g_sq is not None else None, dense(g_sq), score_memory if g_sm is not None else None,
+                       dense(g_sm), E, K, ds_rl=ds_rl, g_loss=g_rl, rl_out=rl_out)
+        dq = torch.empty(N, C, dtype=torch.float32, device=q.device) if ctx.needs_input_grad[0] else None
+        dM = torch.zeros(K, C, dtype=torch.float32, device=q.device) if ctx.needs_input_grad[1] else None
+        capi.score_nhwc_bwd(q, M, E, dq, dM, K)
+        if dq is not None:
+            dq = dq.view(ctx.qshape).to(ctx.qdtype)
+        if dM is not None:
+            dM = dM.to(ctx.mdtype)
+        return dq, dM, None, None, None
