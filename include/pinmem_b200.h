@@ -54,7 +54,7 @@ enum pm_readloss_ws_layout {
 #define PM_COLPART_ROWS 296
 
 /* Bumped with every prototype change; the binding refuses a library whose pm_version() differs. */
-#define PM_ABI_VERSION 211
+#define PM_ABI_VERSION 212
 int pm_version(void);
 const char* pm_status_string(int code);
 /* Row stride (floats) of the internal score buffers for K slots: 20 for K<=19, else 32. */
@@ -492,6 +492,30 @@ int pm_read_bwd_dM_ordered(const void* du, const void* x, const float* score_m, 
 int pm_conv1x1_stats_scratch_bytes(int B, int M, int hw, int dtype);
 int pm_conv1x1_fwd_ordered(const void* X, const void* A_hi, const void* A_lo, void* Y, double* stats, double* scratch, int B,
                            int K, int M, int hw, int dtype, void* stream);
+
+/* The writing net's BatchNorm, residual and ReLU inside the write (memory.py:74-87 then :206-257), fp32 only, hw % 4 == 0
+ * and 16-byte aligned maps. z [B,C,h,w] is the writing net's convolution output, x its input; f = relu(x + BN(z)) is formed
+ * tile by tile in shared memory with pm_bn_apply's expression and never stored. lab_u8 = 0: int64 labels, 1: the packed map.
+ *   pm_write_reduce_bn_fwd  pm_write_reduce_fwd of f, with pm_bn_apply_stats' finalise: mean_out / invstd_out, the running
+ *                           statistics and num_batches_tracked (NULL: none) are written once. _ordered: per-CTA partials to
+ *                           scratch (pm_write_reduce_scratch_bytes) added in CTA order (two launches).
+ *   pm_write_bwd_bn         g = df * [f > 0] (df as pm_write_bwd) into g -- the residual gradient and the BatchNorm's output
+ *                           gradient -- and dbeta = sum g, dgamma = sum g * xhat (per-CTA partials in scratch,
+ *                           pm_write_bwd_bn_scratch_bytes(C), added in CTA order in fp64; two launches). The BatchNorm input
+ *                           gradient is pm_bn_bwd_apply on (g, z) with relu = 0. */
+int pm_write_reduce_bn_fwd(const void* z, const void* x, const void* labels, int lab_u8, float* SD, const double* stats,
+                           double count, const double* count_dev, float eps, const float* gamma, const float* beta,
+                           float* mean_out, float* invstd_out, float* running_mean, float* running_var, float momentum,
+                           long long* num_batches_tracked, int B, int C, int h, int w, int Hm, int Wm, int K, void* stream);
+int pm_write_reduce_bn_fwd_ordered(const void* z, const void* x, const void* labels, int lab_u8, float* SD, float* scratch,
+                                   const double* stats, double count, const double* count_dev, float eps, const float* gamma,
+                                   const float* beta, float* mean_out, float* invstd_out, float* running_mean,
+                                   float* running_var, float momentum, long long* num_batches_tracked, int B, int C, int h,
+                                   int w, int Hm, int Wm, int K, void* stream);
+int pm_write_bwd_bn_scratch_bytes(int C);
+int pm_write_bwd_bn(const float* dS, const void* z, const void* x, const void* labels, int lab_u8, const float* mean,
+                    const float* invstd, const float* gamma, const float* beta, void* g, float* dgamma, float* dbeta,
+                    float* scratch, int B, int C, int h, int w, int Hm, int Wm, int K, void* stream);
 
 #ifdef __cplusplus
 }

@@ -19,7 +19,7 @@ WS_BAD = 2     # PM_WS_BAD
 SEG_WS_WORDS = 4  # PM_SEG_WS_WORDS
 SEG_WS_BAD = 2    # PM_SEG_WS_BAD
 
-ABI_VERSION = 211  # PM_ABI_VERSION of include/pinmem_b200.h the argtypes below were written against
+ABI_VERSION = 212  # PM_ABI_VERSION of include/pinmem_b200.h the argtypes below were written against
 
 _c_p = ctypes.c_void_p
 _c_i = ctypes.c_int
@@ -91,6 +91,10 @@ PROTOTYPES = {
     "pm_score_bwd": [_c_p] * 9 + [_c_i] * 2 + [_c_p],
     "pm_score_nhwc_bwd_scratch_bytes": [_c_i] * 3,
     "pm_score_nhwc_bwd": [_c_p] * 6 + [_c_i] * 3 + [_c_p],
+    "pm_write_reduce_bn_fwd": [_c_p] * 3 + [_c_i] + [_c_p] * 2 + [_c_d, _c_p, _c_f] + [_c_p] * 6 + [_c_f, _c_p] + [_c_i] * 7 + [_c_p],
+    "pm_write_reduce_bn_fwd_ordered": [_c_p] * 3 + [_c_i] + [_c_p] * 3 + [_c_d, _c_p, _c_f] + [_c_p] * 6 + [_c_f, _c_p] + [_c_i] * 7 + [_c_p],
+    "pm_write_bwd_bn_scratch_bytes": [_c_i],
+    "pm_write_bwd_bn": [_c_p] * 4 + [_c_i] + [_c_p] * 8 + [_c_i] * 7 + [_c_p],
 }
 EXPORTED_SYMBOLS = sorted(list(PROTOTYPES) + ["pm_status_string"])
 
@@ -206,7 +210,7 @@ LAUNCHES = 0
 _KERNELS_PER_CALL = {"pm_readloss_fwd_ordered": 2, "pm_readloss_fwd8_ordered": 2, "pm_write_reduce_fwd_ordered": 2,
                      "pm_write_reduce_fwd8_ordered": 2, "pm_read_bwd_dM_ordered": 2, "pm_conv1x1_fwd_ordered": 2,
                      "pm_conv1x1_dgrad_bnbwd": 2, "pm_colsoftmax": 3, "pm_colsoftmax_apply": 1, "pm_read_bwd": 2, "pm_read_bwd_planes": 2, "pm_conv1x1_wgrad": 2,
-                     "pm_score_bwd": 2, "pm_score_nhwc_bwd": 2}
+                     "pm_score_bwd": 2, "pm_score_nhwc_bwd": 2, "pm_write_reduce_bn_fwd_ordered": 2, "pm_write_bwd_bn": 2}
 PLANES = 32  # PM_PLANES: score planes appended to q in the score-plane read
 _timing = None  # name -> list of (start_event, end_event) when enabled
 
@@ -369,6 +373,31 @@ def write_reduce_fwd(f, labels, SD, K):
         return
     _call("pm_write_reduce_fwd8" if labels.dtype == torch.uint8 else "pm_write_reduce_fwd", _ptr(f), _ptr(labels), _ptr(SD), B, C, h, w, Hm, Wm, K, dtype_code(f),
                                       _stream())
+
+
+def write_reduce_bn_fwd(z, x, labels, SD, K, stats, count, eps, gamma, beta, mean_out, invstd_out, running_mean, running_var,
+                        momentum, count_dev=None, num_batches_tracked=None):
+    """Class sums|counts of f = relu(x + BatchNorm(z)) added into SD, f formed in the kernel and never stored; the statistics
+    are finalised from the GEMM epilogue's fp64 sums as bn_apply_stats does (fp32, pipelined-kernel alignment)."""
+    B, C, h, w = z.shape
+    Hm, Wm = labels.shape[1], labels.shape[2]
+    u8 = int(labels.dtype == torch.uint8)
+    tail = (_ptr(stats), float(count), _ptr(count_dev), float(eps), _ptr(gamma), _ptr(beta), _ptr(mean_out), _ptr(invstd_out),
+            _ptr(running_mean), _ptr(running_var), float(momentum), _ptr(num_batches_tracked), B, C, h, w, Hm, Wm, K, _stream())
+    if deterministic():
+        scratch = _scratch(load().pm_write_reduce_scratch_bytes(B, C, h, w, K), z.device, "pm_write_reduce_scratch_bytes")
+        _call("pm_write_reduce_bn_fwd_ordered", _ptr(z), _ptr(x), _ptr(labels), u8, _ptr(SD), _ptr(scratch), *tail)
+        return
+    _call("pm_write_reduce_bn_fwd", _ptr(z), _ptr(x), _ptr(labels), u8, _ptr(SD), *tail)
+
+
+def write_bwd_bn(dS, z, x, labels, mean, invstd, gamma, beta, g, dgamma, dbeta, K):
+    """g = d f * [f > 0] of f = relu(x + BatchNorm(z)) under the write, and dgamma / dbeta (added in a fixed order)."""
+    B, C, h, w = z.shape
+    Hm, Wm = labels.shape[1], labels.shape[2]
+    scratch = _scratch(load().pm_write_bwd_bn_scratch_bytes(C), z.device, "pm_write_bwd_bn_scratch_bytes")
+    _call("pm_write_bwd_bn", _ptr(dS), _ptr(z), _ptr(x), _ptr(labels), int(labels.dtype == torch.uint8), _ptr(mean), _ptr(invstd),
+          _ptr(gamma), _ptr(beta), _ptr(g), _ptr(dgamma), _ptr(dbeta), _ptr(scratch), B, C, h, w, Hm, Wm, K, _stream())
 
 
 def update_aux_floats(K):

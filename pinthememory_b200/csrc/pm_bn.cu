@@ -139,15 +139,7 @@ __global__ void __launch_bounds__(BN_THREADS) bn_stats_kernel(const T* __restric
     }
 }
 
-// one CTA per (b, c) row
-struct BnFinalize {  // stats == nullptr: mean / invstd are given
-    const double* stats;
-    const double* n_dev;  // NULL, or the element count on the device (SyncBatchNorm: the all-reduced global count)
-    double n;
-    float eps, momentum;
-    float *mean_out, *invstd_out, *running_mean, *running_var;
-    long long* num_batches_tracked;  // NULL, or nn.BatchNorm2d's counter: bumped here instead of by a torch add kernel
-};
+// one CTA per (b, c) row (BnFinalize: pm_common.cuh)
 template <typename T, int VN>
 __global__ void __launch_bounds__(256) bn_apply_kernel(const T* __restrict__ x, const float* __restrict__ mean,
                                                        const float* __restrict__ invstd, const float* __restrict__ gamma,
@@ -160,26 +152,13 @@ __global__ void __launch_bounds__(256) bn_apply_kernel(const T* __restrict__ x, 
         // batch statistics straight from the convolution epilogue's fp64 (sum, sum of squares): every CTA finalises its
         // own channel (two loads, a division and a square root) instead of waiting for a finalise launch; the CTAs of
         // image 0 publish mean / invstd for the backward and update the running statistics
-        const double n = fin.n_dev != nullptr ? *fin.n_dev : fin.n;
-        const double m = fin.stats[c] / n;
-        double var = fin.stats[C + c] / n - m * m;
-        if (var < 0.0) var = 0.0;
-        mu = (float)m;
-        is = (float)(1.0 / sqrt(var + (double)fin.eps));
+        bn_finalize_channel(fin, c, C, row < C && threadIdx.x == 0, mu, is);
         if (row == 0 && threadIdx.x == 0 && fin.num_batches_tracked != nullptr) *fin.num_batches_tracked += 1;
-        if (row < C && threadIdx.x == 0) {
-            fin.mean_out[c] = mu;
-            fin.invstd_out[c] = is;
-            if (fin.running_mean != nullptr) {
-                const double unb = n > 1.0 ? var * n / (n - 1.0) : var;
-                fin.running_mean[c] = (float)((1.0 - fin.momentum) * fin.running_mean[c] + fin.momentum * m);
-                fin.running_var[c] = (float)((1.0 - fin.momentum) * fin.running_var[c] + fin.momentum * unb);
-            }
-        }
     } else {
         mu = mean[c], is = invstd[c];
     }
-    const float sc = is * gamma[c], sh = beta[c] - mu * sc;
+    float sc, sh;
+    bn_scale_shift(mu, is, gamma[c], beta[c], sc, sh);
     const size_t base = (size_t)row * hw;
     if constexpr (VN != 0) {
         // relu_mask (optional): 1 bit per element, bit = output > 0, 32 elements per word, rows padded to whole
@@ -197,8 +176,8 @@ __global__ void __launch_bounds__(256) bn_apply_kernel(const T* __restrict__ x, 
                 if (residual) r.load(residual + base + VN * j);
 #pragma unroll
                 for (int e = 0; e < VN; ++e) {
-                    float f = fmaf(v.get(e), sc, sh);
-                    if (residual) f += r.get(e);
+                    float f = bn_affine(v.get(e), sc, sh);
+                    if (residual) f += r.get(e);  // with relu: bn_res_relu, the writing net's fused kernels' expression
                     nib |= (f > 0.f ? 1u : 0u) << e;
                     o.set(e, relu ? fmaxf(f, 0.f) : f);
                 }
@@ -211,7 +190,7 @@ __global__ void __launch_bounds__(256) bn_apply_kernel(const T* __restrict__ x, 
         }
     } else {
         for (int j = threadIdx.x; j < hw; j += 256) {
-            float f = fmaf(ldf(x + base + j), sc, sh);
+            float f = bn_affine(ldf(x + base + j), sc, sh);
             if (residual) f += ldf(residual + base + j);
             stf(y + base + j, relu ? fmaxf(f, 0.f) : f);
         }

@@ -141,6 +141,45 @@ __device__ __forceinline__ void mma_tf32(float (&c)[4], unsigned a0, unsigned a1
         : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
 }
 
+// ---- BatchNorm per-channel step and element expression, shared by every kernel that forms a normalised value ---------
+// (pm_bn.cu's normalise pass and the writing net's fused class-sum / write-backward kernels): one source, so the writing
+// net's features, and the ReLU gate they imply, are the same bits whichever kernel forms them.
+struct BnFinalize {  // stats == nullptr: mean / invstd are given
+    const double* stats;
+    const double* n_dev;  // NULL, or the element count on the device (SyncBatchNorm: the all-reduced global count)
+    double n;
+    float eps, momentum;
+    float *mean_out, *invstd_out, *running_mean, *running_var;
+    long long* num_batches_tracked;  // NULL, or nn.BatchNorm2d's counter: bumped here instead of by a torch add kernel
+};
+// mean and 1/sqrt(var + eps) of channel c from the convolution epilogue's fp64 [sum | sum of squares]; `publish`: also store
+// them for the backward and update the running statistics (exactly one thread per channel and call may publish)
+__device__ __forceinline__ void bn_finalize_channel(const BnFinalize& fin, int c, int C, bool publish, float& mu, float& is) {
+    const double n = fin.n_dev != nullptr ? *fin.n_dev : fin.n;
+    const double m = fin.stats[c] / n;
+    double var = fin.stats[C + c] / n - m * m;
+    if (var < 0.0) var = 0.0;
+    mu = (float)m;
+    is = (float)(1.0 / sqrt(var + (double)fin.eps));
+    if (publish) {
+        fin.mean_out[c] = mu;
+        fin.invstd_out[c] = is;
+        if (fin.running_mean != nullptr) {  // PyTorch: running_var takes the unbiased estimate
+            const double unb = n > 1.0 ? var * n / (n - 1.0) : var;
+            fin.running_mean[c] = (float)((1.0 - fin.momentum) * fin.running_mean[c] + fin.momentum * m);
+            fin.running_var[c] = (float)((1.0 - fin.momentum) * fin.running_var[c] + fin.momentum * unb);
+        }
+    }
+}
+// y = z * sc + sh is the normalise + affine: sc = invstd * gamma, sh = beta - mean * sc
+__device__ __forceinline__ void bn_scale_shift(float mu, float is, float gamma, float beta, float& sc, float& sh) {
+    sc = is * gamma;
+    sh = beta - mu * sc;
+}
+__device__ __forceinline__ float bn_affine(float z, float sc, float sh) { return fmaf(z, sc, sh); }
+// the writing net's output relu(x + BN(z)) (reference memory.py:84-86)
+__device__ __forceinline__ float bn_res_relu(float z, float sc, float sh, float x) { return fmaxf(bn_affine(z, sc, sh) + x, 0.f); }
+
 __device__ __forceinline__ float to_float(float v) { return v; }
 __device__ __forceinline__ float to_float(__nv_bfloat16 v) { return __bfloat162float(v); }
 __device__ __forceinline__ float tile_get(const float* t, int row, int px) { return t[row * 32 + px]; }

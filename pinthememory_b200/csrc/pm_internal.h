@@ -35,6 +35,18 @@ int readloss_gather(const float* tiles, const float* lossp, int ncta, int B, int
 int write_bwd_tiled(const float* dS, const void* f, const void* labels, int lab_u8, void* df, int B, int C, int h, int w, int Hm,
                     int Wm, int K, int dtype, cudaStream_t st);
 
+struct BnFinalize;
+// pm_write_tiled.cu, fp32: the writing net's fused class sums (f = relu(x + BN(z)) formed from the z and x maps; `fin` finalises
+// the statistics, CTA 0 publishes them) and write backward (g = df * [f > 0] into g, then dgamma / dbeta from the per-CTA
+// partials in `part`, write_bwd_bn_scratch_floats(C) floats)
+int write_reduce_bn(const float* z, const float* x, const void* labels, int lab_u8, float* SD, int B, int C, int h, int w, int Hm,
+                    int Wm, int K, const float* gamma, const float* beta, const BnFinalize& fin, cudaStream_t st,
+                    float* part = nullptr, int* ncta = nullptr);
+int write_bwd_bn_scratch_floats(int C);
+int write_bwd_bn(const float* dS, const float* z, const float* x, const void* labels, int lab_u8, const float* mean,
+                 const float* invstd, const float* gamma, const float* beta, float* g, float* dgamma, float* dbeta, float* part,
+                 int B, int C, int h, int w, int Hm, int Wm, int K, cudaStream_t st);
+
 // fills `partial` ([PM_COLPART_ROWS][64]: max at [k], sum at [32+k]) from s (+ gumbel_q) and combines them (row PM_COLPART_ROWS)
 int colsoftmax_stats(const float* s, const float* gumbel_q, float* partial, int N, int K, cudaStream_t st);
 

@@ -36,6 +36,9 @@ __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, i
         "l"(reinterpret_cast<uint64_t>(map)), "r"(c0), "r"(c1), "r"(smem_u32(bar))
         : "memory");
 }
+// generic-proxy writes to shared memory -> visible to the async proxy (TMA loads and stores, tensor-core operand reads);
+// also needed before a TMA load overwrites a box that threads have written into
+__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void bulk_load_1d(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
                  "l"(src), "r"(bytes), "r"(smem_u32(bar))

@@ -686,6 +686,61 @@ extern "C" int pm_write_bwd8(const float* dS, const void* f, const uint8_t* lab8
     return write_bwd_any(dS, f, lab8, 1, df, B, C, h, w, Hm, Wm, K, dtype, stream);
 }
 
+// the writing net's fused passes (fp32, pipelined kernels only: 16-byte rows and pointers)
+static int write_bn_fwd_any(const void* z, const void* x, const void* labels, int lab_u8, float* SD, float* scratch,
+                            const double* stats, double count, const double* count_dev, float eps, const float* gamma,
+                            const float* beta, float* mean_out, float* invstd_out, float* running_mean, float* running_var,
+                            float momentum, long long* num_batches_tracked, int B, int C, int h, int w, int Hm, int Wm, int K,
+                            void* stream) {
+    if (!z || !x || !labels || !SD || !stats || !gamma || !beta || !mean_out || !invstd_out ||
+        ((running_mean == nullptr) != (running_var == nullptr)))
+        return PM_ERR_NULL;
+    if (int e = check_write(B, C, h, w, Hm, Wm, K, PM_F32)) return e;
+    if (!(count > 0.0)) return PM_ERR_SHAPE;
+    if (((uintptr_t)SD | (uintptr_t)scratch) & 15) return PM_ERR_ALIGN;
+    if (!pm::tiled_ok(z, x, nullptr, h * w, PM_F32)) return PM_ERR_ALIGN;
+    const pm::BnFinalize fin{stats, count_dev, count, eps, momentum, mean_out, invstd_out, running_mean, running_var,
+                             num_batches_tracked};
+    cudaStream_t st = (cudaStream_t)stream;
+    int ncta = 0;
+    if (int rc = pm::write_reduce_bn((const float*)z, (const float*)x, labels, lab_u8, SD, B, C, h, w, Hm, Wm, K, gamma, beta,
+                                     fin, st, scratch, scratch ? &ncta : nullptr))
+        return rc;
+    return scratch ? pm::reduce_partials_f32(SD, scratch, ncta, (long long)(K + 1) * (C + 4), st) : 0;
+}
+extern "C" int pm_write_reduce_bn_fwd(const void* z, const void* x, const void* labels, int lab_u8, float* SD, const double* stats,
+                                      double count, const double* count_dev, float eps, const float* gamma, const float* beta,
+                                      float* mean_out, float* invstd_out, float* running_mean, float* running_var, float momentum,
+                                      long long* num_batches_tracked, int B, int C, int h, int w, int Hm, int Wm, int K,
+                                      void* stream) {
+    return write_bn_fwd_any(z, x, labels, lab_u8, SD, nullptr, stats, count, count_dev, eps, gamma, beta, mean_out, invstd_out,
+                            running_mean, running_var, momentum, num_batches_tracked, B, C, h, w, Hm, Wm, K, stream);
+}
+extern "C" int pm_write_reduce_bn_fwd_ordered(const void* z, const void* x, const void* labels, int lab_u8, float* SD,
+                                              float* scratch, const double* stats, double count, const double* count_dev, float eps,
+                                              const float* gamma, const float* beta, float* mean_out, float* invstd_out,
+                                              float* running_mean, float* running_var, float momentum,
+                                              long long* num_batches_tracked, int B, int C, int h, int w, int Hm, int Wm, int K,
+                                              void* stream) {
+    if (!scratch) return PM_ERR_NULL;
+    return write_bn_fwd_any(z, x, labels, lab_u8, SD, scratch, stats, count, count_dev, eps, gamma, beta, mean_out, invstd_out,
+                            running_mean, running_var, momentum, num_batches_tracked, B, C, h, w, Hm, Wm, K, stream);
+}
+extern "C" int pm_write_bwd_bn_scratch_bytes(int C) {
+    if (C != 32 && C != 64 && C != 128 && C != 256) return PM_ERR_CHANNELS;
+    return pm::write_bwd_bn_scratch_floats(C) * (int)sizeof(float);
+}
+extern "C" int pm_write_bwd_bn(const float* dS, const void* z, const void* x, const void* labels, int lab_u8, const float* mean,
+                               const float* invstd, const float* gamma, const float* beta, void* g, float* dgamma, float* dbeta,
+                               float* scratch, int B, int C, int h, int w, int Hm, int Wm, int K, void* stream) {
+    if (!dS || !z || !x || !labels || !mean || !invstd || !gamma || !beta || !g || !dgamma || !dbeta || !scratch)
+        return PM_ERR_NULL;
+    if (int e = check_write(B, C, h, w, Hm, Wm, K, PM_F32)) return e;
+    if (!pm::tiled_ok(z, x, g, h * w, PM_F32) || ((uintptr_t)scratch & 15)) return PM_ERR_ALIGN;
+    return pm::write_bwd_bn(dS, (const float*)z, (const float*)x, labels, lab_u8, mean, invstd, gamma, beta, (float*)g, dgamma,
+                            dbeta, scratch, B, C, h, w, Hm, Wm, K, (cudaStream_t)stream);
+}
+
 extern "C" int pm_update_aux_floats(int K) { return 32 + K * pm::UP_KMAX + 68; }
 
 extern "C" int pm_update_fwd(const float* SD, const float* M_old, float momentum, const float* W_cls,

@@ -212,19 +212,42 @@ __global__ void __launch_bounds__(C) write_reduce_tiled_kernel(const T* __restri
 // fragmented the label map is (the run-length kernel above degenerates on noisy labels).
 
 // The tiles arrive as SWIZZLE_128B tensor-map boxes (16-byte chunk c of row r at chunk c ^ (r & 7)) on an mbarrier ring.
-template <int C, int KP, bool ORD = false>
+//
+// BN = true (the writing net's fused forward, pm_write_reduce_bn_fwd): the boxes are the convolution output z and the
+// writing net's input x, and f = relu(x + BN(z)) is formed in place over the z box before the unchanged body runs, so
+// f never exists in global memory. Each CTA finalises the C channels' statistics in its prologue; CTA 0 publishes
+// mean / invstd and the running statistics and bumps the batch counter. A 2-stage ring of (z, x) pairs (128 KB at C = 256)
+// would leave one CTA per SM; instead there is one z box and one x box, each on its own barrier, and the x box is refilled
+// with the next tile as soon as f is formed, so half of the next tile streams in under the class sums (two CTAs per SM).
+template <int C>
+__host__ __device__ constexpr size_t wr_mma_ring_floats(int nstage) {  // the tile ring, which is also the [32][C+4] class-sum tile at the end
+    return (size_t)nstage * C * 32 > (size_t)32 * (C + 4) ? (size_t)nstage * C * 32 : (size_t)32 * (C + 4);
+}
+template <int C, bool BN>
+constexpr size_t wr_mma_smem_bytes() {
+    constexpr size_t ring = (wr_mma_ring_floats<C>(BN ? 1 : 2) + 255) / 256 * 256;  // x box 1 KB aligned behind it
+    return sizeof(float) * (ring + (BN ? (size_t)C * 32 + 2 * C : 0) + 32 * 40 + (C / 32) * 32 + 32 + 4) + 1024;
+}
+
+template <int C, int KP, bool ORD = false, bool BN = false>
 __global__ void __launch_bounds__(C) write_reduce_mma_kernel(const __grid_constant__ CUtensorMap tm_f,
+                                                              const __grid_constant__ CUtensorMap tm_x,
                                                               const void* __restrict__ labels, int lab_u8,
                                                               float* __restrict__ SD, int h, int w, int Hm, int Wm,
                                                               int K, float sy, float sx, int tiles_per_img,
-                                                              int ntiles) {
-    constexpr int NSTAGE = 2, NW = C / 32, CS = C + 4, OMLD = 40;
+                                                              int ntiles, const float* __restrict__ gamma,
+                                                              const float* __restrict__ beta, BnFinalize fin) {
+    constexpr int NSTAGE = BN ? 1 : 2, NW = C / 32, CS = C + 4, OMLD = 40;
     extern __shared__ __align__(16) unsigned char smraw_[];
     __shared__ __align__(8) uint64_t full[NSTAGE];
+    __shared__ __align__(8) uint64_t fullx;            // BN: the x box has a barrier of its own (refilled before the z box)
     unsigned char* smraw = smem_align(smraw_, 1024);  // the swizzled TMA boxes need 1 KB alignment
     float* ft = reinterpret_cast<float*>(smraw);       // [NSTAGE][C][32] swizzled; reused as S_tile [32][CS] at the end
-    constexpr size_t RING = (size_t)NSTAGE * C * 32 > (size_t)32 * CS ? (size_t)NSTAGE * C * 32 : (size_t)32 * CS;
-    float* om = ft + RING;                             // [32 px][OMLD] dense label weights of the current tile
+    constexpr size_t RING = (wr_mma_ring_floats<C>(NSTAGE) + 255) / 256 * 256;
+    float* xs = ft + RING;                             // BN: [C][32] swizzled x box
+    float* scs = xs + (BN ? C * 32 : 0);               // BN: [C] scale, [C] shift of the normalise
+    float* shs = scs + (BN ? C : 0);
+    float* om = shs + (BN ? C : 0);                    // [32 px][OMLD] dense label weights of the current tile
     float* pn = om + 32 * OMLD;                        // [NW][32]
     float* invr = pn + NW * 32;                        // [32]
     unsigned* cmask = reinterpret_cast<unsigned*>(invr + 32);  // [4]
@@ -262,16 +285,33 @@ __global__ void __launch_bounds__(C) write_reduce_mma_kernel(const __grid_consta
     auto issue = [&](int tl, int s) {  // one thread
         int b, px0;
         tile_coords(tl, b, px0);
+        if constexpr (BN) fence_proxy_async_smem();  // f was written over the z box of the previous tile
         mbar_expect_tx(&full[s], (uint32_t)(C * 32 * sizeof(float)));
         tma_load_2d(ft + s * C * 32, &tm_f, px0, b * C, &full[s]);
+    };
+    auto issue_x = [&](int tl) {  // one thread (BN)
+        int b, px0;
+        tile_coords(tl, b, px0);
+        fence_proxy_async_smem();
+        mbar_expect_tx(&fullx, (uint32_t)(C * 32 * sizeof(float)));
+        tma_load_2d(xs, &tm_x, px0, b * C, &fullx);
     };
     if (tid == 0) {
 #pragma unroll
         for (int s = 0; s < NSTAGE; ++s) mbar_init(&full[s], 1);
+        if constexpr (BN) mbar_init(&fullx, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 #pragma unroll
         for (int s = 0; s < NSTAGE; ++s)
             if (tile + s * (int)gridDim.x < ntiles) issue(tile + s * gridDim.x, s);
+        if constexpr (BN)
+            if (tile < ntiles) issue_x(tile);
+    }
+    if constexpr (BN) {  // thread = channel (blockDim == C)
+        float mu, is;
+        bn_finalize_channel(fin, tid, C, blockIdx.x == 0, mu, is);
+        bn_scale_shift(mu, is, gamma[tid], beta[tid], scs[tid], shs[tid]);
+        if (blockIdx.x == 0 && tid == 0 && fin.num_batches_tracked != nullptr) *fin.num_batches_tracked += 1;
     }
     LabelTaps tcur;
     if (wid == 0) tcur = taps_for(tile);
@@ -283,7 +323,22 @@ __global__ void __launch_bounds__(C) write_reduce_mma_kernel(const __grid_consta
         if (wid == 0) tnext = taps_for(tile + gridDim.x);  // loads in flight across this tile
         __syncthreads();
         mbar_wait(&full[stage], phase);
-        const float* xt = ft + stage * C * 32;
+        float* xt = ft + stage * C * 32;
+        if constexpr (BN) {  // f over the z box: both boxes share the swizzle, so element i of either is channel i / 32
+            mbar_wait(&fullx, phase);
+#pragma unroll 4
+            for (int i = tid; i < C * 8; i += C) {
+                const int c = i >> 3;
+                const float sc = scs[c], sh = shs[c];
+                float4 z = reinterpret_cast<const float4*>(xt)[i];
+                const float4 x = reinterpret_cast<const float4*>(xs)[i];
+                z.x = bn_res_relu(z.x, sc, sh, x.x), z.y = bn_res_relu(z.y, sc, sh, x.y);
+                z.z = bn_res_relu(z.z, sc, sh, x.z), z.w = bn_res_relu(z.w, sc, sh, x.w);
+                reinterpret_cast<float4*>(xt)[i] = z;
+            }
+            __syncthreads();  // x box consumed: the next tile's x streams in under this tile's class sums
+            if (tid == 0 && tile + (int)gridDim.x < ntiles) issue_x(tile + gridDim.x);
+        }
         for (int i = tid; i < 32 * OMLD / 4; i += C) reinterpret_cast<float4*>(om)[i] = make_float4(0.f, 0.f, 0.f, 0.f);
         {  // |f|^2 per pixel: lanes = pixels, each warp sums 32 of the C rows (rows wid, wid+NW, .. share a swizzle
            // phase when NW % 8 == 0)
@@ -618,17 +673,19 @@ int launch_write_reduce_mma16(const void* f, const void* labels, int lab_u8, flo
     return e == cudaSuccess ? 0 : (int)e;
 }
 
-template <int C, int KP>
+// BN: f is relu(x + BN(z)) of the z map `f` and the x map `x` (see write_reduce_mma_kernel)
+template <int C, int KP, bool BN = false>
 int launch_write_reduce_mma(const void* f, const void* labels, int lab_u8, float* SD, int B, int h, int w, int Hm, int Wm, int K,
-                            cudaStream_t st, float* part, int* ncta) {
-    const size_t ring = sizeof(float) * (size_t)2 * C * 32, stile = sizeof(float) * (size_t)32 * (C + 4);
-    const size_t smem = sizeof(float) * (32 * 40 + (C / 32) * 32 + 32 + 4) + (ring > stile ? ring : stile) + 1024;
+                            cudaStream_t st, float* part, int* ncta, const void* x = nullptr, const float* gamma = nullptr,
+                            const float* beta = nullptr, BnFinalize fin = BnFinalize{}) {
+    const size_t smem = wr_mma_smem_bytes<C, BN>();
     const int hw = h * w, tiles = (hw + 31) / 32, ntiles = B * tiles;
     const float sy = h > 1 ? (float)(Hm - 1) / (float)(h - 1) : 0.f;
     const float sx = w > 1 ? (float)(Wm - 1) / (float)(w - 1) : 0.f;
-    CUtensorMap tm_f;
+    CUtensorMap tm_f, tm_x;
     if (!make_map_2d<float>(&tm_f, f, (size_t)B * C, hw, C, 32, true)) return PM_ERR_ALIGN;
-    auto kern = part ? write_reduce_mma_kernel<C, KP, true> : write_reduce_mma_kernel<C, KP>;
+    if (!make_map_2d<float>(&tm_x, BN ? x : f, (size_t)B * C, hw, C, 32, true)) return PM_ERR_ALIGN;
+    auto kern = part ? write_reduce_mma_kernel<C, KP, true, BN> : write_reduce_mma_kernel<C, KP, false, BN>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
     int per_sm = 1;
@@ -642,7 +699,7 @@ int launch_write_reduce_mma(const void* f, const void* labels, int lab_u8, float
         if (grid > PM_ORD_CTAS) grid = PM_ORD_CTAS;
         SD = part, *ncta = grid;
     }
-    kern<<<grid, C, smem, st>>>(tm_f, labels, lab_u8, SD, h, w, Hm, Wm, K, sy, sx, tiles, ntiles);
+    kern<<<grid, C, smem, st>>>(tm_f, tm_x, labels, lab_u8, SD, h, w, Hm, Wm, K, sy, sx, tiles, ntiles, gamma, beta, fin);
     e = cudaGetLastError();
     return e == cudaSuccess ? 0 : (int)e;
 }
@@ -680,21 +737,50 @@ int launch_write_reduce_tiled(const void* f, const void* labels, int lab_u8, flo
 // dS sits in shared memory with row stride C+1 (lanes with different classes hit different banks). The
 // label taps of the next tile are fetched by warp 0 while the current tile is processed.
 
+//
+// BN = true (the writing net's fused backward, pm_write_bwd_bn, fp32): the boxes are z and x of the writing net
+// f = relu(x + BN(z)); f is formed over the x box with the forward's expression (same bits, same gate), and the kernel
+// stores g = df * [f > 0] -- the residual gradient and the BatchNorm's output gradient -- instead of df. It also leaves
+// this CTA's per-channel (sum g, sum g * xhat) in part[blockIdx.x] (lane sums over the tile, added over the CTA's tiles
+// in tile order), which bn_sums_finalize_kernel adds in CTA order. One stage of two boxes keeps two CTAs per SM.
 constexpr int WBT_THREADS = 256, WBT_WARPS = 8, WBT_STAGES = 2;
 
-template <typename T, int C, int KP>
+// v[i] summed over the 32 lanes, scattered: lane l returns the total of v[l % N] (N <= 32, a power of two). Full butterfly
+// sums over the lane bits >= N, then a halving exchange: N - 1 shuffles for N values instead of 5 N.
+template <int N>
+__device__ __forceinline__ float lane_reduce_scatter(float (&v)[N], int lane) {
+#pragma unroll
+    for (int o = 16; o >= N; o >>= 1)
+#pragma unroll
+        for (int i = 0; i < N; ++i) v[i] += __shfl_xor_sync(0xffffffffu, v[i], o);
+#pragma unroll
+    for (int s = N / 2; s >= 1; s >>= 1) {
+        const bool up = (lane & s) != 0;
+#pragma unroll
+        for (int i = 0; i < s; ++i) {
+            const float send = up ? v[i] : v[i + s], keep = up ? v[i + s] : v[i];
+            v[i] = keep + __shfl_xor_sync(0xffffffffu, send, s);
+        }
+    }
+    return v[0];
+}
+
+template <typename T, int C, int KP, bool BN = false>
 __global__ void __launch_bounds__(WBT_THREADS, 2)
-    write_bwd_tiled_kernel(const __grid_constant__ CUtensorMap tm_f, const float* __restrict__ dS,
-                           const void* __restrict__ labels, int lab_u8,
+    write_bwd_tiled_kernel(const __grid_constant__ CUtensorMap tm_f, const __grid_constant__ CUtensorMap tm_x,
+                           const float* __restrict__ dS, const void* __restrict__ labels, int lab_u8,
                            T* __restrict__ df, int h, int w, int Hm, int Wm, int K, float sy, float sx,
-                           int tiles_per_img, int ntiles) {
-    constexpr int NSTAGE = WBT_STAGES, CW = C / WBT_WARPS, LDS_ = C + 1;
+                           int tiles_per_img, int ntiles, const float* __restrict__ mean, const float* __restrict__ invstd,
+                           const float* __restrict__ gamma, const float* __restrict__ beta, float* __restrict__ part) {
+    constexpr int NSTAGE = BN ? 1 : WBT_STAGES, CW = C / WBT_WARPS, LDS_ = C + 1;
     extern __shared__ __align__(16) unsigned char smraw[];
     float* dSs = reinterpret_cast<float*>(smraw);      // [KP][C+1]; rows >= K are zero (ignore class)
     float* pn = dSs + KP * LDS_;                        // [8][32]
     float* pd = pn + WBT_WARPS * 32;                    // [8][32]
-    float2* ent = reinterpret_cast<float2*>(pd + WBT_WARPS * 32 + ((KP * LDS_) & 1));  // [2][32][4]
+    float* bnc = pd + WBT_WARPS * 32;                   // BN: [4][C] scale, shift, mean, invstd
+    float2* ent = reinterpret_cast<float2*>(bnc + (BN ? 4 * C : 0) + ((KP * LDS_) & 1));  // [2][32][4]
     T* ft = reinterpret_cast<T*>(smem_align(reinterpret_cast<unsigned char*>(ent + 2 * 32 * 4), 128));  // [NSTAGE][C][32]
+    T* xs = ft + NSTAGE * C * 32;                       // BN: [C][32] x box, overwritten with f
     __shared__ __align__(8) uint64_t full[NSTAGE];
 
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5, hw = h * w;
@@ -725,8 +811,10 @@ __global__ void __launch_bounds__(WBT_THREADS, 2)
     auto issue = [&](int t, int s) {  // one thread
         int b, px0;
         tile_coords(t, b, px0);
-        mbar_expect_tx(&full[s], (uint32_t)(C * 32 * sizeof(T)));
+        if constexpr (BN) fence_proxy_async_smem();  // f was written over the x box of the previous tile
+        mbar_expect_tx(&full[s], (uint32_t)((BN ? 2 : 1) * C * 32 * sizeof(T)));
         tma_load_2d(ft + s * C * 32, &tm_f, px0, b * C, &full[s]);
+        if constexpr (BN) tma_load_2d(xs, &tm_x, px0, b * C, &full[s]);
     };
     if (tid == 0) {
 #pragma unroll
@@ -740,6 +828,14 @@ __global__ void __launch_bounds__(WBT_THREADS, 2)
         const int k = i / LDS_, c = i - k * LDS_;
         dSs[i] = (k < K && c < C) ? __ldg(dS + (size_t)k * C + c) : 0.f;
     }
+    if constexpr (BN) {
+        for (int c = tid; c < C; c += WBT_THREADS) {
+            const float mu = mean[c], is = invstd[c];
+            bn_scale_shift(mu, is, gamma[c], beta[c], bnc[c], bnc[C + c]);
+            bnc[2 * C + c] = mu, bnc[3 * C + c] = is;
+        }
+    }
+    float accg = 0.f, accgx = 0.f;  // BN: lane l's channel wid * CW + l % CW
     if (wid == 0) {
         LabelTaps t0 = taps_for(tile);
         compact_taps(t0);
@@ -757,6 +853,15 @@ __global__ void __launch_bounds__(WBT_THREADS, 2)
         int b, px0;
         tile_coords(tile, b, px0);
         const int nvalid = min(32, hw - px0);
+        if constexpr (BN) {  // f over the x box; each thread forms (and later reads) only its own column
+            T* fc = xs + wid * CW * 32 + lane;
+            const T* zc = xt + wid * CW * 32 + lane;
+#pragma unroll
+            for (int j = 0; j < CW; ++j) {
+                const int c = wid * CW + j;
+                fc[j * 32] = bn_res_relu(zc[j * 32], bnc[c], bnc[C + c], fc[j * 32]);
+            }
+        }
         // this pixel's taps
         int cls[4];
         float wt[4];
@@ -767,7 +872,7 @@ __global__ void __launch_bounds__(WBT_THREADS, 2)
             wt[j] = e.y;
         }
         const bool multi = wt[1] != 0.f;
-        const T* fcol = xt + wid * CW * 32 + lane;
+        const T* fcol = (BN ? xs : xt) + wid * CW * 32 + lane;
         const float* r0 = dSs + cls[0] * LDS_ + wid * CW;
         float dv[CW], n2 = 0.f, dotf = 0.f;
 #pragma unroll
@@ -797,7 +902,28 @@ __global__ void __launch_bounds__(WBT_THREADS, 2)
         const float nrm = sqrtf(nn), ir = 1.f / fmaxf(nrm, PM_NORM_EPS);
         // v.dv = ir * (f.dv); df = (dv - v (v.dv)) * ir = dv*ir - f * (ir^3 * f.dv)
         const float coef = (nrm <= PM_NORM_EPS) ? 0.f : ir * ir * ir * dd;
-        if (lane < nvalid) {
+        if constexpr (BN) {
+            const T* zc = xt + wid * CW * 32 + lane;
+            float gx[CW];
+#pragma unroll
+            for (int j = 0; j < CW; ++j) {
+                const int c = wid * CW + j;
+                const float fv = fcol[j * 32];
+                const float g = (fv > 0.f && lane < nvalid) ? fmaf(-coef, fv, dv[j] * ir) : 0.f;
+                dv[j] = g;
+                gx[j] = g * ((zc[j * 32] - bnc[2 * C + c]) * bnc[3 * C + c]);
+            }
+            if (lane < nvalid) {
+                T* gp = df + ((size_t)b * C + wid * CW) * hw + px0 + lane;
+#pragma unroll
+                for (int j = 0; j < CW; ++j) {
+                    stf(gp, dv[j]);
+                    gp += hw;
+                }
+            }
+            accg += lane_reduce_scatter<CW>(dv, lane);
+            accgx += lane_reduce_scatter<CW>(gx, lane);
+        } else if (lane < nvalid) {
             T* dfp = df + ((size_t)b * C + wid * CW) * hw + px0 + lane;
 #pragma unroll
             for (int j = 0; j < CW; ++j) {
@@ -815,24 +941,64 @@ __global__ void __launch_bounds__(WBT_THREADS, 2)
         if (++stage == NSTAGE) stage = 0, phase ^= 1u;
         ebuf ^= 1;
     }
+    if constexpr (BN) {
+        if (lane < CW) {
+            part[(size_t)blockIdx.x * 2 * C + wid * CW + lane] = accg;
+            part[(size_t)blockIdx.x * 2 * C + C + wid * CW + lane] = accgx;
+        }
+    }
 }
 
-template <typename T, int C, int KP>
+// dbeta[c] = sum_g part[g][0][c], dgamma[c] = sum_g part[g][1][c] over the G CTA partials of write_bwd_tiled_kernel<BN>,
+// in fp64 and a fixed order: warp w adds the partials g = w, w + 16, ... in ascending order, then thread l of warp 0 adds
+// the 16 warp sums in warp order. A block takes 32 consecutive entries of the [2][C] row.
+__global__ void __launch_bounds__(512) bn_sums_finalize_kernel(const float* __restrict__ part, int G, int C,
+                                                               float* __restrict__ dgamma, float* __restrict__ dbeta) {
+    __shared__ double red[16][32];
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, e = blockIdx.x * 32 + lane;
+    double a = 0.0;
+    if (e < 2 * C) {
+#pragma unroll 4
+        for (int g = wid; g < G; g += 16) a += (double)__ldg(part + (size_t)g * 2 * C + e);
+    }
+    red[wid][lane] = a;
+    __syncthreads();
+    if (wid == 0 && e < 2 * C) {
+        double t = 0.0;
+#pragma unroll
+        for (int i = 0; i < 16; ++i) t += red[i][lane];
+        if (e < C) dbeta[e] = (float)t;
+        else dgamma[e - C] = (float)t;
+    }
+}
+
+// CTAs of the write backward (two per SM); also the number of BatchNorm partials the BN instantiation leaves
+constexpr int WBT_GRID = 2 * 148;
+
+// BN: `f` is z, `x` the writing net's input; df receives g; part [grid][2][C] the CTA partials, then dgamma / dbeta
+template <typename T, int C, int KP, bool BN = false>
 int launch_write_bwd_tiled(const float* dS, const void* f, const void* labels, int lab_u8, void* df, int B, int h, int w, int Hm,
-                           int Wm, int K, cudaStream_t st) {
-    const size_t smem = sizeof(float) * ((size_t)KP * (C + 1) + 2 * WBT_WARPS * 32 + 1) + sizeof(float2) * 2 * 32 * 4 +
-                        sizeof(T) * (size_t)WBT_STAGES * C * 32 + 128;
+                           int Wm, int K, cudaStream_t st, const void* x = nullptr, const float* mean = nullptr,
+                           const float* invstd = nullptr, const float* gamma = nullptr, const float* beta = nullptr,
+                           float* part = nullptr, float* dgamma = nullptr, float* dbeta = nullptr) {
+    const size_t smem = sizeof(float) * ((size_t)KP * (C + 1) + 2 * WBT_WARPS * 32 + (BN ? 4 * C : 0) + 1) +
+                        sizeof(float2) * 2 * 32 * 4 + sizeof(T) * (size_t)(BN ? 2 : WBT_STAGES) * C * 32 + 128;
     const int hw = h * w, tiles = (hw + 31) / 32, ntiles = B * tiles;
-    int grid = 2 * 148;
+    int grid = WBT_GRID;
     if (grid > ntiles) grid = ntiles;
     const float sy = h > 1 ? (float)(Hm - 1) / (float)(h - 1) : 0.f;
     const float sx = w > 1 ? (float)(Wm - 1) / (float)(w - 1) : 0.f;
-    CUtensorMap tm_f;
+    CUtensorMap tm_f, tm_x;
     if (!make_map_2d<T>(&tm_f, f, (size_t)B * C, hw, C, 32, false)) return PM_ERR_ALIGN;
-    auto kern = write_bwd_tiled_kernel<T, C, KP>;
+    if (!make_map_2d<T>(&tm_x, BN ? x : f, (size_t)B * C, hw, C, 32, false)) return PM_ERR_ALIGN;
+    auto kern = write_bwd_tiled_kernel<T, C, KP, BN>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
-    kern<<<grid, WBT_THREADS, smem, st>>>(tm_f, dS, labels, lab_u8, (T*)df, h, w, Hm, Wm, K, sy, sx, tiles, ntiles);
+    kern<<<grid, WBT_THREADS, smem, st>>>(tm_f, tm_x, dS, labels, lab_u8, (T*)df, h, w, Hm, Wm, K, sy, sx, tiles, ntiles, mean,
+                                          invstd, gamma, beta, part);
+    e = cudaGetLastError();
+    if (e != cudaSuccess || !BN) return e == cudaSuccess ? 0 : (int)e;
+    bn_sums_finalize_kernel<<<(2 * C + 31) / 32, 512, 0, st>>>(part, grid, C, dgamma, dbeta);
     e = cudaGetLastError();
     return e == cudaSuccess ? 0 : (int)e;
 }
@@ -877,6 +1043,36 @@ int write_bwd_tiled(const float* dS, const void* f, const void* labels, int lab_
         if (K <= 19) { PM_WT_SWITCH_C(__nv_bfloat16, 20, launch_write_bwd_tiled, dS, f, labels, lab_u8, df, B, h, w, Hm, Wm, K, st) }
         else { PM_WT_SWITCH_C(__nv_bfloat16, 32, launch_write_bwd_tiled, dS, f, labels, lab_u8, df, B, h, w, Hm, Wm, K, st) }
     }
+}
+
+int write_reduce_bn(const float* z, const float* x, const void* labels, int lab_u8, float* SD, int B, int C, int h, int w, int Hm,
+                    int Wm, int K, const float* gamma, const float* beta, const BnFinalize& fin, cudaStream_t st, float* part,
+                    int* ncta) {
+    switch (C) {
+        case 32: return launch_write_reduce_mma<32, 32, true>(z, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st, part, ncta, x, gamma, beta, fin);
+        case 64: return launch_write_reduce_mma<64, 32, true>(z, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st, part, ncta, x, gamma, beta, fin);
+        case 128: return launch_write_reduce_mma<128, 32, true>(z, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st, part, ncta, x, gamma, beta, fin);
+        case 256: return launch_write_reduce_mma<256, 32, true>(z, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st, part, ncta, x, gamma, beta, fin);
+        default: return PM_ERR_CHANNELS;
+    }
+}
+
+int write_bwd_bn_scratch_floats(int C) { return WBT_GRID * 2 * C; }
+
+#define PM_WBN_SWITCH_C(KP)                                                                                                  \
+    switch (C) {                                                                                                             \
+        case 32: return launch_write_bwd_tiled<float, 32, KP, true>(dS, z, labels, lab_u8, g, B, h, w, Hm, Wm, K, st, x, mean, invstd, gamma, beta, part, dgamma, dbeta);   \
+        case 64: return launch_write_bwd_tiled<float, 64, KP, true>(dS, z, labels, lab_u8, g, B, h, w, Hm, Wm, K, st, x, mean, invstd, gamma, beta, part, dgamma, dbeta);   \
+        case 128: return launch_write_bwd_tiled<float, 128, KP, true>(dS, z, labels, lab_u8, g, B, h, w, Hm, Wm, K, st, x, mean, invstd, gamma, beta, part, dgamma, dbeta); \
+        case 256: return launch_write_bwd_tiled<float, 256, KP, true>(dS, z, labels, lab_u8, g, B, h, w, Hm, Wm, K, st, x, mean, invstd, gamma, beta, part, dgamma, dbeta); \
+        default: return PM_ERR_CHANNELS;                                                                                     \
+    }
+
+int write_bwd_bn(const float* dS, const float* z, const float* x, const void* labels, int lab_u8, const float* mean,
+                 const float* invstd, const float* gamma, const float* beta, float* g, float* dgamma, float* dbeta, float* part,
+                 int B, int C, int h, int w, int Hm, int Wm, int K, cudaStream_t st) {
+    if (K <= 19) { PM_WBN_SWITCH_C(20) }
+    else { PM_WBN_SWITCH_C(32) }
 }
 
 }  // namespace pm

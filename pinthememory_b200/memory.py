@@ -251,31 +251,9 @@ class _WriteFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, f, labels, M_old, W, b, momentum, K, group):
-        B, C, h, w = f.shape
-        dev = f.device
-        peer = group.peer if (group is not None and group.world_size > 1) else None
-        # one zeroed allocation: the class sums|counts [K+1, C+4] and the update kernel's scratch
-        nsd = (K + 1) * (C + 4)
-        zbuf = torch.zeros(nsd + capi.update_aux_floats(K), dtype=torch.float32, device=dev)
-        SD, aux = zbuf[:nsd].view(K + 1, C + 4), zbuf[nsd:]
-        M_old = M_old.detach().contiguous()
-        W = W.detach().to(torch.float32).contiguous()
-        b = b.detach().to(torch.float32).contiguous()
-        M_new = torch.empty(K, C, dtype=torch.float32, device=dev)
-        losses = torch.empty(2, dtype=torch.float32, device=dev)
-        saved = torch.empty(2 * K, dtype=torch.float32, device=dev)
-        if peer is not None:
-            # the rank's sums go into its peer-mapped buffer; the update kernel itself gathers and sums all ranks' rows
-            # over NVLink (and leaves the all-reduced sums in SD for the host side)
-            mine = peer.sums_view(K, C)
-            mine.zero_()
-            capi.write_reduce_fwd(f, labels, mine, K)
-            capi.update_fwd_peer(peer, SD, M_old, momentum, W, b, M_new, losses, saved, C, K, aux=aux)
-        else:
-            capi.write_reduce_fwd(f, labels, SD, K)
-            if group is not None:
-                sharding.all_reduce_sum_(SD, group)
-            capi.update_fwd(SD, M_old, momentum, W, b, M_new, losses, saved, C, K, aux=aux)
+        C = f.shape[1]
+        M_new, losses, saved, W, b, SD = _write_update_fwd(lambda sd: capi.write_reduce_fwd(f, labels, sd, K), M_old, W, b,
+                                                           momentum, C, K, group, f.device)
         ctx.K, ctx.momentum, ctx.group = K, momentum, group
         ctx.set_materialize_grads(False)
         ctx.save_for_backward(f, labels, M_new, saved, W, b)
@@ -285,25 +263,136 @@ class _WriteFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dM_new, g_div, g_cls, _g_sd):
         f, labels, M_new, saved, W, b = ctx.saved_tensors
-        K, C = ctx.K, f.shape[1]
-        dev = f.device
-        as32 = lambda t: None if t is None else t.to(torch.float32).contiguous()
-        dS = torch.empty(K, C, dtype=torch.float32, device=dev)
-        dW = torch.empty(K, C, dtype=torch.float32, device=dev)
-        db = torch.empty(K, dtype=torch.float32, device=dev)
-        peer = ctx.group.peer if (ctx.group is not None and ctx.group.world_size > 1) else None
-        if peer is not None:
-            capi.update_bwd_peer(peer, as32(dM_new), as32(g_div), as32(g_cls), M_new, saved, W, b, ctx.momentum, dS, dW, db,
-                                 C, K)
-        else:
-            capi.update_bwd(as32(dM_new), as32(g_div), as32(g_cls), M_new, saved, W, b, ctx.momentum, dS, dW, db, C, K)
-            if ctx.group is not None:
-                sharding.all_reduce_sum_(dS, ctx.group)
+        K = ctx.K
+        dS, dW, db = _write_update_bwd(ctx, dM_new, g_div, g_cls, M_new, saved, W, b, f.shape[1], K)
         df = None
         if ctx.needs_input_grad[0]:
             df = torch.empty_like(f)
             capi.write_bwd(dS, f, labels, df, K)
         return df, None, None, dW, db, None, None, None
+
+
+def _write_update_fwd(reduce, M_old, W, b, momentum, C, K, group, dev):
+    """reduce(sums) adds the class sums|counts into `sums`; then the update (plain, all-reduced or over peer memory).
+    Returns (M_new, losses, saved, W fp32, b fp32, SD)."""
+    peer = group.peer if (group is not None and group.world_size > 1) else None
+    # one zeroed allocation: the class sums|counts [K+1, C+4] and the update kernel's scratch
+    nsd = (K + 1) * (C + 4)
+    zbuf = torch.zeros(nsd + capi.update_aux_floats(K), dtype=torch.float32, device=dev)
+    SD, aux = zbuf[:nsd].view(K + 1, C + 4), zbuf[nsd:]
+    M_old = M_old.detach().contiguous()
+    W = W.detach().to(torch.float32).contiguous()
+    b = b.detach().to(torch.float32).contiguous()
+    M_new = torch.empty(K, C, dtype=torch.float32, device=dev)
+    losses = torch.empty(2, dtype=torch.float32, device=dev)
+    saved = torch.empty(2 * K, dtype=torch.float32, device=dev)
+    if peer is not None:
+        # the rank's sums go into its peer-mapped buffer; the update kernel itself gathers and sums all ranks' rows
+        # over NVLink (and leaves the all-reduced sums in SD for the host side)
+        mine = peer.sums_view(K, C)
+        mine.zero_()
+        reduce(mine)
+        capi.update_fwd_peer(peer, SD, M_old, momentum, W, b, M_new, losses, saved, C, K, aux=aux)
+    else:
+        reduce(SD)
+        if group is not None:
+            sharding.all_reduce_sum_(SD, group)
+        capi.update_fwd(SD, M_old, momentum, W, b, M_new, losses, saved, C, K, aux=aux)
+    return M_new, losses, saved, W, b, SD
+
+
+def _write_update_bwd(ctx, dM_new, g_div, g_cls, M_new, saved, W, b, C, K):
+    """(dS, dW, db) of the update; ctx carries momentum and group."""
+    dev = M_new.device
+    as32 = lambda t: None if t is None else t.to(torch.float32).contiguous()
+    dS = torch.empty(K, C, dtype=torch.float32, device=dev)
+    dW = torch.empty(K, C, dtype=torch.float32, device=dev)
+    db = torch.empty(K, dtype=torch.float32, device=dev)
+    peer = ctx.group.peer if (ctx.group is not None and ctx.group.world_size > 1) else None
+    if peer is not None:
+        capi.update_bwd_peer(peer, as32(dM_new), as32(g_div), as32(g_cls), M_new, saved, W, b, ctx.momentum, dS, dW, db, C, K)
+    else:
+        capi.update_bwd(as32(dM_new), as32(g_div), as32(g_cls), M_new, saved, W, b, ctx.momentum, dS, dW, db, C, K)
+        if ctx.group is not None:
+            sharding.all_reduce_sum_(dS, ctx.group)
+    return dS, dW, db
+
+
+class _WriteNetFn(torch.autograd.Function):
+    """Writingnet then _WriteFn in one Function (fp32): z = conv1x1(x, Wc) with the batch statistics in the GEMM epilogue, then
+    the class sums of f = relu(x + BatchNorm(z)) with f formed inside the class-sum kernel (pm_write_reduce_bn_fwd), then the
+    update. f and its ReLU mask are never stored; the backward forms f again from (z, x) inside the write backward, which
+    also leaves g = df * [f > 0] and the BatchNorm sums (pm_write_bwd_bn), so the BatchNorm backward is one pass
+    (pm_bn_bwd_apply on (g, z)) and the input-gradient GEMM accumulates into g. Saves x and z."""
+
+    @staticmethod
+    def forward(ctx, x, labels, M_old, Wc, gamma, beta, running_mean, running_var, factor, eps, num_batches_tracked, sync_group,
+                W, b, momentum, K, group):
+        B, C, h, w = x.shape
+        dev = x.device
+        W2 = Wc.detach().reshape(C, C).to(torch.float32).contiguous()
+        g32 = gamma.detach().to(torch.float32).contiguous()
+        b32 = beta.detach().to(torch.float32).contiguous()
+        # [sum | sum of squares | element count], cleared by the launch that also splits W and W^T for the two GEMMs
+        stats = torch.empty(2 * C + 1, dtype=torch.float64, device=dev)
+        (hi, lo), ctx.preT = capi.conv1x1_prep_both(W2, torch.float32, zero=stats)
+        z = capi.conv1x1_fwd(x, hi, lo, C, stats=stats)
+        count = None
+        if sync_group is not None:   # as _ConvBnActFn: global statistics
+            import torch.distributed as dist
+
+            stats[2 * C:].fill_(float(B * h * w))
+            dist.all_reduce(stats, group=sync_group)
+            count = stats[2 * C:]
+        mean = torch.empty(C, dtype=torch.float32, device=dev)
+        invstd = torch.empty(C, dtype=torch.float32, device=dev)
+        M_new, losses, saved, W, b, SD = _write_update_fwd(
+            lambda sd: capi.write_reduce_bn_fwd(z, x, labels, sd, K, stats, B * h * w, eps, g32, b32, mean, invstd,
+                                                running_mean, running_var, factor, count_dev=count,
+                                                num_batches_tracked=num_batches_tracked),
+            M_old, W, b, momentum, C, K, group, dev)
+        if GATE_LOG is not None:   # debug only: the gate the kernels applied, formed with the same expression
+            y = torch.empty_like(z)
+            capi.bn_apply(z, mean, invstd, g32, b32, x, y, True)
+            GATE_LOG.setdefault("writenet", []).append(y > 0)
+        ctx.K, ctx.momentum, ctx.group, ctx.sync_group = K, momentum, group, sync_group
+        ctx.wshape, ctx.wdtype = Wc.shape, Wc.dtype
+        ctx.set_materialize_grads(False)
+        ctx.save_for_backward(x, z, labels, M_new, saved, W, b, mean, invstd, g32, b32, count)
+        ctx.mark_non_differentiable(SD)
+        return M_new, losses[0], losses[1], SD
+
+    @staticmethod
+    def backward(ctx, dM_new, g_div, g_cls, _g_sd):
+        x, z, labels, M_new, saved, W, b, mean, invstd, g32, b32, count = ctx.saved_tensors
+        K = ctx.K
+        B, C, h, w = x.shape
+        dev = x.device
+        dS, dW, db = _write_update_bwd(ctx, dM_new, g_div, g_cls, M_new, saved, W, b, C, K)
+        dx = dWc = dgamma = dbeta = None
+        if any(ctx.needs_input_grad[i] for i in (0, 3, 4, 5)):
+            g = torch.empty_like(z)
+            dgamma = torch.empty(C, dtype=torch.float32, device=dev)
+            dbeta = torch.empty(C, dtype=torch.float32, device=dev)
+            capi.write_bwd_bn(dS, z, x, labels, mean, invstd, g32, b32, g, dgamma, dbeta, K)
+            sg, sb = dgamma, dbeta
+            if ctx.sync_group is not None:   # as _ConvBnActFn.backward: input gradient from the sums over all ranks
+                import torch.distributed as dist
+
+                sums = torch.cat([dgamma, dbeta])
+                dist.all_reduce(sums, group=ctx.sync_group)
+                sums = sums * (float(B * h * w) / count).to(torch.float32)
+                sg, sb = sums[:C].contiguous(), sums[C:].contiguous()
+            dz = torch.empty_like(z)
+            capi.bn_bwd_apply(g, None, None, z, mean, invstd, g32, sg, sb, False, True, dz, None)
+            if ctx.needs_input_grad[0]:
+                # dx = g + W^T . dz; before the weight gradient, so that a consumer of dx (the read's backward) is not
+                # queued behind it
+                hiT, loT = ctx.preT
+                dx = capi.conv1x1_fwd(dz, hiT, loT, C, y=g, accumulate=True)
+            if ctx.needs_input_grad[3]:
+                dWc = capi.conv1x1_wgrad(dz, x).view(ctx.wshape).to(ctx.wdtype)
+        return (dx, None, None, dWc, dgamma, dbeta, None, None, None, None, None, None, dW, db, None, None, None)
 
 
 class _MemoryLossFn(torch.autograd.Function):
@@ -900,8 +989,6 @@ class Memory_sup(nn.Module):
         if packed is not None and packed[0] is mask:   # same label tensor as the read of this forward(): reuse its pack
             labels = packed[1]
         self._packed = None
-        f = self.writenet(query)
-        f = _check_features(f, "write feature")
         M_old = self._memory_for_kernels(query.device)
         if M_old.requires_grad and torch.is_grad_enabled():
             # memory.py:236 blends the NON-detached self.m_items[slot]; forward() never gets here with a grad-carrying
@@ -909,11 +996,34 @@ class Memory_sup(nn.Module):
             # drop d loss / d m_items: refuse instead of returning a wrong gradient.
             raise RuntimeError("pinmem_b200: write() on a grad-carrying m_items is not differentiable w.r.t. the old memory "
                                "here; detach it first (forward(..., memory_writing=True) does)")
-        M_new, div_loss, cls_loss, SD = _WriteFn.apply(f, labels, M_old, self.clsfier.weight, self.clsfier.bias,
-                                                       float(self.momentum), self.memory_size, self.shard_group)
+        if self._writenet_fused(query):
+            conv, bn = self.writenet.writefeat[0], self.writenet.writefeat[1]
+            use_batch, rm, rv, factor, nbt = _bn_args(bn, defer_counter=True)
+            M_new, div_loss, cls_loss, SD = _WriteNetFn.apply(
+                query.contiguous(), labels, M_old, conv.weight, bn.weight, bn.bias, rm, rv, factor, float(bn.eps), nbt,
+                _sync_group(bn), self.clsfier.weight, self.clsfier.bias, float(self.momentum), self.memory_size,
+                self.shard_group)
+        else:
+            f = self.writenet(query)
+            f = _check_features(f, "write feature")
+            M_new, div_loss, cls_loss, SD = _WriteFn.apply(f, labels, M_old, self.clsfier.weight, self.clsfier.bias,
+                                                           float(self.momentum), self.memory_size, self.shard_group)
         self.last_class_sums = SD
         self.m_items = M_new.detach() if writing_detach else M_new
         return [div_loss, cls_loss]
+
+    def _writenet_fused(self, x):
+        """The writing net can ride in the write's kernels (_WriteNetFn): an unhooked Writingnet of a 1x1 convolution and a
+        training-mode BatchNorm2d / SyncBatchNorm, fp32 features on the pipelined kernels' alignment. Anything else (bf16,
+        autocast, eval-mode statistics, hooks, odd shapes) runs the Writingnet and _WriteFn as separate steps."""
+        wn = self.writenet
+        if not (type(wn) is Writingnet and _plain(wn) and _plain(wn.writefeat) and len(wn.writefeat) == 2):
+            return False
+        conv, bn = wn.writefeat[0], wn.writefeat[1]
+        C = x.shape[1]
+        return (_pointwise(conv) and _plain(conv) and conv.in_channels == C and conv.out_channels == C and _bn_fast(bn, x)
+                and bn.training and not torch.is_autocast_enabled("cuda") and x.dtype == torch.float32
+                and C in (32, 64, 128, 256) and capi.conv1x1_ok(x, C, C) and capi.planes_ok(x))
 
     # ----------------------------------------------------------------------- external entry points
 
