@@ -28,12 +28,14 @@
 extern "C" {
 #endif
 
-enum pm_dtype { PM_F32 = 0, PM_BF16 = 1 };
+/* PM_F32_TF32: fp32 tensors whose products run as ONE TF32 pass (operands rounded to nearest TF32, fp32 accumulation);
+ * accepted only by the pm_conv1x1_* entries and their size queries, PM_ERR_DTYPE everywhere else. */
+enum pm_dtype { PM_F32 = 0, PM_BF16 = 1, PM_F32_TF32 = 2 };
 
 enum pm_status {
     PM_OK = 0,
     PM_ERR_NULL = -1,      /* a required pointer is NULL */
-    PM_ERR_DTYPE = -2,     /* dtype not PM_F32 / PM_BF16 */
+    PM_ERR_DTYPE = -2,     /* dtype not PM_F32 / PM_BF16 (or PM_F32_TF32 where accepted) */
     PM_ERR_CHANNELS = -3,  /* C not in {32,64,128,256} */
     PM_ERR_SLOTS = -4,     /* K not in 1..31 */
     PM_ERR_SHAPE = -5,     /* a dimension is <= 0 or too large */
@@ -54,7 +56,7 @@ enum pm_readloss_ws_layout {
 #define PM_COLPART_ROWS 296
 
 /* Bumped with every prototype change; the binding refuses a library whose pm_version() differs. */
-#define PM_ABI_VERSION 212
+#define PM_ABI_VERSION 213
 int pm_version(void);
 const char* pm_status_string(int code);
 /* Row stride (floats) of the internal score buffers for K slots: 20 for K<=19, else 32. */
@@ -297,10 +299,13 @@ int pm_bn_bwd_apply(const void* dy, const void* y, const uint32_t* relu_mask, co
  * The two 1x1 convolutions themselves (memory.py:74-75 `Writingnet.writefeat[0]`, memory.py:103-104 `self.output[0]`,
  * both bias-free, applied at memory.py:84/214 and :334) and their autograd, as tcgen05 GEMMs on NCHW activations
  * (csrc/pm_gemm.cu). Per image b:   Y[b] (M x hw) = A (M x K) . X[b] (K x hw).
- *   dtype PM_F32 computes in 3xTF32 (error-compensated, ~fp32 accuracy), PM_BF16 in bf16 with fp32 accumulation.
+ *   dtype PM_F32 computes in 3xTF32 (error-compensated, ~fp32 accuracy), PM_BF16 in bf16 with fp32 accumulation,
+ *   PM_F32_TF32 on fp32 tensors in one TF32 pass (weights and activation tiles rounded to nearest TF32: ~2^-11 per
+ *   product, unbiased; A_lo / At_lo are unused and may be NULL).
  *
  *   pm_conv1x1_prep   A = W (transpose = 0, W is [M,K] fp32) or W^T (transpose = 1, W is [K,M] fp32), padded with
  *                     zero rows to Mpad = ceil(M/128)*128. PM_F32: A_hi, A_lo are fp32 [Mpad,K] (the TF32 split);
+ *                     PM_F32_TF32: A_hi fp32 [Mpad,K] (W rounded to nearest TF32), A_lo unused;
  *                     PM_BF16: A_hi is bf16 [Mpad,K], A_lo unused. transpose = 0 prepares the forward convolution,
  *                     transpose = 1 its input gradient (dX[b] = W^T . dY[b]).
  *   pm_conv1x1_fwd    X [B,K,hw], Y [B,M,hw] in `dtype`; A_hi/A_lo from pm_conv1x1_prep. accumulate != 0 adds into Y

@@ -11,7 +11,7 @@ import torch
 
 from . import build as _build
 
-PM_F32, PM_BF16 = 0, 1
+PM_F32, PM_BF16, PM_F32_TF32 = 0, 1, 2
 WS_WORDS = 40  # PM_WS_WORDS
 WS_HIST = 4    # PM_WS_HIST
 WS_BAD = 2     # PM_WS_BAD
@@ -19,7 +19,7 @@ WS_BAD = 2     # PM_WS_BAD
 SEG_WS_WORDS = 4  # PM_SEG_WS_WORDS
 SEG_WS_BAD = 2    # PM_SEG_WS_BAD
 
-ABI_VERSION = 212  # PM_ABI_VERSION of include/pinmem_b200.h the argtypes below were written against
+ABI_VERSION = 213  # PM_ABI_VERSION of include/pinmem_b200.h the argtypes below were written against
 
 _c_p = ctypes.c_void_p
 _c_i = ctypes.c_int
@@ -260,6 +260,14 @@ def deterministic():
     return torch.are_deterministic_algorithms_enabled()
 
 
+def tf32():
+    """torch's TF32 switches, read at call time: True when torch would run BOTH an fp32 matmul
+    (``torch.backends.cuda.matmul.allow_tf32``, which ``torch.set_float32_matmul_precision("high" / "medium")`` sets) and an
+    fp32 cuDNN convolution (``torch.backends.cudnn.allow_tf32``) in TF32. The fp32 1x1-convolution GEMMs then run one TF32
+    pass instead of 3xTF32. A 1x1 convolution is a convolution to the user and a matmul here, so it takes both."""
+    return bool(torch.backends.cuda.matmul.allow_tf32 and torch.backends.cudnn.allow_tf32)
+
+
 def _scratch(nbytes, device, what):
     """Scratch of an ordered entry from torch's allocator (its contents on entry do not matter)."""
     if nbytes < 0:
@@ -475,35 +483,55 @@ def bn_bwd_apply(dy, y, relu_mask, x, mean, invstd, gamma, dgamma, dbeta, relu, 
 # ------------------------------------------------------------------------ 1x1 convolutions (csrc/pm_gemm.cu)
 
 
-def conv1x1_prep(W2d, transpose, dtype):
+def _prep_code(dtype, tf32):
+    if dtype != torch.float32:
+        return PM_BF16
+    return PM_F32_TF32 if tf32 else PM_F32
+
+
+def conv1x1_prep(W2d, transpose, dtype, tf32=False):
     """W2d fp32 [R,S] -> operand A = W2d (transpose False: M=R, K=S) or W2d^T (True: M=S, K=R), zero-padded to a multiple
-    of 128 rows; fp32 returns (A_hi, A_lo) fp32, bf16 returns (A, None)."""
+    of 128 rows; fp32 returns (A_hi, A_lo) fp32 -- with ``tf32``, (A rounded to TF32, None): the operand of a one-pass TF32
+    GEMM --, bf16 returns (A, None)."""
     R, S = W2d.shape
     M, K = (S, R) if transpose else (R, S)
     Mpad = (M + 127) // 128 * 128
     W2d = _f32c(W2d, "weight")
+    code = _prep_code(dtype, tf32)
     hi = torch.empty(Mpad, K, dtype=dtype, device=W2d.device)
-    lo = torch.empty(Mpad, K, dtype=dtype, device=W2d.device) if dtype == torch.float32 else None
-    _call("pm_conv1x1_prep", _ptr(W2d), M, K, int(bool(transpose)), PM_F32 if dtype == torch.float32 else PM_BF16,
-          _ptr(hi), _ptr(lo), _stream())
+    lo = torch.empty(Mpad, K, dtype=dtype, device=W2d.device) if code == PM_F32 else None
+    _call("pm_conv1x1_prep", _ptr(W2d), M, K, int(bool(transpose)), code, _ptr(hi), _ptr(lo), _stream())
     return hi, lo
 
 
-def conv1x1_prep_both(W2d, dtype, zero=None):
+def conv1x1_prep_both(W2d, dtype, zero=None, tf32=False):
     """((A_hi, A_lo), (At_hi, At_lo)): conv1x1_prep(W2d, False) and conv1x1_prep(W2d, True) from one launch, which also
     clears the float64 buffer ``zero`` (the BatchNorm statistics the forward GEMM's epilogue adds into)."""
     R, S = W2d.shape
     W2d = _f32c(W2d, "weight")
-    f32 = dtype == torch.float32
+    code = _prep_code(dtype, tf32)
     hi = torch.empty((R + 127) // 128 * 128, S, dtype=dtype, device=W2d.device)
-    lo = torch.empty_like(hi) if f32 else None
+    lo = torch.empty_like(hi) if code == PM_F32 else None
     hiT = torch.empty((S + 127) // 128 * 128, R, dtype=dtype, device=W2d.device)
-    loT = torch.empty_like(hiT) if f32 else None
+    loT = torch.empty_like(hiT) if code == PM_F32 else None
     if zero is not None and (zero.dtype != torch.float64 or not zero.is_contiguous()):
         raise ValueError("conv1x1_prep_both: `zero` must be a contiguous float64 tensor")
-    _call("pm_conv1x1_prep_both", _ptr(W2d), R, S, PM_F32 if f32 else PM_BF16, _ptr(hi), _ptr(lo), _ptr(hiT), _ptr(loT),
+    _call("pm_conv1x1_prep_both", _ptr(W2d), R, S, code, _ptr(hi), _ptr(lo), _ptr(hiT), _ptr(loT),
           _ptr(zero), 0 if zero is None else zero.numel(), _stream())
     return (hi, lo), (hiT, loT)
+
+
+def operands_tf32(ops):
+    """True for fp32 operands conv1x1_prep[_both] made with ``tf32`` (no lo part): the GEMMs on them run one TF32 pass."""
+    return ops[0].dtype == torch.float32 and ops[1] is None
+
+
+def _gemm_code(x, A_lo):
+    """dtype code of a GEMM on x with prepared operands: the operands carry the mode they were prepared for, so a
+    forward and the backward that reuses its operands cannot disagree."""
+    if x.dtype == torch.float32 and A_lo is None:
+        return PM_F32_TF32
+    return dtype_code(x)
 
 
 def conv1x1_ok(x, M, K):
@@ -516,30 +544,33 @@ def conv1x1_ok(x, M, K):
 
 
 def conv1x1_fwd(x, A_hi, A_lo, M, y=None, stats=None, accumulate=False):
-    """y[b] (M x hw) (+)= A (M x K) . x[b] (K x hw); stats: zeroed double[2M] receiving per-row sum / sum of squares."""
+    """y[b] (M x hw) (+)= A (M x K) . x[b] (K x hw); stats: zeroed double[2M] receiving per-row sum / sum of squares.
+    The operands choose the mode: fp32 x with A_lo None (conv1x1_prep(..., tf32=True)) runs one TF32 pass, fp32 x with
+    A_lo 3xTF32."""
     B, K, h, w = x.shape
     if y is None:
         y = torch.empty(B, M, h, w, dtype=x.dtype, device=x.device)
     if stats is not None and not accumulate and deterministic():
-        nbytes = load().pm_conv1x1_stats_scratch_bytes(B, M, h * w, dtype_code(x))
+        nbytes = load().pm_conv1x1_stats_scratch_bytes(B, M, h * w, _gemm_code(x, A_lo))
         scratch = _scratch(nbytes, x.device, "pm_conv1x1_stats_scratch_bytes")
         _call("pm_conv1x1_fwd_ordered", _ptr(x), _ptr(A_hi), _ptr(A_lo), _ptr(y), _ptr(stats), _ptr(scratch), B, K, M, h * w,
-              dtype_code(x), _stream())
+              _gemm_code(x, A_lo), _stream())
         return y
     _call("pm_conv1x1_fwd", _ptr(x), _ptr(A_hi), _ptr(A_lo), _ptr(y), _ptr(stats), B, K, M, h * w, int(bool(accumulate)),
-          dtype_code(x), _stream())
+          _gemm_code(x, A_lo), _stream())
     return y
 
 
 def conv1x1_dgrad_bnbwd(dy, z, A_hi, A_lo, M, mean, invstd, gamma, dgamma, dbeta, beta, relu, training):
     """(dx [B,M,h,w], dz [B,K,h,w]): input gradient of conv1x1 -> BatchNorm (-> ReLU) with the BatchNorm backward formed in
-    the GEMM's operand path; dz is stored for the weight-gradient GEMM (fp32 only)."""
+    the GEMM's operand path; dz is stored for the weight-gradient GEMM (fp32 only). A_lo None (operands prepared with
+    ``tf32``): one TF32 pass on the rounded dz; the stored dz is the fp32 value either way."""
     B, K, h, w = dy.shape
     dx = torch.empty(B, M, h, w, dtype=dy.dtype, device=dy.device)
     dz = torch.empty_like(dy)
     _call("pm_conv1x1_dgrad_bnbwd", _ptr(dy), _ptr(z), _ptr(A_hi), _ptr(A_lo), _ptr(dx), _ptr(dz), _ptr(mean), _ptr(invstd),
           _ptr(gamma), _ptr(beta), _ptr(dgamma), _ptr(dbeta), int(bool(relu)), int(bool(training)), B, K, M, h * w,
-          dtype_code(dy), _stream())
+          _gemm_code(dy, A_lo), _stream())
     return dx, dz
 
 
@@ -554,24 +585,25 @@ def bn_eval_affine(gamma, beta, running_mean, running_var, eps):
 
 
 def conv1x1_fwd_affine(x, A_hi, A_lo, M, scale, shift, relu):
-    """y[b] = [relu](scale[m] * (A . x[b]) + shift[m]) -- convolution + eval-mode BatchNorm (+ ReLU) in one kernel."""
+    """y[b] = [relu](scale[m] * (A . x[b]) + shift[m]) -- convolution + eval-mode BatchNorm (+ ReLU) in one kernel; fp32
+    with A_lo None (operands prepared with ``tf32``) runs one TF32 pass."""
     B, K, h, w = x.shape
     y = torch.empty(B, M, h, w, dtype=x.dtype, device=x.device)
     _call("pm_conv1x1_fwd_affine", _ptr(x), _ptr(A_hi), _ptr(A_lo), _ptr(y), _ptr(scale), _ptr(shift), int(bool(relu)), B, K, M,
-          h * w, dtype_code(x), _stream())
+          h * w, _gemm_code(x, A_lo), _stream())
     return y
 
 
-def conv1x1_wgrad(dy, x, dW=None, accumulate=False):
-    """dW [M,N] fp32 (+)= sum_b dy[b] (M x hw) . x[b]^T (hw x N)."""
+def conv1x1_wgrad(dy, x, dW=None, accumulate=False, tf32=False):
+    """dW [M,N] fp32 (+)= sum_b dy[b] (M x hw) . x[b]^T (hw x N); fp32 with ``tf32``: one TF32 pass."""
     B, M, h, w = dy.shape
     N = x.shape[1]
     if dW is None:
         dW = torch.empty(M, N, dtype=torch.float32, device=x.device)
-    nws = load().pm_conv1x1_wgrad_workspace_floats(B, M, N, h * w, dtype_code(x))
+    code = PM_F32_TF32 if (tf32 and x.dtype == torch.float32) else dtype_code(x)
+    nws = load().pm_conv1x1_wgrad_workspace_floats(B, M, N, h * w, code)
     ws = torch.empty(nws, dtype=torch.float32, device=x.device)
-    _call("pm_conv1x1_wgrad", _ptr(dy), _ptr(x), _ptr(ws), _ptr(dW), B, M, N, h * w, int(bool(accumulate)), dtype_code(x),
-          _stream())
+    _call("pm_conv1x1_wgrad", _ptr(dy), _ptr(x), _ptr(ws), _ptr(dW), B, M, N, h * w, int(bool(accumulate)), code, _stream())
     return dW
 
 

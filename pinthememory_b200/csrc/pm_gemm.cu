@@ -16,7 +16,8 @@
 //     fp32): plain TF32 (2^-11 per product) cannot hold the 1e-5 parity bar. The weights are
 //     split once per call by `conv1x1_prep_kernel`; the activation tiles are split in shared memory by four
 //     transform warps (same swizzled offset in a second buffer, so no layout change). bf16 I/O is one
-//     `kind::f16` pass straight from the TMA tiles;
+//     `kind::f16` pass straight from the TMA tiles. PM_F32_TF32 (torch's TF32 switches on) is one `kind::tf32` pass
+//     on fp32 tiles the transform warps round to nearest TF32 in place (element type Tf32OnePass);
 //   * epilogue warps read TMEM with `tcgen05.ld` (thread = output channel, registers = 32 consecutive pixels), so
 //     the per-channel sum and sum of squares of the BatchNorm that follows are thread-local register sums
 //     (fp64 across tiles, one atomicAdd per channel per CTA); the tile goes out through a swizzled shared-memory
@@ -31,6 +32,15 @@ constexpr int GEMM_THREADS = 320;  // warp 0 TMA producer, 1 MMA issuer (+TMEM o
 constexpr int GEMM_RING_BYTES = 192 * 1024;
 constexpr int TILE_A_BYTES = 128 * 128;  // one 128-row K-major operand block: [128 rows][128 bytes]
 
+// fp32 I/O computed in ONE kind::tf32 pass (PM_F32_TF32): the element type of the kernels that run it. BN = the launch
+// forms dz in its operand path (pm_conv1x1_dgrad_bnbwd), which needs a second activation buffer per stage.
+template <bool BN>
+struct Tf32OnePass {
+    float v;
+};
+
+// SPLIT: 3xTF32 (hi/lo operands, three MMAs per K step); XFORM: the transform warps touch every activation tile (split or
+// round it, or form dz); XBUF: activation buffers per stage; BNB: may form dz; MAXST: ring stages at most
 template <typename T>
 struct GemmTraits;
 template <>
@@ -38,14 +48,25 @@ struct GemmTraits<float> {
     static constexpr int PXC = 32;   // elements per 128-byte row
     static constexpr int UK = 8;     // K per tcgen05.mma (32 bytes)
     static constexpr uint32_t FMT = UMMA_FMT_TF32;
-    static constexpr bool SPLIT = true;
+    static constexpr bool SPLIT = true, XFORM = true, BNB = true;
+    static constexpr int XBUF = 2, MAXST = 4;
+};
+template <bool BN>
+struct GemmTraits<Tf32OnePass<BN>> {
+    static constexpr int PXC = 32;
+    static constexpr int UK = 8;
+    static constexpr uint32_t FMT = UMMA_FMT_TF32;
+    static constexpr bool SPLIT = false, XFORM = true, BNB = BN;
+    // without lo buffers a stage is half as large: up to 6 fit the ring (the barrier block holds 4 x 6 + 2 x 2 words)
+    static constexpr int XBUF = BN ? 2 : 1, MAXST = 6;
 };
 template <>
 struct GemmTraits<__nv_bfloat16> {
     static constexpr int PXC = 64;
     static constexpr int UK = 16;
     static constexpr uint32_t FMT = UMMA_FMT_BF16;
-    static constexpr bool SPLIT = false;
+    static constexpr bool SPLIT = false, XFORM = false, BNB = false;
+    static constexpr int XBUF = 1, MAXST = 4;
 };
 
 template <typename T>
@@ -76,6 +97,16 @@ __device__ __forceinline__ void split_tile_trunc(const float4* __restrict__ raw,
     }
 }
 __device__ __forceinline__ float tf32_rn(float x) { return __uint_as_float((__float_as_uint(x) + 0x00001000u) & 0xffffe000u); }
+// one-pass TF32: the activation tile rounded to nearest TF32 in place. Left raw, the tensor core would truncate it, which
+// lowers every operand's magnitude by up to one TF32 ulp (2^-10 relative): a bias, not noise -- a weight gradient, whose
+// operands are both activations, would come out scaled down by a few 1e-4. Rounded, the errors are symmetric and cancel.
+__device__ __forceinline__ void round_tile(float4* __restrict__ raw, int n4, int t, int nthreads) {
+    for (int i = t; i < n4; i += nthreads) {
+        float4 v = raw[i];
+        v.x = tf32_rn(v.x), v.y = tf32_rn(v.y), v.z = tf32_rn(v.z), v.w = tf32_rn(v.w);
+        raw[i] = v;
+    }
+}
 __device__ __forceinline__ void split_tile(float4* __restrict__ raw, float4* __restrict__ lo, int n4, int t, int nthreads) {
     for (int i = t; i < n4; i += nthreads) {
         const float4 v = raw[i];
@@ -101,7 +132,9 @@ struct BnBwdArgs {
     int training, relu;
 };
 
-template <int KB>
+// SPLIT (3xTF32): dz -> dy buffer (the "hi" operand and the stored tile), dz - trunc(dz) -> z buffer ("lo").
+// one pass: tf32_rn(dz) -> dy buffer (the operand), dz -> z buffer (the stored tile keeps every fp32 bit).
+template <int KB, bool SPLIT>
 __device__ __forceinline__ void bnbwd_tile(float4* __restrict__ dy_hi, float4* __restrict__ z_lo, int n4, int t, int nthreads,
                                            int ch0, const BnBwdArgs& bn) {
     // 8 float4 per 128-byte row, KB rows per 32-pixel chunk: float4 i belongs to row (i >> 3) % KB. With 128 threads and
@@ -123,7 +156,8 @@ __device__ __forceinline__ void bnbwd_tile(float4* __restrict__ dy_hi, float4* _
             const float gv = (!bn.relu || fmaf(z.f, sc, sh) > 0.f) ? g.f : 0.f;          \
             const float xh = (z.f - mu) * is;                                            \
             d.f = sc * (gv - k1 - xh * k2);                                              \
-            l.f = d.f - __uint_as_float(__float_as_uint(d.f) & 0xffffe000u);             \
+            if (SPLIT) l.f = d.f - __uint_as_float(__float_as_uint(d.f) & 0xffffe000u);  \
+            else l.f = d.f, d.f = tf32_rn(d.f);                                          \
         }
         PM_BNBWD_ONE(x) PM_BNBWD_ONE(y) PM_BNBWD_ONE(z) PM_BNBWD_ONE(w)
 #undef PM_BNBWD_ONE
@@ -149,18 +183,18 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
                       const __grid_constant__ CUtensorMap mapZ, const __grid_constant__ CUtensorMap mapDZ, const BnBwdArgs bn) {
     using TR = GemmTraits<T>;
     constexpr int PXC = TR::PXC, UK = TR::UK, KSTEPS = KB / UK;
-    const bool bnbwd = TR::SPLIT && bn.mean != nullptr;  // X = dy, Z = saved conv output: dz formed in the split stage
+    const bool bnbwd = TR::BNB && bn.mean != nullptr;  // X = dy, Z = saved conv output: dz formed in the split stage
     constexpr int NCH = NT / PXC;                      // 128-byte pixel chunks per tile
     constexpr int XCHUNK = KB * 128;                   // bytes of one [KB rows][128 B] chunk
     constexpr int XBYTES = NCH * XCHUNK;               // = NT * KB * sizeof(T)
-    constexpr int NOPA = TR::SPLIT ? 2 : 1;
+    constexpr int NOPA = TR::SPLIT ? 2 : 1, XB = TR::XBUF;  // weight operands (hi[, lo]), activation buffers
     // weight block: [128 rows][KB channels] K-major; 128-byte rows use SWIZZLE_128B, 64-byte rows SWIZZLE_64B
     constexpr int AROW = KB * (int)sizeof(T);
     static_assert(AROW == 128 || AROW == 64, "weight rows must be 64 or 128 bytes");
     constexpr int TILE_A = 128 * AROW;
     constexpr uint32_t ASWZ = AROW == 128 ? UMMA_SW128 : UMMA_SW64, ASBO = 8 * AROW;
-    constexpr int STAGE = NOPA * (XBYTES + MT * TILE_A);
-    constexpr int STAGES = (GEMM_RING_BYTES / STAGE) > 4 ? 4 : (GEMM_RING_BYTES / STAGE);
+    constexpr int STAGE = XB * XBYTES + NOPA * MT * TILE_A;
+    constexpr int STAGES = (GEMM_RING_BYTES / STAGE) > TR::MAXST ? TR::MAXST : (GEMM_RING_BYTES / STAGE);
     constexpr int ACC = (512 / (MT * NT)) >= 2 ? 2 : 1;  // accumulator stages in TMEM
     constexpr uint32_t TX = XBYTES + NOPA * MT * TILE_A;
     static_assert(STAGES >= 2, "ring too small");
@@ -173,7 +207,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
     uint64_t* bars = reinterpret_cast<uint64_t*>(stg + 4 * 2 * 4096);
     uint64_t* full = bars;                 // [STAGES] TMA landed
     uint64_t* empty = bars + STAGES;       // [STAGES] MMAs of the stage retired
-    uint64_t* xfull = bars + 2 * STAGES;   // [STAGES] lo parts written (fp32)
+    uint64_t* xfull = bars + 2 * STAGES;   // [STAGES] activation tile transformed (fp32)
     uint64_t* accf = bars + 3 * STAGES;    // [ACC] accumulator complete
     uint64_t* acce = accf + ACC;           // [ACC] accumulator drained
     uint64_t* sfree = acce + ACC;          // [STAGES] the dz store of the stage has left shared memory (bnbwd only)
@@ -222,7 +256,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
                         for (int c = 0; c < NCH; ++c)
                             tma_load_2d(st + XBYTES + c * XCHUNK, &mapZ, px0 + c * PXC, b * K + kb * KB, &full[s]);
                     }
-                    unsigned char* sa = st + NOPA * XBYTES;
+                    unsigned char* sa = st + XB * XBYTES;
 #pragma unroll
                     for (int j = 0; j < NOPA * MT; ++j) {  // weight blocks: [hi of every row tile | lo of every row tile]
                         const int mt = j % MT;
@@ -242,10 +276,10 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
                     const int s = it % STAGES;
                     const uint32_t ph = (it / STAGES) & 1;
                     mbar_wait(&full[s], ph);
-                    if (TR::SPLIT) mbar_wait(&xfull[s], ph);
+                    if (TR::XFORM) mbar_wait(&xfull[s], ph);
                     tc_fence_after();
                     const uint32_t sx = smem_u32(smem + s * STAGE);
-                    const uint32_t sa = sx + NOPA * XBYTES;
+                    const uint32_t sa = sx + XB * XBYTES;
                     int ksteps = (K - kb * KB) / UK;
                     if (ksteps > KSTEPS) ksteps = KSTEPS;
                     for (int ks = 0; ks < ksteps; ++ks) {
@@ -406,8 +440,8 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
                 }
             }
         }
-    } else {  // --------------------------------------------------------------- operand split (fp32 only)
-        if constexpr (TR::SPLIT) {
+    } else {  // ---------------------------------------------------------- operand transform (fp32 only)
+        if constexpr (TR::XFORM) {
             const int t = threadIdx.x - 6 * 32;
             uint32_t it = 0;
             for (int tile = tile0; tile < total_tiles; tile += tile_stride) {
@@ -416,8 +450,9 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
                     const int s = it % STAGES;
                     mbar_wait(&full[s], (it / STAGES) & 1);
                     unsigned char* st = smem + s * STAGE;
-                    if (bnbwd) bnbwd_tile<KB>(reinterpret_cast<float4*>(st), reinterpret_cast<float4*>(st + XBYTES), XBYTES / 16, t, 128, kb * KB, bn);
-                    else split_tile_trunc(reinterpret_cast<float4*>(st), reinterpret_cast<float4*>(st + XBYTES), XBYTES / 16, t, 128);
+                    if (bnbwd) bnbwd_tile<KB, TR::SPLIT>(reinterpret_cast<float4*>(st), reinterpret_cast<float4*>(st + XBYTES), XBYTES / 16, t, 128, kb * KB, bn);
+                    else if (TR::SPLIT) split_tile_trunc(reinterpret_cast<float4*>(st), reinterpret_cast<float4*>(st + XBYTES), XBYTES / 16, t, 128);
+                    else round_tile(reinterpret_cast<float4*>(st), XBYTES / 16, t, 128);
                     fence_proxy_async_smem();
                     __syncwarp();
                     if (lane == 0) mbar_arrive(&xfull[s]);
@@ -427,7 +462,8 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
                         // refilled once the MMAs AND this store have read it
                         mbar_wait(&xfull[s], (it / STAGES) & 1);
 #pragma unroll
-                        for (int c = 0; c < NCH; ++c) tma_store_2d(&mapDZ, px0 + c * PXC, b * K + kb * KB, st + c * XCHUNK);
+                        for (int c = 0; c < NCH; ++c)   // (the fp32 dz: in the dy buffer for 3xTF32, in the z buffer for one pass)
+                            tma_store_2d(&mapDZ, px0 + c * PXC, b * K + kb * KB, st + (TR::SPLIT ? 0 : XBYTES) + c * XCHUNK);
                         bulk_commit();
                         bulk_wait_read<1>();  // every store but the one just issued has left shared memory
                         if (it > 0) mbar_arrive(&sfree[(it - 1) % STAGES]);
@@ -449,8 +485,8 @@ template <typename T, int MT, int NT, int KB>
 constexpr size_t nn_smem_bytes() {
     using TR = GemmTraits<T>;
     constexpr int NOPA = TR::SPLIT ? 2 : 1;
-    constexpr int STAGE = NOPA * (NT * KB * (int)sizeof(T) + MT * 128 * KB * (int)sizeof(T));
-    constexpr int STAGES = (GEMM_RING_BYTES / STAGE) > 4 ? 4 : (GEMM_RING_BYTES / STAGE);
+    constexpr int STAGE = TR::XBUF * NT * KB * (int)sizeof(T) + NOPA * MT * 128 * KB * (int)sizeof(T);
+    constexpr int STAGES = (GEMM_RING_BYTES / STAGE) > TR::MAXST ? TR::MAXST : (GEMM_RING_BYTES / STAGE);
     return (size_t)STAGES * STAGE + 4 * 2 * 4096 + 256 + 1024;
 }
 
@@ -462,7 +498,7 @@ static int launch_nn(const void* X, const void* Ah, const void* Al, void* Y, dou
     CUtensorMap mX, mAh, mAl, mY, mZ, mDZ;
     BnBwdArgs bn{};
     if (bnargs != nullptr && Z != nullptr && DZ != nullptr) {
-        if (!TR::SPLIT || K % KB != 0) return PM_ERR_SHAPE;
+        if (!TR::BNB || K % KB != 0) return PM_ERR_SHAPE;
         bn = *bnargs;
         if (!make_map_2d<T>(&mZ, Z, (size_t)B * K, hw, KB, TR::PXC, 2)) return PM_ERR_ALIGN;
         if (!make_map_2d<T>(&mDZ, DZ, (size_t)B * K, hw, KB, TR::PXC, 2)) return PM_ERR_ALIGN;
@@ -567,7 +603,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
                 const int s = kb % STAGES;
                 const uint32_t ph = (kb / STAGES) & 1;
                 mbar_wait(&full[s], ph);
-                if (TR::SPLIT) mbar_wait(&xfull[s], ph);
+                if (TR::XFORM) mbar_wait(&xfull[s], ph);
                 tc_fence_after();
                 const uint32_t sa = smem_u32(smem + s * STAGE);
                 const uint32_t sb = sa + NOPA * TILE_A_BYTES;
@@ -612,15 +648,20 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
             for (int c = 0; c < N / 4; ++c) *reinterpret_cast<uint4*>(dst + 4 * c) = make_uint4(0u, 0u, 0u, 0u);
         }
     } else {
-        if constexpr (TR::SPLIT) {
+        if constexpr (TR::XFORM) {
             const int t = threadIdx.x - 6 * 32;
             for (int kb = 0; kb < nkb; ++kb) {
                 const int s = kb % STAGES;
                 mbar_wait(&full[s], (kb / STAGES) & 1);
                 unsigned char* st = smem + s * STAGE;
-                split_tile_trunc(reinterpret_cast<float4*>(st), reinterpret_cast<float4*>(st + TILE_A_BYTES), TILE_A_BYTES / 16, t, 128);
-                split_tile_trunc(reinterpret_cast<float4*>(st + 2 * TILE_A_BYTES), reinterpret_cast<float4*>(st + 2 * TILE_A_BYTES + BBYTES),
-                                 N * 8, t, 128);
+                if (TR::SPLIT) {
+                    split_tile_trunc(reinterpret_cast<float4*>(st), reinterpret_cast<float4*>(st + TILE_A_BYTES), TILE_A_BYTES / 16, t, 128);
+                    split_tile_trunc(reinterpret_cast<float4*>(st + 2 * TILE_A_BYTES), reinterpret_cast<float4*>(st + 2 * TILE_A_BYTES + BBYTES),
+                                     N * 8, t, 128);
+                } else {
+                    round_tile(reinterpret_cast<float4*>(st), TILE_A_BYTES / 16, t, 128);
+                    round_tile(reinterpret_cast<float4*>(st + TILE_A_BYTES), N * 8, t, 128);
+                }
                 fence_proxy_async_smem();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&xfull[s]);
@@ -719,7 +760,8 @@ static int launch_wgrad(const void* dY, const void* X, float* part, float* dW, i
 }
 
 // A[m][k] = W[m][k] (transpose = 0, W is [M][K]) or W[k][m] (transpose = 1, W is [K][M]); rows M..Mpad-1 are zero.
-// fp32: hi = W rounded to nearest TF32, lo = W - hi (both fp32 [Mpad][K]); bf16: hi = bf16(W).
+// fp32: hi = W rounded to nearest TF32, lo = W - hi (both fp32 [Mpad][K]; lo == nullptr: one-pass TF32, hi only);
+// bf16: hi = bf16(W).
 template <typename T>
 __global__ void conv1x1_prep_kernel(const float* __restrict__ W, int M, int K, int Mpad, int transpose, T* __restrict__ hi,
                                     T* __restrict__ lo) {
@@ -730,7 +772,7 @@ __global__ void conv1x1_prep_kernel(const float* __restrict__ W, int M, int K, i
     if constexpr (sizeof(T) == 4) {
         const float h = tf32_rn(v);
         hi[i] = h;
-        lo[i] = v - h;
+        if (lo != nullptr) lo[i] = v - h;
     } else {
         hi[i] = __float2bfloat16_rn(v);
     }
@@ -757,7 +799,7 @@ __global__ void conv1x1_prep_both_kernel(const float* __restrict__ W, int R, int
     if constexpr (sizeof(T) == 4) {
         const float h = tf32_rn(v);
         h_out[i] = h;
-        l_out[i] = v - h;
+        if (l_out != nullptr) l_out[i] = v - h;
     } else {
         h_out[i] = __float2bfloat16_rn(v);
     }
@@ -772,13 +814,15 @@ extern "C" {
 int pm_conv1x1_prep_both(const float* W, int R, int S, int dtype, void* A_hi, void* A_lo, void* At_hi, void* At_lo, double* zero,
                          int zero_n, void* stream) {
     if (!W || !A_hi || !At_hi || (dtype == PM_F32 && (!A_lo || !At_lo))) return PM_ERR_NULL;
-    if (dtype != PM_F32 && dtype != PM_BF16) return PM_ERR_DTYPE;
+    if (dtype != PM_F32 && dtype != PM_BF16 && dtype != PM_F32_TF32) return PM_ERR_DTYPE;
     if (R <= 0 || S <= 0 || zero_n < 0 || (zero_n > 0 && !zero)) return PM_ERR_SHAPE;
     const int n0 = (R + 127) / 128 * 128 * S, n1 = (S + 127) / 128 * 128 * R, n = n0 > n1 ? n0 : n1;
     cudaStream_t st = (cudaStream_t)stream;
     const dim3 grid((n + 255) / 256, 2);
     if (dtype == PM_F32)
         conv1x1_prep_both_kernel<float><<<grid, 256, 0, st>>>(W, R, S, (float*)A_hi, (float*)A_lo, (float*)At_hi, (float*)At_lo, zero, zero_n);
+    else if (dtype == PM_F32_TF32)
+        conv1x1_prep_both_kernel<float><<<grid, 256, 0, st>>>(W, R, S, (float*)A_hi, nullptr, (float*)At_hi, nullptr, zero, zero_n);
     else
         conv1x1_prep_both_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(W, R, S, (__nv_bfloat16*)A_hi, nullptr, (__nv_bfloat16*)At_hi, nullptr, zero, zero_n);
     PM_CHECK_LAUNCH();
@@ -787,26 +831,43 @@ int pm_conv1x1_prep_both(const float* W, int R, int S, int dtype, void* A_hi, vo
 
 int pm_conv1x1_prep(const float* W, int M, int K, int transpose, int dtype, void* A_hi, void* A_lo, void* stream) {
     if (!W || !A_hi || (dtype == PM_F32 && !A_lo)) return PM_ERR_NULL;
-    if (dtype != PM_F32 && dtype != PM_BF16) return PM_ERR_DTYPE;
+    if (dtype != PM_F32 && dtype != PM_BF16 && dtype != PM_F32_TF32) return PM_ERR_DTYPE;
     if (M <= 0 || K <= 0) return PM_ERR_SHAPE;
     const int Mpad = (M + 127) / 128 * 128, n = Mpad * K;
     cudaStream_t st = (cudaStream_t)stream;
     if (dtype == PM_F32)
         conv1x1_prep_kernel<float><<<(n + 255) / 256, 256, 0, st>>>(W, M, K, Mpad, transpose, (float*)A_hi, (float*)A_lo);
+    else if (dtype == PM_F32_TF32)
+        conv1x1_prep_kernel<float><<<(n + 255) / 256, 256, 0, st>>>(W, M, K, Mpad, transpose, (float*)A_hi, nullptr);
     else
         conv1x1_prep_kernel<__nv_bfloat16><<<(n + 255) / 256, 256, 0, st>>>(W, M, K, Mpad, transpose, (__nv_bfloat16*)A_hi, nullptr);
     PM_CHECK_LAUNCH();
     return 0;
 }
 
-extern "C++" {  // (a template inside the extern "C" block)
+extern "C++" {  // (templates inside the extern "C" block)
+// the fp32 tile shapes: 256-pixel tiles and 16-channel blocks -- a tile pulls the weights of its row tiles through the
+// SM's L2 port once per 256 pixels instead of once per 128 (the measured bound of the 128-pixel version); small maps keep
+// 128-pixel tiles so that more than a handful of SMs get work
+template <typename T, bool ORD>
+static int launch_f32_tiles(bool wide, int mt, const void* X, const void* A_hi, const void* A_lo, void* Y, double* stats, int B,
+                            int K, int M, int Mpad, int hw, int t0, int accumulate, const float* ep_scale, const float* ep_shift,
+                            int ep_relu, cudaStream_t st, const void* Z, void* DZ, const BnBwdArgs* bn) {
+    if (wide)
+        return mt == 2 ? launch_nn<T, 2, 256, 16, ORD>(X, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st, Z, DZ, bn)
+                       : launch_nn<T, 1, 256, 16, ORD>(X, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st, Z, DZ, bn);
+    return mt == 2 ? launch_nn<T, 2, 128, 32, ORD>(X, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st, Z, DZ, bn)
+                   : launch_nn<T, 1, 128, 32, ORD>(X, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st, Z, DZ, bn);
+}
+
 template <bool ORD = false>
 static int conv1x1_fwd_impl(const void* X, const void* A_hi, const void* A_lo, void* Y, double* stats, int B, int K, int M, int hw,
                             int accumulate, const float* ep_scale, const float* ep_shift, int ep_relu, int dtype, void* stream,
                             const void* Z = nullptr, void* DZ = nullptr, const BnBwdArgs* bn = nullptr) {
     if (!X || !A_hi || !Y || (dtype == PM_F32 && !A_lo) || ((ep_scale == nullptr) != (ep_shift == nullptr))) return PM_ERR_NULL;
-    if (dtype != PM_F32 && dtype != PM_BF16) return PM_ERR_DTYPE;
-    const int esz = dtype == PM_F32 ? 4 : 2, uk = dtype == PM_F32 ? 8 : 16;
+    if (dtype != PM_F32 && dtype != PM_BF16 && dtype != PM_F32_TF32) return PM_ERR_DTYPE;
+    const bool f32 = dtype != PM_BF16;
+    const int esz = f32 ? 4 : 2, uk = f32 ? 8 : 16;
     if (B <= 0 || hw <= 0 || K <= 0 || M <= 0 || K % uk || M % 32 || M > 512) return PM_ERR_SHAPE;
     if ((hw * esz) % 16 || ((uintptr_t)X | (uintptr_t)Y | (uintptr_t)A_hi | (uintptr_t)A_lo) % 16) return PM_ERR_ALIGN;
     cudaStream_t st = (cudaStream_t)stream;
@@ -815,11 +876,8 @@ static int conv1x1_fwd_impl(const void* X, const void* A_hi, const void* A_lo, v
     for (int t0 = 0; t0 < mtiles; t0 += 2) {
         const int mt = mtiles - t0 >= 2 ? 2 : 1;
         int rc;
-        // fp32: 256-pixel tiles and 16-channel blocks -- a tile pulls the (hi, lo) weights of its row tiles through the
-        // SM's L2 port once per 256 pixels instead of once per 128 (the measured bound of the 128-pixel version);
-        // small maps keep 128-pixel tiles so that more than a handful of SMs get work
         const bool wide = (long long)B * ((hw + 255) / 256) >= 96;
-        if (dtype == PM_F32) {
+        if (f32) {
             // fused BatchNorm backward: the FIRST launch forms dz from (X = dy, Z) in its operand path and stores it to DZ
             // (every launch walks all K operand channels of its pixel tiles); the remaining row tiles read DZ
             const bool first = bn != nullptr && t0 == 0;
@@ -827,12 +885,12 @@ static int conv1x1_fwd_impl(const void* X, const void* A_hi, const void* A_lo, v
             const void* Zi = first ? Z : nullptr;
             void* DZo = first ? DZ : nullptr;
             const BnBwdArgs* bi = first ? bn : nullptr;
-            if (wide)
-                rc = mt == 2 ? launch_nn<float, 2, 256, 16, ORD>(Xin, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st, Zi, DZo, bi)
-                             : launch_nn<float, 1, 256, 16, ORD>(Xin, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st, Zi, DZo, bi);
-            else
-                rc = mt == 2 ? launch_nn<float, 2, 128, 32, ORD>(Xin, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st, Zi, DZo, bi)
-                             : launch_nn<float, 1, 128, 32, ORD>(Xin, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st, Zi, DZo, bi);
+            if (dtype == PM_F32)
+                rc = launch_f32_tiles<float, ORD>(wide, mt, Xin, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st, Zi, DZo, bi);
+            else if (bi == nullptr)
+                rc = launch_f32_tiles<Tf32OnePass<false>, ORD>(wide, mt, Xin, A_hi, A_hi, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st, Zi, DZo, bi);
+            else   // (only pm_conv1x1_dgrad_bnbwd forms dz, never with ordered statistics)
+                rc = launch_f32_tiles<Tf32OnePass<true>, false>(wide, mt, Xin, A_hi, A_hi, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st, Zi, DZo, bi);
         } else {
             rc = mt == 2 ? launch_nn<__nv_bfloat16, 2, 128, 64, ORD>(X, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st)
                          : launch_nn<__nv_bfloat16, 1, 128, 64, ORD>(X, A_hi, A_lo, Y, stats, B, K, M, Mpad, hw, t0, accumulate, ep_scale, ep_shift, ep_relu, st);
@@ -850,13 +908,13 @@ int pm_conv1x1_fwd(const void* X, const void* A_hi, const void* A_lo, void* Y, d
 
 // CTAs of the forward GEMM: each stores one [sum | sum of squares] partial in the ordered variant
 static int conv1x1_fwd_ctas(int B, int hw, int dtype) {
-    const bool wide = dtype == PM_F32 && (long long)B * ((hw + 255) / 256) >= 96;   // as conv1x1_fwd_impl chooses NT
+    const bool wide = dtype != PM_BF16 && (long long)B * ((hw + 255) / 256) >= 96;   // as conv1x1_fwd_impl chooses NT
     const long long total = (long long)B * ((hw + (wide ? 255 : 127)) / (wide ? 256 : 128));
     return (int)(total < 148 ? total : 148);
 }
 
 int pm_conv1x1_stats_scratch_bytes(int B, int M, int hw, int dtype) {
-    if (dtype != PM_F32 && dtype != PM_BF16) return PM_ERR_DTYPE;
+    if (dtype != PM_F32 && dtype != PM_BF16 && dtype != PM_F32_TF32) return PM_ERR_DTYPE;
     if (B <= 0 || hw <= 0 || M <= 0 || M % 32 || M > 512) return PM_ERR_SHAPE;
     return conv1x1_fwd_ctas(B, hw, dtype) * 2 * M * (int)sizeof(double);
 }
@@ -875,7 +933,7 @@ int pm_conv1x1_dgrad_bnbwd(const void* dY, const void* Z, const void* A_hi, cons
                            const float* mean, const float* invstd, const float* gamma, const float* beta, const float* dgamma,
                            const float* dbeta, int relu, int training, int B, int K, int M, int hw, int dtype, void* stream) {
     if (!Z || !dZ || !mean || !invstd || !gamma || !beta || !dgamma || !dbeta) return PM_ERR_NULL;
-    if (dtype != PM_F32) return PM_ERR_DTYPE;  // the operand path transforms fp32 tiles; bf16 keeps the separate pass
+    if (dtype != PM_F32 && dtype != PM_F32_TF32) return PM_ERR_DTYPE;  // the operand path transforms fp32 tiles; bf16 keeps the separate pass
     if (K % 32 || ((uintptr_t)Z | (uintptr_t)dZ) % 16) return PM_ERR_ALIGN;
     BnBwdArgs bn{mean, invstd, gamma, beta, dgamma, dbeta, 1.f / ((float)B * (float)hw), training, relu};
     return conv1x1_fwd_impl(dY, A_hi, A_lo, dX, nullptr, B, K, M, hw, 0, nullptr, nullptr, 0, dtype, stream, Z, dZ, &bn);
@@ -890,7 +948,7 @@ int pm_conv1x1_fwd_affine(const void* X, const void* A_hi, const void* A_lo, voi
 int pm_conv1x1_wgrad_workspace_floats(int B, int M, int N, int hw, int dtype) {
     if (B <= 0 || M <= 0 || N <= 0 || hw <= 0) return 0;
     int cpi, bpc;
-    wgrad_split(B, M, hw, dtype == PM_F32 ? 32 : 64, &cpi, &bpc);
+    wgrad_split(B, M, hw, (dtype == PM_F32 || dtype == PM_F32_TF32) ? 32 : 64, &cpi, &bpc);
     const int Mpad = (M + 127) / 128 * 128;
     const int nmax = N > WG_NMAX ? WG_NMAX : N;
     return B * cpi * Mpad * nmax;
@@ -899,8 +957,8 @@ int pm_conv1x1_wgrad_workspace_floats(int B, int M, int N, int hw, int dtype) {
 int pm_conv1x1_wgrad(const void* dY, const void* X, float* workspace, float* dW, int B, int M, int N, int hw, int accumulate,
                      int dtype, void* stream) {
     if (!dY || !X || !workspace || !dW) return PM_ERR_NULL;
-    if (dtype != PM_F32 && dtype != PM_BF16) return PM_ERR_DTYPE;
-    const int esz = dtype == PM_F32 ? 4 : 2;
+    if (dtype != PM_F32 && dtype != PM_BF16 && dtype != PM_F32_TF32) return PM_ERR_DTYPE;
+    const int esz = dtype == PM_BF16 ? 2 : 4;
     if (B <= 0 || hw <= 0 || M <= 0 || N <= 0 || M % 32 || N % 32 || M > 512 || N > 1024) return PM_ERR_SHAPE;
     if ((hw * esz) % 16 || ((uintptr_t)X | (uintptr_t)dY | (uintptr_t)workspace | (uintptr_t)dW) % 16) return PM_ERR_ALIGN;
     cudaStream_t st = (cudaStream_t)stream;
@@ -909,8 +967,9 @@ int pm_conv1x1_wgrad(const void* dY, const void* X, float* workspace, float* dW,
     for (int n0 = 0; n0 < N;) {
         int nb = N - n0;
         if (nb > WG_NMAX) nb = 256;
-        const int rc = dtype == PM_F32 ? launch_wgrad<float>(dY, X, workspace, dW, B, M, N, n0, nb, hw, accumulate, st)
-                                       : launch_wgrad<__nv_bfloat16>(dY, X, workspace, dW, B, M, N, n0, nb, hw, accumulate, st);
+        const int rc = dtype == PM_F32        ? launch_wgrad<float>(dY, X, workspace, dW, B, M, N, n0, nb, hw, accumulate, st)
+                       : dtype == PM_F32_TF32 ? launch_wgrad<Tf32OnePass<false>>(dY, X, workspace, dW, B, M, N, n0, nb, hw, accumulate, st)
+                                              : launch_wgrad<__nv_bfloat16>(dY, X, workspace, dW, B, M, N, n0, nb, hw, accumulate, st);
         if (rc) return rc;
         n0 += nb;
     }

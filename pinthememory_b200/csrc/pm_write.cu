@@ -807,7 +807,7 @@ extern "C" const char* pm_status_string(int code) {
     switch (code) {
         case PM_OK: return "ok";
         case PM_ERR_NULL: return "a required pointer is NULL";
-        case PM_ERR_DTYPE: return "dtype must be PM_F32 (0) or PM_BF16 (1)";
+        case PM_ERR_DTYPE: return "dtype must be PM_F32 (0) or PM_BF16 (1); PM_F32_TF32 (2) only for the pm_conv1x1_* entries";
         case PM_ERR_CHANNELS: return "C (mem_dim) must be one of 32, 64, 128, 256";
         case PM_ERR_SLOTS: return "K (mem_slot) must be in 1..31";
         case PM_ERR_SHAPE: return "a dimension is <= 0 or too large";

@@ -35,6 +35,9 @@ class GraphedStep:
     carry_memory : end the step with ``memory <- updated memory`` (training); False replays from the
                    same memory every time
     autocast_dtype : run the module under ``torch.autocast`` (bf16 feature tensors)
+
+    The modes the module reads from torch at call time -- deterministic algorithms, the TF32 switches (``capi.tf32``) --
+    are fixed when the step is captured; changing them afterwards does not change what a replay runs.
     """
 
     def __init__(self, module, query, mask=None, grad_updated_query=None, loss_weights=(0.02, 0.4, 0.2),

@@ -335,7 +335,8 @@ class _WriteNetFn(torch.autograd.Function):
         b32 = beta.detach().to(torch.float32).contiguous()
         # [sum | sum of squares | element count], cleared by the launch that also splits W and W^T for the two GEMMs
         stats = torch.empty(2 * C + 1, dtype=torch.float64, device=dev)
-        (hi, lo), ctx.preT = capi.conv1x1_prep_both(W2, torch.float32, zero=stats)
+        ctx.tf32 = capi.tf32()   # decided once: the backward's operand W^T is prepared here, in the same mode
+        (hi, lo), ctx.preT = capi.conv1x1_prep_both(W2, torch.float32, zero=stats, tf32=ctx.tf32)
         z = capi.conv1x1_fwd(x, hi, lo, C, stats=stats)
         count = None
         if sync_group is not None:   # as _ConvBnActFn: global statistics
@@ -391,7 +392,7 @@ class _WriteNetFn(torch.autograd.Function):
                 hiT, loT = ctx.preT
                 dx = capi.conv1x1_fwd(dz, hiT, loT, C, y=g, accumulate=True)
             if ctx.needs_input_grad[3]:
-                dWc = capi.conv1x1_wgrad(dz, x).view(ctx.wshape).to(ctx.wdtype)
+                dWc = capi.conv1x1_wgrad(dz, x, tf32=ctx.tf32).view(ctx.wshape).to(ctx.wdtype)
         return (dx, None, None, dWc, dgamma, dbeta, None, None, None, None, None, None, dW, db, None, None, None)
 
 
@@ -473,7 +474,8 @@ class _ConvBnActFn(torch.autograd.Function):
     """y = [relu](BatchNorm2d(conv1x1(x, W)) [+ residual]) -- memory.py:74-87 (Writingnet) and :103-107 (self.output).
 
     The convolution, its input gradient and its weight gradient are the tcgen05 GEMMs of csrc/pm_gemm.cu (3xTF32 in
-    fp32, bf16 otherwise); the forward GEMM's epilogue produces the batch statistics, so the BatchNorm costs one
+    fp32 -- one TF32 pass when torch's TF32 switches allow it (capi.tf32), decided once in the forward --, bf16
+    otherwise); the forward GEMM's epilogue produces the batch statistics, so the BatchNorm costs one
     normalise pass instead of a statistics pass + a normalise pass; when the residual IS the convolution input
     (Writingnet) the input-gradient GEMM accumulates into the residual gradient (TMA reduce-add) instead of leaving an
     element-wise add to autograd."""
@@ -489,8 +491,9 @@ class _ConvBnActFn(torch.autograd.Function):
         b32 = beta.detach().to(torch.float32).contiguous()
         ctx.preT = None
         stats = None
-        if pre is not None and pre[0][0].dtype != x.dtype:
-            pre = None                # prepared for another compute dtype (autocast): redo it here
+        tf32 = x.dtype == torch.float32 and capi.tf32()
+        if pre is not None and (pre[0][0].dtype != x.dtype or capi.operands_tf32(pre[0]) != tf32):
+            pre = None                # prepared for another compute dtype (autocast) or TF32 mode: redo it here
         ctx.w_on_aux = pre is not None
         if pre is not None:           # operands (and the cleared statistics buffer) prepared ahead of time on a side stream
             (hi, lo), ctx.preT, stats = pre
@@ -499,9 +502,9 @@ class _ConvBnActFn(torch.autograd.Function):
         elif ctx.needs_input_grad[0]:   # the input-gradient GEMM's operand W^T comes out of the same launch ...
             if use_batch_stats:       # ... which also clears the statistics buffer (no fill kernel)
                 stats = torch.empty(2 * M + 1, dtype=torch.float64, device=dev)
-            (hi, lo), ctx.preT = capi.conv1x1_prep_both(W2, x.dtype, zero=stats)
+            (hi, lo), ctx.preT = capi.conv1x1_prep_both(W2, x.dtype, zero=stats, tf32=tf32)
         else:
-            hi, lo = capi.conv1x1_prep(W2, False, x.dtype)
+            hi, lo = capi.conv1x1_prep(W2, False, x.dtype, tf32=tf32)
         if use_batch_stats:
             # [sum | sum of squares | element count]: the GEMM epilogue fills the first 2M; with SyncBatchNorm the whole
             # vector is summed over the ranks (fp64, one small all-reduce) and the normalise pass finalises GLOBAL statistics
@@ -536,6 +539,7 @@ class _ConvBnActFn(torch.autograd.Function):
         ctx.relu, ctx.training, ctx.res_is_x, ctx.has_res = relu, use_batch_stats, res_is_x, res is not None
         ctx.use_mask = mask is not None
         ctx.wshape, ctx.wdtype = W.shape, W.dtype
+        ctx.tf32 = tf32
         ctx.sync_group = sync_group if use_batch_stats else None
         ctx.beta32 = b32   # (a detached fp32 copy: only the fused BatchNorm-backward GEMM reads it, to recompute the ReLU gate)
         ctx.save_for_backward(x, W2, xc, mask if mask is not None else y, mean, invstd, g32,
@@ -571,7 +575,7 @@ class _ConvBnActFn(torch.autograd.Function):
         if need_x and not ctx.has_res and xc.dtype == torch.float32 and M % 32 == 0 and ctx.beta32 is not None:
             # blocks without a residual (self.output): the BatchNorm backward rides in the operand path of the
             # input-gradient GEMM, which also stores dz for the weight-gradient GEMM -- no bn_bwd_apply pass
-            hiT, loT = ctx.preT if ctx.preT is not None else capi.conv1x1_prep(W2, True, x.dtype)
+            hiT, loT = ctx.preT if ctx.preT is not None else capi.conv1x1_prep(W2, True, x.dtype, tf32=ctx.tf32)
             dx, dxc = capi.conv1x1_dgrad_bnbwd(dy, xc, hiT, loT, K, mean, invstd, g32, sg, sb, ctx.beta32, ctx.relu,
                                                ctx.training)
             dW = None
@@ -584,19 +588,19 @@ class _ConvBnActFn(torch.autograd.Function):
                     aux = _stream_of(_AUX_STREAMS, x.device)
                     aux.wait_stream(cur)
                     with torch.cuda.stream(aux):
-                        dW = capi.conv1x1_wgrad(dxc, x).view(ctx.wshape).to(ctx.wdtype)
+                        dW = capi.conv1x1_wgrad(dxc, x, tf32=ctx.tf32).view(ctx.wshape).to(ctx.wdtype)
                     dxc.record_stream(aux)
                     x.record_stream(aux)
                 else:
-                    dW = capi.conv1x1_wgrad(dxc, x).view(ctx.wshape).to(ctx.wdtype)
+                    dW = capi.conv1x1_wgrad(dxc, x, tf32=ctx.tf32).view(ctx.wshape).to(ctx.wdtype)
             return dx, dW, dgamma, dbeta, None, None, None, None, None, None, None, None, None, None, None
         capi.bn_bwd_apply(dy, y, mask, xc, mean, invstd, g32, sg, sb, ctx.relu, ctx.training, dxc, dres)
         dW = None
         if ctx.needs_input_grad[1]:
-            dW = capi.conv1x1_wgrad(dxc, x).view(ctx.wshape).to(ctx.wdtype)
+            dW = capi.conv1x1_wgrad(dxc, x, tf32=ctx.tf32).view(ctx.wshape).to(ctx.wdtype)
         dx = None
         if need_x:
-            hiT, loT = ctx.preT if ctx.preT is not None else capi.conv1x1_prep(W2, True, x.dtype)
+            hiT, loT = ctx.preT if ctx.preT is not None else capi.conv1x1_prep(W2, True, x.dtype, tf32=ctx.tf32)
             if ctx.res_is_x:
                 dx = capi.conv1x1_fwd(dxc, hiT, loT, K, y=dres, accumulate=True)   # dres += W^T . dxc
                 dres = None
@@ -712,7 +716,7 @@ def _weight_bn_act(W, bn, x, residual, relu, prepared=None, affine=None, pre=Non
         if _inference_block(bn, x, residual):
             # inference read (BASELINE config 5): the eval-mode BatchNorm and the ReLU ride in the GEMM epilogue
             hi, lo = prepared if prepared is not None else capi.conv1x1_prep(
-                W.detach().reshape(M, K).to(torch.float32).contiguous(), False, x.dtype)
+                W.detach().reshape(M, K).to(torch.float32).contiguous(), False, x.dtype, tf32=capi.tf32())
             scale, shift = affine if affine is not None else _eval_affine(bn)
             return capi.conv1x1_fwd_affine(x, hi, lo, M, scale, shift, relu)
         res_is_x = residual is x or (residual is not None and residual.data_ptr() == x.data_ptr()
@@ -858,16 +862,16 @@ class Memory_sup(nn.Module):
         W = self.output[0].weight
         Co, C, K = W.shape[0], self.feature_dim, self.memory_size
         self._folded_shape = torch.empty(Co, C + capi.PLANES, 0, 0, device="meta")  # shape carrier only (M, K of the GEMM)
-        key = (W, W._version, M, M._version, u.dtype)
+        key = (W, W._version, M, M._version, u.dtype, capi.tf32())   # (an operand split for 3xTF32 has a lo part, one-pass not)
         cached = getattr(self, "_infer_cache", None)
         capturing = torch.cuda.is_current_stream_capturing()
         if (not capturing and cached is not None and cached[0][0] is W and cached[0][2] is M and cached[0][1] == key[1]
-                and cached[0][3] == key[3] and cached[0][4] == key[4]):
+                and cached[0][3] == key[3] and cached[0][4] == key[4] and cached[0][5] == key[5]):
             return cached[1]
         W32 = W.detach().to(torch.float32).contiguous()
         Wp = torch.empty(Co, C + capi.PLANES, dtype=torch.float32, device=W.device)
         capi.fold_weight_fwd(W32, M.detach().to(torch.float32).contiguous(), Wp, Co, C, K)
-        prepared = capi.conv1x1_prep(Wp, False, u.dtype)
+        prepared = capi.conv1x1_prep(Wp, False, u.dtype, tf32=key[5])
         if not capturing:
             self._infer_cache = (key, prepared)
         return prepared
@@ -934,7 +938,7 @@ class Memory_sup(nn.Module):
                 stats = torch.empty(2 * Co + 1, dtype=torch.float64, device=query.device)
                 cdt = torch.get_autocast_dtype("cuda") if torch.is_autocast_enabled("cuda") else query.dtype
                 ops, opsT = capi.conv1x1_prep_both(Wp_early.detach().reshape(Co, C + capi.PLANES).to(torch.float32).contiguous(),
-                                                   cdt, zero=stats)
+                                                   cdt, zero=stats, tf32=capi.tf32())
             wpre = (Wp_early, (ops, opsT, stats))
             for t in (Wp_early, stats, *ops, *opsT):
                 if torch.is_tensor(t):
