@@ -56,7 +56,7 @@ enum pm_readloss_ws_layout {
 #define PM_COLPART_ROWS 296
 
 /* Bumped with every prototype change; the binding refuses a library whose pm_version() differs. */
-#define PM_ABI_VERSION 213
+#define PM_ABI_VERSION 214
 int pm_version(void);
 const char* pm_status_string(int code);
 /* Row stride (floats) of the internal score buffers for K slots: 20 for K<=19, else 32. */
@@ -414,6 +414,58 @@ int pm_update_fwd_peer(const void* peer_bufs, int rank, int world, unsigned* epo
 int pm_update_bwd_peer(const void* peer_bufs, int rank, int world, unsigned* epoch, const float* dM_new, const float* g_div,
                        const float* g_cls, const float* M_new, const float* saved, const float* W_cls, const float* b_cls,
                        float momentum, float* dS, float* dW_cls, float* db_cls, float* aux, int C, int K, void* stream);
+
+/*
+ * Global-batch read for sharded runs (opt-in: sharding.enable_sharded_update(..., global_read=True)). Without it the
+ * read's two reductions over pixels are rank-local: the read loss is a mean over the rank's own valid label pixels
+ * (memory.py:173-176) and score_query a softmax over the rank's own pixels (memory.py:183,186-187). These entries exchange
+ * the small per-rank rows those reductions need, so that every rank computes them over the concatenated global batch:
+ *   readloss       = (sum_r loss_sum_r) / (sum_r V_r), bit-identical on every rank (NaN only when no rank has a valid pixel)
+ *   score_query    = exp(z - m_k) / S_k with the column maximum m_k and sum S_k over all ranks' pixels
+ * and, in the backward, the autograd mirror of an all-reduce: the ranks' upstream gradients of readloss and the column
+ * sums c_k = sum_n p_q[n,k] g_q[n,k] of pm_score_bwd are summed over the ranks. Every sum runs over the ranks in rank
+ * order, in fp64 where the quantity is a sum over pixels, so the results are identical on every rank.
+ *
+ * A row is PM_READ_ROW_FLOATS floats (512 bytes, 16-byte aligned):
+ *   forward   floats [0,32) column maximum m_r, [32,64) column sum S_r (= 1 / the 1/sum pm_read_fwd[_planes] left in
+ *             col_partials), then two doubles at float offset 64: the read-loss sum (ws[PM_WS_LOSS_SUM]) and V_r (the sum of
+ *             the label histogram's bins 0..K-1); both 0 without labels
+ *   backward  doubles [0] the upstream gradient of readloss (0 when NULL), [1, 1+K) the rank's column sums c_k in fp64
+ *             (0 when no partials)
+ * Peer path (peer_bufs != NULL, the symmetric buffers of pm_update_fwd_peer): the rows live at PM_PEER_READ_FWD_OFF /
+ * PM_PEER_READ_BWD_OFF of every rank's buffer, the flags are kinds 4..7 of the flag area (after the update kernels' four
+ * kinds), `epoch` is one device uint32 per entry (zeroed at allocation, owned by the kernel). One CTA writes the rank's
+ * row, raises its flag in every peer's buffer, waits (bounded, like the update kernels) for all ranks, combines, and raises
+ * a "done" flag that the NEXT launch waits for before it overwrites the row. `gathered` is unused.
+ * Gathered path (peer_bufs == NULL, no symmetric memory): pm_read_row_fwd / _bwd write the rank's row into a tensor, the
+ * caller all-gathers the rows into `gathered` [world][PM_READ_ROW_FLOATS] (rank order) and the exchange entry combines them
+ * with the same code that reads peer memory; `rank` and `epoch` are unused.
+ * Every rank of the group must launch the same sequence of these entries.
+ *
+ * pm_read_exchange_fwd: between pm_read_fwd[_planes] (and the read loss, which must have finished: its ws is read) and
+ *   pm_colsoftmax_apply. Rewrites the combined row of col_partials (column maximum, 1/sum) with the global statistics, so
+ *   pm_colsoftmax_apply runs unchanged. ws / out: the read-loss workspace and `out` of pm_readloss_fwd[8][_ordered], or both
+ *   NULL for a read without labels; out[0] = global readloss, out[1] = 1 / (V * temperature) with the global V.
+ * pm_read_exchange_bwd: partials = the workspace pm_score_bwd_partials filled (NULL: score_query has no gradient), g_loss =
+ *   the upstream gradient of readloss (device float, or NULL = 0). Out: g_loss_sum (float[1], the ranks' sum) and colsums
+ *   (double[32], [k < K] the global c_k) for pm_score_bwd_global / pm_read_bwd[_planes].
+ */
+#define PM_READ_ROW_FLOATS 128
+#define PM_PEER_READ_FWD_OFF 98304
+#define PM_PEER_READ_BWD_OFF 98816
+int pm_read_row_fwd(const float* col_partials, const void* ws, float* row, int K, void* stream);
+int pm_read_row_bwd(const float* partials, const float* g_loss, float* row, int K, void* stream);
+int pm_read_exchange_fwd(const void* peer_bufs, int rank, int world, unsigned* epoch, const float* gathered,
+                         float* col_partials, const void* ws, float temperature, float* out, int K, void* stream);
+int pm_read_exchange_bwd(const void* peer_bufs, int rank, int world, unsigned* epoch, const float* gathered,
+                         const float* partials, const float* g_loss, float* g_loss_sum, double* colsums, int K, void* stream);
+/* pm_score_bwd split at its column sums, for the global read: pm_score_bwd_partials is its first launch (the per-CTA fp64
+ * partials of c into `workspace`, pm_score_bwd_workspace_floats(K) floats, 8-byte aligned), pm_score_bwd_global its second
+ * with c[k] = colsums[k] (from pm_read_exchange_bwd) instead of the rank's own partials. Other arguments as pm_score_bwd. */
+int pm_score_bwd_partials(const float* score_q, const float* g_q, float* workspace, int N, int K, void* stream);
+int pm_score_bwd_global(const float* score_q, const float* g_q, const float* score_m, const float* g_m, const float* ds_rl,
+                        const float* g_loss, const float* rl_out, const double* colsums, float* E, int N, int K,
+                        void* stream);
 
 /* 64-bit words of the segmentation-metrics workspace (`ws`, zero it before every pm_seg_eval call). */
 enum pm_seg_eval_ws_layout {

@@ -19,7 +19,7 @@ WS_BAD = 2     # PM_WS_BAD
 SEG_WS_WORDS = 4  # PM_SEG_WS_WORDS
 SEG_WS_BAD = 2    # PM_SEG_WS_BAD
 
-ABI_VERSION = 213  # PM_ABI_VERSION of include/pinmem_b200.h the argtypes below were written against
+ABI_VERSION = 214  # PM_ABI_VERSION of include/pinmem_b200.h the argtypes below were written against
 
 _c_p = ctypes.c_void_p
 _c_i = ctypes.c_int
@@ -95,6 +95,12 @@ PROTOTYPES = {
     "pm_write_reduce_bn_fwd_ordered": [_c_p] * 3 + [_c_i] + [_c_p] * 3 + [_c_d, _c_p, _c_f] + [_c_p] * 6 + [_c_f, _c_p] + [_c_i] * 7 + [_c_p],
     "pm_write_bwd_bn_scratch_bytes": [_c_i],
     "pm_write_bwd_bn": [_c_p] * 4 + [_c_i] + [_c_p] * 8 + [_c_i] * 7 + [_c_p],
+    "pm_read_row_fwd": [_c_p] * 3 + [_c_i, _c_p],
+    "pm_read_row_bwd": [_c_p] * 3 + [_c_i, _c_p],
+    "pm_read_exchange_fwd": [_c_p, _c_i, _c_i] + [_c_p] * 4 + [_c_f, _c_p, _c_i, _c_p],
+    "pm_read_exchange_bwd": [_c_p, _c_i, _c_i] + [_c_p] * 6 + [_c_i, _c_p],
+    "pm_score_bwd_partials": [_c_p] * 3 + [_c_i] * 2 + [_c_p],
+    "pm_score_bwd_global": [_c_p] * 9 + [_c_i] * 2 + [_c_p],
 }
 EXPORTED_SYMBOLS = sorted(list(PROTOTYPES) + ["pm_status_string"])
 
@@ -708,3 +714,56 @@ def update_bwd_peer(peer, dM_new, g_div, g_cls, M_new, saved, W, b, momentum, dS
     _call("pm_update_bwd_peer", peer.bufs_dev, peer.rank, peer.world_size, _ptr(peer.epochs[1:2]), _ptr(dM_new), _ptr(g_div),
           _ptr(g_cls), _ptr(M_new), _ptr(saved), _ptr(W), _ptr(b), float(momentum), _ptr(dS), _ptr(dW), _ptr(db),
           _ptr(update_aux(M_new.device, K)), C, K, _stream())
+
+
+# ------------------------------- global-batch read of a sharded run (csrc/pm_exchange.cu, csrc/pm_score.cu)
+
+READ_ROW_FLOATS = 128                               # PM_READ_ROW_FLOATS
+PEER_READ_FWD_OFF, PEER_READ_BWD_OFF = 98304, 98816  # PM_PEER_READ_*_OFF
+
+
+def read_row_fwd(col_partials, ws, row, K):
+    """This rank's forward row (column statistics, read-loss sum and valid count) into ``row`` [READ_ROW_FLOATS]."""
+    _call("pm_read_row_fwd", _ptr(col_partials), _ptr(ws), _ptr(row), K, _stream())
+
+
+def read_row_bwd(partials, g_loss, row, K):
+    """This rank's backward row (upstream gradient of readloss, column sums of score_query's backward) into ``row``."""
+    _call("pm_read_row_bwd", _ptr(partials), _ptr(g_loss), _ptr(row), K, _stream())
+
+
+def read_exchange_fwd(peer, gathered, world, col_partials, ws, temperature, out, K):
+    """Global column statistics into col_partials' combined row and, with ws / out, the global readloss into out: over
+    peer memory (``peer`` a sharding.PeerExchange) or from the all-gathered rows ``gathered`` [world, READ_ROW_FLOATS]."""
+    if peer is not None:
+        _call("pm_read_exchange_fwd", peer.bufs_dev, peer.rank, peer.world_size, _ptr(peer.epochs[2:3]), None,
+              _ptr(col_partials), _ptr(ws), float(temperature), _ptr(out), K, _stream())
+    else:
+        _call("pm_read_exchange_fwd", None, 0, world, None, _ptr(gathered), _ptr(col_partials), _ptr(ws), float(temperature),
+              _ptr(out), K, _stream())
+
+
+def read_exchange_bwd(peer, gathered, world, partials, g_loss, g_loss_sum, colsums, K):
+    """The ranks' sum of readloss's upstream gradient into g_loss_sum [1] fp32 and the global column sums into colsums
+    [32] fp64 (peer memory, or the all-gathered rows as read_exchange_fwd)."""
+    if peer is not None:
+        _call("pm_read_exchange_bwd", peer.bufs_dev, peer.rank, peer.world_size, _ptr(peer.epochs[3:4]), None, _ptr(partials),
+              _ptr(g_loss), _ptr(g_loss_sum), _ptr(colsums), K, _stream())
+    else:
+        _call("pm_read_exchange_bwd", None, 0, world, None, _ptr(gathered), _ptr(partials), _ptr(g_loss), _ptr(g_loss_sum),
+              _ptr(colsums), K, _stream())
+
+
+def score_bwd_partials(score_q, g_q, K):
+    """First launch of pm_score_bwd alone: the per-CTA fp64 partials of score_query's column sums (returned)."""
+    N = score_q.shape[0]
+    ws = torch.empty(load().pm_score_bwd_workspace_floats(int(K)), dtype=torch.float32, device=score_q.device)
+    _call("pm_score_bwd_partials", _ptr(score_q), _ptr(g_q), _ptr(ws), N, K, _stream())
+    return ws
+
+
+def score_bwd_global(score_q, g_q, score_m, g_m, E, K, colsums, ds_rl=None, g_loss=None, rl_out=None):
+    """score_bwd with the column sums of score_query's backward taken from ``colsums`` (global, read_exchange_bwd)."""
+    N = E.shape[0]
+    _call("pm_score_bwd_global", _ptr(score_q), _ptr(g_q), _ptr(score_m), _ptr(g_m), _ptr(ds_rl), _ptr(g_loss), _ptr(rl_out),
+          _ptr(colsums), _ptr(E), N, K, _stream())

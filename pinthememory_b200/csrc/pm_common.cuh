@@ -288,4 +288,50 @@ __device__ __forceinline__ int compact_taps(LabelTaps& t) {
     return n;
 }
 
+// ---- column sums of score_query's backward (pm_score.cu: pm_score_bwd; pm_exchange.cu: the global read's exchange)
+// SB_PARTS CTAs each leave one fp64 partial per column ([SB_PARTS][32] doubles); the column sum is formed in ONE fixed
+// order everywhere: group j (0..SB_GROUPS-1) adds partials j, j + SB_GROUPS, ... in ascending order, then the groups are
+// added in ascending order. sb_group_sum is one group's term.
+constexpr int SB_PARTS = 148, SB_GROUPS = 8;
+__device__ __forceinline__ double sb_group_sum(const double* part, int k, int j) {
+    double a = 0.0;
+    for (int i = j; i < SB_PARTS; i += SB_GROUPS) a += __ldcg(part + (size_t)i * 32 + k);
+    return a;
+}
+
+// ---- cross-rank flags in the symmetric peer buffer (pm_write.cu: the sharded update; pm_exchange.cu: the global read).
+// flags[kind][row 0..31][rank 0..15] (u32, monotone epochs) at PM_PEER_FLAG_OFF; kinds 0..3 belong to the update kernels,
+// 4..7 to the read exchanges.
+struct PeerCtx {
+    const unsigned long long* bufs;  // device array [world] of symmetric-buffer base addresses; nullptr = not sharded
+    int rank, world;
+    unsigned* epoch;                 // device counter of this kernel's launches (one per kernel kind)
+};
+
+__device__ __forceinline__ unsigned* peer_flag(unsigned long long base, int kind, int row, int rank) {
+    return reinterpret_cast<unsigned*>(base + PM_PEER_FLAG_OFF) + ((kind * 32 + row) * 16 + rank);
+}
+// all threads of the CTA call both; data written by this CTA before peer_signal is visible to the peers after their wait
+__device__ __forceinline__ void peer_signal(const PeerCtx& p, int kind, int row, unsigned e) {
+    __threadfence_system();
+    __syncthreads();
+    if ((int)threadIdx.x < p.world) {
+        unsigned* f = peer_flag(p.bufs[threadIdx.x], kind, row, p.rank);
+        asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(f), "r"(e) : "memory");
+    }
+}
+__device__ __forceinline__ void peer_wait(const PeerCtx& p, int kind, int row, unsigned e) {
+    if ((int)threadIdx.x < p.world) {
+        const unsigned* f = peer_flag(p.bufs[p.rank], kind, row, threadIdx.x);
+        unsigned v = 0;
+        for (unsigned spin = 0;; ++spin) {
+            asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(f) : "memory");
+            if ((int)(v - e) >= 0) break;
+            if (spin > (1u << 27)) __trap();  // a peer that never arrives (crashed rank): fail loudly, do not hang the GPU
+            __nanosleep(32);
+        }
+    }
+    __syncthreads();
+}
+
 }  // namespace pm

@@ -182,7 +182,7 @@ extern "C" int pm_rowsoftmax(const float* s, const float* gumbel_m, float* score
 
 namespace pm {
 
-constexpr int SB_PARTS = 148;
+// (SB_PARTS, SB_GROUPS and the summation order: pm_common.cuh, sb_group_sum)
 
 __global__ void __launch_bounds__(256) score_bwd_colsum_kernel(const float* __restrict__ p, const float* __restrict__ g,
                                                                double* __restrict__ part, int N, int K, int rows_per_cta) {
@@ -202,27 +202,29 @@ __global__ void __launch_bounds__(256) score_bwd_colsum_kernel(const float* __re
     }
 }
 
-template <int KP>
+// GLOBAL: `part` is the double[32] of global column sums pm_read_exchange_bwd left (the global read of a sharded run)
+template <int KP, bool GLOBAL = false>
 __global__ void __launch_bounds__(256)
     score_bwd_apply_kernel(const float* __restrict__ score_q, const float* __restrict__ g_q, const float* __restrict__ score_m,
                            const float* __restrict__ g_m, const float* __restrict__ ds_rl, const float* __restrict__ g_loss,
                            const float* __restrict__ rl_out, const double* __restrict__ part, float* __restrict__ E, int N,
                            int K) {
-    __shared__ double red[8][32];
+    __shared__ double red[SB_GROUPS][32];
     __shared__ float cq[32];
     const int t = threadIdx.x;
-    if (g_q != nullptr) {
-        // c[k]: 8 groups of 32 threads take every 8th partial in ascending order, then the groups in ascending order
+    if (GLOBAL && g_q != nullptr) {
+        if (t < 32) cq[t] = t < K ? (float)__ldcg(part + t) : 0.f;
+        __syncthreads();
+    } else if (g_q != nullptr) {
+        // c[k]: SB_GROUPS groups of 32 threads, one group term each (sb_group_sum), then the groups in ascending order
+        static_assert(SB_GROUPS * 32 == 256, "one group of 32 threads per group term");
         const int k = t & 31, j = t >> 5;
-        double a = 0.0;
-        if (k < K)
-            for (int i = j; i < SB_PARTS; i += 8) a += __ldcg(part + (size_t)i * 32 + k);
-        red[j][k] = a;
+        red[j][k] = k < K ? sb_group_sum(part, k, j) : 0.0;
         __syncthreads();
         if (t < 32) {
             double c = 0.0;
 #pragma unroll
-            for (int i = 0; i < 8; ++i) c += red[i][t];
+            for (int i = 0; i < SB_GROUPS; ++i) c += red[i][t];
             cq[t] = (float)c;
         }
         __syncthreads();
@@ -371,5 +373,36 @@ extern "C" int pm_score_nhwc_bwd(const float* q, const float* M, const float* E,
         pm::score_nhwc_bwd_kernel<32><<<G, tpb, 0, st>>>(q, M, E, dq, part, N, C, K, rows_per_cta);
     PM_CHECK_LAUNCH();
     if (dM) return pm::reduce_partials_f32(dM, scratch, G, (long long)K * C, st);
+    return 0;
+}
+
+extern "C" int pm_score_bwd_partials(const float* score_q, const float* g_q, float* workspace, int N, int K, void* stream) {
+    if (!score_q || !g_q || !workspace) return PM_ERR_NULL;
+    if (K < 1 || K > 31) return PM_ERR_SLOTS;
+    if (N <= 0) return PM_ERR_SHAPE;
+    if ((uintptr_t)workspace & 7) return PM_ERR_ALIGN;
+    const int rows_per_cta = (N + pm::SB_PARTS - 1) / pm::SB_PARTS;
+    pm::score_bwd_colsum_kernel<<<pm::SB_PARTS, K * (256 / K), 0, (cudaStream_t)stream>>>(
+        score_q, g_q, reinterpret_cast<double*>(workspace), N, K, rows_per_cta);
+    PM_CHECK_LAUNCH();
+    return 0;
+}
+
+extern "C" int pm_score_bwd_global(const float* score_q, const float* g_q, const float* score_m, const float* g_m,
+                                   const float* ds_rl, const float* g_loss, const float* rl_out, const double* colsums, float* E,
+                                   int N, int K, void* stream) {
+    if (!E || (g_q && (!score_q || !colsums)) || (g_m && !score_m)) return PM_ERR_NULL;
+    if (K < 1 || K > 31) return PM_ERR_SLOTS;
+    if (N <= 0) return PM_ERR_SHAPE;
+    if (((uintptr_t)E & 15) || ((uintptr_t)ds_rl & 15) || ((uintptr_t)colsums & 7)) return PM_ERR_ALIGN;
+    cudaStream_t st = (cudaStream_t)stream;
+    const int grid = min((N + 255) / 256, 148 * 4);
+    if (K <= 19)
+        pm::score_bwd_apply_kernel<20, true><<<grid, 256, 0, st>>>(score_q, g_q, score_m, g_m, ds_rl, g_loss, rl_out, colsums, E,
+                                                                   N, K);
+    else
+        pm::score_bwd_apply_kernel<32, true><<<grid, 256, 0, st>>>(score_q, g_q, score_m, g_m, ds_rl, g_loss, rl_out, colsums, E,
+                                                                   N, K);
+    PM_CHECK_LAUNCH();
     return 0;
 }

@@ -271,37 +271,7 @@ __device__ __forceinline__ void block_reduce32(float (&v)[32], float* scratch, f
 // so the updated memory is bit-identical across ranks. A second flag round ("done") at the end of the kernel keeps a
 // rank from zeroing / overwriting its buffer for the next step while a slower peer still reads it. No NCCL launch,
 // no extra kernel: ~21 KB per rank cross NVSwitch inside the kernel that needs them.
-struct PeerCtx {
-    const unsigned long long* bufs;  // device array [world] of symmetric-buffer base addresses; nullptr = not sharded
-    int rank, world;
-    unsigned* epoch;                 // device counter of this kernel's launches (one per kernel kind)
-};
-
-__device__ __forceinline__ unsigned* peer_flag(unsigned long long base, int kind, int row, int rank) {
-    return reinterpret_cast<unsigned*>(base + PM_PEER_FLAG_OFF) + ((kind * 32 + row) * 16 + rank);
-}
-// all threads of the CTA call both; data written by this CTA before peer_signal is visible to the peers after their wait
-__device__ __forceinline__ void peer_signal(const PeerCtx& p, int kind, int row, unsigned e) {
-    __threadfence_system();
-    __syncthreads();
-    if ((int)threadIdx.x < p.world) {
-        unsigned* f = peer_flag(p.bufs[threadIdx.x], kind, row, p.rank);
-        asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(f), "r"(e) : "memory");
-    }
-}
-__device__ __forceinline__ void peer_wait(const PeerCtx& p, int kind, int row, unsigned e) {
-    if ((int)threadIdx.x < p.world) {
-        const unsigned* f = peer_flag(p.bufs[p.rank], kind, row, threadIdx.x);
-        unsigned v = 0;
-        for (unsigned spin = 0;; ++spin) {
-            asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(f) : "memory");
-            if ((int)(v - e) >= 0) break;
-            if (spin > (1u << 27)) __trap();  // a peer that never arrives (crashed rank): fail loudly, do not hang the GPU
-            __nanosleep(32);
-        }
-    }
-    __syncthreads();
-}
+// (PeerCtx, peer_signal and peer_wait: pm_common.cuh)
 
 // aux layout (floats, zeroed by the caller): [0] arrival counter (as unsigned), [2 .. 2+32) per-row CE term,
 // [34 .. 34+32) per-row positive off-diagonal Gram sum

@@ -87,10 +87,14 @@ class _ReadFn(torch.autograd.Function):
     last_lab8 = None  # the packed uint8 class map that read produced (None when the first-generation kernel ran)
 
     @staticmethod
-    def forward(ctx, x, M, labels, g_query, g_memory, temperature, K, planes=False, tee=False, branch=False):
+    def forward(ctx, x, M, labels, g_query, g_memory, temperature, K, planes=False, tee=False, branch=False, xg=None):
         """``tee=True`` appends x itself to the outputs: a caller that feeds the same features to a second branch (the
         writing net) hands that branch the tee, so its gradient arrives HERE as an input of backward() and the dx kernel
-        sums it in (``dx_add``) -- instead of autograd adding two feature-sized gradients with an element-wise kernel."""
+        sums it in (``dx_add``) -- instead of autograd adding two feature-sized gradients with an element-wise kernel.
+
+        ``xg``: the shard group of a global read (sharding.enable_sharded_update(global_read=True), more than one rank) or
+        None. The read loss then runs before the column softmax, and one exchange between them turns the rank's column
+        statistics and read-loss sum / valid count into the global batch's (sharding.read_exchange_fwd)."""
         B, C, h, w = x.shape
         N = B * h * w
         dev = x.device
@@ -129,15 +133,27 @@ class _ReadFn(torch.autograd.Function):
             labels.record_stream(side)
             lab8.record_stream(cur)
         capi.read_fwd(x, M, g_memory, u, s, score_m, K, gumbel_q=g_query, col_partials=col_partials, planes=planes)
-        if branch:
-            aux.wait_stream(cur)
-            with torch.cuda.stream(aux):
-                capi.colsoftmax_apply(s, g_query, col_partials, score_q, N, K)
-            for t in (s, g_query, buf, score_q):
-                if torch.is_tensor(t):
-                    t.record_stream(aux)
-        else:
+
+        def column_softmax():
+            if xg is not None:
+                rl_ws = buf[N * KP: N * KP + 2 * capi.WS_WORDS] if labels is not None else None
+                rl_res = buf[N * KP + 2 * capi.WS_WORDS: N * KP + 2 * capi.WS_WORDS + 4] if labels is not None else None
+                sharding.read_exchange_fwd(xg, col_partials, rl_ws, temperature, rl_res, K)
             capi.colsoftmax_apply(s, g_query, col_partials, score_q, N, K)
+
+        def column_softmax_on_stream():
+            if branch:
+                aux.wait_stream(cur)
+                with torch.cuda.stream(aux):
+                    column_softmax()
+                for t in (s, g_query, buf, score_q):
+                    if torch.is_tensor(t):
+                        t.record_stream(aux)
+            else:
+                column_softmax()
+
+        if xg is None:
+            column_softmax_on_stream()
         if labels is not None:
             ds_rl = buf[: N * KP]
             ws = buf[N * KP: N * KP + 2 * capi.WS_WORDS]
@@ -160,7 +176,9 @@ class _ReadFn(torch.autograd.Function):
             ds_rl = rl_out = None
             readloss = torch.zeros((), dtype=torch.float32, device=dev)
             hist = torch.zeros(K + 1, dtype=torch.int64, device=dev)
-        ctx.K, ctx.planes, ctx.UC = K, planes, UC
+        if xg is not None:   # after the read loss: the exchange carries its sum and valid count too
+            column_softmax_on_stream()
+        ctx.K, ctx.planes, ctx.UC, ctx.xg = K, planes, UC, xg
         ctx.has_loss = labels is not None
         ctx.set_materialize_grads(False)  # unused outputs (scores, histogram) arrive as None, not as zero fills
         # score_q is kept for the gradient of score_query (N*K*4 bytes, 5.6 MB at cfg 2: the one cost of differentiable
@@ -186,15 +204,29 @@ class _ReadFn(torch.autograd.Function):
             g_loss = g_loss.to(torch.float32).contiguous()
         else:
             g_loss = None
+        dense = lambda g: None if g is None else g.reshape(N, K).to(torch.float32).contiguous()
+        colsums = None
+        if ctx.xg is not None and (ctx.has_loss or g_sq is not None):
+            # global read: the ranks' upstream gradients of readloss and the column sums of score_query's backward are
+            # summed over the ranks (the autograd mirror of the forward's exchange)
+            g_sq = dense(g_sq)
+            partials = capi.score_bwd_partials(score_q, g_sq, K) if g_sq is not None else None
+            g_sum, colsums = sharding.read_exchange_bwd(ctx.xg, partials, None if g_loss is None else g_loss.reshape(1), K,
+                                                        x.device)
+            if ctx.has_loss:
+                g_loss = g_sum
         if g_loss is None:
             ds_rl = rl_out = None
         if g_sq is not None or g_sm is not None:
             # gradients of score_query / score_memory: their softmax backward (plus the scaled read-loss term) forms one
             # additive similarity gradient E, which the read backward takes in place of ds_rl with a unit scale
-            dense = lambda g: None if g is None else g.reshape(N, K).to(torch.float32).contiguous()
             E = torch.empty(N, capi.score_stride(K), dtype=torch.float32, device=x.device)
-            capi.score_bwd(score_q if g_sq is not None else None, dense(g_sq), score_m if g_sm is not None else None,
-                           dense(g_sm), E, K, ds_rl=ds_rl, g_loss=g_loss, rl_out=rl_out)
+            if colsums is not None and g_sq is not None:
+                capi.score_bwd_global(score_q, g_sq, score_m if g_sm is not None else None, dense(g_sm), E, K, colsums,
+                                      ds_rl=ds_rl, g_loss=g_loss, rl_out=rl_out)
+            else:
+                capi.score_bwd(score_q if g_sq is not None else None, dense(g_sq), score_m if g_sm is not None else None,
+                               dense(g_sm), E, K, ds_rl=ds_rl, g_loss=g_loss, rl_out=rl_out)
             ds_rl = E
             g_loss = rl_out = torch.ones(2, dtype=torch.float32, device=x.device)
         dx = torch.empty_like(x)
@@ -208,7 +240,7 @@ class _ReadFn(torch.autograd.Function):
         if need_dM:
             dM = torch.zeros_like(M)
             capi.read_bwd_dM(None if ctx.planes else du, x, score_m, ds, dM, K)
-        return dx, dM, None, None, None, None, None, None, None, None
+        return dx, dM, None, None, None, None, None, None, None, None, None
 
 
 class _FoldWeightFn(torch.autograd.Function):
@@ -943,8 +975,11 @@ class Memory_sup(nn.Module):
             for t in (Wp_early, stats, *ops, *opsT):
                 if torch.is_tensor(t):
                     t.record_stream(cur)
+        # the global read exchanges only for reads that can feed a training gradient: a read under no_grad (validation,
+        # memory_initalize, a forward-only GraphedStep) stays rank-local, so ranks need not make such reads in lock-step
+        xg = self.shard_group if (torch.is_grad_enabled() and sharding.global_read(self.shard_group)) else None
         outs = _ReadFn.apply(query, M, labels, g_query, g_memory, float(self.temperature), self.memory_size, planes, tee,
-                             _branch)
+                             _branch, xg)
         if wpre is not None:   # (a branched _ReadFn joins the aux stream itself; this covers the read without labels / K > 19)
             torch.cuda.current_stream(query.device).wait_stream(_stream_of(_AUX_STREAMS, query.device))
         u, score_query, score_memory, readloss, hist = outs[:5]

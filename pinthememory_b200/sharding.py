@@ -6,6 +6,10 @@ are all-reduced (sum) over NCCL/NVLink before the momentum update, and -- the au
 gradient w.r.t. the class sums ``[K, C]`` is all-reduced in the backward. Every rank then holds a
 bit-identical ``m_items`` equal to the single-process update on the concatenated global batch.
 The reference has no such collective (each rank silently keeps its own memory, SURVEY.md 2.1).
+
+Opt-in (``global_read=True``): the read loss and score_query, the read's two reductions over pixels, are also taken over
+the global batch -- one small row per rank exchanged before the column softmax and one in the backward
+(csrc/pm_exchange.cu).
 """
 import torch
 import torch.distributed as dist
@@ -28,7 +32,8 @@ class PeerExchange:
         self.handle = symm.rendezvous(self.buffer, pg.group_name)
         self.rank, self.world_size = self.handle.rank, self.handle.world_size
         self.bufs_dev = int(self.handle.buffer_ptrs_dev)      # device array of all ranks' buffer addresses
-        self.epochs = torch.zeros(2, dtype=torch.int32, device=device)
+        # one launch counter per kernel kind: update fwd, update bwd, global-read fwd, global-read bwd
+        self.epochs = torch.zeros(4, dtype=torch.int32, device=device)
         torch.cuda.synchronize(device)
         dist.barrier(group=group)                              # every rank's flags are zero before anyone signals
 
@@ -48,6 +53,7 @@ class ShardGroup:
         self.rank = dist.get_rank(group)
         self.peer = None          # a PeerExchange when the fused exchange is available (CUDA, NVLink peers, <= 16 ranks)
         self.peer_error = None    # why it is not (the NCCL all-reduce is used then)
+        self.global_read = False  # read loss and score_query over the global batch (enable_sharded_update(global_read=True))
 
     def enable_peer_exchange(self, device):
         """Try to set up the fused peer-memory exchange; on any failure keep the NCCL all-reduces (and remember why).
@@ -93,26 +99,99 @@ class AllReduceSum(torch.autograd.Function):
         return all_reduce_sum_(g.contiguous().clone(), ctx.shard), None
 
 
-def enable_sharded_update(module, group=None, peer_exchange=True):
+def enable_sharded_update(module, group=None, peer_exchange=True, global_read=False):
     """Turn on the all-reduce of class sums for every ``Memory_sup`` inside ``module``.
 
     Call after ``init_process_group`` (and after DDP wrapping, or on the bare net) on EVERY rank (collective). Returns
     the (last) ``ShardGroup``. Without this call the module keeps the reference's rank-local update. With
     ``peer_exchange`` (default) the exchange is fused into the update kernels over NVLink peer memory when the platform
     supports it (``ShardGroup.peer``), else two NCCL all-reduces per step are issued.
+
+    ``global_read=True`` also makes the read's two reductions over pixels global: the read loss becomes the mean over the
+    valid label pixels of ALL ranks (memory.py:173-176) and score_query the softmax over all ranks' pixels
+    (memory.py:183,186-187), each bit-identical across ranks; the backward sums the ranks' gradients of both (the autograd
+    mirror of an all-reduce, as for the class sums). Together with the sharded update and SyncBatchNorm, every output and
+    gradient of the module is then independent of the number of GPUs the global batch is split over. It costs two small
+    exchanges per read (one forward, one backward), over the same peer buffers or, without them, NCCL all-gathers. All
+    ranks must pass the same value (checked). ``get_score`` stays rank-local.
+
+    Only reads made with grad mode on exchange (training steps, the meta-test read); a read under ``torch.no_grad()``
+    (validation's ``net(inputs)``, ``memory_initalize``) stays rank-local and needs nothing from the other ranks. Every
+    grad-mode forward of the module is then a collective: all ranks must make the same number of them, in the same order
+    (a training step with the sharded update or SyncBatchNorm already is one; with global_read a grad-mode read without a
+    write is one too). A rank that makes one fewer leaves its peers
+    waiting: on the peer path their exchange kernel gives up after a bounded spin with a device trap (an unrecoverable CUDA
+    error in those processes), on the NCCL path their all-gather waits for NCCL's own timeout.
     """
     from .memory import Memory_sup
 
+    if not isinstance(global_read, bool):
+        raise TypeError(f"enable_sharded_update: global_read must be a bool, got {type(global_read).__name__}")
     mems = [m for m in module.modules() if isinstance(m, Memory_sup)]
     if not mems:
         raise RuntimeError("enable_sharded_update: no Memory_sup inside the given module")
     shard = None
     for m in mems:   # one exchange buffer per memory module (each has its own sums and step order)
         shard = ShardGroup(group)
+        _check_same_on_all_ranks(global_read, shard, m.m_items.device)
+        shard.global_read = global_read
         if peer_exchange and m.m_items.is_cuda:
             shard.enable_peer_exchange(m.m_items.device)
         m.shard_group = shard
     return shard
+
+
+def _check_same_on_all_ranks(flag, shard, device):
+    """Raise on every rank when the ranks passed different values of a collective switch (a rank that exchanges while
+    another does not would wait for a peer that never arrives)."""
+    if shard.world_size == 1:
+        return
+    t = torch.tensor([int(flag), -int(flag)], dtype=torch.int32, device=device)
+    dist.all_reduce(t, op=dist.ReduceOp.MAX, group=shard.group)
+    if int(t[0]) != -int(t[1]):
+        raise ValueError("enable_sharded_update: global_read must be the same on every rank")
+
+
+def global_read(shard):
+    """True when a read under this shard group exchanges its reductions (global_read on, more than one rank)."""
+    return shard is not None and shard.global_read and shard.world_size > 1
+
+
+def gather_rows(row, shard):
+    """[world, n] tensor of every rank's row ``row`` [n], in rank order (one all-gather on the current stream): the
+    layout the exchange kernels read when there is no peer memory."""
+    out = torch.empty(shard.world_size * row.numel(), dtype=row.dtype, device=row.device)
+    dist.all_gather_into_tensor(out, row.contiguous(), group=shard.group)
+    return out.view(shard.world_size, row.numel())
+
+
+def read_exchange_fwd(shard, col_partials, ws, temperature, out, K):
+    """Forward exchange of the global read: col_partials' combined row (and, with the read-loss workspace ws and its
+    out[2], the read loss and its gradient scale) become those of the global batch."""
+    from . import capi
+
+    if shard.peer is not None:
+        capi.read_exchange_fwd(shard.peer, None, shard.world_size, col_partials, ws, temperature, out, K)
+        return
+    row = torch.empty(capi.READ_ROW_FLOATS, dtype=torch.float32, device=col_partials.device)
+    capi.read_row_fwd(col_partials, ws, row, K)
+    capi.read_exchange_fwd(None, gather_rows(row, shard), shard.world_size, col_partials, ws, temperature, out, K)
+
+
+def read_exchange_bwd(shard, partials, g_loss, K, device):
+    """Backward exchange of the global read: (sum over ranks of readloss's upstream gradient, fp32 [1]; global column sums
+    of score_query's backward, fp64 [32]). ``partials`` (capi.score_bwd_partials) and ``g_loss`` may be None (zero)."""
+    from . import capi
+
+    buf = torch.empty(33, dtype=torch.float64, device=device)
+    colsums, g_sum = buf[:32], buf[32:].view(torch.float32)[:1]
+    if shard.peer is not None:
+        capi.read_exchange_bwd(shard.peer, None, shard.world_size, partials, g_loss, g_sum, colsums, K)
+        return g_sum, colsums
+    row = torch.empty(capi.READ_ROW_FLOATS, dtype=torch.float32, device=device)
+    capi.read_row_bwd(partials, g_loss, row, K)
+    capi.read_exchange_bwd(None, gather_rows(row, shard), shard.world_size, partials, g_loss, g_sum, colsums, K)
+    return g_sum, colsums
 
 
 def broadcast_memory(module, src=0, group=None):
