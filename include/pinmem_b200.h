@@ -56,7 +56,7 @@ enum pm_readloss_ws_layout {
 #define PM_COLPART_ROWS 296
 
 /* Bumped with every prototype change; the binding refuses a library whose pm_version() differs. */
-#define PM_ABI_VERSION 214
+#define PM_ABI_VERSION 215
 int pm_version(void);
 const char* pm_status_string(int code);
 /* Row stride (floats) of the internal score buffers for K slots: 20 for K<=19, else 32. */
@@ -399,7 +399,7 @@ int pm_write_bwd8(const float* dS, const void* f, const uint8_t* lab8, void* df,
  *   bytes [PM_PEER_FLAG_OFF, ...) arrival flags, zeroed once at allocation
  * CTA i raises a flag in every peer's buffer, waits for all ranks' flags, reads row i (forward: all rows) out of the
  * peers' buffers and sums in rank order -- identical on every rank, so the new memory is bit-identical across ranks.
- * `epoch`: one device uint32 per kernel kind (two in total), zeroed at allocation, owned by the kernels.
+ * `epoch`: one device uint32 per kernel kind (two for these kernels), zeroed at allocation, owned by the kernels.
  * SD_sum [K+1,C+4] (may be NULL) receives the all-reduced sums|counts; dS [K,C] the all-reduced gradient.
  * Every rank of the group must launch the same sequence of these two kernels (they spin on each other, bounded: a peer
  * that never arrives traps instead of hanging).
@@ -466,6 +466,45 @@ int pm_score_bwd_partials(const float* score_q, const float* g_q, float* workspa
 int pm_score_bwd_global(const float* score_q, const float* g_q, const float* score_m, const float* g_m, const float* ds_rl,
                         const float* g_loss, const float* rl_out, const double* colsums, float* E, int N, int K,
                         void* stream);
+
+/*
+ * SyncBatchNorm over the same symmetric buffers (csrc/pm_bn_exchange.cu). Under the reference's --syncbn
+ * (convert_sync_batchnorm, train.py:95) the module's two BatchNorms normalise with the statistics of the global batch:
+ * the forward sums the GEMM epilogue's fp64 [sum | sum of squares] and the pixel counts over the ranks, the backward sums
+ * (dgamma, dbeta) for the input gradient (the parameter gradients stay local; DDP averages them). When the layer reduces
+ * over the group of the sharded update, these two entries do that over NVLink peer memory instead of two NCCL all-reduces.
+ * Every sum runs over the ranks in rank order in fp64, so the result is bit-identical on every rank.
+ *
+ * `slot` 0 is the module's output block (memory.py:103-107), 1 its writing net (memory.py:74-87). Each (slot, direction)
+ * pair has its own row, its own two flags and its own `epoch` (a device uint32, zeroed at allocation, owned by the kernel):
+ *   flags  kind 8 of the flag area (PM_PEER_BN_FLAG_OFF, 8 rows x 16 ranks of u32): row 2x arrival, row 2x + 1 "done"
+ *          of exchange x = 2 * slot + direction (0 forward, 1 backward)
+ *   rows   forward  PM_PEER_BN_FWD_OFF + slot * PM_BN_FWD_ROW_BYTES: doubles [0, 2M) the rank's [sum | sum of squares],
+ *                   [2M] its pixel count
+ *          backward PM_PEER_BN_BWD_OFF + slot * PM_BN_BWD_ROW_BYTES: floats [0, M) the rank's dgamma, [M, 2M) its dbeta
+ * Protocol as pm_read_exchange_*: one CTA waits for the "done" flags of the previous launch, writes the rank's row, raises
+ * its flag in every peer's buffer, waits (bounded) for all ranks, combines, raises "done". 1 <= M <= PM_BN_MAX_C,
+ * 2 <= world <= 16, slot in {0, 1}. Every rank of the group must launch the same sequence of these entries per slot.
+ *
+ * pm_bn_exchange_fwd: stats double[2M+1], the rank's [sum | sum of squares] in [0, 2M) (pm_conv1x1_fwd[_ordered]'s
+ *   epilogue); count = the rank's pixel count B*h*w. Out, in place: the sums over the ranks and, in stats[2M], the global
+ *   count -- pm_bn_apply_stats / pm_write_reduce_bn_fwd[_ordered] then run unchanged with count_dev = stats + 2M.
+ * pm_bn_exchange_bwd: dgamma, dbeta float[M] of this rank (pm_bn_bwd_reduce_rows / pm_write_bwd_bn); count_global = the
+ *   forward's stats + 2M; local_count = this rank's pixel count. Out: sg, sb float[M] = (sum over ranks, fp64) *
+ *   local_count / count_global, rounded once -- the sums pm_conv1x1_dgrad_bnbwd / pm_bn_bwd_apply take (they divide by the
+ *   local count).
+ */
+#define PM_BN_MAX_C 256
+#define PM_PEER_BN_FLAG_OFF 90112
+#define PM_PEER_BN_FWD_OFF 99328
+#define PM_BN_FWD_ROW_BYTES 4112
+#define PM_PEER_BN_BWD_OFF 107552
+#define PM_BN_BWD_ROW_BYTES 2048
+int pm_bn_exchange_fwd(const void* peer_bufs, int rank, int world, unsigned* epoch, int slot, double* stats, double count, int M,
+                       void* stream);
+int pm_bn_exchange_bwd(const void* peer_bufs, int rank, int world, unsigned* epoch, int slot, const float* dgamma,
+                       const float* dbeta, const double* count_global, double local_count, float* sg, float* sb, int M,
+                       void* stream);
 
 /* 64-bit words of the segmentation-metrics workspace (`ws`, zero it before every pm_seg_eval call). */
 enum pm_seg_eval_ws_layout {

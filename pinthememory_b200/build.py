@@ -15,7 +15,7 @@ PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG_DIR, "csrc")
 LIB_DIR = os.path.join(PKG_DIR, "_lib")
 LIB_PATH = os.path.join(LIB_DIR, "libpinmem_b200.so")
-SOURCES = ["pm_read.cu", "pm_read_tiled.cu", "pm_score.cu", "pm_readloss.cu", "pm_write.cu", "pm_write_tiled.cu", "pm_bn.cu", "pm_fold.cu", "pm_gemm.cu", "pm_losses.cu", "pm_labels.cu", "pm_readloss8.cu", "pm_readloss10.cu", "pm_segeval.cu", "pm_upcat.cu", "pm_ordered.cu", "pm_exchange.cu"]
+SOURCES = ["pm_read.cu", "pm_read_tiled.cu", "pm_score.cu", "pm_readloss.cu", "pm_write.cu", "pm_write_tiled.cu", "pm_bn.cu", "pm_fold.cu", "pm_gemm.cu", "pm_losses.cu", "pm_labels.cu", "pm_readloss8.cu", "pm_readloss10.cu", "pm_segeval.cu", "pm_upcat.cu", "pm_ordered.cu", "pm_exchange.cu", "pm_bn_exchange.cu"]
 ARCH_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a"]
 NVCC_FLAGS = ["-O3", "-lineinfo", "-std=c++17", "--use_fast_math=false", "-Xcompiler", "-fPIC"]
 

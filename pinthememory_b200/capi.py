@@ -19,7 +19,7 @@ WS_BAD = 2     # PM_WS_BAD
 SEG_WS_WORDS = 4  # PM_SEG_WS_WORDS
 SEG_WS_BAD = 2    # PM_SEG_WS_BAD
 
-ABI_VERSION = 214  # PM_ABI_VERSION of include/pinmem_b200.h the argtypes below were written against
+ABI_VERSION = 215  # PM_ABI_VERSION of include/pinmem_b200.h the argtypes below were written against
 
 _c_p = ctypes.c_void_p
 _c_i = ctypes.c_int
@@ -101,6 +101,8 @@ PROTOTYPES = {
     "pm_read_exchange_bwd": [_c_p, _c_i, _c_i] + [_c_p] * 6 + [_c_i, _c_p],
     "pm_score_bwd_partials": [_c_p] * 3 + [_c_i] * 2 + [_c_p],
     "pm_score_bwd_global": [_c_p] * 9 + [_c_i] * 2 + [_c_p],
+    "pm_bn_exchange_fwd": [_c_p, _c_i, _c_i, _c_p, _c_i, _c_p, _c_d, _c_i, _c_p],
+    "pm_bn_exchange_bwd": [_c_p, _c_i, _c_i, _c_p, _c_i] + [_c_p] * 3 + [_c_d, _c_p, _c_p, _c_i, _c_p],
 }
 EXPORTED_SYMBOLS = sorted(list(PROTOTYPES) + ["pm_status_string"])
 
@@ -767,3 +769,31 @@ def score_bwd_global(score_q, g_q, score_m, g_m, E, K, colsums, ds_rl=None, g_lo
     N = E.shape[0]
     _call("pm_score_bwd_global", _ptr(score_q), _ptr(g_q), _ptr(score_m), _ptr(g_m), _ptr(ds_rl), _ptr(g_loss), _ptr(rl_out),
           _ptr(colsums), _ptr(E), N, K, _stream())
+
+
+# ------------------------------- SyncBatchNorm over the sharded update's peer buffers (csrc/pm_bn_exchange.cu)
+
+BN_MAX_C = 256                                           # PM_BN_MAX_C
+PEER_BN_FLAG_OFF = 90112                                 # PM_PEER_BN_FLAG_OFF
+PEER_BN_FWD_OFF, BN_FWD_ROW_BYTES = 99328, 4112          # PM_PEER_BN_FWD_OFF, PM_BN_FWD_ROW_BYTES
+PEER_BN_BWD_OFF, BN_BWD_ROW_BYTES = 107552, 2048         # PM_PEER_BN_BWD_OFF, PM_BN_BWD_ROW_BYTES
+
+
+def _bn_epoch(peer, slot, direction):
+    """The device launch counter of one (slot, direction) exchange: PeerExchange.epochs[4 + 2 * slot + direction]."""
+    i = 4 + 2 * slot + direction
+    return _ptr(peer.epochs[i:i + 1])
+
+
+def bn_exchange_fwd(peer, slot, stats, count, M):
+    """stats [2M+1] fp64 (the rank's [sum | sum of squares] in [0, 2M)) becomes, in place, the sums over the ranks with the
+    global pixel count in stats[2M]; ``count`` is this rank's. slot 0: the output block, 1: the writing net."""
+    _call("pm_bn_exchange_fwd", peer.bufs_dev, peer.rank, peer.world_size, _bn_epoch(peer, slot, 0), int(slot), _ptr(stats),
+          float(count), int(M), _stream())
+
+
+def bn_exchange_bwd(peer, slot, dgamma, dbeta, count_global, local_count, sg, sb, M):
+    """sg, sb [M] fp32 = the ranks' sums of dgamma, dbeta (fp64, rank order) * local_count / count_global (a device fp64
+    scalar: the forward's stats[2M])."""
+    _call("pm_bn_exchange_bwd", peer.bufs_dev, peer.rank, peer.world_size, _bn_epoch(peer, slot, 1), int(slot), _ptr(dgamma),
+          _ptr(dbeta), _ptr(count_global), float(local_count), _ptr(sg), _ptr(sb), int(M), _stream())

@@ -301,7 +301,7 @@ __device__ __forceinline__ double sb_group_sum(const double* part, int k, int j)
 
 // ---- cross-rank flags in the symmetric peer buffer (pm_write.cu: the sharded update; pm_exchange.cu: the global read).
 // flags[kind][row 0..31][rank 0..15] (u32, monotone epochs) at PM_PEER_FLAG_OFF; kinds 0..3 belong to the update kernels,
-// 4..7 to the read exchanges.
+// 4..7 to the read exchanges, rows 0..7 of kind 8 (PM_PEER_BN_FLAG_OFF) to the SyncBatchNorm exchanges (pm_bn_exchange.cu).
 struct PeerCtx {
     const unsigned long long* bufs;  // device array [world] of symmetric-buffer base addresses; nullptr = not sharded
     int rank, world;

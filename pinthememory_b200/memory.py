@@ -371,12 +371,10 @@ class _WriteNetFn(torch.autograd.Function):
         (hi, lo), ctx.preT = capi.conv1x1_prep_both(W2, torch.float32, zero=stats, tf32=ctx.tf32)
         z = capi.conv1x1_fwd(x, hi, lo, C, stats=stats)
         count = None
-        if sync_group is not None:   # as _ConvBnActFn: global statistics
-            import torch.distributed as dist
-
-            stats[2 * C:].fill_(float(B * h * w))
-            dist.all_reduce(stats, group=sync_group)
-            count = stats[2 * C:]
+        ctx.bn_peer = None
+        if sync_group is not None:   # as _ConvBnActFn: global statistics (slot 1 of the shard group's peer buffer)
+            ctx.bn_peer = sharding.bn_peer(group, sync_group, C)
+            count = sharding.bn_stats_exchange(stats, B * h * w, C, sync_group, ctx.bn_peer, 1)
         mean = torch.empty(C, dtype=torch.float32, device=dev)
         invstd = torch.empty(C, dtype=torch.float32, device=dev)
         M_new, losses, saved, W, b, SD = _write_update_fwd(
@@ -410,12 +408,7 @@ class _WriteNetFn(torch.autograd.Function):
             capi.write_bwd_bn(dS, z, x, labels, mean, invstd, g32, b32, g, dgamma, dbeta, K)
             sg, sb = dgamma, dbeta
             if ctx.sync_group is not None:   # as _ConvBnActFn.backward: input gradient from the sums over all ranks
-                import torch.distributed as dist
-
-                sums = torch.cat([dgamma, dbeta])
-                dist.all_reduce(sums, group=ctx.sync_group)
-                sums = sums * (float(B * h * w) / count).to(torch.float32)
-                sg, sb = sums[:C].contiguous(), sums[C:].contiguous()
+                sg, sb = sharding.bn_grad_exchange(dgamma, dbeta, B * h * w, count, ctx.sync_group, ctx.bn_peer, 1)
             dz = torch.empty_like(z)
             capi.bn_bwd_apply(g, None, None, z, mean, invstd, g32, sg, sb, False, True, dz, None)
             if ctx.needs_input_grad[0]:
@@ -514,7 +507,7 @@ class _ConvBnActFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, W, gamma, beta, residual, running_mean, running_var, use_batch_stats, factor, eps, relu,
-                res_is_x, sync_group=None, num_batches_tracked=None, pre=None):
+                res_is_x, sync_group=None, num_batches_tracked=None, pre=None, shard=None, slot=0):
         B, K, h, w = x.shape
         M = W.shape[0]
         dev = x.device
@@ -522,6 +515,7 @@ class _ConvBnActFn(torch.autograd.Function):
         g32 = gamma.detach().to(torch.float32).contiguous()
         b32 = beta.detach().to(torch.float32).contiguous()
         ctx.preT = None
+        ctx.bn_peer, ctx.slot = None, slot
         stats = None
         tf32 = x.dtype == torch.float32 and capi.tf32()
         if pre is not None and (pre[0][0].dtype != x.dtype or capi.operands_tf32(pre[0]) != tf32):
@@ -539,17 +533,15 @@ class _ConvBnActFn(torch.autograd.Function):
             hi, lo = capi.conv1x1_prep(W2, False, x.dtype, tf32=tf32)
         if use_batch_stats:
             # [sum | sum of squares | element count]: the GEMM epilogue fills the first 2M; with SyncBatchNorm the whole
-            # vector is summed over the ranks (fp64, one small all-reduce) and the normalise pass finalises GLOBAL statistics
+            # vector is summed over the ranks (fp64; over the shard group's peer memory when the layer reduces over that
+            # group, else one small all-reduce) and the normalise pass finalises GLOBAL statistics
             if stats is None:
                 stats = torch.zeros(2 * M + 1, dtype=torch.float64, device=dev)
             xc = capi.conv1x1_fwd(x, hi, lo, M, stats=stats)
             count = None
             if sync_group is not None:
-                import torch.distributed as dist
-
-                stats[2 * M:].fill_(float(B * h * w))   # (a fill kernel: capturable, unlike a scalar copy from the host)
-                dist.all_reduce(stats, group=sync_group)
-                count = stats[2 * M:]
+                ctx.bn_peer = sharding.bn_peer(shard, sync_group, M)
+                count = sharding.bn_stats_exchange(stats, B * h * w, M, sync_group, ctx.bn_peer, slot)
             mean = torch.empty(M, dtype=torch.float32, device=dev)
             invstd = torch.empty(M, dtype=torch.float32, device=dev)
         else:
@@ -596,14 +588,10 @@ class _ConvBnActFn(torch.autograd.Function):
         sg, sb = dgamma, dbeta
         if ctx.sync_group is not None:
             # SyncBatchNorm: the input gradient needs the sums over ALL ranks' pixels (the parameter gradients stay
-            # local, DDP averages them -- torch's own SyncBatchNorm does the same). One all-reduce of 2M floats; the
-            # kernel divides by the LOCAL pixel count, so the global sums are pre-scaled by local / global.
-            import torch.distributed as dist
-
-            sums = torch.cat([dgamma, dbeta])
-            dist.all_reduce(sums, group=ctx.sync_group)
-            sums = sums * (float(xc.shape[0] * xc.shape[2] * xc.shape[3]) / count).to(torch.float32)
-            sg, sb = sums[:M].contiguous(), sums[M:].contiguous()
+            # local, DDP averages them -- torch's own SyncBatchNorm does the same); the kernel divides by the LOCAL pixel
+            # count, so the global sums come pre-scaled by local / global
+            sg, sb = sharding.bn_grad_exchange(dgamma, dbeta, xc.shape[0] * xc.shape[2] * xc.shape[3], count, ctx.sync_group,
+                                               ctx.bn_peer, ctx.slot)
         if need_x and not ctx.has_res and xc.dtype == torch.float32 and M % 32 == 0 and ctx.beta32 is not None:
             # blocks without a residual (self.output): the BatchNorm backward rides in the operand path of the
             # input-gradient GEMM, which also stores dz for the weight-gradient GEMM -- no bn_bwd_apply pass
@@ -625,7 +613,7 @@ class _ConvBnActFn(torch.autograd.Function):
                     x.record_stream(aux)
                 else:
                     dW = capi.conv1x1_wgrad(dxc, x, tf32=ctx.tf32).view(ctx.wshape).to(ctx.wdtype)
-            return dx, dW, dgamma, dbeta, None, None, None, None, None, None, None, None, None, None, None
+            return dx, dW, dgamma, dbeta, None, None, None, None, None, None, None, None, None, None, None, None, None
         capi.bn_bwd_apply(dy, y, mask, xc, mean, invstd, g32, sg, sb, ctx.relu, ctx.training, dxc, dres)
         dW = None
         if ctx.needs_input_grad[1]:
@@ -638,7 +626,8 @@ class _ConvBnActFn(torch.autograd.Function):
                 dres = None
             else:
                 dx = capi.conv1x1_fwd(dxc, hiT, loT, K)
-        return dx, dW, dgamma, dbeta, (None if ctx.res_is_x else dres), None, None, None, None, None, None, None, None, None, None
+        return (dx, dW, dgamma, dbeta, (None if ctx.res_is_x else dres), None, None, None, None, None, None, None, None, None, None,
+                None, None)
 
 
 def _plain(m):
@@ -717,11 +706,12 @@ def _sync_group(bn):
     return group if dist.get_world_size(group) > 1 else None
 
 
-def weight_bn_act(W, bn, x, residual, relu, name=None, prepared=None, affine=None, pre=None):
+def weight_bn_act(W, bn, x, residual, relu, name=None, prepared=None, affine=None, pre=None, shard=None, slot=0):
     """[relu](BatchNorm2d(conv1x1(x, W)) [+ residual]) for a [M,K,1,1] weight: everything in this package's kernels
     (tcgen05 GEMM with the statistics in its epilogue + one normalise pass) when the shapes allow, else the library
-    convolution followed by the fused BatchNorm passes."""
-    y = _weight_bn_act(W, bn, x, residual, relu, prepared, affine, pre)
+    convolution followed by the fused BatchNorm passes. ``shard`` / ``slot``: the module's shard group and which of its two
+    blocks this is (0 output, 1 writing net): a SyncBatchNorm over the shard group exchanges over its peer memory."""
+    y = _weight_bn_act(W, bn, x, residual, relu, prepared, affine, pre, shard, slot)
     if GATE_LOG is not None and relu and name is not None:
         GATE_LOG.setdefault(name, []).append(y.detach() > 0)
     return y
@@ -739,7 +729,7 @@ def _inference_block(bn, x, residual):
             and bn.running_var.dtype == torch.float32)
 
 
-def _weight_bn_act(W, bn, x, residual, relu, prepared=None, affine=None, pre=None):
+def _weight_bn_act(W, bn, x, residual, relu, prepared=None, affine=None, pre=None, shard=None, slot=0):
     if torch.is_autocast_enabled("cuda"):  # the nn.Conv2d this replaces would run in the autocast dtype
         x = x.to(torch.get_autocast_dtype("cuda"))
     M, K = W.shape[0], W.shape[1]
@@ -757,16 +747,16 @@ def _weight_bn_act(W, bn, x, residual, relu, prepared=None, affine=None, pre=Non
             residual = residual.to(x.dtype).contiguous()
         use_batch, rm, rv, factor, nbt = _bn_args(bn, defer_counter=True)
         return _ConvBnActFn.apply(x, W, bn.weight, bn.bias, None if res_is_x else residual, rm, rv, use_batch, factor,
-                                  float(bn.eps), relu, res_is_x, _sync_group(bn), nbt, pre)
+                                  float(bn.eps), relu, res_is_x, _sync_group(bn), nbt, pre, shard, slot)
     _warn_once("libconv", "a 1x1 convolution fell back to the library GEMM (feature rows not 16-byte aligned, or an "
                           "unsupported channel count); the BatchNorm passes stay fused")
     return bn_act(F.conv2d(x, W.to(x.dtype)), bn, residual, relu)
 
 
-def conv_bn_act(conv, bn, x, residual, relu, name=None):
-    """conv -> BatchNorm2d (-> + residual) (-> ReLU) for the module's 1x1 blocks."""
+def conv_bn_act(conv, bn, x, residual, relu, name=None, shard=None, slot=0):
+    """conv -> BatchNorm2d (-> + residual) (-> ReLU) for the module's 1x1 blocks (``shard``, ``slot``: see weight_bn_act)."""
     if _pointwise(conv) and _plain(conv):
-        return weight_bn_act(conv.weight, bn, x, residual, relu, name)
+        return weight_bn_act(conv.weight, bn, x, residual, relu, name, shard=shard, slot=slot)
     y = bn_act(conv(x), bn, residual, relu)
     if GATE_LOG is not None and relu and name is not None:
         GATE_LOG.setdefault(name, []).append(y.detach() > 0)
@@ -803,7 +793,9 @@ class Writingnet(nn.Module):
 
     def forward(self, x):
         if x.is_cuda and _plain(self.writefeat) and _plain(self.writefeat[0]):
-            return conv_bn_act(self.writefeat[0], self.writefeat[1], x, x, True, "writenet")
+            # _shard_group: the owning Memory_sup's shard group, set by its write() (a plain attribute: not in state_dict)
+            return conv_bn_act(self.writefeat[0], self.writefeat[1], x, x, True, "writenet",
+                               shard=getattr(self, "_shard_group", None), slot=1)
         return self.relu(x + self.writefeat(x))
 
 
@@ -1010,9 +1002,11 @@ class Memory_sup(nn.Module):
                 Wp = _FoldWeightFn.apply(self.output[0].weight, M)
             updated_query = weight_bn_act(Wp, self.output[1], u, None, True, "output", prepared,   # Wp [C_out, C+32, 1, 1]
                                           pre[1] if infer else None,
-                                          wpre[1] if (wpre is not None and prepared is None) else None)
+                                          wpre[1] if (wpre is not None and prepared is None) else None,
+                                          shard=self.shard_group, slot=0)
         elif plain:
-            updated_query = conv_bn_act(self.output[0], self.output[1], u, None, True, "output")
+            updated_query = conv_bn_act(self.output[0], self.output[1], u, None, True, "output", shard=self.shard_group,
+                                        slot=0)
         else:
             updated_query = self.output(u)
         return updated_query, score_query, score_memory, readloss
@@ -1043,6 +1037,8 @@ class Memory_sup(nn.Module):
                 _sync_group(bn), self.clsfier.weight, self.clsfier.bias, float(self.momentum), self.memory_size,
                 self.shard_group)
         else:
+            if isinstance(self.writenet, Writingnet):
+                self.writenet._shard_group = self.shard_group   # its SyncBatchNorm exchanges over this group's peer memory
             f = self.writenet(query)
             f = _check_features(f, "write feature")
             M_new, div_loss, cls_loss, SD = _WriteFn.apply(f, labels, M_old, self.clsfier.weight, self.clsfier.bias,

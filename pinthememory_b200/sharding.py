@@ -10,6 +10,9 @@ The reference has no such collective (each rank silently keeps its own memory, S
 Opt-in (``global_read=True``): the read loss and score_query, the read's two reductions over pixels, are also taken over
 the global batch -- one small row per rank exchanged before the column softmax and one in the backward
 (csrc/pm_exchange.cu).
+
+SyncBatchNorm layers (``convert_sync_batchnorm``) that reduce over the shard group sum their batch statistics and backward
+sums over the same peer buffers (csrc/pm_bn_exchange.cu; ``bn_peer``), else with NCCL all-reduces.
 """
 import torch
 import torch.distributed as dist
@@ -32,8 +35,9 @@ class PeerExchange:
         self.handle = symm.rendezvous(self.buffer, pg.group_name)
         self.rank, self.world_size = self.handle.rank, self.handle.world_size
         self.bufs_dev = int(self.handle.buffer_ptrs_dev)      # device array of all ranks' buffer addresses
-        # one launch counter per kernel kind: update fwd, update bwd, global-read fwd, global-read bwd
-        self.epochs = torch.zeros(4, dtype=torch.int32, device=device)
+        # one launch counter per kernel kind: update fwd, update bwd, global-read fwd, global-read bwd, then the SyncBatchNorm
+        # exchanges: output block fwd, bwd, writing net fwd, bwd (capi.bn_exchange_*)
+        self.epochs = torch.zeros(8, dtype=torch.int32, device=device)
         torch.cuda.synchronize(device)
         dist.barrier(group=group)                              # every rank's flags are zero before anyone signals
 
@@ -192,6 +196,59 @@ def read_exchange_bwd(shard, partials, g_loss, K, device):
     capi.read_row_bwd(partials, g_loss, row, K)
     capi.read_exchange_bwd(None, gather_rows(row, shard), shard.world_size, partials, g_loss, g_sum, colsums, K)
     return g_sum, colsums
+
+
+def same_group(a, b):
+    """True when two process-group handles name the same group; ``None`` and ``dist.group.WORLD`` are the same group."""
+    if a is b:
+        return True
+    world = dist.group.WORLD if dist.is_available() and dist.is_initialized() else None
+    return (a is None or a is world) and (b is None or b is world)
+
+
+def bn_peer(shard, group, channels):
+    """The PeerExchange a SyncBatchNorm layer of ``channels`` channels that reduces over ``group`` sums through, or None for
+    the NCCL all-reduces. It is the shard group's buffer when that group has one (``enable_sharded_update`` with the peer
+    exchange available), the layer reduces over that same group and has at most capi.BN_MAX_C channels. Decided per call
+    from the live layer, so it does not matter whether ``convert_sync_batchnorm`` ran before or after
+    ``enable_sharded_update``."""
+    from . import capi
+
+    if shard is None or shard.peer is None or shard.world_size < 2 or channels > capi.BN_MAX_C:
+        return None
+    return shard.peer if same_group(group, shard.group) else None
+
+
+def bn_stats_exchange(stats, count, M, group, peer, slot):
+    """SyncBatchNorm forward: stats [2M+1] fp64, the rank's [sum | sum of squares] in [0, 2M), become the sums over the
+    ranks of ``group`` with the global pixel count in stats[2M] (``count`` is the rank's). Over ``peer`` memory when given
+    (slot 0: the output block, 1: the writing net), else one NCCL all-reduce. Returns stats[2M:], the device count the
+    normalise pass takes."""
+    from . import capi
+
+    if peer is not None:
+        capi.bn_exchange_fwd(peer, slot, stats, count, M)
+    else:
+        stats[2 * M:].fill_(float(count))   # (a fill kernel: capturable, unlike a scalar copy from the host)
+        dist.all_reduce(stats, group=group)
+    return stats[2 * M:]
+
+
+def bn_grad_exchange(dgamma, dbeta, local_count, count, group, peer, slot):
+    """SyncBatchNorm backward: (sg, sb), the sums of the rank's dgamma, dbeta [M] over the ranks, scaled by local_count /
+    count (``count`` the device global count of bn_stats_exchange): the input-gradient passes divide by the LOCAL pixel
+    count. The parameter gradients themselves stay local (DDP averages them, as for torch's own SyncBatchNorm)."""
+    from . import capi
+
+    M = dgamma.numel()
+    if peer is not None:
+        out = torch.empty(2 * M, dtype=torch.float32, device=dgamma.device)
+        capi.bn_exchange_bwd(peer, slot, dgamma, dbeta, count, local_count, out[:M], out[M:], M)
+        return out[:M], out[M:]
+    sums = torch.cat([dgamma, dbeta])
+    dist.all_reduce(sums, group=group)
+    sums = sums * (float(local_count) / count).to(torch.float32)
+    return sums[:M].contiguous(), sums[M:].contiguous()
 
 
 def broadcast_memory(module, src=0, group=None):
