@@ -1027,10 +1027,11 @@ int write_reduce_tiled(const void* f, const void* labels, int lab_u8, float* SD,
             case 64: return launch_write_reduce_mma16<64, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st, part, ncta);
             case 128: return launch_write_reduce_mma16<128, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st, part, ncta);
             case 256: return launch_write_reduce_mma16<256, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st, part, ncta);
-            default: break;  // C = 32: the run-length FFMA2 kernel
+            case 32: break;  // the run-length FFMA2 kernel
+            default: return PM_ERR_CHANNELS;
         }
-        if (K <= 19) { PM_WT_SWITCH_C(__nv_bfloat16, 20, launch_write_reduce_tiled, f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st, part, ncta) }
-        else { PM_WT_SWITCH_C(__nv_bfloat16, 32, launch_write_reduce_tiled, f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st, part, ncta) }
+        if (K <= 19) return launch_write_reduce_tiled<__nv_bfloat16, 32, 20>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st, part, ncta);
+        return launch_write_reduce_tiled<__nv_bfloat16, 32, 32>(f, labels, lab_u8, SD, B, h, w, Hm, Wm, K, st, part, ncta);
     }
 }
 
