@@ -527,12 +527,36 @@ static int launch_nn(const void* X, const void* Ah, const void* Al, void* Y, dou
 // =================================================================================================================
 // Form 2: dW (M x N) = sum over (b, pixel) of dY[b] . X[b]^T   (weight gradient). Both operands K-major (K = pixels).
 //   mapG : [B*M rows][hw] output gradient, box [128 rows][PXC pixels]      (A operand)
-//   mapX : [B*Ntot rows][hw] layer input,  box [NW rows][PXC pixels], NI = N / NW boxes per stage   (B operand);
+//   mapX : [B*Ntot rows][hw] layer input,  box [NW/2 rows][PXC pixels], NI = N / NW boxes per stage   (B operand);
 //          this launch covers input channels n0 .. n0+N-1 (N <= 288) of the Ntot
-//   grid : (pixel chunks of every image, M / 128); each CTA writes its [128][N] partial to `part`
-//          part[(chunk * Mpad + row) * N + col]; wgrad_reduce_kernel sums the chunks.
+//   grid : (2 * ceil(mtiles / 2), pixel chunks of every image) in clusters of 2 along x (a launch with the pair along y
+//          is refused as a cluster misconfiguration): SM pair p runs row tiles 2p (rank 0, the leader) and 2p+1 (rank 1)
+//          of one chunk as M = 256 cta_group::2 MMAs. Each CTA stages its own 128 dY rows and HALF of every X box (rows
+//          NW/2 * rank ..), so X crosses L2 -> SM once per chunk and a stage is 34 KB per operand set instead of 52. Each CTA writes its [128][N] partial to `part`
+//          part[(chunk * Mpad + row) * N + col]; wgrad_reduce_kernel sums the chunks. With an odd number of row tiles
+//          the last pair's rank 1 has rows >= Mpad: it loads, splits and takes part in the MMAs, and stores nothing.
+//   protocol: each CTA's producer fills its own stage (local full[s]) once the leader's commit has released it (local
+//          empty[s]); its split warps (bf16: one relay thread) wait on full[s] and arrive on the LEADER's xfull[s]; the
+//          leader's MMA thread waits on xfull[s] only and commits to empty[s] -- and after the last block to accf --
+//          of both CTAs at once (multicast). Before exit each producer waits for the last commits on its empty
+//          barriers, so no arrival is still in flight towards a CTA that has left the SM.
 // =================================================================================================================
 constexpr int WG_NMAX = 288;
+
+template <typename T>
+__host__ __device__ constexpr int wgrad_stage_bytes() {
+    return (GemmTraits<T>::SPLIT ? 2 : 1) * (TILE_A_BYTES + WG_NMAX / 2 * 128);
+}
+template <typename T>
+__host__ __device__ constexpr int wgrad_stages() {  // 3 in 3xTF32 (68 KB stages), 6 in one pass and bf16 (34 KB)
+    return (212992 / wgrad_stage_bytes<T>()) > 6 ? 6 : (212992 / wgrad_stage_bytes<T>());
+}
+
+template <typename T>
+__device__ __forceinline__ void umma_issue_pair(uint32_t d, uint64_t a, uint64_t b, uint32_t idesc, uint32_t acc) {
+    if constexpr (sizeof(T) == 4) umma_tf32_pair(d, a, b, idesc, acc);
+    else umma_bf16_pair(d, a, b, idesc, acc);
+}
 
 template <typename T>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
@@ -542,47 +566,46 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
     using TR = GemmTraits<T>;
     constexpr int PXC = TR::PXC, UK = TR::UK, KSTEPS = PXC / UK;
     constexpr int NOPA = TR::SPLIT ? 2 : 1;
-    constexpr int BBYTES = WG_NMAX * 128;
-    constexpr int STAGE = NOPA * (TILE_A_BYTES + BBYTES);
-    constexpr int STAGES = (212992 / STAGE) > 4 ? 4 : (212992 / STAGE);
+    constexpr int BBYTES = WG_NMAX / 2 * 128;  // this CTA's half of the widest X block
+    constexpr int STAGE = wgrad_stage_bytes<T>();
+    constexpr int STAGES = wgrad_stages<T>();
     static_assert(STAGES >= 2, "ring too small");
 
     extern __shared__ unsigned char smem_raw[];
     unsigned char* smem = smem_align(smem_raw, 1024);
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem + STAGES * STAGE);
-    uint64_t* full = bars;
-    uint64_t* empty = bars + STAGES;
-    uint64_t* xfull = bars + 2 * STAGES;
-    uint64_t* accf = bars + 3 * STAGES;
+    uint64_t* full = bars;                 // [STAGES] this CTA's TMA landed
+    uint64_t* empty = bars + STAGES;       // [STAGES] the pair MMAs of the stage retired (leader's multicast commit)
+    uint64_t* xfull = bars + 2 * STAGES;   // [STAGES] leader only: both CTAs' tiles split (or landed, bf16)
+    uint64_t* accf = bars + 3 * STAGES;    // accumulator complete (leader's multicast commit)
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(accf + 1);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint32_t rank = cluster_ctarank();
     if (threadIdx.x == 0) {
         for (int i = 0; i < STAGES; ++i) {
             mbar_init(&full[i], 1);
             mbar_init(&empty[i], 1);
-            mbar_init(&xfull[i], 4);  // one arrival per operand-split warp
+            mbar_init(&xfull[i], TR::XFORM ? 8 : 2);  // one arrival per split warp (bf16: per relay thread) of either CTA
         }
         mbar_init(accf, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         prefetch_tmap(&mapG);
         prefetch_tmap(&mapX);
     }
-    if (warp == 1) tmem_alloc(tmem_slot, 512);
+    if (warp == 1) tmem_alloc_pair(tmem_slot, 512);
     tc_fence_before();
-    __syncthreads();
+    cluster_sync();  // both CTAs' barriers initialised before either arrives on the other's
     tc_fence_after();
     const uint32_t tmem = *tmem_slot;
 
-    const int chunk = blockIdx.x, mt = blockIdx.y;
+    const int mt = blockIdx.x, chunk = blockIdx.y;
     const int b = chunk / chunks_per_img, cb0 = (chunk - b * chunks_per_img) * blocks_per_chunk;
     const int nblk_img = (hw + PXC - 1) / PXC;
-    int nkb = nblk_img - cb0;
+    int nkb = nblk_img - cb0;  // >= 1: every chunk of wgrad_split starts inside its image
     if (nkb > blocks_per_chunk) nkb = blocks_per_chunk;
-    if (nkb < 0) nkb = 0;
-    const int NI = N / NW;
-    const uint32_t TX = TILE_A_BYTES + (uint32_t)N * 128;
-    const uint32_t IDESC = umma_idesc(TR::FMT, false, false, 128, NW);
+    const int NI = N / NW, NH = NW / 2;
+    const uint32_t TX = TILE_A_BYTES + (uint32_t)(NI * NH) * 128;
 
     if (warp == 0) {
         if (lane == 0) {
@@ -594,16 +617,16 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
                 const int px = (cb0 + kb) * PXC;
                 tma_load_2d(st, &mapG, px, b * M + mt * 128, &full[s]);
                 for (int j = 0; j < NI; ++j)
-                    tma_load_2d(st + NOPA * TILE_A_BYTES + j * NW * 128, &mapX, px, b * Ntot + n0 + j * NW, &full[s]);
+                    tma_load_2d(st + NOPA * TILE_A_BYTES + j * NH * 128, &mapX, px, b * Ntot + n0 + j * NW + (int)rank * NH, &full[s]);
             }
+            for (int kb = nkb; kb < nkb + STAGES; ++kb) mbar_wait(&empty[kb % STAGES], ((kb / STAGES) & 1) ^ 1);
         }
     } else if (warp == 1) {
-        if (lane == 0) {
+        if (lane == 0 && rank == 0) {
+            const uint32_t IDESC = umma_idesc(TR::FMT, false, false, 256, NW);
             for (int kb = 0; kb < nkb; ++kb) {
                 const int s = kb % STAGES;
-                const uint32_t ph = (kb / STAGES) & 1;
-                mbar_wait(&full[s], ph);
-                if (TR::XFORM) mbar_wait(&xfull[s], ph);
+                mbar_wait(&xfull[s], (kb / STAGES) & 1);
                 tc_fence_after();
                 const uint32_t sa = smem_u32(smem + s * STAGE);
                 const uint32_t sb = sa + NOPA * TILE_A_BYTES;
@@ -614,28 +637,27 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
                     const uint32_t first = (kb | ks) ? 1u : 0u;
                     for (int j = 0; j < NI; ++j) {
                         const uint32_t d = tmem + (uint32_t)(j * NW);
-                        const uint64_t bh = umma_desc(sb + j * NW * 128 + ks * 32, 16, 1024);
+                        const uint64_t bh = umma_desc(sb + j * NH * 128 + ks * 32, 16, 1024);
                         if (TR::SPLIT) {
-                            const uint64_t bl = umma_desc(sb + BBYTES + j * NW * 128 + ks * 32, 16, 1024);
-                            umma_issue<T>(d, al, bh, IDESC, first);
-                            umma_issue<T>(d, ah, bl, IDESC, 1u);
-                            umma_issue<T>(d, ah, bh, IDESC, 1u);
+                            const uint64_t bl = umma_desc(sb + BBYTES + j * NH * 128 + ks * 32, 16, 1024);
+                            umma_issue_pair<T>(d, al, bh, IDESC, first);
+                            umma_issue_pair<T>(d, ah, bl, IDESC, 1u);
+                            umma_issue_pair<T>(d, ah, bh, IDESC, 1u);
                         } else {
-                            umma_issue<T>(d, ah, bh, IDESC, first);
+                            umma_issue_pair<T>(d, ah, bh, IDESC, first);
                         }
                     }
                 }
-                umma_commit(&empty[s]);
+                umma_commit_pair(&empty[s], 0x3);
             }
-            umma_commit(accf);
+            umma_commit_pair(accf, 0x3);
         }
     } else if (warp < 6) {
         const int q = warp & 3;
-        const int row = mt * 128 + q * 32 + lane;
-        float* dst = part + ((size_t)chunk * Mpad + row) * N;
-        if (nkb > 0) {
-            mbar_wait(accf, 0);
-            tc_fence_after();
+        mbar_wait(accf, 0);  // (also on an idle rank 1: the MMAs writing its TMEM and reading its tiles are complete)
+        tc_fence_after();
+        if (mt * 128 < Mpad) {
+            float* dst = part + ((size_t)chunk * Mpad + mt * 128 + q * 32 + lane) * N;
             for (int c = 0; c < N / 32; ++c) {
                 uint32_t r[32];
                 tmem_ld32(tmem + ((uint32_t)(q * 32) << 16) + (uint32_t)(c * 32), r);
@@ -644,35 +666,37 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1)
                 for (int j = 0; j < 8; ++j)
                     *reinterpret_cast<uint4*>(dst + c * 32 + 4 * j) = make_uint4(r[4 * j], r[4 * j + 1], r[4 * j + 2], r[4 * j + 3]);
             }
-        } else {
-            for (int c = 0; c < N / 4; ++c) *reinterpret_cast<uint4*>(dst + 4 * c) = make_uint4(0u, 0u, 0u, 0u);
         }
-    } else {
-        if constexpr (TR::XFORM) {
-            const int t = threadIdx.x - 6 * 32;
-            for (int kb = 0; kb < nkb; ++kb) {
-                const int s = kb % STAGES;
-                mbar_wait(&full[s], (kb / STAGES) & 1);
-                unsigned char* st = smem + s * STAGE;
-                if (TR::SPLIT) {
-                    split_tile_trunc(reinterpret_cast<float4*>(st), reinterpret_cast<float4*>(st + TILE_A_BYTES), TILE_A_BYTES / 16, t, 128);
-                    split_tile_trunc(reinterpret_cast<float4*>(st + 2 * TILE_A_BYTES), reinterpret_cast<float4*>(st + 2 * TILE_A_BYTES + BBYTES),
-                                     N * 8, t, 128);
-                } else {
-                    round_tile(reinterpret_cast<float4*>(st), TILE_A_BYTES / 16, t, 128);
-                    round_tile(reinterpret_cast<float4*>(st + TILE_A_BYTES), N * 8, t, 128);
-                }
-                fence_proxy_async_smem();
-                __syncwarp();
-                if (lane == 0) mbar_arrive(&xfull[s]);
+    } else if constexpr (TR::XFORM) {
+        const int t = threadIdx.x - 6 * 32;
+        for (int kb = 0; kb < nkb; ++kb) {
+            const int s = kb % STAGES;
+            mbar_wait(&full[s], (kb / STAGES) & 1);
+            unsigned char* st = smem + s * STAGE;
+            if (TR::SPLIT) {
+                split_tile_trunc(reinterpret_cast<float4*>(st), reinterpret_cast<float4*>(st + TILE_A_BYTES), TILE_A_BYTES / 16, t, 128);
+                split_tile_trunc(reinterpret_cast<float4*>(st + 2 * TILE_A_BYTES), reinterpret_cast<float4*>(st + 2 * TILE_A_BYTES + BBYTES),
+                                 NI * NH * 8, t, 128);
+            } else {
+                round_tile(reinterpret_cast<float4*>(st), TILE_A_BYTES / 16, t, 128);
+                round_tile(reinterpret_cast<float4*>(st + TILE_A_BYTES), NI * NH * 8, t, 128);
             }
+            fence_proxy_async_smem();
+            __syncwarp();
+            if (lane == 0) mbar_arrive_remote(&xfull[s], 0);
+        }
+    } else if (warp == 6 && lane == 0) {  // bf16: the tiles go to the tensor core as they landed; relay "landed" to the leader
+        for (int kb = 0; kb < nkb; ++kb) {
+            const int s = kb % STAGES;
+            mbar_wait(&full[s], (kb / STAGES) & 1);
+            mbar_arrive_remote(&xfull[s], 0);
         }
     }
     tc_fence_before();
-    __syncthreads();
+    cluster_sync();  // the leader's MMAs, the peer's arrivals and every commit are done in both CTAs
     if (warp == 1) {
         tc_fence_after();
-        tmem_dealloc(tmem, 512);
+        tmem_dealloc_pair(tmem, 512);
     }
 }
 
@@ -718,11 +742,7 @@ __global__ void __launch_bounds__(256) wgrad_reduce_kernel(const float* __restri
 
 template <typename T>
 constexpr size_t wgrad_smem_bytes() {
-    using TR = GemmTraits<T>;
-    constexpr int NOPA = TR::SPLIT ? 2 : 1;
-    constexpr int STAGE = NOPA * (TILE_A_BYTES + WG_NMAX * 128);
-    constexpr int STAGES = (212992 / STAGE) > 4 ? 4 : (212992 / STAGE);
-    return (size_t)STAGES * STAGE + 256 + 1024;
+    return (size_t)wgrad_stages<T>() * wgrad_stage_bytes<T>() + 256 + 1024;
 }
 
 static void wgrad_split(int B, int M, int hw, int pxc, int* chunks_per_img, int* blocks_per_chunk) {
@@ -740,18 +760,30 @@ static int launch_wgrad(const void* dY, const void* X, float* part, float* dW, i
                         int accumulate, cudaStream_t st) {
     using TR = GemmTraits<T>;
     const int NI = N > 256 ? 2 : 1, NW = N / NI;
-    const int Mpad = (M + 127) / 128 * 128;
+    // the pair instruction (M = 256) takes N % 16 == 0, N <= 256, and each CTA stages NW/2 rows of X in 8-row swizzle atoms
+    if (N % NI || NW % 16 || NW > 256) return PM_ERR_SHAPE;
+    const int Mpad = (M + 127) / 128 * 128, mtiles = Mpad / 128;
     int cpi, bpc;
     wgrad_split(B, M, hw, TR::PXC, &cpi, &bpc);
     CUtensorMap mG, mX;
-    if (!make_map_2d<T>(&mG, dY, (size_t)B * M, hw, 128, TR::PXC, true)) return PM_ERR_ALIGN;
-    if (!make_map_2d<T>(&mX, X, (size_t)B * Ntot, hw, NW, TR::PXC, true)) return PM_ERR_ALIGN;
+    // 256-byte L2 promotion: a chunk walks its rows 128 bytes (one block) at a time, so every DRAM access also brings in
+    // the block after it (measured: one pass 54.5 -> 50.7 us at 256x288, the other forms unchanged)
+    if (!make_map_2d<T>(&mG, dY, (size_t)B * M, hw, 128, TR::PXC, true, true)) return PM_ERR_ALIGN;
+    if (!make_map_2d<T>(&mX, X, (size_t)B * Ntot, hw, NW / 2, TR::PXC, true, true)) return PM_ERR_ALIGN;
     const size_t smem = wgrad_smem_bytes<T>();
-    dim3 grid(B * cpi, Mpad / 128);
     cudaError_t e = cudaFuncSetAttribute(conv1x1_wgrad_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
-    conv1x1_wgrad_kernel<T><<<grid, GEMM_THREADS, smem, st>>>(mG, mX, M, N, Ntot, n0, NW, hw, cpi, bpc, part, Mpad);
-    e = cudaGetLastError();
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = 2, attr[0].val.clusterDim.y = 1, attr[0].val.clusterDim.z = 1;  // SM pairs: row tiles 2p, 2p+1
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((mtiles + 1) / 2 * 2, B * cpi);
+    cfg.blockDim = dim3(GEMM_THREADS);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = st;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    e = cudaLaunchKernelEx(&cfg, conv1x1_wgrad_kernel<T>, mG, mX, M, N, Ntot, n0, NW, hw, cpi, bpc, part, Mpad);
     if (e != cudaSuccess) return (int)e;
     const int n4 = M * (N / 4);
     wgrad_reduce_kernel<<<(n4 + 31) / 32, 256, 0, st>>>(part, dW, M, N, Mpad, Ntot, n0, B * cpi, accumulate);
@@ -962,7 +994,7 @@ int pm_conv1x1_wgrad(const void* dY, const void* X, float* workspace, float* dW,
     if (B <= 0 || hw <= 0 || M <= 0 || N <= 0 || M % 32 || N % 32 || M > 512 || N > 1024) return PM_ERR_SHAPE;
     if ((hw * esz) % 16 || ((uintptr_t)X | (uintptr_t)dY | (uintptr_t)workspace | (uintptr_t)dW) % 16) return PM_ERR_ALIGN;
     cudaStream_t st = (cudaStream_t)stream;
-    // column blocks of at most WG_NMAX input channels (TMEM: 128 lanes x 512 columns; ring: 2 x 104 KB); blocks wider
+    // column blocks of at most WG_NMAX input channels (TMEM: 128 lanes x 512 columns; ring: 3 x 68 KB); blocks wider
     // than 256 channels take two N/2-wide instructions, so they must be multiples of 32 channels
     for (int n0 = 0; n0 < N;) {
         int nb = N - n0;

@@ -72,23 +72,24 @@ static pm_encode_tiled_fn encode_tiled() {
 struct TensorMapKey {
     const void* base;
     size_t rows, cols;
-    unsigned box_rows, box_cols, esz, swz;
+    unsigned box_rows, box_cols, esz, swz, l2_256;
     bool operator==(const TensorMapKey& o) const {
         return base == o.base && rows == o.rows && cols == o.cols && box_rows == o.box_rows && box_cols == o.box_cols &&
-               esz == o.esz && swz == o.swz;
+               esz == o.esz && swz == o.swz && l2_256 == o.l2_256;
     }
 };
 
 template <typename T>
 static bool make_map_2d(CUtensorMap* map, const void* base, size_t rows, size_t cols, unsigned box_rows, unsigned box_cols,
-                        int swizzle128 /* 0 none, 1 SWIZZLE_128B (16-byte chunks), 2 SWIZZLE_128B_ATOM_32B (32-byte chunks), 3 SWIZZLE_64B */) {
+                        int swizzle128 /* 0 none, 1 SWIZZLE_128B (16-byte chunks), 2 SWIZZLE_128B_ATOM_32B (32-byte chunks), 3 SWIZZLE_64B */,
+                        bool l2_256 = false /* L2 promotion: 256-byte DRAM fetches instead of 128 */) {
     constexpr int SLOTS = 128;
     static std::mutex mu;
     static TensorMapKey keys[SLOTS];
     static CUtensorMap maps[SLOTS];
     static bool used[SLOTS];
     static unsigned next = 0;
-    const TensorMapKey key{base, rows, cols, box_rows, box_cols, (unsigned)sizeof(T), (unsigned)swizzle128};
+    const TensorMapKey key{base, rows, cols, box_rows, box_cols, (unsigned)sizeof(T), (unsigned)swizzle128, (unsigned)l2_256};
     std::lock_guard<std::mutex> lock(mu);
     for (int i = 0; i < SLOTS; ++i)
         if (used[i] && keys[i] == key) {
@@ -107,7 +108,7 @@ static bool make_map_2d(CUtensorMap* map, const void* base, size_t rows, size_t 
             : swizzle128 == 2 ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B
             : swizzle128      ? CU_TENSOR_MAP_SWIZZLE_128B
                               : CU_TENSOR_MAP_SWIZZLE_NONE,
-            CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+            l2_256 ? CU_TENSOR_MAP_L2_PROMOTION_L2_256B : CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
         return false;
     const unsigned slot = next++ % SLOTS;

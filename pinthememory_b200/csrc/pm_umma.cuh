@@ -70,6 +70,59 @@ __device__ __forceinline__ void umma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 
+// ---- SM pairs (cta_group::2): the two CTAs of a 2-CTA cluster run one MMA of M = 256 -------------------------------
+// Rank 0 (the leader) issues every MMA. A's rows 0-127 come from the leader's shared memory and rows 128-255 from the
+// peer's, B's first N/2 rows from the leader and the last N/2 from the peer, each at the same shared-memory offset as
+// the descriptors name; each CTA's TMEM receives its own 128 rows of D. Every tcgen05 instruction of such a kernel uses
+// cta_group::2; alloc, relinquish and dealloc are executed by one warp in EACH CTA of the pair.
+__device__ __forceinline__ uint32_t cluster_ctarank() {
+    uint32_t r;
+    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+    return r;
+}
+// every thread of every CTA of the cluster; orders shared-memory (and mbarrier) accesses across the cluster
+__device__ __forceinline__ void cluster_sync() {
+    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void tmem_alloc_pair(uint32_t* smem_dst, uint32_t ncols) {  // whole warp, in both CTAs
+    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_dst)), "r"(ncols)
+                 : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void tmem_dealloc_pair(uint32_t taddr, uint32_t ncols) {  // whole warp, in both CTAs
+    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+}
+__device__ __forceinline__ void umma_tf32_pair(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
+    asm volatile(
+        "{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\n"
+        "tcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n}" ::"r"(d_tmem),
+        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc)
+        : "memory");
+}
+__device__ __forceinline__ void umma_bf16_pair(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
+    asm volatile(
+        "{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\n"
+        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n}" ::"r"(d_tmem),
+        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc)
+        : "memory");
+}
+// one arrival on the mbarrier at `bar`'s offset in every CTA of `cta_mask` once the pair MMAs issued so far have completed
+__device__ __forceinline__ void umma_commit_pair(uint64_t* bar, uint16_t cta_mask) {
+    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
+                     smem_u32(bar)),
+                 "h"(cta_mask)
+                 : "memory");
+}
+// arrive on the mbarrier at `bar`'s offset in cluster CTA `cta` (release at CTA scope, as a local arrive: a cluster-scope
+// release here costs microseconds per arrival and serialises the split warps -- measured, 3xTF32 wgrad 72 -> 78 us)
+__device__ __forceinline__ void mbar_arrive_remote(uint64_t* bar, uint32_t cta) {
+    asm volatile(
+        "{\n.reg .b32 ra;\nmapa.shared::cluster.u32 ra, %0, %1;\n"
+        "mbarrier.arrive.shared::cluster.b64 _, [ra];\n}" ::"r"(smem_u32(bar)),
+        "r"(cta)
+        : "memory");
+}
+
 // 32 lanes x 32 consecutive columns: thread = lane (row of D), r[j] = column j. Warp w may only touch lanes
 // 32*(w%4) .. 32*(w%4)+31. Follow with tmem_ld_wait() before using r.
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
